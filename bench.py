@@ -6,6 +6,7 @@ N = 1000 sparse random-graph Ising (4-regular, J = +-0.4, h = 0), 1e7-sample his
     python bench.py --impl reference ...                     (CPU oracle port on the host cores)
     python bench.py --config c0|c1|c2|c4                     (time-only lines for the other BASELINE configs, 1 GPU)
     python bench.py --mode node_sharded|sample_sharded|single_process   (multi-GPU partition; default auto)
+    python bench.py --dump-outputs DIR                       (also write the last timed step's matrix to DIR/theta.npy)
 
 A "step" is one full learn(): all node problems solved to the stated tolerance on the resident
 histogram (+ symmetrisation; + the row all-gather in node-sharded mode).  metric = node*sample evals/s
@@ -139,6 +140,23 @@ class ClockSampler(threading.Thread):
         self.join(timeout=5)
         med = float(np.median(self.samples)) if self.samples else None
         return {"sm_mhz": med, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.samples)}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, name: str, a: np.ndarray) -> None:
+    """--dump-outputs: writes `a` as <directory>/<name>.npy in float64, so that two builds can be compared output for
+    output.  Above 64 MB only a fixed, seeded sample of its rows is written, with the row numbers in <name>_rows.npy."""
+    out = pathlib.Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    a = np.asarray(a, dtype=np.float64)
+    if a.nbytes > DUMP_BYTES:
+        row_bytes = a.nbytes // a.shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(a.shape[0], size=DUMP_BYTES // (row_bytes + 8), replace=False))
+        np.save(out / f"{name}_rows.npy", rows.astype(np.float64))
+        a = a[rows]
+    np.save(out / f"{name}.npy", a)
 
 
 def load_peaks():
@@ -363,6 +381,8 @@ def run_b200(args):
         dist.all_reduce(ev)
     value = float(ev.item()) / (ms_step * 1e-3)
     learned = full.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "theta", learned)      # the symmetrised N x N matrix of the last timed step
     recon_err = float(np.abs(learned - np.diag(np.diag(learned)) - truth).max())
     nnz_row = (learned != 0.0).sum(axis=1)          # symmetrised support (union of the two directed estimates)
 
@@ -671,7 +691,12 @@ def main():
     ap.add_argument("--no-coarse", action="store_true")
     ap.add_argument("--warm-start", dest="warm_start", action="store_true", default=None)
     ap.add_argument("--no-warm-start", dest="warm_start", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the learned matrix of the last timed step to DIR/theta.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "c3"):
+        ap.error("--dump-outputs applies to the C3 workload on the GPU")
     if args.impl == "reference":
         run_reference(args)
     elif args.config != "c3":

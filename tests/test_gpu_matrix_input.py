@@ -15,9 +15,9 @@ FORMS = {"RISE": RISE, "logRISE": logRISE, "RPLE": RPLE}
 @pytest.mark.parametrize("dtype", [np.float64, np.int64, np.float32, np.int32])
 @pytest.mark.parametrize("name", ["a", "c", "mvt"])
 def test_matrix_entry_equals_packed_entry_on_goldens(golden, name, dtype):
-    s = golden(f"{name}_samples.csv")
-    if dtype in (np.float32,) and name == "mvt":
-        pytest.skip("mvt counts exceed float32's integer range")
+    # the histogram as the matrix entry receives it: exact in every dtype except float32, which rounds mvt's largest
+    # count (35 712 921 > 2^24) by one -- the packed entry gets the same rounded count
+    s = golden(f"{name}_samples.csv").astype(dtype).astype(np.float64)
     for form in FORMS.values():
         f = form(0.2, False) if name == "mvt" else form()
         packed = gml_b200.learn(s, f, B200(barrier_mu=1e-9))                      # row-major input -> packed entry

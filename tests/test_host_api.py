@@ -2,8 +2,11 @@
 host mirror of the reference interface behaves like the reference, and the product path fails loudly
 (no CPU fallback) when there is no CUDA device."""
 import ctypes
+import os
 import pathlib
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -12,6 +15,15 @@ import gml_b200
 from gml_b200 import _lib
 
 ROOT = pathlib.Path(__file__).resolve().parent.parent
+
+
+def rerun_without_device(request):
+    """On a machine with a CUDA device, runs the calling test again in a child pytest that sees none
+    (CUDA_VISIBLE_DEVICES=""), so the no-device behaviour is checked there too."""
+    assert os.environ.get("CUDA_VISIBLE_DEVICES") != "", "a device is visible with CUDA_VISIBLE_DEVICES=\"\""
+    res = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", f"{request.path}::{request.node.name}"], cwd=ROOT,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0 and "1 passed" in res.stdout, res.stdout[-4000:] + res.stderr[-2000:]
 
 
 def test_library_exports_every_header_symbol():
@@ -86,17 +98,18 @@ def test_nlp_method_is_rejected(golden):
         gml_b200.learn(golden("a_samples.csv"), gml_b200.RISE(), gml_b200.NLP())
 
 
-def test_no_cpu_fallback(golden):
+def test_no_cpu_fallback(golden, request):
     """Without a CUDA device the product must fail loudly, never compute on the CPU."""
     lib = _lib.load()
     if lib.gml_b200_device_count() > 0:
-        pytest.skip("CUDA device present")
+        rerun_without_device(request)
+        return
     with pytest.raises(gml_b200.GMLB200Error) as e:
         gml_b200.learn(golden("a_samples.csv"))
     assert e.value.code == _lib.ECUDA and "no CPU fallback" in str(e.value)
 
 
-def test_matrix_entry_fails_loudly_without_device_and_validates_layout(golden):
+def test_matrix_entry_fails_loudly_without_device_and_validates_layout(golden, request):
     """The reference-typed entry (Fortran-ordered K x (N+1) matrix) has no CPU path either; layout errors are host errors."""
     s = np.asfortranarray(golden("a_samples.csv"))
     with pytest.raises(ValueError):
@@ -105,7 +118,8 @@ def test_matrix_entry_fails_loudly_without_device_and_validates_layout(golden):
         gml_b200.learn_matrix(s.astype(np.float16, order="F"), gml_b200.RISE(), gml_b200.B200())
     lib = _lib.load()
     if lib.gml_b200_device_count() > 0:
-        pytest.skip("CUDA device present")
+        rerun_without_device(request)
+        return
     with pytest.raises(gml_b200.GMLB200Error) as e:
         gml_b200.learn(s, gml_b200.RISE(), gml_b200.B200())        # F-ordered input takes the matrix entry
     assert e.value.code == _lib.ECUDA
