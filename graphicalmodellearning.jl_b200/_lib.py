@@ -120,16 +120,12 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     lib.gml_b200_comm_init.argtypes = [vp, vp, c.c_int32, c.c_int32]
     lib.gml_b200_comm_globalize_histogram.argtypes = [vp]
     lib.gml_b200_comm_attach.argtypes = [vp, vp]
-    for name in EXPORTS:
-        fn = getattr(lib, name)
-        if fn.restype is c.c_int and name not in ("gml_b200_device_count",):
-            fn.restype = c.c_int
     _lib = lib
     return lib
 
 
-def check(rc: int, allow_notconv: bool = False) -> None:
-    if rc == OK or (allow_notconv and rc == ENOTCONV):
+def check(rc: int) -> None:
+    if rc == OK:
         return
     raise GMLB200Error(rc, load().gml_b200_last_error().decode())
 

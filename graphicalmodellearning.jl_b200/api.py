@@ -189,6 +189,18 @@ def regularizer_lambda(c: float, num_spins: int, num_samples: float) -> float:
     return c * math.sqrt(math.log((num_spins ** 2) / 0.05) / num_samples)
 
 
+def _pairwise_id(formulation) -> int:
+    """Formulation id of the C ABI for RISE / logRISE / RPLE."""
+    form_id = {RISE: _lib.RISE_ID, logRISE: _lib.LOGRISE_ID, RPLE: _lib.RPLE_ID}.get(type(formulation))
+    if form_id is None:
+        raise NotImplementedError(f"{type(formulation).__name__} is not on the B200 hot path")
+    return form_id
+
+
+# precision level of Session.eval_pairwise / bench_passes (opts.reserved[5]): fine, coarse, rough
+_LEVELS = {False: 0, True: 1, "rough": 2}
+
+
 def pack_histogram(samples):
     """[count, s_1..s_N] (any real dtype, any memory order -- the Adjoint shim of :73 is a no-op
     here) -> counts float64[K], spins int8 spin-major [N x K]."""
@@ -228,36 +240,37 @@ def learn_packed(counts: np.ndarray, spins: np.ndarray, formulation: GMLFormulat
     ld = spins.strides[0]
     if lam is None:
         lam = regularizer_lambda(formulation.regularizer, N, float(counts.sum()))
+    return _learn_one_shot(lib.gml_b200_learn_multibody, lib.gml_b200_learn_pairwise, (_ptr(counts), _ptr(spins), K, N, ld),
+                           lam, N, formulation, method, return_info, {"lambda": lam})
+
+
+MATRIX_DTYPES = {np.dtype(np.float64): 0, np.dtype(np.int64): 1, np.dtype(np.float32): 2, np.dtype(np.int32): 3,
+                 np.dtype(np.int8): 4}
+
+
+def _learn_one_shot(learn_multibody, learn_pairwise, source: tuple, lam: float, N: int, formulation, method: B200,
+                    return_info: bool, info: dict):
+    """The C call and result of learn_packed / learn_matrix.  learn_multibody / learn_pairwise: their C entry points;
+    source: the leading arguments that locate the histogram; lam: the lambda (packed) or regularizer (matrix) argument;
+    info: what return_info reports besides the objective and the stats."""
     stats = _lib.Stats()
     obj = np.zeros(N)
     opts = method._opts()
     if isinstance(formulation, multiRISE):
         order = int(formulation.interaction_order)
-        n_keys = int(lib.gml_b200_multibody_num_keys(N, order))
-        vals = np.zeros((N, n_keys))
-        rc = lib.gml_b200_learn_multibody(_ptr(counts), _ptr(spins), K, N, ld, order, lam,
-                                          ctypes.byref(opts), _ptr(vals), _ptr(obj), ctypes.byref(stats))
-        method.last_stats = stats.as_dict()
-        _lib.check(rc)
-        result = _multirise_result(vals, N, formulation)
+        vals = np.zeros((N, int(_lib.load().gml_b200_multibody_num_keys(N, order))))
+        rc = learn_multibody(*source, order, lam, ctypes.byref(opts), _ptr(vals), _ptr(obj), ctypes.byref(stats))
     else:
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}.get(type(formulation))
-        if form_id is None:
-            raise NotImplementedError(f"{type(formulation).__name__} is not on the B200 hot path")
+        form_id = _pairwise_id(formulation)
         theta = np.zeros((N, N), order="F")                              # Julia-native column-major
-        rc = lib.gml_b200_learn_pairwise(_ptr(counts), _ptr(spins), K, N, ld, form_id, lam,
-                                         int(bool(formulation.symmetrization)), ctypes.byref(opts),
-                                         _ptr(theta), _ptr(obj), ctypes.byref(stats))
-        method.last_stats = stats.as_dict()
-        _lib.check(rc)
-        result = np.ascontiguousarray(theta)
+        rc = learn_pairwise(*source, form_id, lam, int(bool(formulation.symmetrization)), ctypes.byref(opts),
+                            _ptr(theta), _ptr(obj), ctypes.byref(stats))
+    method.last_stats = stats.as_dict()
+    _lib.check(rc)
+    result = _multirise_result(vals, N, formulation) if isinstance(formulation, multiRISE) else np.ascontiguousarray(theta)
     if return_info:
-        return result, {"lambda": lam, "objective": obj, **method.last_stats}
+        return result, {**info, "objective": obj, **method.last_stats}
     return result
-
-
-MATRIX_DTYPES = {np.dtype(np.float64): 0, np.dtype(np.int64): 1, np.dtype(np.float32): 2, np.dtype(np.int32): 3,
-                 np.dtype(np.int8): 4}
 
 
 def _multirise_result(vals: np.ndarray, N: int, formulation) -> "FactorGraph":
@@ -287,32 +300,9 @@ def learn_matrix(samples: np.ndarray, formulation: GMLFormulation, method: B200,
     if not col_major or samples.dtype not in MATRIX_DTYPES:
         raise ValueError("learn_matrix needs a column-major (Fortran-ordered) matrix of float64 / int64 / float32 / int32 / int8")
     ld = samples.strides[1] // samples.itemsize          # leading dimension >= K (a row range of a taller matrix is fine)
-    stats = _lib.Stats()
-    obj = np.zeros(N)
-    opts = method._opts()
-    dt = MATRIX_DTYPES[samples.dtype]
-    if isinstance(formulation, multiRISE):
-        order = int(formulation.interaction_order)
-        vals = np.zeros((N, int(lib.gml_b200_multibody_num_keys(N, order))))
-        rc = lib.gml_b200_learn_multibody_matrix(_ptr(samples), dt, K, N, ld, order, float(formulation.regularizer),
-                                                 ctypes.byref(opts), _ptr(vals), _ptr(obj), ctypes.byref(stats))
-        method.last_stats = stats.as_dict()
-        _lib.check(rc)
-        result = _multirise_result(vals, N, formulation)
-    else:
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}.get(type(formulation))
-        if form_id is None:
-            raise NotImplementedError(f"{type(formulation).__name__} is not on the B200 hot path")
-        theta = np.zeros((N, N), order="F")
-        rc = lib.gml_b200_learn_pairwise_matrix(_ptr(samples), dt, K, N, ld, form_id, float(formulation.regularizer),
-                                                int(bool(formulation.symmetrization)), ctypes.byref(opts), _ptr(theta),
-                                                _ptr(obj), ctypes.byref(stats))
-        method.last_stats = stats.as_dict()
-        _lib.check(rc)
-        result = np.ascontiguousarray(theta)
-    if return_info:
-        return result, {"objective": obj, **method.last_stats}
-    return result
+    return _learn_one_shot(lib.gml_b200_learn_multibody_matrix, lib.gml_b200_learn_pairwise_matrix,
+                           (_ptr(samples), MATRIX_DTYPES[samples.dtype], K, N, ld), float(formulation.regularizer), N,
+                           formulation, method, return_info, {})
 
 
 def learn(samples, formulation: Optional[GMLFormulation] = None, method: Optional[GMLMethod] = None,
@@ -395,11 +385,14 @@ class Session:
     def num_samples(self) -> float:
         return float(self._lib.gml_b200_num_samples(self._h))
 
+    def _lam(self, formulation, lam: Optional[float]) -> float:
+        """lam, by default the reference's lambda (:157) of the resident histogram"""
+        return regularizer_lambda(formulation.regularizer, self.N, self.num_samples) if lam is None else lam
+
     def solve_pairwise(self, formulation, method: B200, lam: Optional[float] = None, return_info=False):
         N = self.N
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}[type(formulation)]
-        if lam is None:
-            lam = regularizer_lambda(formulation.regularizer, N, self.num_samples)
+        form_id = _pairwise_id(formulation)
+        lam = self._lam(formulation, lam)
         theta = np.zeros((N, N), order="F")
         obj = np.zeros(N)
         st = _lib.Stats()
@@ -413,9 +406,8 @@ class Session:
 
     def solve_pairwise_device(self, formulation, method: B200, d_rows_ptr: int, node_begin: int, node_end: int,
                               lam: Optional[float] = None, stream: int = 0, d_obj_ptr: int = 0):
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}[type(formulation)]
-        if lam is None:
-            lam = regularizer_lambda(formulation.regularizer, self.N, self.num_samples)
+        form_id = _pairwise_id(formulation)
+        lam = self._lam(formulation, lam)
         st = _lib.Stats()
         opts = method._opts(node_begin, node_end, stream)
         rc = self._lib.gml_b200_solve_pairwise_device(self._h, form_id, lam, ctypes.byref(opts),
@@ -430,8 +422,7 @@ class Session:
         (src/GraphicalModelLearning.jl:94-104); Dict assembly / mean-symmetrisation: learn_packed."""
         N = self.N
         order = int(formulation.interaction_order)
-        if lam is None:
-            lam = regularizer_lambda(formulation.regularizer, N, self.num_samples)
+        lam = self._lam(formulation, lam)
         n_keys = int(self._lib.gml_b200_multibody_num_keys(N, order))
         vals, obj = np.zeros((N, n_keys)), np.zeros(N)
         st = _lib.Stats()
@@ -447,8 +438,7 @@ class Session:
         import itertools
         N = self.N
         order = int(formulation.interaction_order)
-        if lam is None:
-            lam = regularizer_lambda(formulation.regularizer, N, self.num_samples)
+        lam = self._lam(formulation, lam)
         n_sym = int(self._lib.gml_b200_multibody_num_sym_keys(N, order))
         vals, obj = np.zeros(n_sym), np.zeros(N)
         st = _lib.Stats()
@@ -473,13 +463,13 @@ class Session:
         """f_u and grad f_u at rows x [N x (N+1)] (couplings then field).  coarse=True evaluates on the tensor-core
         backend's coarse precision level (iterate lattice 2^-22, |x| < 1.95, 16-bit residual digits); "rough": the opt-in
         rough level (lattice 2^-14, one 8-bit residual plane)."""
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}[type(formulation)]
+        form_id = _pairwise_id(formulation)
         x = np.ascontiguousarray(x, dtype=np.float64)
         assert x.shape == (self.N, self.N + 1)
         f = np.zeros(self.N)
         g = np.zeros_like(x) if want_grad else None
         opts = B200(solver=backend)._opts()
-        opts.reserved[5] = {False: 0, True: 1, "rough": 2}[coarse]
+        opts.reserved[5] = _LEVELS[coarse]
         _lib.check(self._lib.gml_b200_eval_pairwise(self._h, form_id, ctypes.byref(opts), _ptr(x), _ptr(f),
                                                     _ptr(g) if want_grad else None))
         return f, g
@@ -487,10 +477,10 @@ class Session:
     def bench_passes(self, formulation, backend: str = "fista_tc", reps: int = 5, node_begin: int = 0, node_end: int = 0,
                      coarse: bool = False):
         """Mean device ms of the contraction kernels: dict(energy_full, grad, energy_obj, full_pass_wall)."""
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}[type(formulation)]
+        form_id = _pairwise_id(formulation)
         out = np.zeros(4)
         opts = B200(solver=backend)._opts(node_begin, node_end)
-        opts.reserved[5] = {False: 0, True: 1, "rough": 2}[coarse]
+        opts.reserved[5] = _LEVELS[coarse]
         _lib.check(self._lib.gml_b200_bench_passes(self._h, form_id, ctypes.byref(opts), reps, _ptr(out)))
         return dict(zip(("energy_full", "grad", "energy_obj", "full_pass_wall"), out.tolist()))
 
@@ -535,7 +525,7 @@ class Session:
         """Regularisation path: one solve per regulariser c (lambda = c*sqrt(log(N^2/0.05)/M), :157), each warm
         started from the previous one.  Returns an array [len(regularizers), N, N]."""
         N = self.N
-        form_id = {RISE: 0, logRISE: 1, RPLE: 2}[type(formulation)]
+        form_id = _pairwise_id(formulation)
         lams = np.array([regularizer_lambda(c, N, self.num_samples) for c in regularizers], dtype=np.float64)
         out = np.zeros((len(lams), N, N))
         st = _lib.Stats()

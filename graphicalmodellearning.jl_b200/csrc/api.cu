@@ -11,6 +11,7 @@
 #include <memory>
 #include <mutex>
 #include <thread>
+#include <tuple>
 
 namespace gml {
 
@@ -225,29 +226,59 @@ void finish_stats(gml_b200_stats* stats, const SolveResult& r, int solver_used, 
     for (int i = 0; i < 4; ++i) stats->reserved_d[i] = r.profile[i];
 }
 
+void throw_if_unconverged(int n_unconverged) {
+    if (n_unconverged == 0) return;
+    set_error("solver did not reach tol within max_iter for " + std::to_string(n_unconverged) + " node(s)");
+    throw CudaError{GML_B200_ENOTCONV};
+}
+
+// 0.5 (R + R') (:185) of the N x N matrix m in place (symmetric in (i, j): row- or column-major alike)
+void launch_symmetrize(double* m, int N, cudaStream_t st) {
+    dim3 b(32, 8), g((unsigned)ceil_div(N, 32), (unsigned)ceil_div(N, 8));
+    symmetrize_kernel<<<g, b, 0, st>>>(m, N);
+    GML_LAUNCHED();
+}
+
+// rows [Nn x N] of the nodes nb.. into the column-major (Julia-native) N x N matrix `out`
+void scatter_rows(const double* rows, int Nn, int N, int nb, double* out) {
+    for (int u = 0; u < Nn; ++u)
+        for (int i = 0; i < N; ++i) out[(size_t)(nb + u) + (size_t)N * i] = rows[(size_t)u * N + i];
+}
+
+// the nodes [nb, ne) a call covers (opts->node_begin / node_end; ne <= 0 = through the last of the N nodes)
+std::pair<int, int> node_range(int nb, int ne, int N) {
+    if (ne <= 0) ne = N;
+    GML_REQUIRE(nb >= 0 && ne <= N && nb < ne, "node shard out of range");
+    return {nb, ne};
+}
+
+// Node problems [nb, ne) of a pairwise formulation over the resident feature matrix [S | 1] (hist.base), with their
+// penalty classes set up on the device.
+void pairwise_problem(NodeProblem& p, Histogram& hist, int formulation, double lambda, int nb, int ne, cudaStream_t st) {
+    GML_REQUIRE(formulation >= GML_B200_RISE && formulation <= GML_B200_RPLE, "unknown formulation id");
+    std::tie(nb, ne) = node_range(nb, ne, hist.N);
+    p.hist = &hist; p.Q = hist.base.p; p.F = hist.N + 1; p.Fp = hist.Fb;
+    p.form = formulation; p.lambda = lambda; p.Nn = ne - nb;
+    p.spin_row.alloc(p.Nn); p.pen.alloc((size_t)p.Nn * p.Fp);
+    pairwise_setup_kernel<<<p.Nn, 128, 0, st>>>(hist.N, p.Fp, nb, p.Nn, p.spin_row.p, p.pen.p);
+    GML_LAUNCHED();
+}
+
 void solve_pairwise_rows_one(gml_b200_handle* h, int formulation, double lambda, const gml_b200_opts& o, int nb, int ne,
                              double* d_rows, double* d_obj, gml_b200_stats* stats, cudaStream_t st, double t0,
                              DevBuf<double>* warm = nullptr /* in: start point (if allocated), out: solution [Nn x Fp] */) {
-    GML_REQUIRE(h->has_hist, "no histogram resident: call gml_b200_upload_histogram first");
-    GML_REQUIRE(formulation >= GML_B200_RISE && formulation <= GML_B200_RPLE, "unknown formulation id");
-    GML_REQUIRE(lambda >= 0.0 && std::isfinite(lambda), "lambda must be finite and >= 0");
     Histogram& hist = h->hist;
     const int N = hist.N;
-    GML_REQUIRE(nb >= 0 && ne <= N && nb < ne, "node shard out of range");
     NodeProblem p;
-    p.hist = &hist; p.Q = hist.base.p; p.F = N + 1; p.Fp = hist.Fb;
-    p.form = formulation; p.lambda = lambda; p.Nn = ne - nb;
     if (o.reserved[2] == 1) {
         GML_REQUIRE(h->comm != nullptr, "sample-sharded solve needs gml_b200_comm_init first");
         GML_REQUIRE(hist.M_local > 0.0, "sample-sharded solve needs gml_b200_comm_globalize_histogram after the upload");
-        GML_REQUIRE(o.solver == GML_B200_SOLVER_FISTA_TC || (o.solver == GML_B200_SOLVER_AUTO && p.F > NEWTON_AUTO_F),
+        GML_REQUIRE(o.solver == GML_B200_SOLVER_FISTA_TC || (o.solver == GML_B200_SOLVER_AUTO && N + 1 > NEWTON_AUTO_F),
                     "sample-sharded mode is implemented for the tensor-core FISTA solver");
         p.comm = h->comm;
     }
-    p.spin_row.alloc(p.Nn); p.pen.alloc((size_t)p.Nn * p.Fp);
     EventTimer timer(st);
-    pairwise_setup_kernel<<<p.Nn, 128, 0, st>>>(N, p.Fp, nb, p.Nn, p.spin_row.p, p.pen.p);
-    GML_LAUNCHED();
+    pairwise_problem(p, hist, formulation, lambda, nb, ne, st);
     SolveResult r;
     // The objective at the returned point costs one more pass over the histogram: only when somebody asked for it.  In a
     // sample-sharded solve that pass contains an all-reduce, so EVERY rank must make the same choice (the callers pass the
@@ -265,22 +296,20 @@ void solve_pairwise_rows_one(gml_b200_handle* h, int formulation, double lambda,
     }
     const double solve_ms = timer.stop();
     finish_stats(stats, r, solver_used, p.Nn, hist.K, solve_ms, 0.0, t0);
-    if (r.n_unconverged > 0) {
-        set_error("solver did not reach tol within max_iter for " + std::to_string(r.n_unconverged) + " node(s)");
-        throw CudaError{GML_B200_ENOTCONV};
-    }
+    throw_if_unconverged(r.n_unconverged);
 }
 
 // Memory-aware front end: the residual limbs of the tensor-core path take nR * nodes * Kp bytes (31 GB at C3 on one
 // GPU).  When a shard would not fit next to the resident histogram copies, its nodes are solved in consecutive
 // chunks (node problems are independent, src/GraphicalModelLearning.jl:161) instead of failing with out-of-memory.
-void solve_pairwise_rows(gml_b200_handle* h, int formulation, double lambda, const gml_b200_opts& o, int nb, int ne,
-                         double* d_rows, double* d_obj, gml_b200_stats* stats, cudaStream_t st, double t0,
+void solve_pairwise_rows(gml_b200_handle* h, int formulation, double lambda, const gml_b200_opts& o, int node_begin,
+                         int node_end, double* d_rows, double* d_obj, gml_b200_stats* stats, cudaStream_t st, double t0,
                          DevBuf<double>* warm = nullptr) {
     GML_REQUIRE(h->has_hist, "no histogram resident: call gml_b200_upload_histogram first");
+    GML_REQUIRE(lambda >= 0.0 && std::isfinite(lambda), "lambda must be finite and >= 0");
     const Histogram& hist = h->hist;
     const int N = hist.N;
-    GML_REQUIRE(nb >= 0 && ne <= N && nb < ne, "node shard out of range");
+    const auto [nb, ne] = node_range(node_begin, node_end, N);
     const int F = N + 1;
     int solver = pick_solver(o, F);
     int chunk = ne - nb;
@@ -329,10 +358,7 @@ void solve_pairwise_rows(gml_b200_handle* h, int formulation, double lambda, con
     acc.kernel_launches = g_launches;
     acc.total_ms = now_ms() - t0;
     if (stats) *stats = acc;
-    if (unconverged > 0) {
-        set_error("solver did not reach tol within max_iter for " + std::to_string(unconverged) + " node(s)");
-        throw CudaError{GML_B200_ENOTCONV};
-    }
+    throw_if_unconverged(unconverged);
 }
 
 // base features of multiRISE order p: all subsets of [N] of size <= p-1, by size then lexicographic
@@ -385,6 +411,111 @@ MultibodyLayout multibody_layout(int N, int order) {
         L.n_keys = count;
     }
     return L;
+}
+
+// The eval / bench entry points: node problems opts->node_begin..node_end and the evaluation backend opts->solver
+// names, on the precision level opts->reserved[5] asks for.
+std::unique_ptr<EvalBackend> eval_backend(gml_b200_handle* h, int formulation, const gml_b200_opts& o, NodeProblem& p,
+                                          cudaStream_t st) {
+    GML_REQUIRE(o.solver == GML_B200_SOLVER_FISTA_CC || o.solver == GML_B200_SOLVER_FISTA_TC,
+                "eval and bench need solver = FISTA_CC or FISTA_TC");
+    pairwise_problem(p, h->hist, formulation, 0.0, o.node_begin, o.node_end, st);
+    std::unique_ptr<EvalBackend> be(o.solver == GML_B200_SOLVER_FISTA_TC ? make_backend_tc(p, st) : make_backend_cc(p, st));
+    if (o.reserved[5] == 1)      // the coarse precision level (lattice 2^-22, |x| < 1.95)
+        GML_REQUIRE(be->set_level(0, st), "this backend has no coarse precision level");
+    if (o.reserved[5] == 2)      // the rough level (lattice 2^-14, |x| < 1.95, one residual digit plane)
+        GML_REQUIRE(be->set_level(-1, st), "the rough precision level is not available for this backend / histogram (it needs near-uniform counts)");
+    return be;
+}
+
+// Host upload of a K-row histogram: fill(d_counts, d_base, Kp) writes the counts and the spin rows of `base` (pitch Kp)
+// and returns its host-side time (stats->h2d_ms); validation and padding then run in place.  The handle holds no
+// histogram until that has succeeded.
+template <class Fill> void upload_histogram_with(gml_b200_handle* h, int64_t K, int32_t N, gml_b200_stats* stats, Fill&& fill) {
+    const double t0 = now_ms();
+    GML_CUDA(cudaSetDevice(h->device));
+    DevBuf<double> dc;
+    dc.alloc(K);
+    Histogram& hist = h->hist;
+    const int64_t Kp = round_up(K, KPAD);
+    h->has_hist = false;
+    hist.base.alloc((size_t)round_up(N + 1, FPAD) * Kp);
+    const double h2d = fill(dc.p, hist.base.p, Kp);
+    gml_b200_stats tmp;
+    const int rc = gml_b200_attach_histogram_device(h, dc.p, hist.base.p, K, N, Kp, &tmp);
+    if (rc != GML_B200_OK) throw CudaError{rc};
+    if (stats) {
+        *stats = tmp;
+        stats->h2d_ms = h2d;
+        stats->total_ms = now_ms() - t0;
+    }
+}
+
+// where the histogram of a one-shot call comes from: packed (counts + int8 spins) or the reference's K x (N+1) matrix
+struct HostSource {
+    const double* counts = nullptr; const int8_t* spins = nullptr;     // packed form
+    const void* matrix = nullptr; int dtype = 0;                       // matrix form
+    int64_t ld = 0;
+    double regularizer = -1.0;      // >= 0: lambda = regularizer*sqrt(log(N^2/0.05)/M) (:157) from the global sample count
+    int upload(gml_b200_handle* h, int64_t k0, int64_t k1, int32_t N, gml_b200_stats* up) const {
+        if (matrix) return gml_b200_upload_matrix(h, matrix, dtype, k0, k1 - k0, N, ld, up);
+        return gml_b200_upload_histogram(h, counts + k0, spins + k0, k1 - k0, N, ld, up);
+    }
+    double lambda_for(double lambda, int32_t N, double M) const {
+        return regularizer >= 0.0 ? regularizer * std::sqrt(std::log(((double)N * (double)N) / 0.05) / M) : lambda;
+    }
+};
+
+// One-shot call on one device: its own handle, the upload of all K rows of `src`, then solve(handle, lambda, stats);
+// the stats add the upload's to the solve's.
+template <class Solve> int learn_one_device(int device, const HostSource& src, int64_t K, int32_t N, double lambda,
+                                            gml_b200_stats* stats, Solve&& solve) {
+    gml_b200_handle* h = nullptr;
+    int rc = gml_b200_create(&h, device);
+    if (rc != GML_B200_OK) return rc;
+    gml_b200_stats up{}, so{};
+    rc = src.upload(h, 0, K, N, &up);
+    if (rc == GML_B200_OK) rc = solve(h, src.lambda_for(lambda, N, gml_b200_num_samples(h)), &so);
+    if (stats) {
+        *stats = so;
+        stats->pack_ms = up.pack_ms; stats->h2d_ms = up.h2d_ms;
+        stats->kernel_launches += up.kernel_launches;
+        stats->total_ms += up.total_ms;
+    }
+    gml_b200_destroy(h);
+    return rc;
+}
+
+// Runs body(r) -> status for the devices first_device + r, r < n_dev, on one host thread each.  The combined status is
+// the first failure other than ENOTCONV, else ENOTCONV if a device did not converge; the error names the device.
+template <class Body> int on_each_device(int first_device, int n_dev, Body&& body) {
+    std::vector<int> rcs(n_dev, GML_B200_OK);
+    std::vector<std::string> errs(n_dev);
+    std::vector<std::thread> threads;
+    for (int r = 0; r < n_dev; ++r)
+        threads.emplace_back([&, r] {
+            rcs[r] = body(r);
+            if (rcs[r] != GML_B200_OK) errs[r] = gml_b200_last_error();
+        });
+    for (auto& t : threads) t.join();
+    int rc = GML_B200_OK;
+    for (int r = 0; r < n_dev; ++r)
+        if (rcs[r] != GML_B200_OK && (rc == GML_B200_OK || rc == GML_B200_ENOTCONV)) { rc = rcs[r]; set_error("device " + std::to_string(first_device + r) + ": " + errs[r]); }
+    return rc;
+}
+
+// devices of a one-shot call: opts->reserved[4] from opts->device on, as far as they exist
+int one_shot_devices(const gml_b200_opts* opts) {
+    if (!opts || opts->reserved[4] <= 1) return 1;
+    return std::min<int>(opts->reserved[4], std::max(1, gml_b200_device_count() - opts->device));
+}
+
+// Partition (SURVEY 8e): sample slices when the tensor-core solver runs and every device still gets a GPU-filling
+// number of rows -- each device then streams K/n rows per pass instead of all K.
+bool use_sample_slices(const gml_b200_opts* opts, int64_t K, int32_t N, int n_dev) {
+    if (n_dev <= 1) return false;
+    const bool tc = (opts->solver == GML_B200_SOLVER_AUTO && N + 1 > NEWTON_AUTO_F) || opts->solver == GML_B200_SOLVER_FISTA_TC;
+    return tc && K / n_dev >= 65536 && opts->barrier_mu == 0.0;
 }
 
 }  // namespace
@@ -471,28 +602,15 @@ int gml_b200_upload_histogram(gml_b200_handle* h, const double* counts, const in
     return guarded([&] {
         GML_REQUIRE(h && counts && spins, "null argument");
         GML_REQUIRE(K >= 1 && N >= 1 && ld >= K, "histogram needs K >= 1, N >= 1, ld >= K");
-        const double t0 = now_ms();
-        GML_CUDA(cudaSetDevice(h->device));
-        cudaStream_t st = h->own_stream;
-        DevBuf<double> dc;
-        dc.alloc(K);
         // the spins land directly in their final place (rows of `base`, pitch Kp); validation and padding
         // then run in place -- no staging copy of the histogram on the device
-        Histogram& hist = h->hist;
-        const int64_t Kp = round_up(K, KPAD);
-        hist.base.alloc((size_t)round_up(N + 1, FPAD) * Kp);
-        EventTimer timer(st);
-        GML_CUDA(cudaMemcpyAsync(dc.p, counts, sizeof(double) * K, cudaMemcpyHostToDevice, st));
-        GML_CUDA(cudaMemcpy2DAsync(hist.base.p, Kp, spins, ld, K, N, cudaMemcpyHostToDevice, st));
-        const double h2d = timer.stop();
-        gml_b200_stats tmp;
-        const int rc = gml_b200_attach_histogram_device(h, dc.p, hist.base.p, K, N, Kp, &tmp);
-        if (rc != GML_B200_OK) throw CudaError{rc};
-        if (stats) {
-            *stats = tmp;
-            stats->h2d_ms = h2d;
-            stats->total_ms = now_ms() - t0;
-        }
+        upload_histogram_with(h, K, N, stats, [&](double* d_counts, int8_t* d_base, int64_t Kp) {
+            cudaStream_t st = h->own_stream;
+            EventTimer timer(st);
+            GML_CUDA(cudaMemcpyAsync(d_counts, counts, sizeof(double) * K, cudaMemcpyHostToDevice, st));
+            GML_CUDA(cudaMemcpy2DAsync(d_base, Kp, spins, ld, K, N, cudaMemcpyHostToDevice, st));
+            return timer.stop();
+        });
     });
 }
 
@@ -501,24 +619,11 @@ int gml_b200_upload_matrix(gml_b200_handle* h, const void* samples, int32_t dtyp
     return guarded([&] {
         GML_REQUIRE(h && samples, "null argument");
         GML_REQUIRE(K >= 1 && N >= 1 && row_begin >= 0 && ld >= row_begin + K, "samples matrix needs K >= 1, N >= 1, ld >= row_begin + K");
-        const double t0 = now_ms();
-        GML_CUDA(cudaSetDevice(h->device));
-        DevBuf<double> dc;
-        dc.alloc(K);
-        Histogram& hist = h->hist;
-        const int64_t Kp = round_up(K, KPAD);
-        h->has_hist = false;
-        hist.base.alloc((size_t)round_up(N + 1, FPAD) * Kp);
-        double host_ms = 0.0;
-        ingest_matrix(samples, dtype, ld, row_begin, K, N, hist.base.p, Kp, dc.p, 0, &host_ms);
-        gml_b200_stats tmp;
-        const int rc = gml_b200_attach_histogram_device(h, dc.p, hist.base.p, K, N, Kp, &tmp);     // validate + pad in place
-        if (rc != GML_B200_OK) throw CudaError{rc};
-        if (stats) {
-            *stats = tmp;
-            stats->h2d_ms = host_ms;
-            stats->total_ms = now_ms() - t0;
-        }
+        upload_histogram_with(h, K, N, stats, [&](double* d_counts, int8_t* d_base, int64_t Kp) {
+            double host_ms = 0.0;
+            ingest_matrix(samples, dtype, ld, row_begin, K, N, d_base, Kp, d_counts, 0, &host_ms);
+            return host_ms;
+        });
     });
 }
 
@@ -531,8 +636,8 @@ int gml_b200_solve_pairwise_device(gml_b200_handle* h, int32_t formulation, doub
         gml_b200_opts o; fill_opts(o, opts);
         GML_CUDA(cudaSetDevice(h->device));
         if (stats) std::memset(stats, 0, sizeof(*stats));
-        const int nb = o.node_begin, ne = o.node_end > 0 ? o.node_end : h->hist.N;
-        solve_pairwise_rows(h, formulation, lambda, o, nb, ne, d_out_rows, d_out_objective, stats, stream_of(h, o), t0);
+        solve_pairwise_rows(h, formulation, lambda, o, o.node_begin, o.node_end, d_out_rows, d_out_objective, stats,
+                            stream_of(h, o), t0);
     });
 }
 
@@ -548,8 +653,7 @@ int gml_b200_solve_pairwise(gml_b200_handle* h, int32_t formulation, double lamb
         cudaStream_t st = stream_of(h, o);
         if (stats) std::memset(stats, 0, sizeof(*stats));
         const int N = h->hist.N;
-        const int nb = o.node_begin, ne = o.node_end > 0 ? o.node_end : N;
-        GML_REQUIRE(nb >= 0 && ne <= N && nb < ne, "node shard out of range");
+        const auto [nb, ne] = node_range(o.node_begin, o.node_end, N);
         const int Nn = ne - nb;
         DevBuf<double> rows, obj;
         rows.alloc((size_t)Nn * N); obj.alloc(Nn);
@@ -561,17 +665,12 @@ int gml_b200_solve_pairwise(gml_b200_handle* h, int32_t formulation, double lamb
             rc = e.code;   // still hand back the best iterate, then report
         }
         EventTimer timer(st);
-        if (symmetrize && Nn == N) {
-            dim3 b(32, 8), g((unsigned)ceil_div(N, 32), (unsigned)ceil_div(N, 8));
-            symmetrize_kernel<<<g, b, 0, st>>>(rows.p, N);
-            GML_LAUNCHED();
-        }
+        if (symmetrize && Nn == N) launch_symmetrize(rows.p, N, st);
         std::vector<double> hrows((size_t)Nn * N);
         GML_CUDA(cudaMemcpyAsync(hrows.data(), rows.p, sizeof(double) * Nn * N, cudaMemcpyDeviceToHost, st));
         if (out_objective) GML_CUDA(cudaMemcpyAsync(out_objective + nb, obj.p, sizeof(double) * Nn, cudaMemcpyDeviceToHost, st));
         const double d2h = timer.stop();
-        for (int u = 0; u < Nn; ++u)
-            for (int i = 0; i < N; ++i) out_theta[(size_t)(nb + u) + (size_t)N * i] = hrows[(size_t)u * N + i];
+        scatter_rows(hrows.data(), Nn, N, nb, out_theta);
         if (stats) { stats->d2h_ms = d2h; stats->kernel_launches = g_launches; stats->total_ms = now_ms() - t0; }
         if (rc != GML_B200_OK) throw CudaError{rc};
     });
@@ -596,16 +695,10 @@ int gml_b200_solve_pairwise_path(gml_b200_handle* h, int32_t formulation, const 
         for (int li = 0; li < n_lambda; ++li) {
             std::memset(&cur, 0, sizeof(cur));
             solve_pairwise_rows(h, formulation, lambdas[li], o, 0, N, rows.p, nullptr, &cur, st, now_ms(), &warm);   // warm start
-            if (symmetrize) {
-                dim3 b(32, 8), g((unsigned)ceil_div(N, 32), (unsigned)ceil_div(N, 8));
-                symmetrize_kernel<<<g, b, 0, st>>>(rows.p, N);
-                GML_LAUNCHED();
-            }
+            if (symmetrize) launch_symmetrize(rows.p, N, st);
             GML_CUDA(cudaMemcpyAsync(hrows.data(), rows.p, sizeof(double) * N * N, cudaMemcpyDeviceToHost, st));
             GML_CUDA(cudaStreamSynchronize(st));
-            double* out = out_thetas + (size_t)li * N * N;
-            for (int u = 0; u < N; ++u)
-                for (int i = 0; i < N; ++i) out[(size_t)u + (size_t)N * i] = hrows[(size_t)u * N + i];
+            scatter_rows(hrows.data(), N, N, 0, out_thetas + (size_t)li * N * N);
             acc.iterations += cur.iterations; acc.n_fg_passes += cur.n_fg_passes; acc.n_f_passes += cur.n_f_passes;
             acc.evals += cur.evals; acc.solve_ms += cur.solve_ms; acc.solver_used = cur.solver_used;
             acc.max_residual = std::max(acc.max_residual, cur.max_residual);
@@ -682,10 +775,7 @@ static int solve_multibody_impl(gml_b200_handle* h, int32_t order, double lambda
         if (out_objective) GML_CUDA(cudaMemcpyAsync(out_objective, r.objective.p, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
         const double d2h = t2.stop();
         finish_stats(stats, r, solver_used, N, hist.K, solve_ms, d2h, t0);
-        if (r.n_unconverged > 0) {
-            set_error("solver did not reach tol within max_iter for " + std::to_string(r.n_unconverged) + " node(s)");
-            throw CudaError{GML_B200_ENOTCONV};
-        }
+        throw_if_unconverged(r.n_unconverged);
     });
 }
 
@@ -738,28 +828,13 @@ int gml_b200_eval_pairwise(gml_b200_handle* h, int32_t formulation, const gml_b2
     return guarded([&] {
         GML_REQUIRE(h && x && f_out, "null argument");
         GML_REQUIRE(h->has_hist, "no histogram resident: call gml_b200_upload_histogram first");
-        GML_REQUIRE(formulation >= GML_B200_RISE && formulation <= GML_B200_RPLE, "unknown formulation id");
         g_launches = 0;
         gml_b200_opts o; fill_opts(o, opts);
-        GML_REQUIRE(o.solver == GML_B200_SOLVER_FISTA_CC || o.solver == GML_B200_SOLVER_FISTA_TC,
-                    "eval needs solver = FISTA_CC or FISTA_TC");
         GML_CUDA(cudaSetDevice(h->device));
         cudaStream_t st = stream_of(h, o);
-        Histogram& hist = h->hist;
-        const int N = hist.N, F = N + 1;
-        const int nb = o.node_begin, ne = o.node_end > 0 ? o.node_end : N;
-        GML_REQUIRE(nb >= 0 && ne <= N && nb < ne, "node shard out of range");
         NodeProblem p;
-        p.hist = &hist; p.Q = hist.base.p; p.F = F; p.Fp = hist.Fb;
-        p.form = formulation; p.lambda = 0.0; p.Nn = ne - nb;
-        p.spin_row.alloc(p.Nn); p.pen.alloc((size_t)p.Nn * p.Fp);
-        pairwise_setup_kernel<<<p.Nn, 128, 0, st>>>(N, p.Fp, nb, p.Nn, p.spin_row.p, p.pen.p);
-        GML_LAUNCHED();
-        std::unique_ptr<EvalBackend> be(o.solver == GML_B200_SOLVER_FISTA_TC ? make_backend_tc(p, st) : make_backend_cc(p, st));
-        if (o.reserved[5] == 1)      // evaluate on the coarse precision level (lattice 2^-22, |x| < 1.95)
-            GML_REQUIRE(be->set_level(0, st), "this backend has no coarse precision level");
-        if (o.reserved[5] == 2)      // ... on the rough level (lattice 2^-14, |x| < 1.95, one residual digit plane)
-            GML_REQUIRE(be->set_level(-1, st), "the rough precision level is not available for this backend / histogram (it needs near-uniform counts)");
+        const std::unique_ptr<EvalBackend> be = eval_backend(h, formulation, o, p, st);
+        const int nb = o.node_begin, F = p.F;
         std::vector<double> hx((size_t)p.Nn * p.Fp, 0.0);
         const double lat = be->lattice(), xmax = be->x_range();
         for (int u = 0; u < p.Nn; ++u)
@@ -793,27 +868,14 @@ int gml_b200_bench_passes(gml_b200_handle* h, int32_t formulation, const gml_b20
         GML_REQUIRE(h->has_hist, "no histogram resident: call gml_b200_upload_histogram first");
         g_launches = 0;
         gml_b200_opts o; fill_opts(o, opts);
-        GML_REQUIRE(o.solver == GML_B200_SOLVER_FISTA_CC || o.solver == GML_B200_SOLVER_FISTA_TC,
-                    "bench needs solver = FISTA_CC or FISTA_TC");
         GML_CUDA(cudaSetDevice(h->device));
         cudaStream_t st = stream_of(h, o);
-        Histogram& hist = h->hist;
-        const int N = hist.N;
-        const int nb = o.node_begin, ne = o.node_end > 0 ? o.node_end : N;
-        GML_REQUIRE(nb >= 0 && ne <= N && nb < ne, "node shard out of range");
         NodeProblem p;
-        p.hist = &hist; p.Q = hist.base.p; p.F = N + 1; p.Fp = hist.Fb;
-        p.form = formulation; p.lambda = 0.0; p.Nn = ne - nb;
-        p.spin_row.alloc(p.Nn); p.pen.alloc((size_t)p.Nn * p.Fp);
-        pairwise_setup_kernel<<<p.Nn, 128, 0, st>>>(N, p.Fp, nb, p.Nn, p.spin_row.p, p.pen.p);
-        GML_LAUNCHED();
-        std::unique_ptr<EvalBackend> be(o.solver == GML_B200_SOLVER_FISTA_TC ? make_backend_tc(p, st) : make_backend_cc(p, st));
+        const std::unique_ptr<EvalBackend> be = eval_backend(h, formulation, o, p, st);
         DevBuf<double> dx, df, dg;
         const size_t nx = (size_t)p.Nn * p.Fp;
         dx.alloc(nx); df.alloc(p.Nn); dg.alloc(nx);
         GML_CUDA(cudaMemsetAsync(dx.p, 0, sizeof(double) * nx, st));
-        if (o.reserved[5] == 1) be->set_level(0, st);   // time the coarse precision level
-        if (o.reserved[5] == 2) be->set_level(-1, st);  // ... the rough one
         be->eval(dx.p, true, df.p, dg.p, st);    // warm-up
         be->eval(dx.p, false, df.p, nullptr, st);
         be->set_profiling(true);
@@ -831,9 +893,7 @@ int gml_b200_bench_passes(gml_b200_handle* h, int32_t formulation, const gml_b20
 int gml_b200_symmetrize_device(double* d_theta, int32_t N, void* stream) {
     return guarded([&] {
         GML_REQUIRE(d_theta && N >= 1, "bad argument");
-        dim3 b(32, 8), g((unsigned)ceil_div(N, 32), (unsigned)ceil_div(N, 8));
-        symmetrize_kernel<<<g, b, 0, (cudaStream_t)stream>>>(d_theta, N);
-        GML_LAUNCHED();
+        launch_symmetrize(d_theta, N, (cudaStream_t)stream);
     });
 }
 
@@ -841,14 +901,11 @@ int gml_b200_symmetrize_device(double* d_theta, int32_t N, void* stream) {
 // device, each with its own handle, the histogram replicated, node shards with 16-aligned cuts; every thread writes
 // its rows straight into the caller's matrix, the symmetrisation of the N x N result runs on the host.  This is what a
 // single Julia process uses; multi-process launches (torchrun) use gml_b200_solve_pairwise_device + an all-gather.
-static int learn_pairwise_multi_device(const double* counts, const int8_t* spins, int64_t K, int32_t N, int64_t ld,
-                                       int32_t formulation, double lambda, int32_t symmetrize, const gml_b200_opts& base,
-                                       int n_dev, double* out_theta, double* out_objective, gml_b200_stats* stats) {
+static int learn_pairwise_multi_device(const HostSource& src, int64_t K, int32_t N, int32_t formulation, double lambda,
+                                       int32_t symmetrize, const gml_b200_opts& base, int n_dev, double* out_theta,
+                                       double* out_objective, gml_b200_stats* stats) {
     const double t0 = now_ms();
-    std::vector<int> rcs(n_dev, GML_B200_OK);
-    std::vector<std::string> errs(n_dev);
     std::vector<gml_b200_stats> sts(n_dev);
-    std::vector<std::thread> threads;
     auto cut = [&](int r) {            // same rule as distributed.shard_bounds
         const int per = N / n_dev, extra = N % n_dev;
         int b = r * per + std::min(r, extra), e = b + per + (r < extra ? 1 : 0);
@@ -858,40 +915,31 @@ static int learn_pairwise_multi_device(const double* counts, const int8_t* spins
         }
         return std::make_pair(b, e);
     };
-    for (int r = 0; r < n_dev; ++r)
-        threads.emplace_back([&, r] {
-            gml_b200_handle* h = nullptr;
-            gml_b200_opts o = base;
-            o.device = base.device + r;
-            const auto be = cut(r);
-            o.node_begin = be.first; o.node_end = be.second; o.stream = nullptr;
-            int rc = gml_b200_create(&h, o.device);
-            gml_b200_stats up{};
-            std::memset(&sts[r], 0, sizeof(gml_b200_stats));
-            if (rc == GML_B200_OK && be.first < be.second) {
-                rc = gml_b200_upload_histogram(h, counts, spins, K, N, ld, &up);
-                if (rc == GML_B200_OK)
-                    rc = gml_b200_solve_pairwise(h, formulation, lambda, 0, &o, out_theta, out_objective, &sts[r]);
-                sts[r].pack_ms = up.pack_ms; sts[r].h2d_ms = up.h2d_ms; sts[r].kernel_launches += up.kernel_launches;
-            }
-            if (rc != GML_B200_OK) errs[r] = gml_b200_last_error();
-            rcs[r] = rc;
-            gml_b200_destroy(h);
-        });
-    for (auto& t : threads) t.join();
-    int rc = GML_B200_OK;
-    for (int r = 0; r < n_dev; ++r)
-        if (rcs[r] != GML_B200_OK && (rc == GML_B200_OK || rc == GML_B200_ENOTCONV)) { rc = rcs[r]; set_error("device " + std::to_string(base.device + r) + ": " + errs[r]); }
+    int rc = on_each_device(base.device, n_dev, [&](int r) {
+        gml_b200_handle* h = nullptr;
+        gml_b200_opts o = base;
+        o.device = base.device + r;
+        const auto be = cut(r);
+        o.node_begin = be.first; o.node_end = be.second; o.stream = nullptr;
+        int rc = gml_b200_create(&h, o.device);
+        gml_b200_stats up{};
+        if (rc == GML_B200_OK && be.first < be.second) {
+            rc = src.upload(h, 0, K, N, &up);
+            if (rc == GML_B200_OK)
+                rc = gml_b200_solve_pairwise(h, formulation, lambda, 0, &o, out_theta, out_objective, &sts[r]);
+            sts[r].pack_ms = up.pack_ms; sts[r].h2d_ms = up.h2d_ms; sts[r].kernel_launches += up.kernel_launches;
+        }
+        gml_b200_destroy(h);
+        return rc;
+    });
     if (symmetrize && (rc == GML_B200_OK || rc == GML_B200_ENOTCONV)) {
-        // 0.5 (R + R') (:185) on the first device: the rows of all shards are already in the caller's matrix
+        // on the first device: the rows of all shards are already in the caller's matrix
         const int rs = guarded([&] {
             GML_CUDA(cudaSetDevice(base.device));
             DevBuf<double> m;
             m.alloc((size_t)N * N);
             GML_CUDA(cudaMemcpy(m.p, out_theta, sizeof(double) * N * N, cudaMemcpyHostToDevice));
-            dim3 b(32, 8), g((unsigned)ceil_div(N, 32), (unsigned)ceil_div(N, 8));
-            symmetrize_kernel<<<g, b>>>(m.p, N);       // symmetric in (i, j): the column-major matrix is symmetrised in place
-            GML_LAUNCHED();
+            launch_symmetrize(m.p, N, 0);
             GML_CUDA(cudaMemcpy(out_theta, m.p, sizeof(double) * N * N, cudaMemcpyDeviceToHost));
         });
         if (rs != GML_B200_OK) rc = rs;
@@ -920,21 +968,6 @@ static int learn_pairwise_multi_device(const double* counts, const int8_t* spins
 // rows (one pass over the host link per byte, no replication), the threads join one NCCL communicator and advance all
 // node problems in lockstep (all-reduce of the exact int64 gradient sums per pass, csrc/comm.cu).  Every device ends
 // with the full solution; device `base.device` symmetrises it on the device (:184-186) and writes the caller's matrix.
-// where the histogram comes from: packed (counts + int8 spins) or the reference's K x (N+1) matrix
-struct HostSource {
-    const double* counts = nullptr; const int8_t* spins = nullptr;     // packed form
-    const void* matrix = nullptr; int dtype = 0;                       // matrix form
-    int64_t ld = 0;
-    double regularizer = -1.0;      // >= 0: lambda = regularizer*sqrt(log(N^2/0.05)/M) (:157) from the global sample count
-    int upload(gml_b200_handle* h, int64_t k0, int64_t k1, int32_t N, gml_b200_stats* up) const {
-        if (matrix) return gml_b200_upload_matrix(h, matrix, dtype, k0, k1 - k0, N, ld, up);
-        return gml_b200_upload_histogram(h, counts + k0, spins + k0, k1 - k0, N, ld, up);
-    }
-    double lambda_for(double lambda, int32_t N, double M) const {
-        return regularizer >= 0.0 ? regularizer * std::sqrt(std::log(((double)N * (double)N) / 0.05) / M) : lambda;
-    }
-};
-
 static int learn_pairwise_multi_device_samples(const HostSource& src, int64_t K, int32_t N,
                                                int32_t formulation, double lambda, int32_t symmetrize, const gml_b200_opts& base,
                                                int n_dev, double* out_theta, double* out_objective, gml_b200_stats* stats) {
@@ -949,61 +982,51 @@ static int learn_pairwise_multi_device_samples(const HostSource& src, int64_t K,
     uint8_t ident[128];
     if (!have_comm && gml_b200_comm_unique_id(ident) != GML_B200_OK) { comm_cache.erase(std::make_pair((int)base.device, n_dev)); return -1; }   // no NCCL: node shards
     if (!have_comm) cached.assign(n_dev, nullptr);
-    std::vector<int> rcs(n_dev, GML_B200_OK);
-    std::vector<std::string> errs(n_dev);
     std::vector<gml_b200_stats> sts(n_dev);
-    std::vector<std::thread> threads;
     const int64_t per = round_up(ceil_div(K, n_dev), 256);
-    for (int r = 0; r < n_dev; ++r)
-        threads.emplace_back([&, r] {
-            gml_b200_handle* h = nullptr;
-            gml_b200_opts o = base;
-            o.device = base.device + r; o.stream = nullptr;
-            o.node_begin = 0; o.node_end = 0; o.reserved[2] = 1; o.reserved[4] = 0;
-            o.solver = GML_B200_SOLVER_FISTA_TC;
-            const int64_t k0 = std::min<int64_t>(K, r * per), k1 = std::min<int64_t>(K, (r + 1) * per);
-            std::memset(&sts[r], 0, sizeof(gml_b200_stats));
-            gml_b200_stats up{};
-            int rc = gml_b200_create(&h, o.device);
-            if (rc == GML_B200_OK) rc = src.upload(h, k0, k1, N, &up);
-            // every thread must reach the communicator set-up, also after a failed upload (the others would wait for ever)
-            int rc_comm = GML_B200_ECUDA;
-            if (h && have_comm) { h->comm = cached[r]; h->owns_comm = false; rc_comm = GML_B200_OK; }
-            else if (h) {
-                rc_comm = gml_b200_comm_init(h, ident, r, n_dev);
-                if (rc_comm == GML_B200_OK) { cached[r] = h->comm; h->owns_comm = false; }      // the cache owns it from now on
+    const int rc = on_each_device(base.device, n_dev, [&](int r) {
+        gml_b200_handle* h = nullptr;
+        gml_b200_opts o = base;
+        o.device = base.device + r; o.stream = nullptr;
+        o.node_begin = 0; o.node_end = 0; o.reserved[2] = 1; o.reserved[4] = 0;
+        o.solver = GML_B200_SOLVER_FISTA_TC;
+        const int64_t k0 = std::min<int64_t>(K, r * per), k1 = std::min<int64_t>(K, (r + 1) * per);
+        gml_b200_stats up{};
+        int rc = gml_b200_create(&h, o.device);
+        if (rc == GML_B200_OK) rc = src.upload(h, k0, k1, N, &up);
+        // every thread must reach the communicator set-up, also after a failed upload (the others would wait for ever)
+        int rc_comm = GML_B200_ECUDA;
+        if (h && have_comm) { h->comm = cached[r]; h->owns_comm = false; rc_comm = GML_B200_OK; }
+        else if (h) {
+            rc_comm = gml_b200_comm_init(h, ident, r, n_dev);
+            if (rc_comm == GML_B200_OK) { cached[r] = h->comm; h->owns_comm = false; }      // the cache owns it from now on
+        }
+        if (rc == GML_B200_OK) rc = rc_comm;
+        if (rc_comm == GML_B200_OK) {       // leave together if any device failed so far
+            int agreed = rc;
+            if (guarded([&] { agreed = comm_agree_max(h->comm, rc, h->own_stream); }) == GML_B200_OK && agreed != GML_B200_OK && rc == GML_B200_OK) {
+                rc = agreed; set_error("another device of the multi-device solve failed");
             }
-            if (rc == GML_B200_OK) rc = rc_comm;
-            if (rc_comm == GML_B200_OK) {       // leave together if any device failed so far
-                int agreed = rc;
-                if (guarded([&] { agreed = comm_agree_max(h->comm, rc, h->own_stream); }) == GML_B200_OK && agreed != GML_B200_OK && rc == GML_B200_OK) {
-                    rc = agreed; set_error("another device of the multi-device solve failed");
-                }
+        }
+        if (rc == GML_B200_OK) rc = gml_b200_comm_globalize_histogram(h);
+        if (rc == GML_B200_OK) {
+            const double lam = src.lambda_for(lambda, N, gml_b200_num_samples(h));     // global M after the globalize step
+            if (r == 0) rc = gml_b200_solve_pairwise(h, formulation, lam, symmetrize, &o, out_theta, out_objective, &sts[r]);
+            else {
+                DevBuf<double> rows, obj_scratch;
+                try { rows.alloc((size_t)N * N); if (out_objective) obj_scratch.alloc(N); } catch (const CudaError& e) { rc = e.code; }
+                if (rc == GML_B200_OK)      // same passes as device 0: the objective pass is a collective
+                    rc = gml_b200_solve_pairwise_device(h, formulation, lam, &o, rows.p, out_objective ? obj_scratch.p : nullptr, &sts[r]);
+                cudaStreamSynchronize(h->own_stream);
             }
-            if (rc == GML_B200_OK) rc = gml_b200_comm_globalize_histogram(h);
-            if (rc == GML_B200_OK) {
-                const double lam = src.lambda_for(lambda, N, gml_b200_num_samples(h));     // global M after the globalize step
-                if (r == 0) rc = gml_b200_solve_pairwise(h, formulation, lam, symmetrize, &o, out_theta, out_objective, &sts[r]);
-                else {
-                    DevBuf<double> rows, obj_scratch;
-                    try { rows.alloc((size_t)N * N); if (out_objective) obj_scratch.alloc(N); } catch (const CudaError& e) { rc = e.code; }
-                    if (rc == GML_B200_OK)      // same passes as device 0: the objective pass is a collective
-                        rc = gml_b200_solve_pairwise_device(h, formulation, lam, &o, rows.p, out_objective ? obj_scratch.p : nullptr, &sts[r]);
-                    cudaStreamSynchronize(h->own_stream);
-                }
-                sts[r].pack_ms = up.pack_ms; sts[r].h2d_ms = up.h2d_ms; sts[r].kernel_launches += up.kernel_launches;
-            }
-            if (rc != GML_B200_OK) errs[r] = gml_b200_last_error();
-            rcs[r] = rc;
-            gml_b200_destroy(h);
-        });
-    for (auto& t : threads) t.join();
+            sts[r].pack_ms = up.pack_ms; sts[r].h2d_ms = up.h2d_ms; sts[r].kernel_launches += up.kernel_launches;
+        }
+        gml_b200_destroy(h);
+        return rc;
+    });
     if (!have_comm)
         for (int r = 0; r < n_dev; ++r)
             if (!cached[r]) { comm_cache.erase(std::make_pair((int)base.device, n_dev)); break; }      // set-up failed on some device: retry next call
-    int rc = GML_B200_OK;
-    for (int r = 0; r < n_dev; ++r)
-        if (rcs[r] != GML_B200_OK && (rc == GML_B200_OK || rc == GML_B200_ENOTCONV)) { rc = rcs[r]; set_error("device " + std::to_string(base.device + r) + ": " + errs[r]); }
     if (stats) {
         *stats = sts[0];
         for (int r = 1; r < n_dev; ++r) {
@@ -1021,56 +1044,31 @@ static int learn_pairwise_multi_device_samples(const HostSource& src, int64_t K,
 int gml_b200_learn_pairwise(const double* counts, const int8_t* spins, int64_t K, int32_t N, int64_t ld,
                             int32_t formulation, double lambda, int32_t symmetrize, const gml_b200_opts* opts,
                             double* out_theta, double* out_objective, gml_b200_stats* stats) {
-    if (opts && opts->reserved[4] > 1) {
-        const int n_dev = std::min<int>(opts->reserved[4], std::max(1, gml_b200_device_count() - opts->device));
-        // Partition (SURVEY 8e): sample slices when every device still gets a GPU-filling number of rows -- each device
-        // then streams K/n rows per pass instead of all K -- else node shards with the histogram replicated.
-        // opts->reserved[2] = 2 forces node shards.
-        const bool tc = (opts->solver == GML_B200_SOLVER_AUTO && N + 1 > NEWTON_AUTO_F) || opts->solver == GML_B200_SOLVER_FISTA_TC;
-        if (n_dev > 1 && tc && opts->reserved[2] != 2 && K / n_dev >= 65536 && opts->barrier_mu == 0.0) {
-            HostSource src;
-            src.counts = counts; src.spins = spins; src.ld = ld;
-            const int rc = learn_pairwise_multi_device_samples(src, K, N, formulation, lambda, symmetrize, *opts,
-                                                               n_dev, out_theta, out_objective, stats);
-            if (rc >= 0) return rc;
-        }
-        if (n_dev > 1 && N >= 2 * n_dev)
-            return learn_pairwise_multi_device(counts, spins, K, N, ld, formulation, lambda, symmetrize, *opts, n_dev,
-                                               out_theta, out_objective, stats);
+    HostSource src;
+    src.counts = counts; src.spins = spins; src.ld = ld;
+    const int n_dev = one_shot_devices(opts);
+    // else node shards with the histogram replicated; opts->reserved[2] = 2 forces them
+    if (use_sample_slices(opts, K, N, n_dev) && opts->reserved[2] != 2) {
+        const int rc = learn_pairwise_multi_device_samples(src, K, N, formulation, lambda, symmetrize, *opts,
+                                                           n_dev, out_theta, out_objective, stats);
+        if (rc >= 0) return rc;
     }
-    gml_b200_handle* h = nullptr;
-    int rc = gml_b200_create(&h, opts ? opts->device : 0);
-    if (rc != GML_B200_OK) return rc;
-    gml_b200_stats up{}, so{};
-    rc = gml_b200_upload_histogram(h, counts, spins, K, N, ld, &up);
-    if (rc == GML_B200_OK) rc = gml_b200_solve_pairwise(h, formulation, lambda, symmetrize, opts, out_theta, out_objective, &so);
-    if (stats) {
-        *stats = so;
-        stats->pack_ms = up.pack_ms; stats->h2d_ms = up.h2d_ms;
-        stats->kernel_launches += up.kernel_launches;
-        stats->total_ms += up.total_ms;
-    }
-    gml_b200_destroy(h);
-    return rc;
+    if (n_dev > 1 && N >= 2 * n_dev)
+        return learn_pairwise_multi_device(src, K, N, formulation, lambda, symmetrize, *opts, n_dev, out_theta,
+                                           out_objective, stats);
+    return learn_one_device(opts ? opts->device : 0, src, K, N, lambda, stats, [&](gml_b200_handle* h, double lam, gml_b200_stats* so) {
+        return gml_b200_solve_pairwise(h, formulation, lam, symmetrize, opts, out_theta, out_objective, so);
+    });
 }
 
 int gml_b200_learn_multibody(const double* counts, const int8_t* spins, int64_t K, int32_t N, int64_t ld,
                              int32_t order, double lambda, const gml_b200_opts* opts, double* out_vals,
                              double* out_objective, gml_b200_stats* stats) {
-    gml_b200_handle* h = nullptr;
-    int rc = gml_b200_create(&h, opts ? opts->device : 0);
-    if (rc != GML_B200_OK) return rc;
-    gml_b200_stats up{}, so{};
-    rc = gml_b200_upload_histogram(h, counts, spins, K, N, ld, &up);
-    if (rc == GML_B200_OK) rc = gml_b200_solve_multibody(h, order, lambda, opts, out_vals, out_objective, &so);
-    if (stats) {
-        *stats = so;
-        stats->pack_ms = up.pack_ms; stats->h2d_ms = up.h2d_ms;
-        stats->kernel_launches += up.kernel_launches;
-        stats->total_ms += up.total_ms;
-    }
-    gml_b200_destroy(h);
-    return rc;
+    HostSource src;
+    src.counts = counts; src.spins = spins; src.ld = ld;
+    return learn_one_device(opts ? opts->device : 0, src, K, N, lambda, stats, [&](gml_b200_handle* h, double lam, gml_b200_stats* so) {
+        return gml_b200_solve_multibody(h, order, lam, opts, out_vals, out_objective, so);
+    });
 }
 
 int gml_b200_learn_pairwise_matrix(const void* samples, int32_t dtype, int64_t K, int32_t N, int64_t ld,
@@ -1079,34 +1077,15 @@ int gml_b200_learn_pairwise_matrix(const void* samples, int32_t dtype, int64_t K
     if (!(regularizer >= 0.0) || !std::isfinite(regularizer)) { set_error("regularizer must be finite and >= 0"); return GML_B200_EINVAL; }
     HostSource src;
     src.matrix = samples; src.dtype = dtype; src.ld = ld; src.regularizer = regularizer;
-    if (opts && opts->reserved[4] > 1) {
-        const int n_dev = std::min<int>(opts->reserved[4], std::max(1, gml_b200_device_count() - opts->device));
-        const bool tc = (opts->solver == GML_B200_SOLVER_AUTO && N + 1 > NEWTON_AUTO_F) || opts->solver == GML_B200_SOLVER_FISTA_TC;
-        if (n_dev > 1 && tc && K / n_dev >= 65536 && opts->barrier_mu == 0.0) {
-            const int rc = learn_pairwise_multi_device_samples(src, K, N, formulation, 0.0, symmetrize, *opts, n_dev, out_theta,
-                                                               out_objective, stats);
-            if (rc >= 0) return rc;
-        }
+    const int n_dev = one_shot_devices(opts);
+    if (use_sample_slices(opts, K, N, n_dev)) {
+        const int rc = learn_pairwise_multi_device_samples(src, K, N, formulation, 0.0, symmetrize, *opts, n_dev, out_theta,
+                                                           out_objective, stats);
+        if (rc >= 0) return rc;
     }
-    gml_b200_handle* h = nullptr;
-    int rc = gml_b200_create(&h, opts ? opts->device : 0);
-    if (rc != GML_B200_OK) return rc;
-    gml_b200_stats up{}, so{};
-    rc = src.upload(h, 0, K, N, &up);
-    if (rc == GML_B200_OK) {
-        gml_b200_opts o; fill_opts(o, opts);
-        o.reserved[4] = 0;
-        rc = gml_b200_solve_pairwise(h, formulation, src.lambda_for(0.0, N, gml_b200_num_samples(h)), symmetrize, &o, out_theta,
-                                     out_objective, &so);
-    }
-    if (stats) {
-        *stats = so;
-        stats->pack_ms = up.pack_ms; stats->h2d_ms = up.h2d_ms;
-        stats->kernel_launches += up.kernel_launches;
-        stats->total_ms += up.total_ms;
-    }
-    gml_b200_destroy(h);
-    return rc;
+    return learn_one_device(opts ? opts->device : 0, src, K, N, 0.0, stats, [&](gml_b200_handle* h, double lam, gml_b200_stats* so) {
+        return gml_b200_solve_pairwise(h, formulation, lam, symmetrize, opts, out_theta, out_objective, so);
+    });
 }
 
 int gml_b200_learn_multibody_matrix(const void* samples, int32_t dtype, int64_t K, int32_t N, int64_t ld, int32_t order,
@@ -1115,21 +1094,9 @@ int gml_b200_learn_multibody_matrix(const void* samples, int32_t dtype, int64_t 
     if (!(regularizer >= 0.0) || !std::isfinite(regularizer)) { set_error("regularizer must be finite and >= 0"); return GML_B200_EINVAL; }
     HostSource src;
     src.matrix = samples; src.dtype = dtype; src.ld = ld; src.regularizer = regularizer;
-    gml_b200_handle* h = nullptr;
-    int rc = gml_b200_create(&h, opts ? opts->device : 0);
-    if (rc != GML_B200_OK) return rc;
-    gml_b200_stats up{}, so{};
-    rc = src.upload(h, 0, K, N, &up);
-    if (rc == GML_B200_OK)
-        rc = gml_b200_solve_multibody(h, order, src.lambda_for(0.0, N, gml_b200_num_samples(h)), opts, out_vals, out_objective, &so);
-    if (stats) {
-        *stats = so;
-        stats->pack_ms = up.pack_ms; stats->h2d_ms = up.h2d_ms;
-        stats->kernel_launches += up.kernel_launches;
-        stats->total_ms += up.total_ms;
-    }
-    gml_b200_destroy(h);
-    return rc;
+    return learn_one_device(opts ? opts->device : 0, src, K, N, 0.0, stats, [&](gml_b200_handle* h, double lam, gml_b200_stats* so) {
+        return gml_b200_solve_multibody(h, order, lam, opts, out_vals, out_objective, so);
+    });
 }
 
 int gml_b200_sample_gibbs_device(int32_t device, int32_t N, const int32_t* row_ptr, const int32_t* col_idx,

@@ -102,8 +102,6 @@ void comm_destroy(Comm* c) {
     delete c;
 }
 
-int comm_world(const Comm* c) { return c ? c->world : 1; }
-
 // several collectives issued between start / end go out as ONE NCCL launch
 void comm_group_start(Comm* c) { if (c && c->world > 1) nccl_check(api().GroupStart(), "ncclGroupStart"); }
 void comm_group_end(Comm* c) { if (c && c->world > 1) nccl_check(api().GroupEnd(), "ncclGroupEnd"); }

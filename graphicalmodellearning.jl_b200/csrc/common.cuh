@@ -201,9 +201,6 @@ struct EvalBackend {
 EvalBackend* make_backend_cc(const NodeProblem& p, cudaStream_t st);
 EvalBackend* make_backend_tc(const NodeProblem& p, cudaStream_t st);
 
-// --- output.cu
-void symmetrize_rowmajor(double* d_theta, int N, cudaStream_t st);
-
 // --- histogram.cu : raw samples -> deduplicated histogram (returns the number of distinct configurations)
 int64_t build_histogram(const int8_t* d_samples, int64_t M, int N, int64_t ld, int8_t* d_out_spins, int64_t ld_out,
                         double* d_out_counts, cudaStream_t st);
@@ -212,7 +209,6 @@ int64_t build_histogram(const int8_t* d_samples, int64_t M, int N, int64_t ld, i
 void comm_unique_id(uint8_t* out128);
 Comm* comm_create(const uint8_t* id128, int rank, int world);
 void comm_destroy(Comm* c);
-int comm_world(const Comm* c);
 void comm_group_start(Comm* c);
 void comm_group_end(Comm* c);
 void comm_allreduce_sum_i64(Comm* c, long long* buf, size_t n, cudaStream_t st);

@@ -89,8 +89,19 @@ def test_passes_at_headline_shapes(monkeypatch, n, kernel, level, form):
 
 def test_rough_level_is_refused_for_strongly_weighted_histograms():
     _, _, x = eval_case(300)
+    sess = eval_session(300)
     with pytest.raises(gml_b200.GMLB200Error):
-        eval_session(300).eval_pairwise(RISE(), x, "fista_tc", coarse="rough")
+        sess.eval_pairwise(RISE(), x, "fista_tc", coarse="rough")
+    # bench_passes takes the same levels as eval_pairwise: a refused one is an error, not a timing of the fine level
+    with pytest.raises(gml_b200.GMLB200Error):
+        sess.bench_passes(RISE(), "fista_tc", reps=1, coarse="rough")
+    with pytest.raises(gml_b200.GMLB200Error) as e:
+        sess.bench_passes(RISE(), "fista_cc", reps=1, coarse=True)      # the CUDA-core backend has no coarse level
+    assert e.value.code == 1
+    opts, out = B200(solver="fista_tc")._opts(), np.zeros(4)
+    assert _lib.load().gml_b200_bench_passes(sess._h, 7, ctypes.byref(opts), 1, ctypes.c_void_p(out.ctypes.data)) == 1   # unknown formulation id
+    ms = sess.bench_passes(RISE(), "fista_tc", reps=1, coarse=True)
+    assert len(ms) == 4 and all(np.isfinite(v) and v >= 0.0 for v in ms.values()) and ms["full_pass_wall"] > 0.0
 
 
 @pytest.mark.parametrize("kernel", ["pair", "streaming"])

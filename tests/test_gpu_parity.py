@@ -186,6 +186,13 @@ def test_edge_cases(golden):
     with pytest.raises(gml_b200.GMLB200Error) as e:
         gml_b200.learn(hist, RISE(), B200(solver="fista_cc", max_iter=2))
     assert e.value.code == 3
+    # the pairwise Session methods refuse multiRISE like learn() refuses a formulation it cannot run
+    sess = gml_b200.Session().upload(counts, spins)
+    for call in (lambda f: sess.solve_pairwise(f, B200()), lambda f: sess.solve_pairwise_device(f, B200(), 0, 0, 3),
+                 lambda f: sess.eval_pairwise(f, np.zeros((3, 4))), lambda f: sess.bench_passes(f),
+                 lambda f: sess.solve_path(f, B200(), [0.2])):
+        with pytest.raises(NotImplementedError):
+            call(multiRISE())
 
 
 @pytest.mark.parametrize("form", list(FORMS))
