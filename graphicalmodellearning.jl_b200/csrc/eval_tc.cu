@@ -281,15 +281,13 @@ __global__ void __launch_bounds__(128) tc_quantize_x_kernel(const double* __rest
 // GEMM-1: energies + fused epilogue
 // ------------------------------------------------------------------------------------------
 struct EnergyParams {
-    int64_t Kp;
-    int Fp, Fspin, Nn, n_tiles, node_begin_row;   // node tile t covers spin rows node_begin_row + 64 t ... of each [Fspin x 128] block
+    int Fp, Fspin, n_tiles, node_begin_row;        // node tile t covers spin rows node_begin_row + 64 t ... of each [Fspin x 128] block
     int spin_vec;                          // 1: the spin tile comes from P, sample-major [128 samples][64 nodes] (16 B per thread)
     int n_groups;                          // sample ranges; work item = (group, node tile)
     int n_waves, g_main;                   // CTA-pair kernel: wave-aligned item schedule (pair_schedule)
     int64_t sample_blocks;                 // sample blocks of this pass (Kp / 128 / block_stride)
     int64_t block_stride;                  // pass b uses histogram block b * block_stride (strided subsample)
     int64_t r_rows_per_limb;               // Nn_pad2
-    int nR, form;
     float lattice;                         // value of one unit of the combined integer energy
     const float* w32;
     uint8_t* R;                            // residual digit planes [SB][nR][Nn_pad2][128]
@@ -311,10 +309,8 @@ struct EnergyParams {
 #endif
 
 constexpr int E_STAGES = 4;
-#ifndef GML_E_EPI_WARPS
-#define GML_E_EPI_WARPS 16   // measured: full pass 4.17 ms (8 warps) -> 3.50 ms (16 warps) at N=1000, K=1e6
-#endif
-constexpr int E_EPI_WARPS = GML_E_EPI_WARPS;         // E_EPI_WARPS/4 per TMEM lane quarter, 64/(E_EPI_WARPS/4) nodes each
+constexpr int E_EPI_WARPS = 16;     // 4 per TMEM lane quarter; measured: full pass 4.17 ms (8 warps) -> 3.50 ms (16 warps) at N=1000, K=1e6
+constexpr int E_NPT = NODE_TILE1 / (E_EPI_WARPS / 4);   // nodes per epilogue thread: 16, i.e. four words of spin bytes
 constexpr int E_THREADS = 64 + 32 * E_EPI_WARPS;
 constexpr int E_A_BYTES = 128 * 128, E_B_BYTES = 256 * 128, E_STAGE_BYTES = E_A_BYTES + E_B_BYTES;
 constexpr int E_S_BYTES = NODE_TILE1 * 128;          // spins tile of the node block
@@ -356,75 +352,142 @@ __device__ __forceinline__ float fast_lg2(float x) {
     return y;
 }
 
-// Per-block epilogue math of one thread: NPT nodes of one sample (TMEM lane).  Reads the XL limb accumulators,
-// recombines them exactly, applies the node sign, evaluates the objective / residual terms, accumulates the
-// objective into facc and (GRAD) writes the NR residual digits (bytes of q + BIAS, most significant first) of every
-// node straight to global memory at rg (+ node * 128, + digit * limb_stride): a warp covers one full 32-byte sector
-// per store, and no staging tile, proxy fence, block barrier or TMA store sits between the epilogue warps and the
-// next block.  `release` is called once, right after the last TMEM read.
-template <int FORM, bool GRAD, int XL, int NR, int NPT, class Release>
-__device__ __forceinline__ void energy_epilogue_math(const EnergyParams& p, uint32_t tbase, uint32_t spin_addr, uint32_t scale_addr,
-                                                     uint8_t* __restrict__ rg, int64_t limb_stride, float wk, float (&facc)[NPT], Release release) {
+// Per-block epilogue math of one thread: NODES nodes of one sample (TMEM lane) whose XL limb sums are already in
+// registers (a[limb][node]), sw = their spin bytes (0x01 / 0xFF; 0x00 for padding nodes), four to a word.  Recombines
+// the limb sums exactly, applies the node sign, evaluates the objective / residual terms, accumulates the objective
+// into facc and (GRAD) writes the NR residual digits (bytes of q + BIAS, most significant first) of every node straight
+// to global memory at rgp[digit] + (node0 + node) * 128: a warp covers one full 32-byte sector per store, and no staging
+// tile, proxy fence, block barrier or TMA store sits between the epilogue warps and the next block.
+template <int FORM, bool GRAD, int XL, int NR, int NODES>
+__device__ __forceinline__ void energy_epilogue(const EnergyParams& p, const int32_t (&a)[4][NODES], const uint32_t* sw, uint32_t scale_addr,
+                                                uint8_t* const (&rgp)[4] /* per digit plane: address of this thread's byte of node 0 */,
+                                                int node0, float wk, float* __restrict__ facc) {
     const float c_arg = -p.lattice * 1.4426950408889634f;      // exp(-t) = ex2(c_arg * s_u * E_int)
     constexpr unsigned R_BIAS = r_bias(NR);
+    if (GML_DBG(p, 32)) { facc[0] += __int_as_float(a[0][0] ^ a[1][3] ^ (XL >= 3 ? a[2][7] : 0) ^ (XL == 4 ? a[3][5] : 0)); return; }   // ablation: TMEM reads only
 #pragma unroll
-    for (int c = 0; c < NPT / 16; ++c) {
-        uint32_t sw[4];                       // the 16 spin bytes of this chunk, packed
-        if (p.spin_vec) {
-            const uint4 v = lds128(spin_addr ^ (uint32_t)(c * 16));   // c * 16 stays inside the thread's 64-byte row
-            sw[0] = v.x; sw[1] = v.y; sw[2] = v.z; sw[3] = v.w;
+    for (int i = 0; i < NODES; ++i) {
+        const uint32_t w = sw[i >> 2];
+        const uint32_t sb_top = (i & 3) == 3 ? w : (w << (24 - 8 * (i & 3)));      // spin byte in the top byte: its sign bit is that of s_u
+        // recombine the limb sums: exact integers, at most one rounding
+        float e;
+        if (XL == 2) e = __int2float_rn(join2(a[0][i], a[1][i]));
+        else if (XL == 3) e = __int2float_rn(join2(join2(a[0][i], a[1][i]), a[2][i]));       // exact in fp32 while |E| < 4
+        else e = fmaf(__int2float_rn(join2(a[0][i], a[1][i])), 65536.f, __int2float_rn(join2(a[2][i], a[3][i])));
+        const float es = flip_sign(e, sb_top);                  // s_u * E / lattice
+        float fterm, gterm;
+        if (FORM == GML_B200_RPLE) {
+            const float t2 = -2.f * p.lattice * es;
+            const float ex = fast_ex2(-fabsf(t2) * 1.4426950408889634f);
+            fterm = wk * fmaf(fast_lg2(1.f + ex), 0.6931471805599453f, fmaxf(t2, 0.f));
+            gterm = __fdividef(2.f * wk * (t2 > 0.f ? 1.f : ex), 1.f + ex);   // 2 w sigma(-2t)
         } else {
-#pragma unroll
-            for (int w = 0; w < 4; ++w) {
-                const uint32_t b = spin_addr + (c * 16 + 4 * w) * 128;
-                sw[w] = lds_u8(b) | (lds_u8(b + 128) << 8) | (lds_u8(b + 256) << 16) | (lds_u8(b + 384) << 24);
-            }
+            // no clamp: |t| <= |x_u|_1 keeps the argument in range; an overflow for a wild trial point (|x_u|_1 > 80) gives
+            // f = inf, which the driver's descent test rejects
+            fterm = wk * fast_ex2(es * c_arg);
+            gterm = fterm;
         }
-        int32_t a0[16], a1[16], a2[16], a3[16];
-        tmem_ld16(tbase + 0 * NODE_TILE1 + c * 16, a0);
-        tmem_ld16(tbase + 1 * NODE_TILE1 + c * 16, a1);
-        if (XL >= 3) tmem_ld16(tbase + 2 * NODE_TILE1 + c * 16, a2);
-        if (XL == 4) tmem_ld16(tbase + 3 * NODE_TILE1 + c * 16, a3);
-        tmem_ld_wait();
-        if (c == NPT / 16 - 1) release();         // accumulator fully read: hand it back to the MMA warp
-        if (GML_DBG(p, 32)) { facc[0] += __int_as_float(a0[0] ^ a1[3] ^ (XL >= 3 ? a2[7] : 0) ^ (XL == 4 ? a3[11] : 0)); continue; }   // ablation: TMEM reads only
+        facc[i] += fterm;
+        if (GRAD) {
+            // r = s_u * gterm in units of the node's residual grid, rounded to nearest, plus the
+            // bias that makes all balanced digits non-negative
+            const float sscale = flip_sign(lds_f32(scale_addr + 4 * i), sb_top);      // s_u / deltaR
+            unsigned qb;      // low NR bytes = q + BIAS
+            if (NR == 4) qb = (unsigned)__float2int_rn(gterm * sscale) + R_BIAS;
+            else qb = (unsigned)__float_as_int(fmaf(gterm, sscale, r_magic(NR)));   // round to nearest, |q| < 2^22; bias from the constant
+            if (!GML_DBG(p, 64)) {
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const int nit = c * 16 + i;                           // node within this thread's slice
-            // sign bit of s_u (bytes are 0x01 / 0xFF; 0x00 for padding nodes)
-            const uint32_t sgn = ((i & 3) == 3 ? sw[i >> 2] : (sw[i >> 2] << (24 - 8 * (i & 3)))) & 0x80000000u;
-            // recombine the limb sums: exact integers, at most one rounding
-            float e;
-            if (XL == 2) e = __int2float_rn(join2(a0[i], a1[i]));
-            else if (XL == 3) e = __int2float_rn(join2(join2(a0[i], a1[i]), a2[i]));       // exact in fp32 while |E| < 4
-            else e = fmaf(__int2float_rn(join2(a0[i], a1[i])), 65536.f, __int2float_rn(join2(a2[i], a3[i])));
-            const float es = __uint_as_float(__float_as_uint(e) ^ sgn);        // s_u * E / lattice
-            float fterm, gterm;
-            if (FORM == GML_B200_RPLE) {
-                const float a = -2.f * p.lattice * es;
-                const float ex = fast_ex2(-fabsf(a) * 1.4426950408889634f);
-                fterm = wk * fmaf(fast_lg2(1.f + ex), 0.6931471805599453f, fmaxf(a, 0.f));
-                gterm = __fdividef(2.f * wk * (a > 0.f ? 1.f : ex), 1.f + ex);   // 2 w sigma(-2t)
-            } else {
-                fterm = wk * fast_ex2(fminf(es * c_arg, 115.f));
-                gterm = fterm;
-            }
-            facc[nit] += fterm;
-            if (GRAD) {
-                // r = s_u * gterm in units of the node's residual grid, rounded to nearest, plus the
-                // bias that makes all balanced digits non-negative
-                const float sscale = __uint_as_float(__float_as_uint(lds_f32(scale_addr + 4 * nit)) ^ sgn);      // s_u / deltaR
-                unsigned qb;      // low NR bytes = q + BIAS
-                if (NR == 4) qb = (unsigned)__float2int_rn(gterm * sscale) + R_BIAS;
-                else qb = (unsigned)__float_as_int(fmaf(gterm, sscale, r_magic(NR)));      // round to nearest, |q| < 2^22; bias from the constant
-                uint8_t* dst = rg + nit * 128;
-#pragma unroll
-                for (int j = 0; j < NR; ++j)      // plane 0 = most significant byte
-                    if (!GML_DBG(p, 64) || qb == 0xFFFFFFFFu) dst[j * limb_stride] = (uint8_t)(qb >> (8 * (NR - 1 - j)));
+                for (int j = 0; j < NR; ++j) rgp[j][(node0 + i) * 128] = (uint8_t)(qb >> (8 * (NR - 1 - j)));      // plane 0 = most significant byte
             }
         }
     }
 }
+// TMEM loads of the XL limb sums of NODES (8 or 16) consecutive accumulator columns from tchunk on
+template <int XL, int NODES>
+__device__ __forceinline__ void epi_issue(uint32_t tchunk, int32_t (&a)[4][NODES]) {
+    static_assert(NODES == 8 || NODES == 16, "TMEM loads come in x8 and x16 groups");
+#pragma unroll
+    for (int j = 0; j < XL; ++j) {
+        if constexpr (NODES == 16) tmem_ld16(tchunk + j * NODE_TILE1, a[j]);
+        else tmem_ld8(tchunk + j * NODE_TILE1, a[j]);
+    }
+}
+template <int XL>
+__device__ __forceinline__ void epi_wait(int32_t (&a)[4][8]) {
+    tmem_ld_wait_on(a[0]);
+#pragma unroll
+    for (int j = 1; j < XL; ++j) reg_fence(a[j]);
+}
+
+// Producer side: the spin tile of node tile nt for histogram block sb, landing on `bar`.  From P itself (sample-major,
+// box {64 nodes, 128 samples}) when the shard's first spin column is 16-byte aligned, else from the sample-blocked
+// spin rows (node-major, box 64 rows).
+__device__ __forceinline__ void load_spin_tile(const EnergyParams& p, void* dst, const CUtensorMap* tmS, const CUtensorMap* tmSv,
+                                               uint64_t* bar, int nt, int64_t sb, uint32_t pred) {
+    mbar_expect_tx_if(bar, E_S_BYTES, pred);
+    if (p.spin_vec) tma_load_2d_if(dst, tmSv, bar, p.node_begin_row + nt * NODE_TILE1, (int)(sb * 128), pred);
+    else tma_load_2d_if(dst, tmS, bar, 0, (int)(sb * p.Fspin) + p.node_begin_row + nt * NODE_TILE1, pred);
+}
+// Epilogue side: the spin bytes of the thread's E_NPT nodes from node0 on at sample `row` of the spin tile at `tile`, four
+// to a word: 16 contiguous bytes of the sample-major tile [128 samples][64 nodes] (64B swizzle: 16-byte chunk index
+// ^= (row >> 1) & 3), or one byte per node at column `row` of the node-major tile [64 nodes][128 samples].
+__device__ __forceinline__ void spin_words(const EnergyParams& p, uint32_t tile, int row, int node0, uint32_t (&sw)[4]) {
+    if (p.spin_vec) {
+        const uint4 v = lds128(tile + row * NODE_TILE1 + (node0 ^ (((row >> 1) & 3) << 4)));
+        sw[0] = v.x; sw[1] = v.y; sw[2] = v.z; sw[3] = v.w;
+    } else {
+        const uint32_t sa = tile + node0 * 128 + row;
+#pragma unroll
+        for (int w = 0; w < 4; ++w)
+            sw[w] = lds_u8(sa + 4 * w * 128) | (lds_u8(sa + (4 * w + 1) * 128) << 8) | (lds_u8(sa + (4 * w + 2) * 128) << 16) | (lds_u8(sa + (4 * w + 3) * 128) << 24);
+    }
+}
+// Per digit plane, the address of the thread's byte of node node0 of node tile nt in sample block sb:
+// R[((sb * NR + digit) * rows + node) * 128 + sample].  A block that must not be stored (!valid) goes to a scratch tile.
+template <int NR>
+__device__ __forceinline__ void digit_planes(const EnergyParams& p, bool valid, int64_t sb, int nt, int node0, int row, uint8_t* (&rgp)[4]) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        rgp[j] = valid ? p.R + (((sb * NR + j) * p.r_rows_per_limb + nt * NODE_TILE1 + node0) * 128 + row)
+                       : p.r_scratch + ((j * NODE_TILE1 + node0) * 128 + row);
+}
+
+// Objective sums of one epilogue thread over one work item (its E_NPT nodes of node tile nt): fp32 per-thread partial
+// sums over at most 32 sample blocks, then fp64 warp sums added to fsum.
+struct ItemObjective {
+    float facc[E_NPT];
+    int since_flush;
+    double* fsum;                             // objective sum of the thread's first node
+    // start of an item; GRAD: also refill the node tile's residual scales
+    template <bool GRAD>
+    __device__ __forceinline__ void begin(const EnergyParams& p, int nt, int node0, float* s_scale) {
+#pragma unroll
+        for (int i = 0; i < E_NPT; ++i) facc[i] = 0.f;
+        if (GRAD) {
+            const int et = threadIdx.x - 64;
+            named_bar_sync(1, 32 * E_EPI_WARPS);          // previous item's readers are done with s_scale
+            if (et < NODE_TILE1) s_scale[et] = p.inv_dr[nt * NODE_TILE1 + et];
+            named_bar_sync(1, 32 * E_EPI_WARPS);
+        }
+        since_flush = 0;
+        fsum = p.fsum + (int64_t)nt * NODE_TILE1 + node0;
+    }
+    // before each sample block
+    __device__ __forceinline__ void next_block() {
+        if (since_flush >= 32) { flush(); since_flush = 0; }
+        ++since_flush;
+    }
+    // after the item's last block
+    __device__ __forceinline__ void flush() {
+#pragma unroll
+        for (int i = 0; i < E_NPT; ++i) {
+            double v = (double)facc[i];
+            for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            if ((threadIdx.x & 31) == 0) atomicAdd(fsum + i, v);
+            facc[i] = 0.f;
+        }
+    }
+};
 
 // Work decomposition: item = (sample range g, node tile nt), ordered group-major and dealt round-robin,
 // so CTAs that run concurrently stream the SAME sample blocks for different node tiles (the P tiles are
@@ -487,9 +550,7 @@ __global__ void __launch_bounds__(E_THREADS, 1) tc_energy_kernel(const __grid_co
             for (int64_t eb = b0; eb < b1; ++eb) {
                 const int64_t sb = eb * p.block_stride;
                 mbar_wait(&sempty[slot], sphase ^ 1);
-                mbar_expect_tx_if(&sfull[slot], E_S_BYTES, leader);
-                if (p.spin_vec) tma_load_2d_if(s_spin + slot * E_S_BYTES, &tmSv, &sfull[slot], p.node_begin_row + nt * NODE_TILE1, (int)(sb * 128), leader);
-                else tma_load_2d_if(s_spin + slot * E_S_BYTES, &tmS, &sfull[slot], 0, (int)(sb * p.Fspin) + p.node_begin_row + nt * NODE_TILE1, leader);
+                load_spin_tile(p, s_spin + slot * E_S_BYTES, &tmS, &tmSv, &sfull[slot], nt, sb, leader);
                 if (++slot == 2) { slot = 0; sphase ^= 1; }
                 for (int kb = 0; kb < kblocks; ++kb) {
                     mbar_wait(&empty[stage], phase ^ 1);
@@ -531,43 +592,20 @@ __global__ void __launch_bounds__(E_THREADS, 1) tc_energy_kernel(const __grid_co
             }
         }
     } else {
-        // ================= epilogue warps 2..9: TMEM lane quarter = warp % 4, node half = (warp-2)/4 =========
+        // ================= epilogue warps 2..17: TMEM lane quarter = warp % 4, node slice = (warp-2)/4 =========
         const int quarter = warp & 3;
-        const int half = (warp - 2) >> 2;                // which slice of the node tile this warp owns
+        const int node0 = ((warp - 2) >> 2) * E_NPT;     // first node of the slice of the node tile this warp owns
         const int row = quarter * 32 + lane;            // sample within the block == TMEM lane
-        const int et = threadIdx.x - 64;                // 0..255
-        constexpr int NPT = NODE_TILE1 / (E_EPI_WARPS / 4);   // nodes per thread
-        constexpr int ACC_STAGES = 2;
-        constexpr int EPI_THREADS = 32 * E_EPI_WARPS;
-        float facc[NPT];
+        ItemObjective obj;
         int as = 0; uint32_t aphase = 0;
         int slot = 0; uint32_t sphase = 0;
-        const int64_t limb_stride = p.r_rows_per_limb * 128;
         for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
             int nt; int64_t b0, b1;
             item_range(item, nt, b0, b1);
-#pragma unroll
-            for (int i = 0; i < NPT; ++i) facc[i] = 0.f;
-            if (GRAD) {
-                named_bar_sync(1, EPI_THREADS);          // previous item's readers are done with s_scale
-                if (et < NODE_TILE1) s_scale[et] = p.inv_dr[nt * NODE_TILE1 + et];
-                named_bar_sync(1, EPI_THREADS);
-            }
-            int since_flush = 0;
-            auto flush = [&]() {
-#pragma unroll
-                for (int i = 0; i < NPT; ++i) {
-                    double v = (double)facc[i];
-                    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-                    if (lane == 0) atomicAdd(p.fsum + (int64_t)nt * NODE_TILE1 + half * NPT + i, v);
-                    facc[i] = 0.f;
-                }
-            };
+            obj.begin<GRAD>(p, nt, node0, s_scale);
             for (int64_t eb = b0; eb < b1; ++eb) {
                 const int64_t sb = eb * p.block_stride;
-                // objective terms: fp32 per-thread partial sums over at most 32 sample blocks, then fp64
-                if (since_flush >= 32) { flush(); since_flush = 0; }
-                ++since_flush;
+                obj.next_block();
                 const float wk = p.w32[sb * 128 + row];
                 mbar_wait(&sfull[slot], sphase);
                 mbar_wait(&tfull[as], aphase);
@@ -576,89 +614,32 @@ __global__ void __launch_bounds__(E_THREADS, 1) tc_energy_kernel(const __grid_co
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) { mbar_arrive(&tempty[as]); mbar_arrive(&sempty[slot]); }
-                    if (++as == ACC_STAGES) { as = 0; aphase ^= 1; }
+                    if (++as == 2) { as = 0; aphase ^= 1; }
                     if (++slot == 2) { slot = 0; sphase ^= 1; }
                     continue;
                 }
-                // residual digits of this thread: R[((sb * NR + digit) * rows + node) * 128 + sample]
-                uint8_t* rg = p.R + ((sb * NR * p.r_rows_per_limb + nt * NODE_TILE1 + half * NPT) * 128 + row);
-                // spins of this thread's nodes: either 16 contiguous bytes of the sample-major tile [128 samples][64 nodes]
-                // or one byte per node at column `row` of the node-major tile [64 nodes][128 samples]
-                const uint32_t spin_base = smem_u32(s_spin) + slot * E_S_BYTES;
-                const uint32_t spin_addr = p.spin_vec ? spin_base + row * NODE_TILE1 + ((half * NPT) ^ (((row >> 1) & 3) << 4)) : spin_base + half * NPT * 128 + row;
-                const uint32_t scale_addr = smem_u32(s_scale) + 4 * half * NPT;
-                const uint32_t tbase = tmem_base + ((uint32_t)(quarter * 32) << 16) + as * 256 + half * NPT;
-                energy_epilogue_math<FORM, GRAD, XL, NR, NPT>(p, tbase, spin_addr, scale_addr, rg, limb_stride, wk, facc, [&] {
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&tempty[as]);
-                });
+                uint8_t* rgp[4];
+                digit_planes<NR>(p, true, sb, nt, node0, row, rgp);
+                uint32_t sw[4];
+                spin_words(p, smem_u32(s_spin) + slot * E_S_BYTES, row, node0, sw);
+                int32_t a[4][E_NPT];
+                epi_issue<XL>(tmem_base + ((uint32_t)(quarter * 32) << 16) + as * 256 + node0, a);
+                tmem_ld_wait();
+                tc_fence_before();                       // accumulator fully read: hand it back to the MMA warp
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&tempty[as]);
+                energy_epilogue<FORM, GRAD, XL, NR>(p, a, sw, smem_u32(s_scale) + 4 * node0, rgp, 0, wk, obj.facc);
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&sempty[slot]);
                 if (++as == 2) { as = 0; aphase ^= 1; }
                 if (++slot == 2) { slot = 0; sphase ^= 1; }
             }
-            flush();
+            obj.flush();
         }
     }
     tc_fence_before();
     __syncthreads();
     if (warp == 1) tmem_dealloc(tmem_base, 512);
-}
-
-// Chunked form of the epilogue math for software-pipelined epilogues: 8 nodes of one sample whose XL limb sums
-// are already in registers (a[limb][node]); sw0 / sw1 = the 8 spin bytes.  Same arithmetic as above.
-template <int FORM, bool GRAD, int XL, int NR>
-__device__ __forceinline__ void energy_chunk_math(const EnergyParams& p, int32_t (&a)[4][8], uint32_t sw0, uint32_t sw1, uint32_t scale_addr,
-                                                  uint8_t* const (&rgp)[4] /* per digit plane: address of this thread's byte of node 0 */,
-                                                  int node0, float wk, float* __restrict__ facc) {
-    const float c_arg = -p.lattice * 1.4426950408889634f;
-    constexpr unsigned R_BIAS = r_bias(NR);
-    if (GML_DBG(p, 32)) { facc[0] += __int_as_float(a[0][0] ^ a[1][3] ^ (XL >= 3 ? a[2][7] : 0) ^ (XL == 4 ? a[3][5] : 0)); return; }
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const uint32_t w = i < 4 ? sw0 : sw1;
-        const uint32_t sb_top = (i & 3) == 3 ? w : (w << (24 - 8 * (i & 3)));      // spin byte (0x01 / 0xFF / 0x00) in the top byte
-        float e;
-        if (XL == 2) e = __int2float_rn(join2(a[0][i], a[1][i]));
-        else if (XL == 3) e = __int2float_rn(join2(join2(a[0][i], a[1][i]), a[2][i]));
-        else e = fmaf(__int2float_rn(join2(a[0][i], a[1][i])), 65536.f, __int2float_rn(join2(a[2][i], a[3][i])));
-        const float es = flip_sign(e, sb_top);
-        float fterm, gterm;
-        if (FORM == GML_B200_RPLE) {
-            const float t2 = -2.f * p.lattice * es;
-            const float ex = fast_ex2(-fabsf(t2) * 1.4426950408889634f);
-            fterm = wk * fmaf(fast_lg2(1.f + ex), 0.6931471805599453f, fmaxf(t2, 0.f));
-            gterm = __fdividef(2.f * wk * (t2 > 0.f ? 1.f : ex), 1.f + ex);
-        } else {
-            // no clamp: |t| <= |x_u|_1 keeps the argument in range; an overflow for a wild trial point (|x_u|_1 > 80) gives
-            // f = inf, which the driver's descent test rejects
-            fterm = wk * fast_ex2(es * c_arg);
-            gterm = fterm;
-        }
-        facc[i] += fterm;
-        if (GRAD) {
-            const float sscale = flip_sign(lds_f32(scale_addr + 4 * i), sb_top);      // s_u / deltaR
-            unsigned qb;      // low NR bytes = q + BIAS
-            if (NR == 4) qb = (unsigned)__float2int_rn(gterm * sscale) + R_BIAS;
-            else qb = (unsigned)__float_as_int(fmaf(gterm, sscale, r_magic(NR)));   // round to nearest, |q| < 2^22; bias from the constant
-            if (!GML_DBG(p, 64)) {
-#pragma unroll
-                for (int j = 0; j < NR; ++j) rgp[j][(node0 + i) * 128] = (uint8_t)(qb >> (8 * (NR - 1 - j)));      // plane 0 = most significant byte
-            }
-        }
-    }
-}
-template <int XL>
-__device__ __forceinline__ void epi_issue(uint32_t tchunk, int32_t (&a)[4][8]) {
-#pragma unroll
-    for (int j = 0; j < XL; ++j) tmem_ld8(tchunk + j * NODE_TILE1, a[j]);
-}
-template <int XL>
-__device__ __forceinline__ void epi_wait(int32_t (&a)[4][8]) {
-    tmem_ld_wait_on(a[0]);
-#pragma unroll
-    for (int j = 1; j < XL; ++j) reg_fence(a[j]);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -778,9 +759,7 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                 const int64_t eb = min(2 * pb + (int64_t)rank, p.sample_blocks - 1);    // an odd tail re-reads the last block (its epilogue is skipped)
                 const int64_t sb = eb * p.block_stride;
                 mbar_wait(&sempty[slot], sphase ^ 1);
-                mbar_expect_tx_if(&sfull[slot], E_S_BYTES, lane_leader);
-                if (p.spin_vec) tma_load_2d_if(s_spin + slot * E_S_BYTES, &tmSv, &sfull[slot], p.node_begin_row + nt * NODE_TILE1, (int)(sb * 128), lane_leader);
-                else tma_load_2d_if(s_spin + slot * E_S_BYTES, &tmS, &sfull[slot], 0, (int)(sb * p.Fspin) + p.node_begin_row + nt * NODE_TILE1, lane_leader);
+                load_spin_tile(p, s_spin + slot * E_S_BYTES, &tmS, &tmSv, &sfull[slot], nt, sb, lane_leader);
                 if (++slot == 2) { slot = 0; sphase ^= 1; }
                 for (int kb = 0; kb < kblocks; ++kb) {
                     mbar_wait(&empty[stage], phase ^ 1);
@@ -828,36 +807,18 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
     } else {
         // ================= epilogue warps of this CTA: its own 128 samples of every pair-step =================
         const int quarter = warp & 3;
-        const int half = (warp - 2) >> 2;
+        const int node0 = ((warp - 2) >> 2) * E_NPT;
         const int row = quarter * 32 + lane;
-        const int et = threadIdx.x - 64;
-        constexpr int NPT = NODE_TILE1 / (E_EPI_WARPS / 4);
-        constexpr int EPI_THREADS = 32 * E_EPI_WARPS;
-        float facc[NPT];
+        ItemObjective obj;
         int as = 0; uint32_t aphase = 0;
         int slot = 0; uint32_t sphase = 0;
-        const int64_t limb_stride = p.r_rows_per_limb * 128;
         const uint32_t tempty_leader0 = mapa_rank(smem_u32(&tempty[0]), 0), tempty_leader1 = mapa_rank(smem_u32(&tempty[1]), 0);
+        const uint32_t tlane = tmem_base + ((uint32_t)(quarter * 32) << 16) + node0;
+        const uint32_t scale_addr = smem_u32(s_scale) + 4 * node0;
         for (int w = 0; w < p.n_waves; ++w) {
             int nt; int64_t b0, b1;
             if (!wave_item(w, nt, b0, b1)) continue;
-#pragma unroll
-            for (int i = 0; i < NPT; ++i) facc[i] = 0.f;
-            if (GRAD) {
-                named_bar_sync(1, EPI_THREADS);
-                if (et < NODE_TILE1) s_scale[et] = p.inv_dr[nt * NODE_TILE1 + et];
-                named_bar_sync(1, EPI_THREADS);
-            }
-            int since_flush = 0;
-            auto flush = [&]() {
-#pragma unroll
-                for (int i = 0; i < NPT; ++i) {
-                    double v = (double)facc[i];
-                    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-                    if (lane == 0) atomicAdd(p.fsum + (int64_t)nt * NODE_TILE1 + half * NPT + i, v);
-                    facc[i] = 0.f;
-                }
-            };
+            obj.begin<GRAD>(p, nt, node0, s_scale);
             auto block_of = [&](int64_t pb) { return min(2 * pb + (int64_t)rank, p.sample_blocks - 1) * p.block_stride; };
             if (GML_DBG(p, 1)) {                        // ablation: no epilogue, only the barrier hand-shakes
                 for (int64_t pb = b0; pb < b1; ++pb) {
@@ -872,10 +833,6 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                 }
                 continue;
             }
-            // Software pipeline over half-blocks (8 of the thread's 16 nodes): the TMEM loads of the next chunk are in
-            // flight while the current chunk is evaluated -- also across block boundaries when the next accumulator is
-            // already published -- so TMEM read latency / bandwidth overlaps the math instead of preceding it.
-            static_assert(NPT == 16, "the pipelined epilogue is written for 16 nodes per thread");
             if (XL == 4) {
                 // 4-limb passes: plain form (one x16 load group per block); the pipelined form below needs 2 x 32
                 // accumulator registers there, spills, and measured slower (5.6 vs 5.0 ms at K = 2e6)
@@ -883,8 +840,7 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                 for (int64_t pb = b0; pb < b1; ++pb) {
                     const bool valid = 2 * pb + (int64_t)rank < p.sample_blocks;
                     const int64_t sb = block_of(pb);
-                    if (since_flush >= 32) { flush(); since_flush = 0; }
-                    ++since_flush;
+                    obj.next_block();
                     const float wk = wk_next;
                     if (pb + 1 < b1) wk_next = __ldg(p.w32 + block_of(pb + 1) * 128 + row);
                     mbar_wait(&sfull[slot], sphase);
@@ -896,27 +852,30 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                         __syncwarp();
                         if (lane == 0) { mbar_arrive_cluster(tempty_leader); mbar_arrive(&sempty[slot]); }
                     } else {
-                        uint8_t* rg = p.R + ((sb * NR * p.r_rows_per_limb + nt * NODE_TILE1 + half * NPT) * 128 + row);
-                        const uint32_t spin_base = smem_u32(s_spin) + slot * E_S_BYTES;
-                        const uint32_t spin_addr = p.spin_vec ? spin_base + row * NODE_TILE1 + ((half * NPT) ^ (((row >> 1) & 3) << 4)) : spin_base + half * NPT * 128 + row;
-                        const uint32_t tbase = tmem_base + ((uint32_t)(quarter * 32) << 16) + as * 256 + half * NPT;
-                        energy_epilogue_math<FORM, GRAD, XL, NR, NPT>(p, tbase, spin_addr, smem_u32(s_scale) + 4 * half * NPT, rg, limb_stride, wk, facc, [&] {
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) mbar_arrive_cluster(tempty_leader);
-                        });
+                        uint8_t* rgp[4];
+                        digit_planes<NR>(p, true, sb, nt, node0, row, rgp);
+                        uint32_t sw[4];
+                        spin_words(p, smem_u32(s_spin) + slot * E_S_BYTES, row, node0, sw);
+                        int32_t a[4][E_NPT];
+                        epi_issue<XL>(tlane + as * 256, a);
+                        tmem_ld_wait();
+                        tc_fence_before();                   // accumulator fully read: hand it back to the MMA warp
+                        __syncwarp();
+                        if (lane == 0) mbar_arrive_cluster(tempty_leader);
+                        energy_epilogue<FORM, GRAD, XL, NR>(p, a, sw, scale_addr, rgp, 0, wk, obj.facc);
                         __syncwarp();
                         if (lane == 0) mbar_arrive(&sempty[slot]);
                     }
                     if (++as == 2) { as = 0; aphase ^= 1; }
                     if (++slot == 2) { slot = 0; sphase ^= 1; }
                 }
-                flush();
+                obj.flush();
                 continue;
             }
+            // Software pipeline over half-blocks (8 of the thread's 16 nodes): the TMEM loads of the next chunk are in
+            // flight while the current chunk is evaluated -- also across block boundaries when the next accumulator is
+            // already published -- so TMEM read latency / bandwidth overlaps the math instead of preceding it.
             int32_t ra[4][8], rb[4][8];
-            const uint32_t tlane = tmem_base + ((uint32_t)(quarter * 32) << 16) + half * NPT;
-            const uint32_t scale_addr = smem_u32(s_scale) + 4 * half * NPT;
             float wk_next = b0 < b1 ? __ldg(p.w32 + block_of(b0) * 128 + row) : 0.f;
             if (b0 < b1) {
                 mbar_wait(&sfull[slot], sphase);
@@ -927,27 +886,13 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
             for (int64_t pb = b0; pb < b1; ++pb) {
                 const bool valid = 2 * pb + (int64_t)rank < p.sample_blocks;      // false: second block of an odd tail (nothing is stored or summed)
                 const int64_t sb = block_of(pb);
-                if (since_flush >= 32) { flush(); since_flush = 0; }
-                ++since_flush;
+                obj.next_block();
                 const float wk = valid ? wk_next : 0.f;
                 if (pb + 1 < b1) wk_next = __ldg(p.w32 + block_of(pb + 1) * 128 + row);
-                // digit planes of this thread's first node; the duplicate block of an odd tail writes to a scratch tile instead
                 uint8_t* rgp[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-                    rgp[j] = valid ? p.R + (((sb * NR + j) * p.r_rows_per_limb + nt * NODE_TILE1 + half * NPT) * 128 + row)
-                                   : p.r_scratch + ((j * NODE_TILE1 + half * NPT) * 128 + row);
-                const uint32_t spin_base = smem_u32(s_spin) + slot * E_S_BYTES;
+                digit_planes<NR>(p, valid, sb, nt, node0, row, rgp);
                 uint32_t sw[4];
-                if (p.spin_vec) {
-                    const uint4 v = lds128(spin_base + row * NODE_TILE1 + ((half * NPT) ^ (((row >> 1) & 3) << 4)));
-                    sw[0] = v.x; sw[1] = v.y; sw[2] = v.z; sw[3] = v.w;
-                } else {
-                    const uint32_t sa = spin_base + half * NPT * 128 + row;
-#pragma unroll
-                    for (int w = 0; w < 4; ++w)
-                        sw[w] = lds_u8(sa + 4 * w * 128) | (lds_u8(sa + (4 * w + 1) * 128) << 8) | (lds_u8(sa + (4 * w + 2) * 128) << 16) | (lds_u8(sa + (4 * w + 3) * 128) << 24);
-                }
+                spin_words(p, smem_u32(s_spin) + slot * E_S_BYTES, row, node0, sw);
                 // The 16 spin bytes of this thread are in registers: hand the slot back NOW.  Releasing it only after the
                 // block's math (as the first version did) chains the TMA producer -- which loads spin tile b+2 in order
                 // with the histogram tiles of block b+2 -- to the END of epilogue b, and the MMA warp then starts every
@@ -957,7 +902,7 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                 // ---- nodes 0..7 (in ra); nodes 8..15 start loading
                 epi_wait<XL>(ra);
                 epi_issue<XL>(tlane + as * 256 + 8, rb);
-                energy_chunk_math<FORM, GRAD, XL, NR>(p, ra, sw[0], sw[1], scale_addr, rgp, 0, wk, facc);
+                energy_epilogue<FORM, GRAD, XL, NR>(p, ra, sw, scale_addr, rgp, 0, wk, obj.facc);
                 // ---- nodes 8..15 (in rb): the accumulator is now fully read
                 epi_wait<XL>(rb);
                 tc_fence_before();
@@ -970,7 +915,7 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                     pre = __all_sync(0xffffffffu, mbar_test(&tfull[as_n], aphase_n) && mbar_test(&sfull[slot_n], sphase_n));
                     if (pre) { tc_fence_after(); epi_issue<XL>(tlane + as_n * 256, ra); }
                 }
-                energy_chunk_math<FORM, GRAD, XL, NR>(p, rb, sw[2], sw[3], scale_addr + 32, rgp, 8, wk, facc + 8);
+                energy_epilogue<FORM, GRAD, XL, NR>(p, rb, sw + 2, scale_addr + 32, rgp, 8, wk, obj.facc + 8);
                 as = as_n; aphase = aphase_n; slot = slot_n; sphase = sphase_n;
                 if (pb + 1 < b1 && !pre) {
                     mbar_wait(&sfull[slot], sphase);
@@ -979,7 +924,7 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
                     epi_issue<XL>(tlane + as * 256, ra);
                 }
             }
-            flush();
+            obj.flush();
         }
     }
     tc_fence_before();
@@ -991,7 +936,7 @@ tc_energy_pair_kernel(const __grid_constant__ CUtensorMap tmA,    // P  [Kp x Fp
 // GEMM-2: gradient contraction, split over sample ranges
 // ------------------------------------------------------------------------------------------
 struct GradParams {
-    int Fp, m_tiles, f_tiles, nR;
+    int Fp, m_tiles, f_tiles;
     int64_t r_rows_per_limb;      // Nn_pad2
     int n_splits;                 // sample ranges; work item = (split, output tile)
     int64_t sample_blocks, block_stride;   // as in EnergyParams
@@ -1241,12 +1186,53 @@ CUtensorMap make_map_2d(const void* base, uint64_t inner, uint64_t outer, uint32
     return m;
 }
 
+// ---- the kernel instantiations, each named once; BackendTC::configure() and eval() both go through the lookups below
+using EnergyKernel = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, EnergyParams);
+using GradKernel = void (*)(CUtensorMap, CUtensorMap, GradParams);
+template <class K> struct Launch { K kernel; int smem; };   // kernel and its dynamic shared memory
+
+// form: RPLE, or RISE for both RISE and logRISE; xl = iterate limbs (4 fine, 3 coarse, 2 rough level); nr = residual
+// digit planes, read by the gradient passes only (the rough level has one)
+struct EnergyInstance { int form; bool grad; int xl, nr; EnergyKernel stream, pair; };
+template <int FORM, bool GRAD, int XL, int NR>
+EnergyInstance energy_instance() { return {FORM, GRAD, XL, NR, tc_energy_kernel<FORM, GRAD, XL, NR>, tc_energy_pair_kernel<FORM, GRAD, XL, NR>}; }
+const EnergyInstance ENERGY_KERNELS[] = {
+    energy_instance<GML_B200_RISE, false, 4, 2>(), energy_instance<GML_B200_RISE, true, 4, 2>(),
+    energy_instance<GML_B200_RISE, true, 4, 3>(), energy_instance<GML_B200_RISE, true, 4, 4>(),
+    energy_instance<GML_B200_RISE, false, 3, 2>(), energy_instance<GML_B200_RISE, true, 3, 2>(),
+    energy_instance<GML_B200_RISE, true, 3, 3>(), energy_instance<GML_B200_RISE, true, 3, 4>(),
+    energy_instance<GML_B200_RISE, false, 2, 1>(), energy_instance<GML_B200_RISE, true, 2, 1>(),
+    energy_instance<GML_B200_RPLE, false, 4, 2>(), energy_instance<GML_B200_RPLE, true, 4, 2>(),
+    energy_instance<GML_B200_RPLE, true, 4, 3>(), energy_instance<GML_B200_RPLE, true, 4, 4>(),
+    energy_instance<GML_B200_RPLE, false, 3, 2>(), energy_instance<GML_B200_RPLE, true, 3, 2>(),
+    energy_instance<GML_B200_RPLE, true, 3, 3>(), energy_instance<GML_B200_RPLE, true, 3, 4>(),
+    energy_instance<GML_B200_RPLE, false, 2, 1>(), energy_instance<GML_B200_RPLE, true, 2, 1>()};
+Launch<EnergyKernel> energy_kernel(int form, bool grad, int xl, int nr, bool pair) {
+    const int kform = form == GML_B200_RPLE ? GML_B200_RPLE : GML_B200_RISE;
+    for (const EnergyInstance& k : ENERGY_KERNELS)
+        if (k.form == kform && k.grad == grad && k.xl == xl && (k.nr == nr || !grad))    // one objective-only kernel serves every nr
+            return pair ? Launch<EnergyKernel>{k.pair, e2_smem(xl)} : Launch<EnergyKernel>{k.stream, E_SMEM};
+    GML_REQUIRE(false, "no tensor-core energy kernel for this formulation and precision level");
+    return {nullptr, 0};
+}
+
+// nr = residual digit planes, ft = feature-tile width
+struct GradInstance { int nr, ft; GradKernel kernel; };
+const GradInstance GRAD_KERNELS[] = {{1, 128, tc_grad_kernel<1, 128>}, {1, 256, tc_grad_kernel<1, 256>}, {2, 128, tc_grad_kernel<2, 128>},
+                                     {2, 256, tc_grad_kernel<2, 256>}, {3, 128, tc_grad_kernel<3, 128>}, {4, 128, tc_grad_kernel<4, 128>}};
+Launch<GradKernel> grad_kernel(int nr, int ft) {
+    for (const GradInstance& k : GRAD_KERNELS)
+        if (k.nr == nr && k.ft == ft) return {k.kernel, g_stages(nr, ft) * g_stage_bytes(nr, ft) + 1024 + 128};
+    GML_REQUIRE(false, "no tensor-core gradient kernel for this residual width");
+    return {nullptr, 0};
+}
+
 struct BackendTC : EvalBackend {
     const NodeProblem& p;
     int Nn_pad1, Nn_pad2, nR, n_sms;   // nR: residual limbs of the fine level
     int level = 1;                      // 0 = coarse (3-limb iterate, nR-1 residual limbs), 1 = fine
     int32_t first_row = 0;   // spin rows of this shard are contiguous in `base`: spin_row[u] = first_row + u
-    DevBuf<int8_t> X4, X3, X2, R;
+    DevBuf<int8_t> X, R;                // X: iterate limbs, room for 4; each pass's quantiser rewrites the rows its limb count uses
     DevBuf<float> inv_dr;
     DevBuf<double> delta;
     DevBuf<double> fsum;
@@ -1265,7 +1251,8 @@ struct BackendTC : EvalBackend {
     const int8_t* spin_blocked = nullptr;
     int Fspin = 0;
     DevBuf<int8_t> base_blocked;
-    CUtensorMap tmA, tmB, tmB3, tmB2, tmBh, tmB3h, tmB2h, tmS, tmSv, tmRa, tmQ, tmQ256;
+    CUtensorMap tmB[3], tmBh[3];        // limb tile / half limb tile of xl = 2, 3, 4 iterate limbs, at [xl - 2]
+    CUtensorMap tmA, tmS, tmSv, tmRa, tmQ, tmQ256;
     bool pair_ok = false;               // the CTA-pair energy kernel applies (limb half-tile fits: Fp <= E2_MAX_FP)
     bool spin_vec = false;
 
@@ -1280,9 +1267,7 @@ struct BackendTC : EvalBackend {
         GML_CUDA(cudaGetDevice(&dev));
         GML_CUDA(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, dev));
         P = ensure_P(h, p.Q, p.Fp, st);
-        X4.alloc((size_t)Nn_pad1 * 4 * p.Fp);
-        X3.alloc((size_t)Nn_pad1 * 3 * p.Fp);
-        X2.alloc((size_t)Nn_pad1 * 2 * p.Fp);
+        X.alloc((size_t)Nn_pad1 * X_LIMBS_MAX * p.Fp);
         R.alloc((size_t)nR * Nn_pad2 * h.Kp);
         inv_dr.alloc(Nn_pad1); delta.alloc(Nn_pad1);
         fsum.alloc(Nn_pad1);
@@ -1294,12 +1279,10 @@ struct BackendTC : EvalBackend {
         // rows of R that belong to padding nodes are never written by GEMM-1 tiles beyond Nn_pad1: clear once
         GML_CUDA(cudaMemsetAsync(R.p, 0, (size_t)nR * Nn_pad2 * h.Kp, st));
         tmA = make_map_2d(P, p.Fp, h.Kp, 128, 128, CU_TENSOR_MAP_SWIZZLE_128B);
-        tmB = make_map_2d(X4.p, p.Fp, (uint64_t)Nn_pad1 * 4, 128, 4 * NODE_TILE1, CU_TENSOR_MAP_SWIZZLE_128B);
-        tmB3 = make_map_2d(X3.p, p.Fp, (uint64_t)Nn_pad1 * 3, 128, 3 * NODE_TILE1, CU_TENSOR_MAP_SWIZZLE_128B);
-        tmBh = make_map_2d(X4.p, p.Fp, (uint64_t)Nn_pad1 * 4, 128, 4 * 32, CU_TENSOR_MAP_SWIZZLE_128B);
-        tmB3h = make_map_2d(X3.p, p.Fp, (uint64_t)Nn_pad1 * 3, 128, 3 * 32, CU_TENSOR_MAP_SWIZZLE_128B);
-        tmB2 = make_map_2d(X2.p, p.Fp, (uint64_t)Nn_pad1 * 2, 128, 2 * NODE_TILE1, CU_TENSOR_MAP_SWIZZLE_128B);
-        tmB2h = make_map_2d(X2.p, p.Fp, (uint64_t)Nn_pad1 * 2, 128, 2 * 32, CU_TENSOR_MAP_SWIZZLE_128B);
+        for (int xl = 2; xl <= X_LIMBS_MAX; ++xl) {
+            tmB[xl - 2] = make_map_2d(X.p, p.Fp, (uint64_t)Nn_pad1 * xl, 128, xl * NODE_TILE1, CU_TENSOR_MAP_SWIZZLE_128B);
+            tmBh[xl - 2] = make_map_2d(X.p, p.Fp, (uint64_t)Nn_pad1 * xl, 128, xl * 32, CU_TENSOR_MAP_SWIZZLE_128B);
+        }
         pair_ok = p.Fp <= E2_MAX_FP && !std::getenv("GML_B200_NO_PAIR");
         // Sample-blocked layouts: every TMA box is one contiguous 8/16 KB chunk (one 2 MB page) instead of
         // 64/128 rows that are Kp bytes apart.
@@ -1329,35 +1312,16 @@ struct BackendTC : EvalBackend {
         configure();
     }
 
-    template <class K> static void set_smem(K kernel, int bytes) {
-        GML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    template <class K> static void set_smem(Launch<K> k) {
+        GML_CUDA(cudaFuncSetAttribute(k.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem));
     }
     void configure() {
-#define GML_TC_SET(FORM, XL)                                               \
-        set_smem(tc_energy_kernel<FORM, false, XL, 2>, E_SMEM);                \
-        set_smem(tc_energy_kernel<FORM, true, XL, 2>, E_SMEM);                 \
-        set_smem(tc_energy_kernel<FORM, true, XL, 3>, E_SMEM);                 \
-        set_smem(tc_energy_kernel<FORM, true, XL, 4>, E_SMEM);                 \
-        set_smem(tc_energy_pair_kernel<FORM, false, XL, 2>, e2_smem(XL));           \
-        set_smem(tc_energy_pair_kernel<FORM, true, XL, 2>, e2_smem(XL));            \
-        set_smem(tc_energy_pair_kernel<FORM, true, XL, 3>, e2_smem(XL));            \
-        set_smem(tc_energy_pair_kernel<FORM, true, XL, 4>, e2_smem(XL))
-        GML_TC_SET(GML_B200_RISE, 3); GML_TC_SET(GML_B200_RISE, 4);
-        GML_TC_SET(GML_B200_RPLE, 3); GML_TC_SET(GML_B200_RPLE, 4);
-#undef GML_TC_SET
-        // rough level: 2 iterate limbs, 1 residual digit plane
-        set_smem(tc_energy_kernel<GML_B200_RISE, false, 2, 1>, E_SMEM); set_smem(tc_energy_kernel<GML_B200_RISE, true, 2, 1>, E_SMEM);
-        set_smem(tc_energy_kernel<GML_B200_RPLE, false, 2, 1>, E_SMEM); set_smem(tc_energy_kernel<GML_B200_RPLE, true, 2, 1>, E_SMEM);
-        set_smem(tc_energy_pair_kernel<GML_B200_RISE, false, 2, 1>, e2_smem(2)); set_smem(tc_energy_pair_kernel<GML_B200_RISE, true, 2, 1>, e2_smem(2));
-        set_smem(tc_energy_pair_kernel<GML_B200_RPLE, false, 2, 1>, e2_smem(2)); set_smem(tc_energy_pair_kernel<GML_B200_RPLE, true, 2, 1>, e2_smem(2));
-        set_smem(tc_grad_kernel<1, 256>, grad_smem(1, 256));
-        set_smem(tc_grad_kernel<1, 128>, grad_smem(1, 128));
-        set_smem(tc_grad_kernel<2, 128>, grad_smem(2, 128));
-        set_smem(tc_grad_kernel<2, 256>, grad_smem(2, 256));
-        set_smem(tc_grad_kernel<3, 128>, grad_smem(3, 128));
-        set_smem(tc_grad_kernel<4, 128>, grad_smem(4, 128));
+        for (const EnergyInstance& k : ENERGY_KERNELS) {
+            set_smem(energy_kernel(k.form, k.grad, k.xl, k.nr, false));
+            set_smem(energy_kernel(k.form, k.grad, k.xl, k.nr, true));
+        }
+        for (const GradInstance& k : GRAD_KERNELS) set_smem(grad_kernel(k.nr, k.ft));
     }
-    static int grad_smem(int nr, int ft) { return g_stages(nr, ft) * g_stage_bytes(nr, ft) + 1024 + 128; }
     // Number of sample ranges for `tiles` output tiles on n_sms persistent CTAs: the smallest count from one
     // wave upwards whose items fill the last wave to >= 96 % (items are dealt round-robin, range-major).
     static int balanced_splits(int tiles, int n_sms, int64_t max_splits) {
@@ -1378,8 +1342,8 @@ struct BackendTC : EvalBackend {
     // HBM about twice (ncu: 20.1 GB read for a 10.2 GB histogram).  Ranges of at most ITEM_STEPS pair-steps bound the
     // drift; the limb-tile reload per item (96 KB against 256 KB of histogram tiles per step) stays below 0.2 %.
     static int pair_groups(int tiles, int n_pairs, int64_t pair_blocks) {
-        static const int item_steps = [] { const char* e = std::getenv("GML_B200_ITEM_STEPS"); return e ? std::max(1, std::atoi(e)) : 256; }();
-        const int64_t g_min = std::max<int64_t>(1, ceil_div(pair_blocks, item_steps));
+        constexpr int ITEM_STEPS = 256;
+        const int64_t g_min = std::max<int64_t>(1, ceil_div(pair_blocks, ITEM_STEPS));
         const int wave = balanced_splits(tiles, n_pairs, pair_blocks);
         if (g_min <= wave) return wave;
         int64_t best = g_min; double best_eff = 0.0;
@@ -1467,13 +1431,13 @@ struct BackendTC : EvalBackend {
         const int nr = level_nr();                                  // residual digit planes of this pass
         const int n_nodes = act_idx ? n_act : p.Nn;                // slots of this pass
         const int pad1 = (int)round_up(n_nodes, NODE_TILE1), pad2 = (int)round_up(n_nodes, NODE_TILE2);
-        tc_quantize_x_kernel<<<pad1, 128, 0, st>>>(x, n_nodes, p.Fp, p.form, h.wmax, nr, xl, NODE_TILE1, 1.0 / lattice(), xl == 2 ? X2.p : (xl == 3 ? X3.p : X4.p),
+        tc_quantize_x_kernel<<<pad1, 128, 0, st>>>(x, n_nodes, p.Fp, p.form, h.wmax, nr, xl, NODE_TILE1, 1.0 / lattice(), X.p,
                                                    inv_dr.p, delta.p, flags.p, act_idx);
         GML_LAUNCHED();
         GML_CUDA(cudaMemsetAsync(fsum.p, 0, sizeof(double) * pad1, st));
         EnergyParams ep{};
-        ep.Kp = h.Kp; ep.Fp = p.Fp; ep.Fspin = Fspin; ep.Nn = n_nodes; ep.n_tiles = pad1 / NODE_TILE1;
-        ep.block_stride = stride; ep.sample_blocks = ceil_div(h.Kp / 128, stride); ep.r_rows_per_limb = Nn_pad2; ep.nR = nr; ep.form = p.form; ep.lattice = (float)lattice();
+        ep.Fp = p.Fp; ep.Fspin = Fspin; ep.n_tiles = pad1 / NODE_TILE1;
+        ep.block_stride = stride; ep.sample_blocks = ceil_div(h.Kp / 128, stride); ep.r_rows_per_limb = Nn_pad2; ep.lattice = (float)lattice();
         ep.w32 = h.w32.p; ep.inv_dr = inv_dr.p; ep.fsum = fsum.p; ep.R = reinterpret_cast<uint8_t*>(R.p); ep.r_scratch = r_scratch.p;
         ep.node_begin_row = act_idx ? 0 : first_row; ep.spin_vec = (act_idx || spin_vec) ? 1 : 0;
         const CUtensorMap& tmSvUse = act_idx ? tmSvAct : tmSv;
@@ -1490,28 +1454,9 @@ struct BackendTC : EvalBackend {
             const int m = used / T;                   // whole ranges per wave (0: more tiles than pairs -> round robin)
             ep.g_main = m ? std::min(ep.n_groups, ep.n_waves * m) : 0;
         }
-        const bool rple = p.form == GML_B200_RPLE;
+        const Launch<EnergyKernel> ek = energy_kernel(p.form, want_grad, xl, nr, pair);
         span_begin(want_grad ? 0 : 2, st);
-#define GML_TC_ENERGY(FORM, GRAD, XL, NRL, MAPB, MAPBH)                                                                          \
-        do {                                                                                                                      \
-            if (pair) tc_energy_pair_kernel<FORM, GRAD, XL, NRL><<<grid1, E_THREADS, e2_smem(XL), st>>>(tmA, MAPBH, tmS, tmSvUse, ep); \
-            else tc_energy_kernel<FORM, GRAD, XL, NRL><<<grid1, E_THREADS, E_SMEM, st>>>(tmA, MAPB, tmS, tmSvUse, ep);             \
-        } while (0)
-#define GML_TC_BY_NR(FORM, XL, MAPB, MAPBH)                                                 \
-        do {                                                                                \
-            if (!want_grad) GML_TC_ENERGY(FORM, false, XL, 2, MAPB, MAPBH);                 \
-            else if (nr == 2) GML_TC_ENERGY(FORM, true, XL, 2, MAPB, MAPBH);                \
-            else if (nr == 3) GML_TC_ENERGY(FORM, true, XL, 3, MAPB, MAPBH);                \
-            else GML_TC_ENERGY(FORM, true, XL, 4, MAPB, MAPBH);                             \
-        } while (0)
-        if (xl == 4) { if (rple) GML_TC_BY_NR(GML_B200_RPLE, 4, tmB, tmBh); else GML_TC_BY_NR(GML_B200_RISE, 4, tmB, tmBh); }
-        else if (xl == 3) { if (rple) GML_TC_BY_NR(GML_B200_RPLE, 3, tmB3, tmB3h); else GML_TC_BY_NR(GML_B200_RISE, 3, tmB3, tmB3h); }
-        else {      // rough level: always one residual plane (objective-only passes have no residual at all)
-            if (rple) { if (want_grad) GML_TC_ENERGY(GML_B200_RPLE, true, 2, 1, tmB2, tmB2h); else GML_TC_ENERGY(GML_B200_RPLE, false, 2, 1, tmB2, tmB2h); }
-            else { if (want_grad) GML_TC_ENERGY(GML_B200_RISE, true, 2, 1, tmB2, tmB2h); else GML_TC_ENERGY(GML_B200_RISE, false, 2, 1, tmB2, tmB2h); }
-        }
-#undef GML_TC_BY_NR
-#undef GML_TC_ENERGY
+        ek.kernel<<<grid1, E_THREADS, ek.smem, st>>>(tmA, pair ? tmBh[xl - 2] : tmB[xl - 2], tmS, tmSvUse, ep);
         GML_LAUNCHED();
         span_end(st);
         if (want_grad) {
@@ -1528,20 +1473,16 @@ struct BackendTC : EvalBackend {
                 GML_LAUNCHED();
             }
             GradParams gp{};
-            const int ft = (nr <= 2 && p.Fp % 256 == 0 && !std::getenv("GML_B200_GRAD_FT128")) ? 256 : 128;   // feature-tile width
-            gp.Fp = p.Fp; gp.m_tiles = pad2 / 128; gp.f_tiles = p.Fp / ft; gp.nR = nr;
+            const int ft = (nr <= 2 && p.Fp % 256 == 0) ? 256 : 128;   // feature-tile width
+            gp.Fp = p.Fp; gp.m_tiles = pad2 / 128; gp.f_tiles = p.Fp / ft;
             gp.r_rows_per_limb = Nn_pad2; gp.block_stride = stride; gp.sample_blocks = ceil_div(h.Kp / 128, stride); gp.G = G64.p;
             gp.dbg = ep.dbg;
             const int tiles = gp.m_tiles * gp.f_tiles;
             gp.n_splits = balanced_splits(tiles, n_sms, gp.sample_blocks);
             const int grid2 = std::min(n_sms, tiles * gp.n_splits);
+            const Launch<GradKernel> gk = grad_kernel(nr, ft);
             span_begin(1, st);
-            if (nr == 1 && ft == 256) tc_grad_kernel<1, 256><<<grid2, 192, grad_smem(1, 256), st>>>(tmRa, tmQ256, gp);
-            else if (nr == 1) tc_grad_kernel<1, 128><<<grid2, 192, grad_smem(1, 128), st>>>(tmRa, tmQ, gp);
-            else if (nr == 2 && ft == 256) tc_grad_kernel<2, 256><<<grid2, 192, grad_smem(2, 256), st>>>(tmRa, tmQ256, gp);
-            else if (nr == 2) tc_grad_kernel<2, 128><<<grid2, 192, grad_smem(2, 128), st>>>(tmRa, tmQ, gp);
-            else if (nr == 3) tc_grad_kernel<3, 128><<<grid2, 192, grad_smem(3, 128), st>>>(tmRa, tmQ, gp);
-            else tc_grad_kernel<4, 128><<<grid2, 192, grad_smem(4, 128), st>>>(tmRa, tmQ, gp);
+            gk.kernel<<<grid2, 192, gk.smem, st>>>(tmRa, ft == 256 ? tmQ256 : tmQ, gp);
             GML_LAUNCHED();
             span_end(st);
         }
