@@ -347,6 +347,89 @@ def sample_terms_device(terms: Dict[Tuple[int, ...], float], num_spins: int, n_s
     return out
 
 
+# ---- samplers (src/sampling.jl:1-3, 90-106) ---------------------------------------------------
+class GMLSampler:
+    pass
+
+
+@dataclass
+class Gibbs(GMLSampler):
+    """The reference's CPU sampler (enumeration of all 2^N configurations on one thread); not available here."""
+
+
+@dataclass
+class B200Exact(GMLSampler):
+    """Exact iid sampler on the device (csrc/exact_sampler.cu): the reference's distribution, drawn by enumerating all
+    2^N configurations in blocks, for N <= 40.  The draws depend only on (model, number_sample, replicates, seed)."""
+    seed: int = 0
+    device: int = 0
+
+
+def _exact_call(gm: FactorGraph, number_sample: int, replicates: int, sampler):
+    """Validates the arguments of sample / sample_device and runs gml_b200_sample_exact_device into device buffers sized
+    for the largest possible result (min(n, 2^N) rows per replicate).  Returns (counts, spins, K, log_z)."""
+    import torch
+    sampler = B200Exact() if sampler is None else sampler
+    if isinstance(sampler, Gibbs):
+        raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact() as the sampler")
+    if not isinstance(sampler, B200Exact):
+        raise TypeError("sampler must be a GMLSampler")
+    if gm.alphabet != "spin":                                                    # src/sampling.jl:95-97
+        raise ValueError(f"sampling of a FactorGraph is only supported for the spin alphabet, not {gm.alphabet!r}")
+    N, n, reps = int(gm.varible_count), int(number_sample), int(replicates)
+    if not 1 <= N <= _lib.EXACT_MAX_N:
+        raise ValueError(f"the exact sampler supports 1 <= N <= {_lib.EXACT_MAX_N} spins, got {N}")
+    if n < 1 or reps < 1:
+        raise ValueError("number_sample and replicates must be >= 1")
+    order = max((len(k) for k in gm.terms), default=1)
+    idx = -np.ones((max(len(gm.terms), 1), order), dtype=np.int32)
+    wts = np.zeros(max(len(gm.terms), 1), dtype=np.float64)
+    for t, (k, v) in enumerate(gm.terms.items()):
+        if min(k, default=1) < 1:
+            raise ValueError(f"FactorGraph keys are 1-based spin labels, got {k}")
+        idx[t, :len(k)] = np.asarray(k, dtype=np.int64) - 1                     # the library refuses labels > N
+        wts[t] = v
+    ld = reps * min(n, 1 << N)
+    dev = f"cuda:{int(sampler.device)}"
+    counts = torch.empty(ld, dtype=torch.float64, device=dev)
+    spins = torch.empty((N, ld), dtype=torch.int8, device=dev)
+    K = np.zeros(reps, dtype=np.int64)
+    log_z = ctypes.c_double(0.0)
+    _lib.check(_lib.load().gml_b200_sample_exact_device(int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts), n,
+                                                        reps, int(sampler.seed) & (2 ** 64 - 1), _ptr(K), ctypes.byref(log_z),
+                                                        ctypes.c_void_p(counts.data_ptr()), ctypes.c_void_p(spins.data_ptr()),
+                                                        ld, None))
+    return counts, spins, K, log_z.value
+
+
+def sample_device(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Optional[GMLSampler] = None,
+                  return_log_z: bool = False):
+    """Device-resident form of `sample`: the packed histogram (counts float64[K], spins int8 [N x K] spin-major, a view with
+    leading dimension spins.stride(0)) as torch tensors on the sampler's device, rows in increasing configuration index.
+    Session.attach_device(counts.data_ptr(), spins.data_ptr(), K, N, spins.stride(0)) takes it without a host copy.
+    A list of (counts, spins) when replicates > 1; with return_log_z, also log Z (natural log of the partition function)."""
+    counts, spins, K, log_z = _exact_call(gm, number_sample, replicates, sampler)
+    ends = np.cumsum(K)
+    hists = [(counts[e - k:e], spins[:, e - k:e]) for k, e in zip(K.tolist(), ends.tolist())]
+    out = hists[0] if replicates == 1 else hists
+    return (out, log_z) if return_log_z else out
+
+
+def sample(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Optional[GMLSampler] = None,
+           return_log_z: bool = False):
+    """sample(gm, number_sample[, replicates[, sampler]]) -- src/sampling.jl:90-106.  Returns the reference's int64
+    K x (N+1) matrix [count, s_1..s_N] (rows in increasing configuration index, spin_i = 2*bit_i - 1), or a list of them
+    when replicates > 1; learn() takes it as it is.  The default sampler is B200Exact(seed=0, device=0)."""
+    counts, spins, K, log_z = _exact_call(gm, number_sample, replicates, sampler)
+    rows = int(K.sum())
+    c = counts[:rows].cpu().numpy().astype(np.int64)
+    s = spins[:, :rows].cpu().numpy().astype(np.int64)
+    ends = np.cumsum(K)
+    hists = [np.concatenate([c[e - k:e, None], s[:, e - k:e].T], axis=1) for k, e in zip(K.tolist(), ends.tolist())]
+    out = hists[0] if replicates == 1 else hists
+    return (out, log_z) if return_log_z else out
+
+
 class Session:
     """Handle API (include/gml_b200.h): keeps the histogram resident in HBM across calls."""
 

@@ -1170,6 +1170,54 @@ int gml_b200_sample_gibbs_terms_device(int32_t device, int32_t N, int32_t order,
     });
 }
 
+int gml_b200_sample_exact_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                 const double* term_weight, int64_t n_samples, int32_t replicates, uint64_t seed,
+                                 int64_t* out_K, double* out_log_z, double* d_counts, int8_t* d_spins, int64_t ld,
+                                 void* stream) {
+    return guarded([&] {
+        GML_REQUIRE(N >= 1 && N <= GML_B200_EXACT_MAX_N, "exact sampler needs 1 <= N <= " + std::to_string(GML_B200_EXACT_MAX_N));
+        GML_REQUIRE(order >= 1 && order <= GML_B200_EXACT_MAX_N && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)) && out_K,
+                    "bad sampler argument");
+        GML_REQUIRE(n_samples >= 1 && replicates >= 1 && n_samples <= (INT64_C(1) << 62) / replicates, "bad sampler sizes");
+        GML_REQUIRE(!d_counts || (d_spins && ld >= 1), "d_counts needs d_spins and ld >= 1");
+        std::vector<uint64_t> masks(n_terms, 0);
+        std::vector<double> weights(term_weight, term_weight + n_terms);
+        double abs_sum = 0.0;
+        for (int t = 0; t < n_terms; ++t) {
+            for (int m = 0; m < order; ++m) {
+                const int i = term_idx[(size_t)t * order + m];
+                if (i == -1) continue;
+                GML_REQUIRE(i >= 0 && i < N, "sampler term refers to a spin outside [0, N)");
+                GML_REQUIRE(!((masks[t] >> i) & 1ull), "sampler term repeats a spin");
+                masks[t] |= 1ull << i;
+            }
+            GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
+            abs_sum += std::fabs(weights[t]);
+        }
+        GML_REQUIRE(std::isfinite(abs_sum), "sum of |term weights| is not finite");
+        GML_CUDA(cudaSetDevice(device));
+        cudaStream_t st = (cudaStream_t)stream;
+        // host buffers: the rows are emitted into device staging buffers and copied back
+        cudaPointerAttributes attr{};
+        const bool on_host = d_counts && (cudaPointerGetAttributes(&attr, d_counts) != cudaSuccess ||
+                                          (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged));
+        cudaGetLastError();   // an unregistered host pointer may leave an error behind
+        DevBuf<double> stage_c;
+        DevBuf<int8_t> stage_s;
+        if (on_host) { stage_c.alloc(ld); stage_s.alloc((size_t)N * ld); }
+        const double log_z = sample_exact(N, masks, weights, n_samples, replicates, seed, out_K, on_host ? stage_c.p : d_counts,
+                                          on_host ? stage_s.p : d_spins, ld, st);
+        if (on_host) {
+            int64_t rows = 0;
+            for (int r = 0; r < replicates; ++r) rows += out_K[r];
+            GML_CUDA(cudaMemcpyAsync(d_counts, stage_c.p, sizeof(double) * rows, cudaMemcpyDeviceToHost, st));
+            GML_CUDA(cudaMemcpy2DAsync(d_spins, ld, stage_s.p, ld, rows, N, cudaMemcpyDeviceToHost, st));
+            GML_CUDA(cudaStreamSynchronize(st));
+        }
+        if (out_log_z) *out_log_z = log_z;
+    });
+}
+
 int gml_b200_build_histogram_device(int32_t device, const int8_t* d_samples, int64_t M, int32_t N, int64_t ld,
                                     int8_t* d_out_spins, int64_t ld_out, double* d_out_counts, int64_t* out_K,
                                     void* stream) {

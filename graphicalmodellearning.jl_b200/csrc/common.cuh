@@ -225,4 +225,10 @@ void sample_gibbs(int N, const int32_t* d_row_ptr, const int32_t* d_col, const f
 void sample_gibbs_terms(int N, int width, const int32_t* d_row_ptr, const int32_t* d_others, const float* d_weight,
                         int64_t n_samples, int sweeps, uint64_t seed, int8_t* d_spins, int64_t ld, cudaStream_t st);
 
+// --- exact_sampler.cu : iid draws from the exact distribution by enumeration (term t = spins of masks[t]); fills
+// out_K[replicates] and, when d_counts is set, the histograms at consecutive rows; returns log Z.  N <= GML_B200_EXACT_MAX_N.
+double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights, int64_t n_samples,
+                    int replicates, uint64_t seed, int64_t* out_K, double* d_counts, int8_t* d_spins, int64_t ld,
+                    cudaStream_t st);
+
 }  // namespace gml

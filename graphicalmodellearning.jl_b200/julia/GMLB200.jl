@@ -156,3 +156,56 @@ function learn(samples::Array{T,2}, formulation::multiRISE, method::B200) where 
 
     return FactorGraph(inter_order, num_spins, :spin, reconstruction)                       # :151
 end
+
+"""
+    B200Exact(; seed=0, device=0)
+
+Exact iid sampler on the GPU: the distribution of the reference's `sample` (src/sampling.jl:58-106), drawn by enumerating
+all 2^N configurations in blocks on the device, for N <= 40.  The draws depend only on (model, number_sample, replicates,
+seed); rows come out in increasing configuration index.
+"""
+struct B200Exact <: GMLSampler
+    seed::UInt64
+    device::Int
+end
+B200Exact(; seed=0, device=0) = B200Exact(UInt64(seed), device)
+
+function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer, sampler::B200Exact) where T <: Real
+    if gm.alphabet != :spin                                                                 # src/sampling.jl:95-97
+        error("sampling is only supported for spin alphabets, not $(gm.alphabet)")
+    end
+    num_spins = gm.varible_count
+    order = maximum(length(k) for k in keys(gm.terms); init=1)
+    n_terms = length(gm.terms)
+    term_idx = fill(Int32(-1), order, max(n_terms, 1))     # column t = term t: the C side's n_terms x order row-major array
+    term_weight = zeros(Float64, max(n_terms, 1))
+    for (t, (key, weight)) in enumerate(gm.terms)
+        for (m, i) in enumerate(key)
+            term_idx[m, t] = Int32(i - 1)
+        end
+        term_weight[t] = Float64(weight)
+    end
+    rows = replicates * min(number_sample, 2^min(num_spins, 62))
+    out_K = zeros(Int64, replicates)
+    # host buffers of the largest possible size (min(n, 2^N) rows per replicate); the library stages them on the device
+    counts = Array{Float64}(undef, rows)
+    spins = Array{Int8}(undef, rows, num_spins)              # column-major: spins[:, i] == the C side's row i (ld = rows)
+    GC.@preserve term_idx term_weight out_K counts spins begin
+        rc = ccall((:gml_b200_sample_exact_device, _libgml_b200), Cint,
+                   (Int32, Int32, Int32, Int32, Ptr{Int32}, Ptr{Cdouble}, Int64, Int32, UInt64, Ptr{Int64}, Ptr{Cdouble},
+                    Ptr{Cdouble}, Ptr{Int8}, Int64, Ptr{Cvoid}),
+                   sampler.device, num_spins, order, n_terms, term_idx, term_weight, number_sample, replicates, sampler.seed,
+                   out_K, C_NULL, counts, spins, rows, C_NULL)
+    end
+    _gml_b200_check(rc)
+    out = Vector{Array{Int64,2}}(undef, replicates)
+    first = 1
+    for r in 1:replicates
+        last = first + out_K[r] - 1
+        out[r] = hcat(Int64.(counts[first:last]), Int64.(spins[first:last, :]))   # [count, s_1..s_N], src/sampling.jl:53-54
+        first = last + 1
+    end
+    return out
+end
+
+sample(gm::FactorGraph, number_sample::Integer, sampler::B200Exact) = sample(gm, number_sample, 1, sampler)[1]

@@ -233,6 +233,27 @@ int gml_b200_sample_gibbs_terms_device(int32_t device, int32_t N, int32_t order,
                                        const float* term_weight, int64_t n_samples, int32_t sweeps, uint64_t seed,
                                        int8_t* d_spins, int64_t ld, void* stream);
 
+/* Exact iid sampler: the reference's `sample(gm, number_sample, replicates)` (src/sampling.jl:58-106) on the device, for the
+ * same term lists as gml_b200_sample_gibbs_terms_device but with fp64 weights.  p(s) ~ exp(sum_t w_t prod_{i in t} s_i),
+ * drawn exactly by enumerating all 2^N configurations (never stored: they are recomputed in blocks of 2^12).
+ * Configuration c has spin_i = 2*bit_i(c) - 1 (bit 0 = spin 1, src/sampling.jl:11-14).  Replicate r is the histogram of
+ * draws [r*n_samples, (r+1)*n_samples) of one counter-based stream; its rows are the configurations drawn at least once,
+ * in increasing c.  The output depends only on (terms, n_samples, replicates, seed).
+ *   - out_K[replicates] receives the rows of every replicate, *out_log_z (nullable) the natural log of the partition
+ *     function.  With d_counts == NULL nothing else is written; with buffers (the histogram layout above, ld >= sum of
+ *     out_K, e.g. replicates * min(n_samples, 2^N)), replicate r's rows follow those of replicate r-1.  The buffers are
+ *     device memory of `device` (written in place) or host memory (staged on the device and copied back).
+ *     A count-only call costs as much as a full one: callers that can afford the bound should pass buffers at once.
+ *   - N <= 40 (GML_B200_EXACT_MAX_N).  Cost ~ 2^N * n_terms fp64 sign+add (plus the same again for the blocks that
+ *     receive draws); device memory ~ 40 * 2^(N-12) bytes + 10 bytes per draw.
+ *   - GML_B200_EINVAL: N outside [1, 40], an index outside [-1, N) or repeated in a term, a non-finite weight (or sum of
+ *     |weights|), n_samples < 1, replicates < 1, or ld smaller than the rows (out_K is then filled). */
+#define GML_B200_EXACT_MAX_N 40
+int gml_b200_sample_exact_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                 const double* term_weight, int64_t n_samples, int32_t replicates, uint64_t seed,
+                                 int64_t* out_K /* [replicates] */, double* out_log_z /* nullable */,
+                                 double* d_counts, int8_t* d_spins, int64_t ld, void* stream);
+
 /* ---- sample-sharded mode (SURVEY 8e): histogram rows split over ranks, every rank solves all nodes; per pass
  * the int64 gradient sums and fp64 objective sums are combined with NCCL all-reduces on the solve stream.
  *   rank 0: gml_b200_comm_unique_id(id) -> broadcast the 128 bytes with any transport -> every rank:
