@@ -365,22 +365,24 @@ class B200Exact(GMLSampler):
     device: int = 0
 
 
-def _exact_call(gm: FactorGraph, number_sample: int, replicates: int, sampler):
-    """Validates the arguments of sample / sample_device and runs gml_b200_sample_exact_device into device buffers sized
-    for the largest possible result (min(n, 2^N) rows per replicate).  Returns (counts, spins, K, log_z)."""
-    import torch
-    sampler = B200Exact() if sampler is None else sampler
-    if isinstance(sampler, Gibbs):
-        raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact() as the sampler")
-    if not isinstance(sampler, B200Exact):
-        raise TypeError("sampler must be a GMLSampler")
-    if gm.alphabet != "spin":                                                    # src/sampling.jl:95-97
-        raise ValueError(f"sampling of a FactorGraph is only supported for the spin alphabet, not {gm.alphabet!r}")
-    N, n, reps = int(gm.varible_count), int(number_sample), int(replicates)
-    if not 1 <= N <= _lib.EXACT_MAX_N:
-        raise ValueError(f"the exact sampler supports 1 <= N <= {_lib.EXACT_MAX_N} spins, got {N}")
-    if n < 1 or reps < 1:
-        raise ValueError("number_sample and replicates must be >= 1")
+@dataclass
+class B200Gibbs(GMLSampler):
+    """Multi-sample Gibbs sampler on the device (csrc/mcmc_sampler.cu) for N <= 4096 spins and terms of order <= 8.  Each
+    of `chains` chains (0 = min(round_up(number_sample, 32), 2^17)) runs `burn_in` systematic-scan sweeps from a random
+    start, then records its configuration after every `thin`-th sweep.  The draws depend only on (model, number_sample,
+    replicates, seed, chains, burn_in, thin).  The draws are correlated and only as good as the chains' mixing:
+    last_rhat holds, per replicate of the last call, the split-R-hat (energy, magnetisation) over the chains' halves."""
+    seed: int = 0
+    device: int = 0
+    chains: int = 0
+    burn_in: int = 200
+    thin: int = 10
+    last_rhat: list = field(default_factory=list, repr=False, compare=False)
+
+
+def _term_arrays(gm: FactorGraph):
+    """The term lists of the sampler entry points: (order, term_idx int32 [n_terms x order] 0-based, -1 padded,
+    term_weight float64 [n_terms])."""
     order = max((len(k) for k in gm.terms), default=1)
     idx = -np.ones((max(len(gm.terms), 1), order), dtype=np.int32)
     wts = np.zeros(max(len(gm.terms), 1), dtype=np.float64)
@@ -389,26 +391,65 @@ def _exact_call(gm: FactorGraph, number_sample: int, replicates: int, sampler):
             raise ValueError(f"FactorGraph keys are 1-based spin labels, got {k}")
         idx[t, :len(k)] = np.asarray(k, dtype=np.int64) - 1                     # the library refuses labels > N
         wts[t] = v
+    return order, idx, wts
+
+
+def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, return_log_z: bool):
+    """Validates the arguments of sample / sample_device and runs the sampler's C entry point into device buffers sized
+    for the largest possible result (min(n, 2^N) rows per replicate).  Returns (counts, spins, K, log_z); log_z is None
+    for B200Gibbs, which also records its R-hat in sampler.last_rhat."""
+    import torch
+    sampler = B200Exact() if sampler is None else sampler
+    if isinstance(sampler, Gibbs):
+        raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact() "
+                                  "(N <= 40) or B200Gibbs() (MCMC) as the sampler")
+    if not isinstance(sampler, (B200Exact, B200Gibbs)):
+        raise TypeError("sampler must be a GMLSampler")
+    mcmc = isinstance(sampler, B200Gibbs)
+    if mcmc:
+        sampler.last_rhat = []
+        if return_log_z:
+            raise ValueError("B200Gibbs is an MCMC sampler and has no partition function: return_log_z needs B200Exact")
+    if gm.alphabet != "spin":                                                    # src/sampling.jl:95-97
+        raise ValueError(f"sampling of a FactorGraph is only supported for the spin alphabet, not {gm.alphabet!r}")
+    N, n, reps = int(gm.varible_count), int(number_sample), int(replicates)
+    cap = _lib.MCMC_MAX_N if mcmc else _lib.EXACT_MAX_N
+    if not 1 <= N <= cap:
+        raise ValueError(f"the {type(sampler).__name__} sampler supports 1 <= N <= {cap} spins, got {N}")
+    if n < 1 or reps < 1:
+        raise ValueError("number_sample and replicates must be >= 1")
+    if mcmc:
+        if sampler.chains < 0 or sampler.burn_in < 0 or sampler.thin < 1:
+            raise ValueError("B200Gibbs needs chains >= 0, burn_in >= 0 and thin >= 1")
+        if N <= 64 and n >= 2 ** 31:
+            raise ValueError("B200Gibbs builds the histogram of N <= 64 spins from fewer than 2^31 draws per replicate")
+    order, idx, wts = _term_arrays(gm)
     ld = reps * min(n, 1 << N)
     dev = f"cuda:{int(sampler.device)}"
     counts = torch.empty(ld, dtype=torch.float64, device=dev)
     spins = torch.empty((N, ld), dtype=torch.int8, device=dev)
     K = np.zeros(reps, dtype=np.int64)
-    log_z = ctypes.c_double(0.0)
-    _lib.check(_lib.load().gml_b200_sample_exact_device(int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts), n,
-                                                        reps, int(sampler.seed) & (2 ** 64 - 1), _ptr(K), ctypes.byref(log_z),
-                                                        ctypes.c_void_p(counts.data_ptr()), ctypes.c_void_p(spins.data_ptr()),
-                                                        ld, None))
-    return counts, spins, K, log_z.value
+    lib = _lib.load()
+    head = (int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts), n, reps)
+    tail = (ctypes.c_void_p(counts.data_ptr()), ctypes.c_void_p(spins.data_ptr()), ld, None)
+    if not mcmc:
+        log_z = ctypes.c_double(0.0)
+        _lib.check(lib.gml_b200_sample_exact_device(*head, int(sampler.seed) & (2 ** 64 - 1), _ptr(K), ctypes.byref(log_z), *tail))
+        return counts, spins, K, log_z.value
+    rhat = np.zeros((reps, 2))
+    _lib.check(lib.gml_b200_sample_mcmc_device(*head, int(sampler.chains), int(sampler.burn_in), int(sampler.thin),
+                                               int(sampler.seed) & (2 ** 64 - 1), _ptr(K), _ptr(rhat), *tail))
+    sampler.last_rhat = [tuple(r) for r in rhat.tolist()]
+    return counts, spins, K, None
 
 
 def sample_device(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Optional[GMLSampler] = None,
                   return_log_z: bool = False):
     """Device-resident form of `sample`: the packed histogram (counts float64[K], spins int8 [N x K] spin-major, a view with
-    leading dimension spins.stride(0)) as torch tensors on the sampler's device, rows in increasing configuration index.
-    Session.attach_device(counts.data_ptr(), spins.data_ptr(), K, N, spins.stride(0)) takes it without a host copy.
-    A list of (counts, spins) when replicates > 1; with return_log_z, also log Z (natural log of the partition function)."""
-    counts, spins, K, log_z = _exact_call(gm, number_sample, replicates, sampler)
+    leading dimension spins.stride(0)) as torch tensors on the sampler's device.  Session.attach_device(counts.data_ptr(),
+    spins.data_ptr(), K, N, spins.stride(0)) takes it without a host copy.  A list of (counts, spins) when replicates > 1;
+    with return_log_z (B200Exact only), also log Z (natural log of the partition function)."""
+    counts, spins, K, log_z = _sample_call(gm, number_sample, replicates, sampler, return_log_z)
     ends = np.cumsum(K)
     hists = [(counts[e - k:e], spins[:, e - k:e]) for k, e in zip(K.tolist(), ends.tolist())]
     out = hists[0] if replicates == 1 else hists
@@ -418,9 +459,10 @@ def sample_device(gm: FactorGraph, number_sample: int, replicates: int = 1, samp
 def sample(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Optional[GMLSampler] = None,
            return_log_z: bool = False):
     """sample(gm, number_sample[, replicates[, sampler]]) -- src/sampling.jl:90-106.  Returns the reference's int64
-    K x (N+1) matrix [count, s_1..s_N] (rows in increasing configuration index, spin_i = 2*bit_i - 1), or a list of them
-    when replicates > 1; learn() takes it as it is.  The default sampler is B200Exact(seed=0, device=0)."""
-    counts, spins, K, log_z = _exact_call(gm, number_sample, replicates, sampler)
+    K x (N+1) matrix [count, s_1..s_N] (spin_i = 2*bit_i - 1), or a list of them when replicates > 1; learn() takes it as it
+    is.  Rows are in increasing configuration index, except for B200Gibbs beyond 64 spins, whose rows are the draws in
+    order with count 1.  The default sampler is B200Exact(seed=0, device=0)."""
+    counts, spins, K, log_z = _sample_call(gm, number_sample, replicates, sampler, return_log_z)
     rows = int(K.sum())
     c = counts[:rows].cpu().numpy().astype(np.int64)
     s = spins[:, :rows].cpu().numpy().astype(np.int64)

@@ -226,6 +226,27 @@ void finish_stats(gml_b200_stats* stats, const SolveResult& r, int solver_used, 
     for (int i = 0; i < 4; ++i) stats->reserved_d[i] = r.profile[i];
 }
 
+// Runs fill(counts, spins) on the output buffers of a sampler entry point: device buffers as they are; host buffers through
+// device staging buffers, of which the first sum(out_K) rows are copied back; null buffers (a count-only call) as null.
+template <class Fill> void into_sample_buffers(double* d_counts, int8_t* d_spins, int64_t ld, int N, int replicates,
+                                               const int64_t* out_K, cudaStream_t st, Fill&& fill) {
+    cudaPointerAttributes attr{};
+    const bool on_host = d_counts && (cudaPointerGetAttributes(&attr, d_counts) != cudaSuccess ||
+                                      (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged));
+    cudaGetLastError();   // an unregistered host pointer may leave an error behind
+    DevBuf<double> stage_c;
+    DevBuf<int8_t> stage_s;
+    if (on_host) { stage_c.alloc(ld); stage_s.alloc((size_t)N * ld); }
+    fill(on_host ? stage_c.p : d_counts, on_host ? stage_s.p : d_spins);
+    if (on_host) {
+        int64_t rows = 0;
+        for (int r = 0; r < replicates; ++r) rows += out_K[r];
+        GML_CUDA(cudaMemcpyAsync(d_counts, stage_c.p, sizeof(double) * rows, cudaMemcpyDeviceToHost, st));
+        GML_CUDA(cudaMemcpy2DAsync(d_spins, ld, stage_s.p, ld, rows, N, cudaMemcpyDeviceToHost, st));
+        GML_CUDA(cudaStreamSynchronize(st));
+    }
+}
+
 void throw_if_unconverged(int n_unconverged) {
     if (n_unconverged == 0) return;
     set_error("solver did not reach tol within max_iter for " + std::to_string(n_unconverged) + " node(s)");
@@ -1132,40 +1153,17 @@ int gml_b200_sample_gibbs_terms_device(int32_t device, int32_t N, int32_t order,
         GML_REQUIRE(n_samples >= 1 && ld >= n_samples && sweeps >= 1, "bad sampler sizes");
         GML_CUDA(cudaSetDevice(device));
         cudaStream_t st = (cudaStream_t)stream;
-        // per-site incidence lists: (weight, the other members of the term)
-        const int width = std::max(1, order - 1);
-        std::vector<int32_t> row_ptr(N + 1, 0);
-        for (int t = 0; t < n_terms; ++t)
-            for (int m = 0; m < order; ++m) {
-                const int i = term_idx[(size_t)t * order + m];
-                if (i < 0) continue;
-                GML_REQUIRE(i < N, "sampler term refers to a spin >= N");
-                for (int m2 = 0; m2 < m; ++m2) GML_REQUIRE(term_idx[(size_t)t * order + m2] != i, "sampler term repeats a spin");
-                ++row_ptr[i + 1];
-            }
-        for (int i = 0; i < N; ++i) row_ptr[i + 1] += row_ptr[i];
-        const int nnz = row_ptr[N];
-        std::vector<int32_t> others((size_t)std::max(nnz, 1) * width, -1), fill(row_ptr.begin(), row_ptr.end() - 1);
-        std::vector<float> weight(std::max(nnz, 1), 0.f);
-        for (int t = 0; t < n_terms; ++t)
-            for (int m = 0; m < order; ++m) {
-                const int i = term_idx[(size_t)t * order + m];
-                if (i < 0) continue;
-                const int q = fill[i]++;
-                weight[q] = term_weight[t];
-                int w = 0;
-                for (int m2 = 0; m2 < order; ++m2) {
-                    const int j = term_idx[(size_t)t * order + m2];
-                    if (j >= 0 && m2 != m) others[(size_t)q * width + w++] = j;
-                }
-            }
+        const Incidence inc = build_incidence(N, order, n_terms, term_idx);
+        std::vector<float> weight(inc.term.size(), 0.f);
+        for (size_t q = 0; q < inc.term.size(); ++q)
+            if (inc.term[q] >= 0) weight[q] = term_weight[inc.term[q]];
         DevBuf<int32_t> rp, ot;
         DevBuf<float> ww;
-        rp.alloc(N + 1); ot.alloc(others.size()); ww.alloc(weight.size());
-        GML_CUDA(cudaMemcpyAsync(rp.p, row_ptr.data(), sizeof(int32_t) * (N + 1), cudaMemcpyHostToDevice, st));
-        GML_CUDA(cudaMemcpyAsync(ot.p, others.data(), sizeof(int32_t) * others.size(), cudaMemcpyHostToDevice, st));
+        rp.alloc(N + 1); ot.alloc(inc.others.size()); ww.alloc(weight.size());
+        GML_CUDA(cudaMemcpyAsync(rp.p, inc.row_ptr.data(), sizeof(int32_t) * (N + 1), cudaMemcpyHostToDevice, st));
+        GML_CUDA(cudaMemcpyAsync(ot.p, inc.others.data(), sizeof(int32_t) * inc.others.size(), cudaMemcpyHostToDevice, st));
         GML_CUDA(cudaMemcpyAsync(ww.p, weight.data(), sizeof(float) * weight.size(), cudaMemcpyHostToDevice, st));
-        sample_gibbs_terms(N, width, rp.p, ot.p, ww.p, n_samples, sweeps, seed, d_spins, ld, st);
+        sample_gibbs_terms(N, inc.width, rp.p, ot.p, ww.p, n_samples, sweeps, seed, d_spins, ld, st);
         GML_CUDA(cudaStreamSynchronize(st));
     });
 }
@@ -1197,24 +1195,47 @@ int gml_b200_sample_exact_device(int32_t device, int32_t N, int32_t order, int32
         GML_REQUIRE(std::isfinite(abs_sum), "sum of |term weights| is not finite");
         GML_CUDA(cudaSetDevice(device));
         cudaStream_t st = (cudaStream_t)stream;
-        // host buffers: the rows are emitted into device staging buffers and copied back
-        cudaPointerAttributes attr{};
-        const bool on_host = d_counts && (cudaPointerGetAttributes(&attr, d_counts) != cudaSuccess ||
-                                          (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged));
-        cudaGetLastError();   // an unregistered host pointer may leave an error behind
-        DevBuf<double> stage_c;
-        DevBuf<int8_t> stage_s;
-        if (on_host) { stage_c.alloc(ld); stage_s.alloc((size_t)N * ld); }
-        const double log_z = sample_exact(N, masks, weights, n_samples, replicates, seed, out_K, on_host ? stage_c.p : d_counts,
-                                          on_host ? stage_s.p : d_spins, ld, st);
-        if (on_host) {
-            int64_t rows = 0;
-            for (int r = 0; r < replicates; ++r) rows += out_K[r];
-            GML_CUDA(cudaMemcpyAsync(d_counts, stage_c.p, sizeof(double) * rows, cudaMemcpyDeviceToHost, st));
-            GML_CUDA(cudaMemcpy2DAsync(d_spins, ld, stage_s.p, ld, rows, N, cudaMemcpyDeviceToHost, st));
-            GML_CUDA(cudaStreamSynchronize(st));
-        }
+        double log_z = 0.0;
+        into_sample_buffers(d_counts, d_spins, ld, N, replicates, out_K, st, [&](double* c, int8_t* sp) {
+            log_z = sample_exact(N, masks, weights, n_samples, replicates, seed, out_K, c, sp, ld, st);
+        });
         if (out_log_z) *out_log_z = log_z;
+    });
+}
+
+int gml_b200_sample_mcmc_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                const double* term_weight, int64_t n_samples, int32_t replicates, int64_t chains, int32_t burn_in,
+                                int32_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* d_counts, int8_t* d_spins,
+                                int64_t ld, void* stream) {
+    return guarded([&] {
+        GML_REQUIRE(N >= 1 && N <= GML_B200_MCMC_MAX_N, "MCMC sampler needs 1 <= N <= " + std::to_string(GML_B200_MCMC_MAX_N));
+        GML_REQUIRE(order >= 1 && order <= 8 && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)) && out_K,
+                    "bad sampler argument");
+        GML_REQUIRE(n_samples >= 1 && replicates >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1,
+                    "bad sampler sizes");
+        GML_REQUIRE(N > 64 || n_samples < (INT64_C(1) << 31), "the histogram of N <= 64 spins takes fewer than 2^31 draws per replicate");
+        GML_REQUIRE(!d_counts || (d_spins && ld >= 1), "d_counts needs d_spins and ld >= 1");
+        if (chains == 0) chains = mcmc_auto_chains(n_samples);
+        const double steps = ((double)burn_in + (double)thin * (double)ceil_div(n_samples, chains)) * N;
+        GML_REQUIRE(steps * replicates < 0x1.0p62, "too many sweeps");
+        std::vector<int32_t> idx(term_idx, term_idx + (size_t)n_terms * order);
+        std::vector<double> weights(term_weight, term_weight + n_terms);
+        for (int t = 0; t < n_terms; ++t) {
+            for (int m = 0; m < order; ++m) GML_REQUIRE(idx[(size_t)t * order + m] >= -1, "sampler term refers to a spin outside [0, N)");
+            GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
+        }
+        const Incidence inc = build_incidence(N, order, n_terms, idx.data());
+        if (N > 64 && d_counts && ld < n_samples * replicates) {
+            for (int r = 0; r < replicates; ++r) out_K[r] = n_samples;
+            GML_REQUIRE(false, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(n_samples * replicates) +
+                               " rows of the replicates (out_K holds their sizes)");
+        }
+        GML_CUDA(cudaSetDevice(device));
+        cudaStream_t st = (cudaStream_t)stream;
+        into_sample_buffers(d_counts, d_spins, ld, N, replicates, out_K, st, [&](double* c, int8_t* sp) {
+            sample_mcmc(N, order, idx, weights, inc, n_samples, replicates, chains, burn_in, thin, seed, out_K, out_rhat, c, sp,
+                        ld, st);
+        });
     });
 }
 

@@ -204,6 +204,16 @@ EvalBackend* make_backend_tc(const NodeProblem& p, cudaStream_t st);
 // --- histogram.cu : raw samples -> deduplicated histogram (returns the number of distinct configurations)
 int64_t build_histogram(const int8_t* d_samples, int64_t M, int N, int64_t ld, int8_t* d_out_spins, int64_t ld_out,
                         double* d_out_counts, cudaStream_t st);
+// The tail of build_histogram, for callers that produce the 64-bit configuration keys (bit i = spin i+1 up) themselves:
+// sort_key_runs sorts M < 2^31 keys of N bits and run-length encodes them (runs.K distinct keys, increasing);
+// unpack_key_runs writes the runs as histogram rows [counts, spins] at rows [0, runs.K) of the output.
+struct KeyRuns {
+    DevBuf<unsigned long long> uniq;
+    DevBuf<int> run_len;
+    int64_t K = 0;
+};
+void sort_key_runs(const unsigned long long* d_keys, int64_t M, int N, KeyRuns& runs, cudaStream_t st);
+void unpack_key_runs(const KeyRuns& runs, int N, int8_t* d_out_spins, int64_t ld_out, double* d_out_counts, cudaStream_t st);
 
 // --- comm.cu : NCCL plumbing of the sample-sharded mode
 void comm_unique_id(uint8_t* out128);
@@ -224,6 +234,27 @@ void sample_gibbs(int N, const int32_t* d_row_ptr, const int32_t* d_col, const f
 
 void sample_gibbs_terms(int N, int width, const int32_t* d_row_ptr, const int32_t* d_others, const float* d_weight,
                         int64_t n_samples, int sweeps, uint64_t seed, int8_t* d_spins, int64_t ld, cudaStream_t st);
+
+// Per-site incidence lists (CSR) of a term list term_idx [n_terms x order] (0-based spin ids, negative = padding):
+// entry q in [row_ptr[i], row_ptr[i+1]) of site i is term term[q], with its width = max(1, order-1) other members in
+// others[q*width ..] (-1 padded).  Refuses an index >= N or a spin repeated in a term.  With no entries, one padding
+// entry (term -1) keeps the arrays non-empty.
+struct Incidence {
+    int width = 1;
+    std::vector<int32_t> row_ptr, others, term;
+};
+Incidence build_incidence(int N, int order, int n_terms, const int32_t* term_idx);
+
+// --- mcmc_sampler.cu : multi-sample Gibbs sampler (one warp = 32 chains, state in shared memory); fills out_K and
+// out_rhat (nullable, [replicates][2]: split-R-hat of the energy and of the magnetisation) and, when d_counts is set,
+// the replicates' rows at consecutive rows: N <= 64 deduplicated histograms, N > 64 one row per draw.
+// N <= GML_B200_MCMC_MAX_N; term weights are rounded once to fp32.
+constexpr int64_t MCMC_AUTO_CHAINS = 1 << 17;
+int64_t mcmc_auto_chains(int64_t n_samples);
+void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                 const Incidence& inc, int64_t n_samples, int replicates, int64_t chains, int64_t burn_in, int64_t thin,
+                 uint64_t seed, int64_t* out_K, double* out_rhat, double* d_counts, int8_t* d_spins, int64_t ld,
+                 cudaStream_t st);
 
 // --- exact_sampler.cu : iid draws from the exact distribution by enumeration (term t = spins of masks[t]); fills
 // out_K[replicates] and, when d_counts is set, the histograms at consecutive rows; returns log Z.  N <= GML_B200_EXACT_MAX_N.

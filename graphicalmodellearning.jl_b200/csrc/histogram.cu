@@ -37,35 +37,51 @@ __global__ void unpack_keys_kernel(const unsigned long long* __restrict__ keys, 
 
 }  // namespace
 
+void sort_key_runs(const unsigned long long* d_keys, int64_t M, int N, KeyRuns& runs, cudaStream_t st) {
+    DevBuf<unsigned long long> keys_sorted;
+    DevBuf<int> n_runs;
+    keys_sorted.alloc(M); runs.uniq.alloc(M); runs.run_len.alloc(M); n_runs.alloc(1);
+    size_t tmp_bytes = 0, tmp2 = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, d_keys, keys_sorted.p, (int)M, 0, N, st);
+    cub::DeviceRunLengthEncode::Encode(nullptr, tmp2, keys_sorted.p, runs.uniq.p, runs.run_len.p, n_runs.p, (int)M, st);
+    DevBuf<uint8_t> tmp;
+    tmp.alloc(std::max(tmp_bytes, tmp2));
+    GML_CUDA(cub::DeviceRadixSort::SortKeys(tmp.p, tmp_bytes, d_keys, keys_sorted.p, (int)M, 0, N, st));
+    ++g_launches;
+    GML_CUDA(cub::DeviceRunLengthEncode::Encode(tmp.p, tmp2, keys_sorted.p, runs.uniq.p, runs.run_len.p, n_runs.p, (int)M, st));
+    ++g_launches;
+    int hk = 0;
+    GML_CUDA(cudaMemcpyAsync(&hk, n_runs.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GML_CUDA(cudaStreamSynchronize(st));
+    runs.K = hk;
+}
+
+void unpack_key_runs(const KeyRuns& runs, int N, int8_t* d_out_spins, int64_t ld_out, double* d_out_counts, cudaStream_t st) {
+    unpack_keys_kernel<<<(unsigned)ceil_div(runs.K, 256), 256, 0, st>>>(runs.uniq.p, runs.run_len.p, runs.K, N, ld_out,
+                                                                        d_out_spins, d_out_counts);
+    GML_LAUNCHED();
+}
+
 int64_t build_histogram(const int8_t* d_samples, int64_t M, int N, int64_t ld, int8_t* d_out_spins, int64_t ld_out,
                         double* d_out_counts, cudaStream_t st) {
     GML_REQUIRE(N >= 1 && N <= 64, "device histogram builder supports 1 <= N <= 64 spins (64-bit keys)");
     GML_REQUIRE(M >= 1 && M < (1ll << 31), "device histogram builder supports up to 2^31-1 samples per call");
-    DevBuf<unsigned long long> keys, keys_sorted, uniq;
-    DevBuf<int> run_len, n_runs, flags;
-    keys.alloc(M); keys_sorted.alloc(M); uniq.alloc(M); run_len.alloc(M); n_runs.alloc(1); flags.alloc(1);
+    DevBuf<unsigned long long> keys;
+    DevBuf<int> flags;
+    keys.alloc(M); flags.alloc(1);
     GML_CUDA(cudaMemsetAsync(flags.p, 0, sizeof(int), st));
     pack_keys_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, st>>>(d_samples, ld, M, N, keys.p, flags.p);
     GML_LAUNCHED();
-    size_t tmp_bytes = 0, tmp2 = 0;
-    cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, keys.p, keys_sorted.p, (int)M, 0, N, st);
-    cub::DeviceRunLengthEncode::Encode(nullptr, tmp2, keys_sorted.p, uniq.p, run_len.p, n_runs.p, (int)M, st);
-    DevBuf<uint8_t> tmp;
-    tmp.alloc(std::max(tmp_bytes, tmp2));
-    GML_CUDA(cub::DeviceRadixSort::SortKeys(tmp.p, tmp_bytes, keys.p, keys_sorted.p, (int)M, 0, N, st));
-    ++g_launches;
-    GML_CUDA(cub::DeviceRunLengthEncode::Encode(tmp.p, tmp2, keys_sorted.p, uniq.p, run_len.p, n_runs.p, (int)M, st));
-    ++g_launches;
-    int hk = 0, hf = 0;
-    GML_CUDA(cudaMemcpyAsync(&hk, n_runs.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    KeyRuns runs;
+    sort_key_runs(keys.p, M, N, runs, st);
+    int hf = 0;
     GML_CUDA(cudaMemcpyAsync(&hf, flags.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     GML_CUDA(cudaStreamSynchronize(st));
     GML_REQUIRE(hf == 0, "samples must be exactly -1 or +1");
-    GML_REQUIRE(ld_out >= hk, "output leading dimension smaller than the number of distinct configurations");
-    unpack_keys_kernel<<<(unsigned)ceil_div(hk, 256), 256, 0, st>>>(uniq.p, run_len.p, hk, N, ld_out, d_out_spins, d_out_counts);
-    GML_LAUNCHED();
+    GML_REQUIRE(ld_out >= runs.K, "output leading dimension smaller than the number of distinct configurations");
+    unpack_key_runs(runs, N, d_out_spins, ld_out, d_out_counts, st);
     GML_CUDA(cudaStreamSynchronize(st));
-    return hk;
+    return runs.K;
 }
 
 }  // namespace gml

@@ -5,6 +5,8 @@
 // produce the N = 100 / N = 1000 benchmark inputs; here every chain is one thread, its spins are
 // bit-packed in thread-local words, and one sample per chain is emitted after `sweeps` sweeps from
 // a random start.  Counter-based RNG: results depend only on (seed, chain, sweep, site).
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace gml {
@@ -82,6 +84,39 @@ __global__ void __launch_bounds__(128) gibbs_terms_kernel(int N, int width, cons
 }
 
 }  // namespace
+
+Incidence build_incidence(int N, int order, int n_terms, const int32_t* term_idx) {
+    Incidence inc;
+    inc.width = std::max(1, order - 1);
+    const int width = inc.width;
+    inc.row_ptr.assign(N + 1, 0);
+    for (int t = 0; t < n_terms; ++t)
+        for (int m = 0; m < order; ++m) {
+            const int i = term_idx[(size_t)t * order + m];
+            if (i < 0) continue;
+            GML_REQUIRE(i < N, "sampler term refers to a spin >= N");
+            for (int m2 = 0; m2 < m; ++m2) GML_REQUIRE(term_idx[(size_t)t * order + m2] != i, "sampler term repeats a spin");
+            ++inc.row_ptr[i + 1];
+        }
+    for (int i = 0; i < N; ++i) inc.row_ptr[i + 1] += inc.row_ptr[i];
+    const int nnz = inc.row_ptr[N];
+    inc.others.assign((size_t)std::max(nnz, 1) * width, -1);
+    inc.term.assign(std::max(nnz, 1), -1);
+    std::vector<int32_t> fill(inc.row_ptr.begin(), inc.row_ptr.end() - 1);
+    for (int t = 0; t < n_terms; ++t)
+        for (int m = 0; m < order; ++m) {
+            const int i = term_idx[(size_t)t * order + m];
+            if (i < 0) continue;
+            const int q = fill[i]++;
+            inc.term[q] = t;
+            int w = 0;
+            for (int m2 = 0; m2 < order; ++m2) {
+                const int j = term_idx[(size_t)t * order + m2];
+                if (j >= 0 && m2 != m) inc.others[(size_t)q * width + w++] = j;
+            }
+        }
+    return inc;
+}
 
 void sample_gibbs_terms(int N, int width, const int32_t* d_row_ptr, const int32_t* d_others, const float* d_weight,
                         int64_t n_samples, int sweeps, uint64_t seed, int8_t* d_spins, int64_t ld, cudaStream_t st) {

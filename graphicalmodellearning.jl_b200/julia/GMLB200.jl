@@ -170,11 +170,11 @@ struct B200Exact <: GMLSampler
 end
 B200Exact(; seed=0, device=0) = B200Exact(UInt64(seed), device)
 
-function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer, sampler::B200Exact) where T <: Real
+# the term lists of the sampler entry points: n_terms x order 0-based spin ids (-1 padded) and fp64 weights
+function _gml_b200_terms(gm::FactorGraph)
     if gm.alphabet != :spin                                                                 # src/sampling.jl:95-97
         error("sampling is only supported for spin alphabets, not $(gm.alphabet)")
     end
-    num_spins = gm.varible_count
     order = maximum(length(k) for k in keys(gm.terms); init=1)
     n_terms = length(gm.terms)
     term_idx = fill(Int32(-1), order, max(n_terms, 1))     # column t = term t: the C side's n_terms x order row-major array
@@ -185,6 +185,24 @@ function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer,
         end
         term_weight[t] = Float64(weight)
     end
+    return order, n_terms, term_idx, term_weight
+end
+
+# the replicates' [count, s_1..s_N] matrices (src/sampling.jl:53-54) from the rows the library wrote at consecutive offsets
+function _gml_b200_replicates(counts, spins, out_K)
+    out = Vector{Array{Int64,2}}(undef, length(out_K))
+    first = 1
+    for r in eachindex(out_K)
+        last = first + out_K[r] - 1
+        out[r] = hcat(Int64.(counts[first:last]), Int64.(spins[first:last, :]))
+        first = last + 1
+    end
+    return out
+end
+
+function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer, sampler::B200Exact) where T <: Real
+    num_spins = gm.varible_count
+    order, n_terms, term_idx, term_weight = _gml_b200_terms(gm)
     rows = replicates * min(number_sample, 2^min(num_spins, 62))
     out_K = zeros(Int64, replicates)
     # host buffers of the largest possible size (min(n, 2^N) rows per replicate); the library stages them on the device
@@ -198,14 +216,49 @@ function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer,
                    out_K, C_NULL, counts, spins, rows, C_NULL)
     end
     _gml_b200_check(rc)
-    out = Vector{Array{Int64,2}}(undef, replicates)
-    first = 1
-    for r in 1:replicates
-        last = first + out_K[r] - 1
-        out[r] = hcat(Int64.(counts[first:last]), Int64.(spins[first:last, :]))   # [count, s_1..s_N], src/sampling.jl:53-54
-        first = last + 1
-    end
-    return out
+    return _gml_b200_replicates(counts, spins, out_K)
 end
 
 sample(gm::FactorGraph, number_sample::Integer, sampler::B200Exact) = sample(gm, number_sample, 1, sampler)[1]
+
+"""
+    B200Gibbs(; seed=0, device=0, chains=0, burn_in=200, thin=10)
+
+Multi-sample Gibbs sampler on the GPU for N <= 4096 spins and terms of order <= 8.  Each of `chains` chains (0 selects
+min(round_up(number_sample, 32), 2^17)) runs `burn_in` systematic-scan sweeps from a random start, then records its
+configuration after every `thin`-th sweep.  The draws depend only on (model, number_sample, replicates, seed, chains,
+burn_in, thin).  Up to 64 spins each replicate is a histogram in increasing configuration index; beyond, one row of count 1
+per draw.  `rhat` receives, per replicate of the last call, the split-R-hat (energy, magnetisation) over the chains' halves.
+"""
+mutable struct B200Gibbs <: GMLSampler
+    seed::UInt64
+    device::Int
+    chains::Int
+    burn_in::Int
+    thin::Int
+    rhat::Vector{NTuple{2,Float64}}
+end
+B200Gibbs(; seed=0, device=0, chains=0, burn_in=200, thin=10) =
+    B200Gibbs(UInt64(seed), device, chains, burn_in, thin, NTuple{2,Float64}[])
+
+function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer, sampler::B200Gibbs) where T <: Real
+    num_spins = gm.varible_count
+    order, n_terms, term_idx, term_weight = _gml_b200_terms(gm)
+    rows = replicates * (num_spins <= 62 ? min(number_sample, 2^num_spins) : number_sample)
+    out_K = zeros(Int64, replicates)
+    rhat = zeros(Float64, 2, replicates)
+    counts = Array{Float64}(undef, rows)
+    spins = Array{Int8}(undef, rows, num_spins)
+    GC.@preserve term_idx term_weight out_K rhat counts spins begin
+        rc = ccall((:gml_b200_sample_mcmc_device, _libgml_b200), Cint,
+                   (Int32, Int32, Int32, Int32, Ptr{Int32}, Ptr{Cdouble}, Int64, Int32, Int64, Int32, Int32, UInt64, Ptr{Int64},
+                    Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int8}, Int64, Ptr{Cvoid}),
+                   sampler.device, num_spins, order, n_terms, term_idx, term_weight, number_sample, replicates, sampler.chains,
+                   sampler.burn_in, sampler.thin, sampler.seed, out_K, rhat, counts, spins, rows, C_NULL)
+    end
+    _gml_b200_check(rc)
+    sampler.rhat = [(rhat[1, r], rhat[2, r]) for r in 1:replicates]
+    return _gml_b200_replicates(counts, spins, out_K)
+end
+
+sample(gm::FactorGraph, number_sample::Integer, sampler::B200Gibbs) = sample(gm, number_sample, 1, sampler)[1]

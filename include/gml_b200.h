@@ -254,6 +254,32 @@ int gml_b200_sample_exact_device(int32_t device, int32_t N, int32_t order, int32
                                  int64_t* out_K /* [replicates] */, double* out_log_z /* nullable */,
                                  double* d_counts, int8_t* d_spins, int64_t ld, void* stream);
 
+/* Multi-sample Gibbs sampler: `sample(gm, number_sample, replicates)` by MCMC for models beyond the exact sampler's cap, on
+ * the term lists of gml_b200_sample_exact_device (fp64 weights, rounded once to fp32 on the device).  Systematic-scan
+ * single-site Gibbs; one warp advances 32 chains with their spins in shared memory.  Each chain runs burn_in sweeps from a
+ * random start, then records its configuration at the end of every thin-th sweep; draw d = r*chains + c is chain c's r-th
+ * record and the first n_samples draws form a replicate.  Replicate r runs chains [r*chains, (r+1)*chains) of one
+ * counter-based stream, so replicates are independent and replicate 0 equals a single-replicate call.  chains = 0 picks
+ * min(round_up(n_samples, 32), 2^17).  The output depends only on (terms, n_samples, replicates, chains, burn_in, thin,
+ * seed).
+ *   - N <= 64: each replicate is a deduplicated histogram, rows in increasing configuration index (the layout of
+ *     gml_b200_sample_exact_device).  N > 64: each replicate is n_samples rows of count 1, draw order; repeated
+ *     configurations are not merged (learn() weighs a repeated row exactly like one row with the summed count).
+ *   - out_K[replicates] receives the rows of every replicate; out_rhat (nullable) [replicates][2] the split-R-hat of the
+ *     energy sum_t w_t prod s and of the magnetisation sum_i s_i over the 2*chains half-chains of the floor(n_samples /
+ *     chains) records every chain holds (NaN when a half holds fewer than 2; when no half-chain varies, 1 if they all
+ *     hold the same value and +inf if not).  Buffers as gml_b200_sample_exact_device:
+ *     d_counts == NULL is a count-only call, device buffers are written in place, host buffers are staged on the device.
+ *   - GML_B200_EINVAL: N outside [1, GML_B200_MCMC_MAX_N], order outside [1, 8], an index outside [-1, N) or repeated in a
+ *     term, a non-finite weight, n_samples < 1, replicates < 1, chains < 0, burn_in < 0, thin < 1, N <= 64 with
+ *     n_samples >= 2^31, or ld smaller than the rows (out_K is then filled). */
+#define GML_B200_MCMC_MAX_N 4096
+int gml_b200_sample_mcmc_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                const double* term_weight, int64_t n_samples, int32_t replicates, int64_t chains,
+                                int32_t burn_in, int32_t thin, uint64_t seed, int64_t* out_K /* [replicates] */,
+                                double* out_rhat /* nullable, [replicates][2]: energy, magnetisation */, double* d_counts,
+                                int8_t* d_spins, int64_t ld, void* stream);
+
 /* ---- sample-sharded mode (SURVEY 8e): histogram rows split over ranks, every rank solves all nodes; per pass
  * the int64 gradient sums and fp64 objective sums are combined with NCCL all-reduces on the solve stream.
  *   rank 0: gml_b200_comm_unique_id(id) -> broadcast the 128 bytes with any transport -> every rank:
