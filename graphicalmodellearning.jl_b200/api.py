@@ -380,6 +380,39 @@ class B200Gibbs(GMLSampler):
     last_rhat: list = field(default_factory=list, repr=False, compare=False)
 
 
+@dataclass
+class B200Tempering(GMLSampler):
+    """Replica-exchange (parallel tempering) sampler on the device (csrc/mcmc_sampler.cu) for models whose B200Gibbs chains
+    do not mix, such as ferromagnets below T_c and low-temperature spin glasses; N <= 4096, terms of order <= 8.  Each
+    chain is a ladder of replicas at the inverse temperatures `betas` (betas[0] = 1, strictly decreasing, non-negative, 2,
+    4, 8, 16 or 32 rungs; None = the library's default, 16 rungs geometric from 1 to 0.1) that exchange states between
+    adjacent rungs after every sweep; only the beta = 1 replica records.  chains = 0 picks min(round_up(number_sample,
+    32/R), 2^17/R) ladders of R rungs.  A draw costs about R times a B200Gibbs draw at the same thin.  The draws depend only
+    on (model, number_sample, replicates, seed, chains, burn_in, thin, betas).  last_rhat holds, per replicate of the last
+    call, the split-R-hat (energy, magnetisation) of the recorded chains; last_swap_rate the fraction of accepted swaps of
+    each adjacent pair of rungs after burn_in (R - 1 floats)."""
+    seed: int = 0
+    device: int = 0
+    chains: int = 0
+    burn_in: int = 200
+    thin: int = 10
+    betas: Optional[list] = None
+    last_rhat: list = field(default_factory=list, repr=False, compare=False)
+    last_swap_rate: list = field(default_factory=list, repr=False, compare=False)
+
+
+def _ladder(sampler: B200Tempering) -> np.ndarray:
+    """The betas of a B200Tempering as float64 (empty: the library default); ValueError for a ladder the library refuses."""
+    if sampler.betas is None:
+        return np.zeros(0)
+    b = np.asarray(sampler.betas, dtype=np.float64).ravel()
+    if len(b) not in (2, 4, 8, 16, 32):
+        raise ValueError(f"B200Tempering needs 2, 4, 8, 16 or 32 betas, got {len(b)}")
+    if b[0] != 1.0 or not np.isfinite(b).all() or (b < 0).any() or (np.diff(b) >= 0).any():
+        raise ValueError("B200Tempering betas must start at 1 and be finite, non-negative and strictly decreasing")
+    return b
+
+
 def _term_arrays(gm: FactorGraph):
     """The term lists of the sampler entry points: (order, term_idx int32 [n_terms x order] 0-based, -1 padded,
     term_weight float64 [n_terms])."""
@@ -397,32 +430,37 @@ def _term_arrays(gm: FactorGraph):
 def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, return_log_z: bool):
     """Validates the arguments of sample / sample_device and runs the sampler's C entry point into device buffers sized
     for the largest possible result (min(n, 2^N) rows per replicate).  Returns (counts, spins, K, log_z); log_z is None
-    for B200Gibbs, which also records its R-hat in sampler.last_rhat."""
+    for the MCMC samplers, which record their R-hat in sampler.last_rhat (B200Tempering: also last_swap_rate)."""
     import torch
     sampler = B200Exact() if sampler is None else sampler
     if isinstance(sampler, Gibbs):
         raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact() "
                                   "(N <= 40) or B200Gibbs() (MCMC) as the sampler")
-    if not isinstance(sampler, (B200Exact, B200Gibbs)):
+    if not isinstance(sampler, (B200Exact, B200Gibbs, B200Tempering)):
         raise TypeError("sampler must be a GMLSampler")
-    mcmc = isinstance(sampler, B200Gibbs)
+    mcmc = isinstance(sampler, (B200Gibbs, B200Tempering))
+    tempering = isinstance(sampler, B200Tempering)
+    name = type(sampler).__name__
     if mcmc:
         sampler.last_rhat = []
+        if tempering:
+            sampler.last_swap_rate = []
         if return_log_z:
-            raise ValueError("B200Gibbs is an MCMC sampler and has no partition function: return_log_z needs B200Exact")
+            raise ValueError(f"{name} is an MCMC sampler and has no partition function: return_log_z needs B200Exact")
     if gm.alphabet != "spin":                                                    # src/sampling.jl:95-97
         raise ValueError(f"sampling of a FactorGraph is only supported for the spin alphabet, not {gm.alphabet!r}")
     N, n, reps = int(gm.varible_count), int(number_sample), int(replicates)
     cap = _lib.MCMC_MAX_N if mcmc else _lib.EXACT_MAX_N
     if not 1 <= N <= cap:
-        raise ValueError(f"the {type(sampler).__name__} sampler supports 1 <= N <= {cap} spins, got {N}")
+        raise ValueError(f"the {name} sampler supports 1 <= N <= {cap} spins, got {N}")
     if n < 1 or reps < 1:
         raise ValueError("number_sample and replicates must be >= 1")
     if mcmc:
         if sampler.chains < 0 or sampler.burn_in < 0 or sampler.thin < 1:
-            raise ValueError("B200Gibbs needs chains >= 0, burn_in >= 0 and thin >= 1")
+            raise ValueError(f"{name} needs chains >= 0, burn_in >= 0 and thin >= 1")
         if N <= 64 and n >= 2 ** 31:
-            raise ValueError("B200Gibbs builds the histogram of N <= 64 spins from fewer than 2^31 draws per replicate")
+            raise ValueError(f"{name} builds the histogram of N <= 64 spins from fewer than 2^31 draws per replicate")
+    betas = _ladder(sampler) if tempering else None
     order, idx, wts = _term_arrays(gm)
     ld = reps * min(n, 1 << N)
     dev = f"cuda:{int(sampler.device)}"
@@ -437,8 +475,14 @@ def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, 
         _lib.check(lib.gml_b200_sample_exact_device(*head, int(sampler.seed) & (2 ** 64 - 1), _ptr(K), ctypes.byref(log_z), *tail))
         return counts, spins, K, log_z.value
     rhat = np.zeros((reps, 2))
-    _lib.check(lib.gml_b200_sample_mcmc_device(*head, int(sampler.chains), int(sampler.burn_in), int(sampler.thin),
-                                               int(sampler.seed) & (2 ** 64 - 1), _ptr(K), _ptr(rhat), *tail))
+    run = (int(sampler.chains), int(sampler.burn_in), int(sampler.thin), int(sampler.seed) & (2 ** 64 - 1), _ptr(K), _ptr(rhat))
+    if tempering:
+        swap = np.zeros((reps, (len(betas) or _lib.TEMPERING_DEFAULT_RUNGS) - 1))
+        _lib.check(lib.gml_b200_sample_tempering_device(*head[:6], len(betas), _ptr(betas) if len(betas) else None, *head[6:],
+                                                        *run, _ptr(swap), *tail))
+        sampler.last_swap_rate = swap.tolist()
+    else:
+        _lib.check(lib.gml_b200_sample_mcmc_device(*head, *run, *tail))
     sampler.last_rhat = [tuple(r) for r in rhat.tolist()]
     return counts, spins, K, None
 
@@ -460,8 +504,8 @@ def sample(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Op
            return_log_z: bool = False):
     """sample(gm, number_sample[, replicates[, sampler]]) -- src/sampling.jl:90-106.  Returns the reference's int64
     K x (N+1) matrix [count, s_1..s_N] (spin_i = 2*bit_i - 1), or a list of them when replicates > 1; learn() takes it as it
-    is.  Rows are in increasing configuration index, except for B200Gibbs beyond 64 spins, whose rows are the draws in
-    order with count 1.  The default sampler is B200Exact(seed=0, device=0)."""
+    is.  Rows are in increasing configuration index, except for B200Gibbs and B200Tempering beyond 64 spins, whose rows
+    are the draws in order with count 1.  The default sampler is B200Exact(seed=0, device=0)."""
     counts, spins, K, log_z = _sample_call(gm, number_sample, replicates, sampler, return_log_z)
     rows = int(K.sum())
     c = counts[:rows].cpu().numpy().astype(np.int64)

@@ -247,6 +247,43 @@ template <class Fill> void into_sample_buffers(double* d_counts, int8_t* d_spins
     }
 }
 
+// The MCMC entry points (betas = {1}: gml_b200_sample_mcmc_device; R > 1 rungs: gml_b200_sample_tempering_device, whose
+// ladder the caller has checked): argument checks, then the sampler into the caller's buffers.
+void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx, const double* term_weight,
+              const std::vector<double>& betas, int64_t n_samples, int32_t replicates, int64_t chains, int32_t burn_in,
+              int32_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate, double* d_counts,
+              int8_t* d_spins, int64_t ld, void* stream) {
+    GML_REQUIRE(N >= 1 && N <= GML_B200_MCMC_MAX_N, "MCMC sampler needs 1 <= N <= " + std::to_string(GML_B200_MCMC_MAX_N));
+    GML_REQUIRE(order >= 1 && order <= 8 && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)) && out_K,
+                "bad sampler argument");
+    GML_REQUIRE(n_samples >= 1 && replicates >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1,
+                "bad sampler sizes");
+    GML_REQUIRE(N > 64 || n_samples < (INT64_C(1) << 31), "the histogram of N <= 64 spins takes fewer than 2^31 draws per replicate");
+    GML_REQUIRE(!d_counts || (d_spins && ld >= 1), "d_counts needs d_spins and ld >= 1");
+    const int rungs = (int)betas.size();
+    if (chains == 0) chains = mcmc_auto_chains(n_samples, rungs);
+    const double steps = ((double)burn_in + (double)thin * (double)ceil_div(n_samples, chains)) * N;
+    GML_REQUIRE(steps * replicates < 0x1.0p62, "too many sweeps");
+    std::vector<int32_t> idx(term_idx, term_idx + (size_t)n_terms * order);
+    std::vector<double> weights(term_weight, term_weight + n_terms);
+    for (int t = 0; t < n_terms; ++t) {
+        for (int m = 0; m < order; ++m) GML_REQUIRE(idx[(size_t)t * order + m] >= -1, "sampler term refers to a spin outside [0, N)");
+        GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
+    }
+    const Incidence inc = build_incidence(N, order, n_terms, idx.data());
+    if (N > 64 && d_counts && ld < n_samples * replicates) {
+        for (int r = 0; r < replicates; ++r) out_K[r] = n_samples;
+        GML_REQUIRE(false, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(n_samples * replicates) +
+                           " rows of the replicates (out_K holds their sizes)");
+    }
+    GML_CUDA(cudaSetDevice(device));
+    cudaStream_t st = (cudaStream_t)stream;
+    into_sample_buffers(d_counts, d_spins, ld, N, replicates, out_K, st, [&](double* c, int8_t* sp) {
+        sample_mcmc(N, order, idx, weights, inc, betas, n_samples, replicates, chains, burn_in, thin, seed, out_K, out_rhat,
+                    out_swap_rate, c, sp, ld, st);
+    });
+}
+
 void throw_if_unconverged(int n_unconverged) {
     if (n_unconverged == 0) return;
     set_error("solver did not reach tol within max_iter for " + std::to_string(n_unconverged) + " node(s)");
@@ -1208,34 +1245,33 @@ int gml_b200_sample_mcmc_device(int32_t device, int32_t N, int32_t order, int32_
                                 int32_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* d_counts, int8_t* d_spins,
                                 int64_t ld, void* stream) {
     return guarded([&] {
-        GML_REQUIRE(N >= 1 && N <= GML_B200_MCMC_MAX_N, "MCMC sampler needs 1 <= N <= " + std::to_string(GML_B200_MCMC_MAX_N));
-        GML_REQUIRE(order >= 1 && order <= 8 && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)) && out_K,
-                    "bad sampler argument");
-        GML_REQUIRE(n_samples >= 1 && replicates >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1,
-                    "bad sampler sizes");
-        GML_REQUIRE(N > 64 || n_samples < (INT64_C(1) << 31), "the histogram of N <= 64 spins takes fewer than 2^31 draws per replicate");
-        GML_REQUIRE(!d_counts || (d_spins && ld >= 1), "d_counts needs d_spins and ld >= 1");
-        if (chains == 0) chains = mcmc_auto_chains(n_samples);
-        const double steps = ((double)burn_in + (double)thin * (double)ceil_div(n_samples, chains)) * N;
-        GML_REQUIRE(steps * replicates < 0x1.0p62, "too many sweeps");
-        std::vector<int32_t> idx(term_idx, term_idx + (size_t)n_terms * order);
-        std::vector<double> weights(term_weight, term_weight + n_terms);
-        for (int t = 0; t < n_terms; ++t) {
-            for (int m = 0; m < order; ++m) GML_REQUIRE(idx[(size_t)t * order + m] >= -1, "sampler term refers to a spin outside [0, N)");
-            GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
+        run_mcmc(device, N, order, n_terms, term_idx, term_weight, {1.0}, n_samples, replicates, chains, burn_in, thin, seed,
+                 out_K, out_rhat, nullptr, d_counts, d_spins, ld, stream);
+    });
+}
+
+int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                     const double* term_weight, int32_t n_rungs, const double* betas, int64_t n_samples,
+                                     int32_t replicates, int64_t chains, int32_t burn_in, int32_t thin, uint64_t seed,
+                                     int64_t* out_K, double* out_rhat, double* out_swap_rate, double* d_counts, int8_t* d_spins,
+                                     int64_t ld, void* stream) {
+    return guarded([&] {
+        GML_REQUIRE(n_rungs == 0 || n_rungs == 2 || n_rungs == 4 || n_rungs == 8 || n_rungs == 16 || n_rungs == 32,
+                    "n_rungs must be 0 (the default ladder) or one of 2, 4, 8, 16, 32");
+        GML_REQUIRE((n_rungs == 0) == (betas == nullptr), "n_rungs = 0 goes with betas = NULL (the default ladder) and only with it");
+        std::vector<double> ladder;
+        if (n_rungs == 0) {                          // the default ladder: geometric from 1 to 0.1
+            constexpr int R = GML_B200_TEMPERING_DEFAULT_RUNGS;
+            for (int k = 0; k < R; ++k) ladder.push_back(std::pow(0.1, (double)k / (R - 1)));
+        } else {
+            ladder.assign(betas, betas + n_rungs);
+            GML_REQUIRE(ladder[0] == 1.0, "betas[0] must be 1 (the rung that records)");
+            for (int k = 1; k < n_rungs; ++k)
+                GML_REQUIRE(std::isfinite(ladder[k]) && ladder[k] >= 0.0 && ladder[k] < ladder[k - 1],
+                            "betas must be finite, non-negative and strictly decreasing");
         }
-        const Incidence inc = build_incidence(N, order, n_terms, idx.data());
-        if (N > 64 && d_counts && ld < n_samples * replicates) {
-            for (int r = 0; r < replicates; ++r) out_K[r] = n_samples;
-            GML_REQUIRE(false, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(n_samples * replicates) +
-                               " rows of the replicates (out_K holds their sizes)");
-        }
-        GML_CUDA(cudaSetDevice(device));
-        cudaStream_t st = (cudaStream_t)stream;
-        into_sample_buffers(d_counts, d_spins, ld, N, replicates, out_K, st, [&](double* c, int8_t* sp) {
-            sample_mcmc(N, order, idx, weights, inc, n_samples, replicates, chains, burn_in, thin, seed, out_K, out_rhat, c, sp,
-                        ld, st);
-        });
+        run_mcmc(device, N, order, n_terms, term_idx, term_weight, ladder, n_samples, replicates, chains, burn_in, thin, seed,
+                 out_K, out_rhat, out_swap_rate, d_counts, d_spins, ld, stream);
     });
 }
 

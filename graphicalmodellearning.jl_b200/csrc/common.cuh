@@ -245,16 +245,19 @@ struct Incidence {
 };
 Incidence build_incidence(int N, int order, int n_terms, const int32_t* term_idx);
 
-// --- mcmc_sampler.cu : multi-sample Gibbs sampler (one warp = 32 chains, state in shared memory); fills out_K and
-// out_rhat (nullable, [replicates][2]: split-R-hat of the energy and of the magnetisation) and, when d_counts is set,
-// the replicates' rows at consecutive rows: N <= 64 deduplicated histograms, N > 64 one row per draw.
+// --- mcmc_sampler.cu : multi-sample Gibbs sampler (one warp = 32 chains, state in shared memory) and its replica-exchange
+// form (betas.size() = R > 1 rungs: a ladder of R lanes per chain, only rung 0 = betas[0] = 1 records); fills out_K and
+// out_rhat (nullable, [replicates][2]: split-R-hat of the energy and of the magnetisation), out_swap_rate (nullable, R > 1,
+// [replicates][R-1]: accepted / proposed swaps of each adjacent pair after burn_in) and, when d_counts is set, the
+// replicates' rows at consecutive rows: N <= 64 deduplicated histograms, N > 64 one row per draw.
 // N <= GML_B200_MCMC_MAX_N; term weights are rounded once to fp32.
 constexpr int64_t MCMC_AUTO_CHAINS = 1 << 17;
-int64_t mcmc_auto_chains(int64_t n_samples);
+constexpr int TEMPERING_MAX_RUNGS = GML_B200_TEMPERING_MAX_RUNGS;
+int64_t mcmc_auto_chains(int64_t n_samples, int rungs);
 void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
-                 const Incidence& inc, int64_t n_samples, int replicates, int64_t chains, int64_t burn_in, int64_t thin,
-                 uint64_t seed, int64_t* out_K, double* out_rhat, double* d_counts, int8_t* d_spins, int64_t ld,
-                 cudaStream_t st);
+                 const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int replicates, int64_t chains,
+                 int64_t burn_in, int64_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate,
+                 double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st);
 
 // --- exact_sampler.cu : iid draws from the exact distribution by enumeration (term t = spins of masks[t]); fills
 // out_K[replicates] and, when d_counts is set, the histograms at consecutive rows; returns log Z.  N <= GML_B200_EXACT_MAX_N.

@@ -262,3 +262,57 @@ function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer,
 end
 
 sample(gm::FactorGraph, number_sample::Integer, sampler::B200Gibbs) = sample(gm, number_sample, 1, sampler)[1]
+
+const GML_B200_TEMPERING_DEFAULT_RUNGS = 16   # include/gml_b200.h
+
+"""
+    B200Tempering(; seed=0, device=0, chains=0, burn_in=200, thin=10, betas=Float64[])
+
+Replica-exchange (parallel tempering) sampler on the GPU for models whose B200Gibbs chains do not mix; N <= 4096 spins,
+terms of order <= 8.  Each chain is a ladder of replicas at the inverse temperatures `betas` (betas[1] = 1, strictly
+decreasing, non-negative; 2, 4, 8, 16 or 32 rungs; empty selects the library's default, 16 rungs geometric from 1 to 0.1)
+that exchange states between adjacent rungs after every sweep; only the beta = 1 replica records.  `chains` = 0 selects
+min(round_up(number_sample, 32/R), 2^17/R) ladders of R rungs; a draw costs about R times a B200Gibbs draw.  `rhat`
+receives, per replicate of the last call, the split-R-hat (energy, magnetisation); `swap_rate` the fraction of accepted
+swaps of each adjacent pair of rungs after burn_in.
+"""
+mutable struct B200Tempering <: GMLSampler
+    seed::UInt64
+    device::Int
+    chains::Int
+    burn_in::Int
+    thin::Int
+    betas::Vector{Float64}
+    rhat::Vector{NTuple{2,Float64}}
+    swap_rate::Vector{Vector{Float64}}
+end
+B200Tempering(; seed=0, device=0, chains=0, burn_in=200, thin=10, betas=Float64[]) =
+    B200Tempering(UInt64(seed), device, chains, burn_in, thin, Float64.(betas), NTuple{2,Float64}[], Vector{Float64}[])
+
+function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer, sampler::B200Tempering) where T <: Real
+    num_spins = gm.varible_count
+    order, n_terms, term_idx, term_weight = _gml_b200_terms(gm)
+    rows = replicates * (num_spins <= 62 ? min(number_sample, 2^num_spins) : number_sample)
+    n_rungs = length(sampler.betas)
+    pairs = (n_rungs == 0 ? GML_B200_TEMPERING_DEFAULT_RUNGS : n_rungs) - 1
+    betas = sampler.betas
+    out_K = zeros(Int64, replicates)
+    rhat = zeros(Float64, 2, replicates)
+    swap = zeros(Float64, pairs, replicates)
+    counts = Array{Float64}(undef, rows)
+    spins = Array{Int8}(undef, rows, num_spins)
+    GC.@preserve term_idx term_weight betas out_K rhat swap counts spins begin
+        rc = ccall((:gml_b200_sample_tempering_device, _libgml_b200), Cint,
+                   (Int32, Int32, Int32, Int32, Ptr{Int32}, Ptr{Cdouble}, Int32, Ptr{Cdouble}, Int64, Int32, Int64, Int32, Int32,
+                    UInt64, Ptr{Int64}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int8}, Int64, Ptr{Cvoid}),
+                   sampler.device, num_spins, order, n_terms, term_idx, term_weight, n_rungs,
+                   n_rungs == 0 ? Ptr{Cdouble}(C_NULL) : pointer(betas), number_sample, replicates, sampler.chains,
+                   sampler.burn_in, sampler.thin, sampler.seed, out_K, rhat, swap, counts, spins, rows, C_NULL)
+    end
+    _gml_b200_check(rc)
+    sampler.rhat = [(rhat[1, r], rhat[2, r]) for r in 1:replicates]
+    sampler.swap_rate = [swap[:, r] for r in 1:replicates]
+    return _gml_b200_replicates(counts, spins, out_K)
+end
+
+sample(gm::FactorGraph, number_sample::Integer, sampler::B200Tempering) = sample(gm, number_sample, 1, sampler)[1]

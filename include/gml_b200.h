@@ -280,6 +280,30 @@ int gml_b200_sample_mcmc_device(int32_t device, int32_t N, int32_t order, int32_
                                 double* out_rhat /* nullable, [replicates][2]: energy, magnetisation */, double* d_counts,
                                 int8_t* d_spins, int64_t ld, void* stream);
 
+/* Replica-exchange (parallel tempering) sampler: gml_b200_sample_mcmc_device for models whose single-site Gibbs chains do
+ * not mix (strong ferromagnets, low-temperature glasses).  A chain is a ladder of n_rungs replicas of the model at the
+ * inverse temperatures betas[0] = 1 > betas[1] > ... >= 0 (replica k draws from p(s)^betas[k]); after every sweep the
+ * adjacent pairs (k, k+1) with k = sweep (mod 2) propose to exchange their states (deterministic even-odd scheme), accepted
+ * with probability min(1, exp((beta_k - beta_{k+1}) (E_{k+1} - E_k))), E = sum_t w_t prod s.  Only the beta = 1 replica
+ * records: draw d = r*chains + c is ladder c's r-th record.  n_rungs = 0 with betas = NULL selects the default ladder:
+ * 16 rungs geometric from 1 to 0.1 (beta_k = 0.1^(k/15)).  chains = 0 picks min(round_up(n_samples, 32/R), 2^17/R) ladders
+ * of R rungs.  Each ladder yields one draw per record step, so a draw costs about R times a gml_b200_sample_mcmc_device
+ * draw at the same thin.  The output depends only on (terms, n_samples, replicates, chains, burn_in, thin, betas, seed).
+ *   - Output layout, out_K, out_rhat (of the beta = 1 records) and the buffers as gml_b200_sample_mcmc_device.
+ *   - out_swap_rate (nullable) [replicates][n_rungs - 1] (default ladder: GML_B200_TEMPERING_DEFAULT_RUNGS - 1): per
+ *     adjacent pair, the fraction of the swaps proposed after burn_in that were accepted (NaN when none was proposed).
+ *   - GML_B200_EINVAL: everything gml_b200_sample_mcmc_device refuses, n_rungs not in {0, 2, 4, 8, 16, 32}, exactly one of
+ *     n_rungs == 0 and betas == NULL, betas[0] != 1, betas not strictly decreasing, or a negative or non-finite beta. */
+#define GML_B200_TEMPERING_MAX_RUNGS 32
+#define GML_B200_TEMPERING_DEFAULT_RUNGS 16
+int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                     const double* term_weight, int32_t n_rungs, const double* betas /* [n_rungs] */,
+                                     int64_t n_samples, int32_t replicates, int64_t chains, int32_t burn_in, int32_t thin,
+                                     uint64_t seed, int64_t* out_K /* [replicates] */,
+                                     double* out_rhat /* nullable [replicates][2] */,
+                                     double* out_swap_rate /* nullable [replicates][n_rungs - 1] */, double* d_counts,
+                                     int8_t* d_spins, int64_t ld, void* stream);
+
 /* ---- sample-sharded mode (SURVEY 8e): histogram rows split over ranks, every rank solves all nodes; per pass
  * the int64 gradient sums and fp64 objective sums are combined with NCCL all-reduces on the solve stream.
  *   rank 0: gml_b200_comm_unique_id(id) -> broadcast the 128 bytes with any transport -> every rank:
