@@ -375,19 +375,21 @@ __device__ __forceinline__ void energy_epilogue(const EnergyParams& p, const int
         else if (XL == 3) e = __int2float_rn(join2(join2(a[0][i], a[1][i]), a[2][i]));       // exact in fp32 while |E| < 4
         else e = fmaf(__int2float_rn(join2(a[0][i], a[1][i])), 65536.f, __int2float_rn(join2(a[2][i], a[3][i])));
         const float es = flip_sign(e, sb_top);                  // s_u * E / lattice
-        float fterm, gterm;
+        float gterm;
         if (FORM == GML_B200_RPLE) {
             const float t2 = -2.f * p.lattice * es;
             const float ex = fast_ex2(-fabsf(t2) * 1.4426950408889634f);
-            fterm = wk * fmaf(fast_lg2(1.f + ex), 0.6931471805599453f, fmaxf(t2, 0.f));
+            facc[i] += wk * fmaf(fast_lg2(1.f + ex), 0.6931471805599453f, fmaxf(t2, 0.f));
             gterm = __fdividef(2.f * wk * (t2 > 0.f ? 1.f : ex), 1.f + ex);   // 2 w sigma(-2t)
         } else {
             // no clamp: |t| <= |x_u|_1 keeps the argument in range; an overflow for a wild trial point (|x_u|_1 > 80) gives
-            // f = inf, which the driver's descent test rejects
-            fterm = wk * fast_ex2(es * c_arg);
-            gterm = fterm;
+            // f = inf, which the driver's descent test rejects.  The objective term is one fma in every instantiation: with
+            // a separately rounded product (the residual) the full passes and the objective-only passes of the line
+            // search would differ by ~3e-9 relative
+            const float ex = fast_ex2(es * c_arg);
+            facc[i] = fmaf(wk, ex, facc[i]);
+            gterm = wk * ex;
         }
-        facc[i] += fterm;
         if (GRAD) {
             // r = s_u * gterm in units of the node's residual grid, rounded to nearest, plus the
             // bias that makes all balanced digits non-negative
@@ -1192,20 +1194,18 @@ using GradKernel = void (*)(CUtensorMap, CUtensorMap, GradParams);
 template <class K> struct Launch { K kernel; int smem; };   // kernel and its dynamic shared memory
 
 // form: RPLE, or RISE for both RISE and logRISE; xl = iterate limbs (4 fine, 3 coarse, 2 rough level); nr = residual
-// digit planes, read by the gradient passes only (the rough level has one)
+// digit planes, read by the gradient passes only.  The gradient kernels are the ones BackendTC::level_nr() can select:
+// fine nr = nR in {3, 4}, coarse nr = max(2, nR - 1) in {2, 3}, rough nr = 1 (tests/test_gpu_tc_passes.py checks that
+// every instantiation here is launched by some pass).
 struct EnergyInstance { int form; bool grad; int xl, nr; EnergyKernel stream, pair; };
 template <int FORM, bool GRAD, int XL, int NR>
 EnergyInstance energy_instance() { return {FORM, GRAD, XL, NR, tc_energy_kernel<FORM, GRAD, XL, NR>, tc_energy_pair_kernel<FORM, GRAD, XL, NR>}; }
 const EnergyInstance ENERGY_KERNELS[] = {
-    energy_instance<GML_B200_RISE, false, 4, 2>(), energy_instance<GML_B200_RISE, true, 4, 2>(),
-    energy_instance<GML_B200_RISE, true, 4, 3>(), energy_instance<GML_B200_RISE, true, 4, 4>(),
-    energy_instance<GML_B200_RISE, false, 3, 2>(), energy_instance<GML_B200_RISE, true, 3, 2>(),
-    energy_instance<GML_B200_RISE, true, 3, 3>(), energy_instance<GML_B200_RISE, true, 3, 4>(),
+    energy_instance<GML_B200_RISE, false, 4, 2>(), energy_instance<GML_B200_RISE, true, 4, 3>(), energy_instance<GML_B200_RISE, true, 4, 4>(),
+    energy_instance<GML_B200_RISE, false, 3, 2>(), energy_instance<GML_B200_RISE, true, 3, 2>(), energy_instance<GML_B200_RISE, true, 3, 3>(),
     energy_instance<GML_B200_RISE, false, 2, 1>(), energy_instance<GML_B200_RISE, true, 2, 1>(),
-    energy_instance<GML_B200_RPLE, false, 4, 2>(), energy_instance<GML_B200_RPLE, true, 4, 2>(),
-    energy_instance<GML_B200_RPLE, true, 4, 3>(), energy_instance<GML_B200_RPLE, true, 4, 4>(),
-    energy_instance<GML_B200_RPLE, false, 3, 2>(), energy_instance<GML_B200_RPLE, true, 3, 2>(),
-    energy_instance<GML_B200_RPLE, true, 3, 3>(), energy_instance<GML_B200_RPLE, true, 3, 4>(),
+    energy_instance<GML_B200_RPLE, false, 4, 2>(), energy_instance<GML_B200_RPLE, true, 4, 3>(), energy_instance<GML_B200_RPLE, true, 4, 4>(),
+    energy_instance<GML_B200_RPLE, false, 3, 2>(), energy_instance<GML_B200_RPLE, true, 3, 2>(), energy_instance<GML_B200_RPLE, true, 3, 3>(),
     energy_instance<GML_B200_RPLE, false, 2, 1>(), energy_instance<GML_B200_RPLE, true, 2, 1>()};
 Launch<EnergyKernel> energy_kernel(int form, bool grad, int xl, int nr, bool pair) {
     const int kform = form == GML_B200_RPLE ? GML_B200_RPLE : GML_B200_RISE;
