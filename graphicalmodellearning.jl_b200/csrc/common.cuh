@@ -127,7 +127,7 @@ struct SolveResult {
     int iterations = 0, n_fg = 0, n_f = 0, n_unconverged = 0;
     int n_stalled = 0;        // nodes accepted at the gradient noise floor with tol < residual <= 10 tol
     int n_out_of_range = 0;   // nodes re-solved by the CUDA-core backend because they left the fixed-point range
-    int n_unpolished = 0;     // support polish: nodes whose support exceeded the reduced solver's 64 features (FISTA point kept)
+    int n_unpolished = 0;     // support polish: nodes whose support exceeded the reduced solver's NEWTON_MAX_F = 128 features (FISTA point kept)
     DevBuf<double> grad;      // [Nn x Fp] gradient of the smooth part at x (filled by solve_fista when want_grad_at_x)
     bool want_grad_at_x = false;
     bool want_objective = true;   // false: the FISTA driver skips the final objective pass (`objective` is then not filled)

@@ -14,6 +14,12 @@ namespace {
 constexpr int TS = 128;        // samples per staged tile
 constexpr int NT = 256;        // threads per accumulation CTA
 constexpr int NALPHA = 12;     // step sizes 1, 1/2, ..., 2^-11 tried per line-search pass
+// Barrier phase stall rule.  The phase stops at a Newton step below 1e-15, but at some nodes rounding keeps the step at a
+// few 1e-15 (the direction is computed from fp64 sums over K rows) and the merit stops moving.  A node whose step stays
+// below STALL_STEP with a merit change within the line search's summation slack for STALL_ITERS consecutive iterations
+// is converged at the rounding floor: accepted and counted in stats.n_stalled, not run out to max_iter.
+constexpr double STALL_STEP = 1e-13;
+constexpr int STALL_ITERS = 4;
 
 struct NewtonParams {
     const int8_t* Q;           // [Fp x Kp]
@@ -36,6 +42,7 @@ struct NewtonParams {
     double* obj;               // [Nn]
     double* resid;             // [Nn] last step size
     int* conv;                 // [Nn]
+    int* idle;                 // [Nn] consecutive barrier iterations at the rounding floor (STALL_ITERS: stalled)
     int* n_active;             // [1]
 };
 
@@ -432,7 +439,14 @@ __device__ __forceinline__ void newton_update_body(const NewtonParams& p, int fo
     for (int o = 16; o; o >>= 1) step = fmax(step, __shfl_xor_sync(0xffffffffu, step, o));
     if (lane == 0) {
         p.resid[u] = step;
-        if (p.barrier && step < p.tol) p.conv[u] = 1;
+        bool done = false;
+        if (p.barrier) {
+            const double f0 = p.fcur[u];
+            const bool flat = step >= p.tol && step < STALL_STEP && fabs(f0 - last_merit) <= 1e-13 * fmax(fabs(f0), 1.0);
+            p.idle[u] = flat ? p.idle[u] + 1 : 0;
+            done = step < p.tol || p.idle[u] >= STALL_ITERS;
+        }
+        if (done) p.conv[u] = 1;
         else atomicAdd(p.n_active, 1);
     }
 }
@@ -505,6 +519,16 @@ void launch_accum(const NewtonParams& P, int form, cudaStream_t st) {
     GML_LAUNCHED();
 }
 
+// nodes whose barrier phase stopped at the rounding floor (synchronises the stream)
+int count_stalled(const int* d_idle, int Nn, cudaStream_t st) {
+    std::vector<int> h(Nn);
+    GML_CUDA(cudaMemcpyAsync(h.data(), d_idle, sizeof(int) * Nn, cudaMemcpyDeviceToHost, st));
+    GML_CUDA(cudaStreamSynchronize(st));
+    int n = 0;
+    for (int v : h) n += v >= STALL_ITERS;
+    return n;
+}
+
 }  // namespace
 
 void solve_newton(const NodeProblem& prob, const gml_b200_opts& o, SolveResult& r, cudaStream_t st) {
@@ -524,18 +548,19 @@ void solve_newton(const NodeProblem& prob, const gml_b200_opts& o, SolveResult& 
     chunks = ceil_div(h.Kp, chunk_len);
 
     DevBuf<double> d, part, part_ls, fcur, slope, resid;
-    DevBuf<int> conv, n_active;
+    DevBuf<int> conv, idle, n_active;
     r.x.alloc((size_t)Nn * Fp);
     r.objective.alloc(Nn);
     d.alloc((size_t)Nn * Fp);
     part.alloc((size_t)Nn * chunks * Ptot);
     part_ls.alloc((size_t)Nn * chunks * NALPHA);
     fcur.alloc(Nn); slope.alloc(Nn); resid.alloc(Nn);
-    conv.alloc(Nn); n_active.alloc(1);
+    conv.alloc(Nn); idle.alloc(Nn); n_active.alloc(1);
     if (prob.x0) GML_CUDA(cudaMemcpyAsync(r.x.p, prob.x0, sizeof(double) * Nn * Fp, cudaMemcpyDeviceToDevice, st));
     else GML_CUDA(cudaMemsetAsync(r.x.p, 0, sizeof(double) * Nn * Fp, st));
     GML_CUDA(cudaMemsetAsync(d.p, 0, sizeof(double) * Nn * Fp, st));
     GML_CUDA(cudaMemsetAsync(conv.p, 0, sizeof(int) * Nn, st));
+    GML_CUDA(cudaMemsetAsync(idle.p, 0, sizeof(int) * Nn, st));
     GML_CUDA(cudaMemsetAsync(resid.p, 0, sizeof(double) * Nn, st));
 
     NewtonParams P{};
@@ -543,7 +568,7 @@ void solve_newton(const NodeProblem& prob, const gml_b200_opts& o, SolveResult& 
     P.Kp = h.Kp; P.F = F; P.Fp = Fp; P.Nn = Nn; P.chunks = (int)chunks; P.chunk_len = chunk_len;
     P.lambda = prob.lambda; P.mu = o.barrier_mu;
     P.x = r.x.p; P.d = d.p; P.part = part.p; P.part_ls = part_ls.p; P.fcur = fcur.p; P.slope = slope.p;
-    P.obj = r.objective.p; P.resid = resid.p; P.conv = conv.p; P.n_active = n_active.p;
+    P.obj = r.objective.p; P.resid = resid.p; P.conv = conv.p; P.idle = idle.p; P.n_active = n_active.p;
 
     const size_t dir_smem = sizeof(double) * ((size_t)F * F + 4 * F);
     const int form = prob.form;
@@ -584,12 +609,13 @@ void solve_newton(const NodeProblem& prob, const gml_b200_opts& o, SolveResult& 
         std::vector<double> hres(Nn);
         GML_CUDA(cudaMemcpyAsync(hinfo.data(), info.p, sizeof(int) * 2 * Nn, cudaMemcpyDeviceToHost, st));
         GML_CUDA(cudaMemcpyAsync(hres.data(), resid.p, sizeof(double) * Nn, cudaMemcpyDeviceToHost, st));
-        GML_CUDA(cudaStreamSynchronize(st));
+        const int stalled = count_stalled(idle.p, Nn, st);
         int unconv = 0, iters = 0;
         double mr = 0.0;
         for (int u = 0; u < Nn; ++u) { iters = std::max(iters, hinfo[2 * u]); unconv += hinfo[2 * u + 1]; mr = std::max(mr, hres[u]); }
         const bool two_phase = o.barrier_mu > 0.0 && prob.lambda > 0.0;
         r.iterations = iters; r.n_fg = iters + (two_phase ? 2 : 1); r.n_f = iters; r.n_unconverged = unconv; r.max_residual = mr;
+        r.n_stalled = stalled;
         return;
     }
     run_phase(0, tol_exact);
@@ -610,10 +636,11 @@ void solve_newton(const NodeProblem& prob, const gml_b200_opts& o, SolveResult& 
 
     std::vector<double> hres(Nn);
     GML_CUDA(cudaMemcpyAsync(hres.data(), resid.p, sizeof(double) * Nn, cudaMemcpyDeviceToHost, st));
-    GML_CUDA(cudaStreamSynchronize(st));
+    const int stalled = count_stalled(idle.p, Nn, st);
     double mr = 0.0;
     for (double v : hres) mr = std::max(mr, v);
     r.iterations = total_iter; r.n_fg = n_fg; r.n_f = n_f; r.n_unconverged = unconverged; r.max_residual = mr;
+    r.n_stalled = stalled;
 }
 
 }  // namespace gml

@@ -85,7 +85,9 @@ typedef struct gml_b200_stats {
     int32_t n_unconverged;    /* nodes that missed tol (the call then returns GML_B200_ENOTCONV) */
     int32_t n_stalled;        /* FISTA: nodes whose gradient mapping stopped improving at the backend's gradient noise floor
                                  with tol < residual <= 10*tol; they are ACCEPTED (not counted in n_unconverged) and their
-                                 residual is part of max_residual -- callers that need tol strictly check n_stalled == 0 */
+                                 residual is part of max_residual -- callers that need tol strictly check n_stalled == 0.
+                                 Newton, barrier_mu > 0: nodes whose barrier Newton step stayed between 1e-15 (the stop) and
+                                 1e-13 with a flat merit for 4 iterations (the fp64 rounding floor); also accepted */
     int64_t kernel_launches;  /* kernels of this library launched by the call */
     double evals;             /* node*sample evals = nodes*K*(fg + 0.5*f), passes weighted by the fraction of
                                  the histogram they swept (coarse continuation levels count 1/stride)  (SURVEY 8d) */

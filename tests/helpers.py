@@ -1,4 +1,8 @@
 """Seeded synthetic inputs shared by the tests (BASELINE.json configs, reduced where noted)."""
+import re
+import shutil
+import subprocess
+
 import numpy as np
 
 import gml_oracle as o
@@ -127,3 +131,23 @@ def three_body_model(n, seed, n_triples=None):
         t = tuple(sorted(int(x) + 1 for x in rng.choice(n, 3, replace=False)))
         terms[t] = float(rng.choice([-0.4, 0.4]))
     return terms
+
+
+# ---- which kernels ran, which are compiled ------------------------------------------------------------------------------
+def profiled_kernel_names(fn):
+    """fn()'s result and the names of the CUDA kernels it launched (torch.profiler)"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        out = fn()
+        torch.cuda.synchronize()
+    return out, [ev.key for ev in prof.key_averages()]
+
+
+def compiled_kernel_names(lib_path):
+    """the (mangled) names of the kernels compiled into the library at lib_path, read with cuobjdump; None without it"""
+    tool = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
+    if not shutil.which(tool):
+        return None
+    out = subprocess.run([tool, "-sass", str(lib_path)], capture_output=True, text=True, check=True).stdout
+    return re.findall(r"Function : (\S+)", out)

@@ -101,7 +101,7 @@ def test_multirise_order4_recovers_truth():
 
 
 def test_multirise_order3_larger_fista():
-    """C4-style (reduced): N=10 three-body model, order 3, F=46 base features -> Newton; and the FISTA
+    """C4-style (reduced): N=10 three-body model, order 3, F=56 base features -> Newton; and the FISTA
     backends agree with it."""
     n = 10
     terms = three_body_model(n, 30)
@@ -113,8 +113,9 @@ def test_multirise_order3_larger_fista():
 
 
 def test_multirise_c4_reduced_tensor_path():
-    """BASELINE config C4 reduced to N=12 (exactly samplable): order 3 -> 79 base features, beyond the Newton
-    solver's 64, so the auto solver takes the tensor-core FISTA path; checked against the oracle key by key."""
+    """BASELINE config C4 reduced to N=12 (exactly samplable): order 3 -> 79 base features (the subsets of size <= 2;
+    each node has 67 keys among them), beyond AUTO's Newton limit of 64, so the auto solver takes the tensor-core FISTA
+    path; checked against the oracle key by key."""
     n = 12
     terms = three_body_model(n, 30)
     hist = o.sample_exact(terms, n, 200_000, np.random.default_rng(32))

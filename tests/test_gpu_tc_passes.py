@@ -22,8 +22,6 @@ Histograms:
 import ctypes
 import functools
 import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
@@ -31,8 +29,8 @@ import pytest
 import c_oracle as c
 import gml_b200
 from gml_b200 import B200, RISE, RPLE, _lib, logRISE
-from helpers import (TC_F_REL, random_spins, tc_f_err, tc_grad_bar, tc_level_nr, tc_pass_terms,
-                     tc_residual_limbs)
+from helpers import (TC_F_REL, compiled_kernel_names, profiled_kernel_names, random_spins, tc_f_err, tc_grad_bar, tc_level_nr,
+                     tc_pass_terms, tc_residual_limbs)
 
 pytestmark = pytest.mark.gpu
 FORMS = {"RISE": RISE, "logRISE": logRISE, "RPLE": RPLE}
@@ -125,12 +123,8 @@ def tc_kernels(names):
 
 def profiled(fn):
     """fn()'s result and the tensor-core kernels it launched"""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = fn()
-        torch.cuda.synchronize()
-    return out, tc_kernels(ev.key for ev in prof.key_averages())
+    out, names = profiled_kernel_names(fn)
+    return out, tc_kernels(names)
 
 
 def expected_kernels(counts, n, level, form, want_grad, pair_allowed):
@@ -155,11 +149,8 @@ def use_kernel(monkeypatch, kernel):
 
 def compiled_kernels():
     """the tensor-core pass instantiations in the in-tree library, or None without cuobjdump"""
-    tool = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
-    if not shutil.which(tool):
-        return None
-    out = subprocess.run([tool, "-sass", str(_lib.LIB_PATH)], capture_output=True, text=True, check=True).stdout
-    return tc_kernels(re.findall(r"Function : (\S+)", out))
+    names = compiled_kernel_names(_lib.LIB_PATH)
+    return None if names is None else tc_kernels(names)
 
 
 # ------------------------------------------------------------------------------------------------
