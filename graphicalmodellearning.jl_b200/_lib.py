@@ -16,6 +16,7 @@ RISE_ID, LOGRISE_ID, RPLE_ID = 0, 1, 2
 EXACT_MAX_N = 40   # GML_B200_EXACT_MAX_N
 MCMC_MAX_N = 4096  # GML_B200_MCMC_MAX_N
 TEMPERING_DEFAULT_RUNGS = 16  # GML_B200_TEMPERING_DEFAULT_RUNGS
+LOG_Z_DEFAULT_RUNGS = 32  # GML_B200_LOG_Z_DEFAULT_RUNGS
 SOLVER_AUTO, SOLVER_NEWTON, SOLVER_FISTA_CC, SOLVER_FISTA_TC = 0, 1, 2, 3
 
 # every symbol include/gml_b200.h declares
@@ -29,7 +30,7 @@ EXPORTS = (
     "gml_b200_multibody_num_sym_keys", "gml_b200_threshold_device", "gml_b200_eval_pairwise", "gml_b200_bench_passes",
     "gml_b200_symmetrize_device",
     "gml_b200_sample_gibbs_device", "gml_b200_sample_gibbs_terms_device", "gml_b200_sample_exact_device",
-    "gml_b200_sample_mcmc_device", "gml_b200_sample_tempering_device",
+    "gml_b200_sample_mcmc_device", "gml_b200_sample_tempering_device", "gml_b200_log_partition_tempering",
     "gml_b200_build_histogram_device",
     "gml_b200_comm_unique_id", "gml_b200_comm_init", "gml_b200_comm_globalize_histogram", "gml_b200_comm_attach",
 )
@@ -126,6 +127,8 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     lib.gml_b200_sample_tempering_device.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, vp,
                                                      c.c_int64, c.c_int32, c.c_int64, c.c_int32, c.c_int32, c.c_uint64, vp, vp,
                                                      vp, vp, vp, c.c_int64, vp]
+    lib.gml_b200_log_partition_tempering.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, vp,
+                                                     c.c_int64, c.c_int32, c.c_int64, c.c_uint64, vp, vp, vp, vp, vp]
     lib.gml_b200_build_histogram_device.argtypes = [c.c_int32, vp, c.c_int64, c.c_int32, c.c_int64, vp, c.c_int64, vp,
                                                     c.POINTER(c.c_int64), vp]
     lib.gml_b200_comm_unique_id.argtypes = [vp]

@@ -516,6 +516,66 @@ def sample(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Op
     return (out, log_z) if return_log_z else out
 
 
+def log_partition(gm: FactorGraph, sampler: Optional[GMLSampler] = None, sweeps: int = 1000, return_info: bool = False):
+    """(log Z, stderr): the natural log of the partition function Z = sum_s exp(sum_t w_t prod s) of a spin model and its
+    standard error.  The held-out log-likelihood of a model is then the mean over rows of E(s) = sum_t w_t prod s, minus
+    log Z.
+
+    - None or B200Tempering: bridge sampling along a replica-exchange ladder that ends at beta = 0, where log Z = N log 2
+      (gml_b200_log_partition_tempering, N <= 4096, terms of order <= 8).  Uses the sampler's seed, device, chains (0 =
+      2^17 / R ladders), burn_in and betas (None = the log Z default: 32 rungs evenly spaced from 1 to 0; a given ladder
+      must end at 0); thin is ignored.  Each ladder runs burn_in + `sweeps` sweeps; the standard error is the delta-method
+      error over the independent ladders.  The estimate is of the model with fp32-rounded weights, which the chains sample:
+      it differs from log Z of the fp64 weights by at most sum_t |w_t - fl32(w_t)|.  The result depends only on (model,
+      betas, chains, burn_in, sweeps, seed).
+    - B200Exact: enumeration (N <= 40); stderr 0.0.
+    - return_info (B200Tempering) adds a dict: log_ratio and log_ratio_stderr (log Z_k - log Z_{k+1} per adjacent pair of
+      rungs and its standard error), swap_rate (per pair), betas, ladders and sweeps.  A ladder too coarse for the model
+      shows there as small swap rates and large per-pair errors.  With B200Exact the dict is empty."""
+    sampler = B200Tempering() if sampler is None else sampler
+    if isinstance(sampler, B200Gibbs):
+        raise ValueError("B200Gibbs has no temperature ladder to bridge: log_partition needs B200Tempering or B200Exact")
+    if not isinstance(sampler, (B200Exact, B200Tempering)):
+        raise TypeError("log_partition needs a B200Tempering or B200Exact sampler")
+    if gm.alphabet != "spin":
+        raise ValueError(f"log_partition is only supported for the spin alphabet, not {gm.alphabet!r}")
+    exact = isinstance(sampler, B200Exact)
+    N = int(gm.varible_count)
+    cap = _lib.EXACT_MAX_N if exact else _lib.MCMC_MAX_N
+    name = type(sampler).__name__
+    if not 1 <= N <= cap:
+        raise ValueError(f"log_partition with {name} supports 1 <= N <= {cap} spins, got {N}")
+    order, idx, wts = _term_arrays(gm)
+    lib = _lib.load()
+    seed = int(sampler.seed) & (2 ** 64 - 1)
+    log_z = ctypes.c_double(0.0)
+    if exact:
+        K = np.zeros(1, dtype=np.int64)
+        _lib.check(lib.gml_b200_sample_exact_device(int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts), 1, 1,
+                                                    seed, _ptr(K), ctypes.byref(log_z), None, None, 0, None))
+        return (log_z.value, 0.0, {}) if return_info else (log_z.value, 0.0)
+    betas = _ladder(sampler)
+    if len(betas) and betas[-1] != 0.0:
+        raise ValueError("log_partition needs a ladder whose last rung is beta = 0")
+    sweeps = int(sweeps)
+    if sweeps < 1 or sampler.chains < 0 or sampler.chains == 1 or sampler.burn_in < 0:
+        raise ValueError("log_partition needs sweeps >= 1, burn_in >= 0 and chains = 0 or >= 2 (the standard error is "
+                         "taken over the ladders)")
+    R = len(betas) or _lib.LOG_Z_DEFAULT_RUNGS
+    stderr = ctypes.c_double(0.0)
+    ratio, swap = np.zeros((R - 1, 2)), np.zeros(R - 1)
+    _lib.check(lib.gml_b200_log_partition_tempering(int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts),
+                                                    len(betas), _ptr(betas) if len(betas) else None, int(sampler.chains),
+                                                    int(sampler.burn_in), sweeps, seed, ctypes.byref(log_z),
+                                                    ctypes.byref(stderr), _ptr(ratio), _ptr(swap), None))
+    if not return_info:
+        return log_z.value, stderr.value
+    info = {"log_ratio": ratio[:, 0].tolist(), "log_ratio_stderr": ratio[:, 1].tolist(), "swap_rate": swap.tolist(),
+            "betas": betas.tolist() if len(betas) else [1.0 - k / (R - 1) for k in range(R)],
+            "ladders": int(sampler.chains) or (1 << 17) // R, "sweeps": sweeps}
+    return log_z.value, stderr.value, info
+
+
 class Session:
     """Handle API (include/gml_b200.h): keeps the histogram resident in HBM across calls."""
 

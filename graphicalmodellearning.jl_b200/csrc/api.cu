@@ -247,15 +247,51 @@ template <class Fill> void into_sample_buffers(double* d_counts, int8_t* d_spins
     }
 }
 
+// A term list of the MCMC entry points, checked, with its incidence lists
+struct McmcModel {
+    std::vector<int32_t> idx;
+    std::vector<double> weights;
+    Incidence inc;
+};
+
+McmcModel mcmc_model(int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx, const double* term_weight) {
+    GML_REQUIRE(N >= 1 && N <= GML_B200_MCMC_MAX_N, "MCMC sampler needs 1 <= N <= " + std::to_string(GML_B200_MCMC_MAX_N));
+    GML_REQUIRE(order >= 1 && order <= 8 && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)),
+                "bad sampler argument");
+    McmcModel m;
+    m.idx.assign(term_idx, term_idx + (size_t)n_terms * order);
+    m.weights.assign(term_weight, term_weight + n_terms);
+    for (int t = 0; t < n_terms; ++t) {
+        for (int k = 0; k < order; ++k) GML_REQUIRE(m.idx[(size_t)t * order + k] >= -1, "sampler term refers to a spin outside [0, N)");
+        GML_REQUIRE(std::isfinite(m.weights[t]), "sampler term weight is not finite");
+    }
+    m.inc = build_incidence(N, order, n_terms, m.idx.data());
+    return m;
+}
+
+// The ladder of a replica-exchange entry point: n_rungs = 0 with betas = NULL selects `fallback` (the entry point's
+// default); otherwise 2, 4, 8, 16 or 32 betas from 1, strictly decreasing, finite and non-negative.
+std::vector<double> tempering_ladder(int32_t n_rungs, const double* betas, std::vector<double> fallback) {
+    GML_REQUIRE(n_rungs == 0 || n_rungs == 2 || n_rungs == 4 || n_rungs == 8 || n_rungs == 16 || n_rungs == 32,
+                "n_rungs must be 0 (the default ladder) or one of 2, 4, 8, 16, 32");
+    GML_REQUIRE((n_rungs == 0) == (betas == nullptr), "n_rungs = 0 goes with betas = NULL (the default ladder) and only with it");
+    if (n_rungs == 0) return fallback;
+    std::vector<double> ladder(betas, betas + n_rungs);
+    GML_REQUIRE(ladder[0] == 1.0, "betas[0] must be 1 (the rung that records)");
+    for (int k = 1; k < n_rungs; ++k)
+        GML_REQUIRE(std::isfinite(ladder[k]) && ladder[k] >= 0.0 && ladder[k] < ladder[k - 1],
+                    "betas must be finite, non-negative and strictly decreasing");
+    return ladder;
+}
+
 // The MCMC entry points (betas = {1}: gml_b200_sample_mcmc_device; R > 1 rungs: gml_b200_sample_tempering_device, whose
 // ladder the caller has checked): argument checks, then the sampler into the caller's buffers.
 void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx, const double* term_weight,
               const std::vector<double>& betas, int64_t n_samples, int32_t replicates, int64_t chains, int32_t burn_in,
               int32_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate, double* d_counts,
               int8_t* d_spins, int64_t ld, void* stream) {
-    GML_REQUIRE(N >= 1 && N <= GML_B200_MCMC_MAX_N, "MCMC sampler needs 1 <= N <= " + std::to_string(GML_B200_MCMC_MAX_N));
-    GML_REQUIRE(order >= 1 && order <= 8 && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)) && out_K,
-                "bad sampler argument");
+    const McmcModel m = mcmc_model(N, order, n_terms, term_idx, term_weight);
+    GML_REQUIRE(out_K, "bad sampler argument");
     GML_REQUIRE(n_samples >= 1 && replicates >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1,
                 "bad sampler sizes");
     GML_REQUIRE(N > 64 || n_samples < (INT64_C(1) << 31), "the histogram of N <= 64 spins takes fewer than 2^31 draws per replicate");
@@ -264,13 +300,6 @@ void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const i
     if (chains == 0) chains = mcmc_auto_chains(n_samples, rungs);
     const double steps = ((double)burn_in + (double)thin * (double)ceil_div(n_samples, chains)) * N;
     GML_REQUIRE(steps * replicates < 0x1.0p62, "too many sweeps");
-    std::vector<int32_t> idx(term_idx, term_idx + (size_t)n_terms * order);
-    std::vector<double> weights(term_weight, term_weight + n_terms);
-    for (int t = 0; t < n_terms; ++t) {
-        for (int m = 0; m < order; ++m) GML_REQUIRE(idx[(size_t)t * order + m] >= -1, "sampler term refers to a spin outside [0, N)");
-        GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
-    }
-    const Incidence inc = build_incidence(N, order, n_terms, idx.data());
     if (N > 64 && d_counts && ld < n_samples * replicates) {
         for (int r = 0; r < replicates; ++r) out_K[r] = n_samples;
         GML_REQUIRE(false, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(n_samples * replicates) +
@@ -279,8 +308,8 @@ void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const i
     GML_CUDA(cudaSetDevice(device));
     cudaStream_t st = (cudaStream_t)stream;
     into_sample_buffers(d_counts, d_spins, ld, N, replicates, out_K, st, [&](double* c, int8_t* sp) {
-        sample_mcmc(N, order, idx, weights, inc, betas, n_samples, replicates, chains, burn_in, thin, seed, out_K, out_rhat,
-                    out_swap_rate, c, sp, ld, st);
+        sample_mcmc(N, order, m.idx, m.weights, m.inc, betas, n_samples, replicates, chains, burn_in, thin, seed, out_K,
+                    out_rhat, out_swap_rate, c, sp, ld, st);
     });
 }
 
@@ -1256,22 +1285,34 @@ int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, i
                                      int64_t* out_K, double* out_rhat, double* out_swap_rate, double* d_counts, int8_t* d_spins,
                                      int64_t ld, void* stream) {
     return guarded([&] {
-        GML_REQUIRE(n_rungs == 0 || n_rungs == 2 || n_rungs == 4 || n_rungs == 8 || n_rungs == 16 || n_rungs == 32,
-                    "n_rungs must be 0 (the default ladder) or one of 2, 4, 8, 16, 32");
-        GML_REQUIRE((n_rungs == 0) == (betas == nullptr), "n_rungs = 0 goes with betas = NULL (the default ladder) and only with it");
-        std::vector<double> ladder;
-        if (n_rungs == 0) {                          // the default ladder: geometric from 1 to 0.1
-            constexpr int R = GML_B200_TEMPERING_DEFAULT_RUNGS;
-            for (int k = 0; k < R; ++k) ladder.push_back(std::pow(0.1, (double)k / (R - 1)));
-        } else {
-            ladder.assign(betas, betas + n_rungs);
-            GML_REQUIRE(ladder[0] == 1.0, "betas[0] must be 1 (the rung that records)");
-            for (int k = 1; k < n_rungs; ++k)
-                GML_REQUIRE(std::isfinite(ladder[k]) && ladder[k] >= 0.0 && ladder[k] < ladder[k - 1],
-                            "betas must be finite, non-negative and strictly decreasing");
-        }
+        std::vector<double> fallback;               // the default ladder: geometric from 1 to 0.1
+        constexpr int R = GML_B200_TEMPERING_DEFAULT_RUNGS;
+        for (int k = 0; k < R; ++k) fallback.push_back(std::pow(0.1, (double)k / (R - 1)));
+        const std::vector<double> ladder = tempering_ladder(n_rungs, betas, fallback);
         run_mcmc(device, N, order, n_terms, term_idx, term_weight, ladder, n_samples, replicates, chains, burn_in, thin, seed,
                  out_K, out_rhat, out_swap_rate, d_counts, d_spins, ld, stream);
+    });
+}
+
+int gml_b200_log_partition_tempering(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                     const double* term_weight, int32_t n_rungs, const double* betas, int64_t chains,
+                                     int32_t burn_in, int64_t sweeps, uint64_t seed, double* out_log_z, double* out_stderr,
+                                     double* out_log_ratio, double* out_swap_rate, void* stream) {
+    return guarded([&] {
+        std::vector<double> fallback;               // the default ladder: evenly spaced from 1 to 0
+        constexpr int R = GML_B200_LOG_Z_DEFAULT_RUNGS;
+        for (int k = 0; k < R; ++k) fallback.push_back(1.0 - (double)k / (R - 1));
+        const std::vector<double> ladder = tempering_ladder(n_rungs, betas, fallback);
+        GML_REQUIRE(ladder.back() == 0.0, "the last rung of a log Z ladder must be beta = 0");
+        const McmcModel m = mcmc_model(N, order, n_terms, term_idx, term_weight);
+        GML_REQUIRE(out_log_z, "null out_log_z");
+        GML_REQUIRE(chains >= 0 && chains != 1 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && sweeps >= 1,
+                    "bad log Z sizes (chains = 1 leaves no standard error)");
+        GML_REQUIRE(((double)burn_in + (double)sweeps) * N < 0x1.0p62, "too many sweeps");
+        if (chains == 0) chains = MCMC_AUTO_CHAINS / (int64_t)ladder.size();
+        GML_CUDA(cudaSetDevice(device));
+        log_partition_tempering(N, order, m.idx, m.weights, m.inc, ladder, chains, burn_in, sweeps, seed, out_log_z, out_stderr,
+                                out_log_ratio, out_swap_rate, (cudaStream_t)stream);
     });
 }
 

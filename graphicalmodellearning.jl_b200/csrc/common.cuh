@@ -258,6 +258,13 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
                  const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int replicates, int64_t chains,
                  int64_t burn_in, int64_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate,
                  double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st);
+// log Z of the model by bridge sampling along a replica-exchange ladder betas[0] = 1 > ... > betas[R-1] = 0 (R > 1):
+// `chains` ladders, burn_in sweeps, then `sweeps` sweeps that feed the bridge sums; fills *out_log_z and the nullable
+// out_stderr, out_log_ratio [R-1][2] (estimate, stderr of log Z_k - log Z_{k+1}) and out_swap_rate [R-1].  chains >= 2.
+void log_partition_tempering(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                             const Incidence& inc, const std::vector<double>& betas, int64_t chains, int64_t burn_in,
+                             int64_t sweeps, uint64_t seed, double* out_log_z, double* out_stderr, double* out_log_ratio,
+                             double* out_swap_rate, cudaStream_t st);
 
 // --- exact_sampler.cu : iid draws from the exact distribution by enumeration (term t = spins of masks[t]); fills
 // out_K[replicates] and, when d_counts is set, the histograms at consecutive rows; returns log Z.  N <= GML_B200_EXACT_MAX_N.

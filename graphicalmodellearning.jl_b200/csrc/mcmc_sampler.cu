@@ -23,6 +23,11 @@
 //     k = sw (mod 2) are proposed (deterministic even-odd scheme) and accepted with probability
 //     min(1, exp((beta_k - beta_{k+1}) (E_{k+1} - E_k))), E from an fp64 term-list pass after every sweep.  Only the lane
 //     at rung 0 (beta = 1) records: draw d = r * ladders + ladder.  Order within a sweep: sweep, record, swap.
+//   - Partition function (R > 1, BRIDGE, log_partition(gm, B200Tempering())): on every sweep after burn_in,
+//     before the swap, the lane at slot k < R-1 adds x = +dbeta_k E_{k+1} / 2 and y = -dbeta_k E_k / 2 (dbeta_k = beta_k -
+//     beta_{k+1}) to two running log-sum-exps (running maximum, so nothing overflows) and finally writes their log-means:
+//     the two halves of the geometric bridge log Z_k - log Z_{k+1} = log E_{k+1}[e^x] - log E_k[e^y] (Meng & Wong 1996).
+//     The RNG streams and the swap decisions are those of the sampler.
 #include <cmath>
 #include <type_traits>
 
@@ -74,6 +79,7 @@ struct McmcParams {
                                // squares and of the half-chain variances over the warp's chains
     unsigned long long* swap_acc;   // R > 1: [warps x (R-1)] swaps of pair (k, k+1) accepted after burn_in
     double beta[TEMPERING_MAX_RUNGS];  // R > 1: inverse temperature of each rung, beta[0] = 1
+    double* bridge;            // BRIDGE: [chains x (R-1) x 2] per ladder and pair k the log-means of e^x and e^y
 };
 
 // parity (1 = odd) of the down spins of lane `lane` among the members m of a list (entries < 0 are padding)
@@ -115,14 +121,24 @@ __device__ __forceinline__ T term_energy(const uint32_t* __restrict__ s, const M
     return energy;
 }
 
+// adds x to the running log-sum-exp  m + log(sum).  One exp on either side of the maximum (m = -inf: e = 0), in fp32:
+// e is in (0, 1], its relative error ~1e-7 moves the log-sum by as little, and an fp64 exp's constants would take the
+// registers of the sweep loop.
+__device__ __forceinline__ void log_sum_exp_add(double x, double& m, double& sum) {
+    const double e = expf((float)-fabs(x - m));
+    sum = x > m ? fma(sum, e, 1.0) : sum + e;
+    m = fmax(m, x);
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
     return v;
 }
 
-// R = 1: multi-sample Gibbs, one chain per lane.  R > 1: one ladder of R rungs per R consecutive lanes (see the top).
-template <bool KEYS, int R>
+// R = 1: multi-sample Gibbs, one chain per lane.  R > 1: one ladder of R rungs per R consecutive lanes (see the top);
+// BRIDGE adds the sums of the log Z estimator (a separate instantiation: the sampler's registers stay as they are).
+template <bool KEYS, int R, bool BRIDGE = false>
 __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
     using Energy = typename std::conditional<R == 1, float, double>::type;
     constexpr int LADDERS = 32 / R;                           // ladders (chains) per warp
@@ -142,6 +158,7 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
     float beta = 1.f;
     uint64_t ladder_key = 0;
     unsigned long long n_acc = 0;                             // accepted swaps of pair (slot, slot + 1) after burn_in
+    double a_max = -INFINITY, a_sum = 0, b_max = -INFINITY, b_sum = 0;   // the bridge sums of pair (slot, slot + 1)
     if constexpr (R > 1) {
         ladder_key = __shfl_sync(FULL, (unsigned long long)key, 0, R);
         beta = (float)p.beta[slot];
@@ -214,6 +231,11 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
             const double e_k = __shfl_sync(FULL, energy_now, who, R);
             const double e_k1 = __shfl_down_sync(FULL, e_k, 1, R);
             const int who_up = __shfl_down_sync(FULL, who, 1, R), who_down = __shfl_up_sync(FULL, who, 1, R);
+            if (BRIDGE && sw > p.burn_in && slot + 1 < R) {
+                const double half = 0.5 * (p.beta[slot] - p.beta[slot + 1]);
+                log_sum_exp_add(half * e_k1, a_max, a_sum);
+                log_sum_exp_add(-half * e_k, b_max, b_sum);
+            }
             bool acc = false;
             if (((slot ^ (int)sw) & 1) == 0 && slot + 1 < R) {
                 const double x = (p.beta[slot] - p.beta[slot + 1]) * (e_k1 - e_k);
@@ -233,6 +255,12 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
 #pragma unroll
         for (int o = R; o < 32; o <<= 1) n_acc += __shfl_xor_sync(FULL, n_acc, o);
         if (lane < R - 1) p.swap_acc[warp * (R - 1) + lane] = n_acc;
+        if (BRIDGE && live && slot + 1 < R) {               // log-means over the records * thin sweeps after burn_in
+            const double log_s = log((double)(p.records * p.thin));
+            double* o = p.bridge + (c * (R - 1) + slot) * 2;
+            o[0] = a_max + log(a_sum) - log_s;
+            o[1] = b_max + log(b_sum) - log_s;
+        }
     }
     if (h < 2) return;
     double em = 0, em2 = 0, ev = 0, mm = 0, mm2 = 0, mv = 0;
@@ -280,6 +308,60 @@ template <bool KEYS> void (*ladder_kernel(int rungs))(McmcParams) {
         default: return mcmc_kernel<KEYS, 32>;
     }
 }
+
+void (*bridge_kernel(int rungs))(McmcParams) {
+    switch (rungs) {
+        case 2: return mcmc_kernel<false, 2, true>;
+        case 4: return mcmc_kernel<false, 4, true>;
+        case 8: return mcmc_kernel<false, 8, true>;
+        case 16: return mcmc_kernel<false, 16, true>;
+        default: return mcmc_kernel<false, 32, true>;
+    }
+}
+
+// A model on the device for mcmc_kernel: the incidence lists and the term list with weights rounded once to fp32, and the
+// parameters that describe the model and the ladder.  The caller fills in the run.
+struct DeviceModel {
+    DevBuf<int32_t> rp, ot, ti;
+    DevBuf<float> ww, tw;
+    std::vector<float> w32, inc_w;                    // the host sources of the fp32 weights
+    McmcParams p{};
+
+    DeviceModel(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                const Incidence& inc, const std::vector<double>& betas, cudaStream_t st)
+        : w32(term_weight.begin(), term_weight.end()), inc_w(inc.term.size()) {
+        const int n_terms = (int)term_weight.size();
+        for (size_t q = 0; q < inc.term.size(); ++q) inc_w[q] = inc.term[q] >= 0 ? (float)term_weight[inc.term[q]] : 0.f;
+        rp.alloc(inc.row_ptr.size()); ot.alloc(inc.others.size()); ww.alloc(inc_w.size());
+        ti.alloc(std::max<size_t>(term_idx.size(), 1)); tw.alloc(std::max<size_t>(w32.size(), 1));
+        GML_CUDA(cudaMemcpyAsync(rp.p, inc.row_ptr.data(), sizeof(int32_t) * inc.row_ptr.size(), cudaMemcpyHostToDevice, st));
+        GML_CUDA(cudaMemcpyAsync(ot.p, inc.others.data(), sizeof(int32_t) * inc.others.size(), cudaMemcpyHostToDevice, st));
+        GML_CUDA(cudaMemcpyAsync(ww.p, inc_w.data(), sizeof(float) * inc_w.size(), cudaMemcpyHostToDevice, st));
+        if (n_terms) {
+            GML_CUDA(cudaMemcpyAsync(ti.p, term_idx.data(), sizeof(int32_t) * term_idx.size(), cudaMemcpyHostToDevice, st));
+            GML_CUDA(cudaMemcpyAsync(tw.p, w32.data(), sizeof(float) * n_terms, cudaMemcpyHostToDevice, st));
+        }
+        p.N = N; p.order = order; p.width = inc.width; p.n_terms = n_terms;
+        p.row_ptr = rp.p; p.others = ot.p; p.weight = ww.p; p.term_idx = ti.p; p.term_w = tw.p;
+        for (size_t k = 0; k < betas.size(); ++k) p.beta[k] = betas[k];
+    }
+};
+
+// per adjacent pair, accepted / proposed swaps after burn_in from the per-warp counts of swap_acc
+void swap_rates(const unsigned long long* swap_acc, int64_t warps, int rungs, int64_t chains, int64_t burn_in, int64_t sweeps,
+                double* out, cudaStream_t st) {
+    std::vector<unsigned long long> accepted(warps * (rungs - 1));
+    GML_CUDA(cudaMemcpyAsync(accepted.data(), swap_acc, sizeof(unsigned long long) * accepted.size(), cudaMemcpyDeviceToHost, st));
+    GML_CUDA(cudaStreamSynchronize(st));
+    auto with_parity = [](int64_t x, int par) { return par ? (x + 1) / 2 : x / 2; };   // sw in [1, x] with sw = par (mod 2)
+    for (int k = 0; k + 1 < rungs; ++k) {
+        unsigned long long a = 0;
+        for (int64_t w = 0; w < warps; ++w) a += accepted[w * (rungs - 1) + k];
+        // the sweeps sw in (burn_in, sweeps] with sw = k (mod 2) propose pair k in every ladder
+        const int64_t proposals = with_parity(sweeps, k % 2) - with_parity(burn_in, k % 2);
+        out[k] = proposals > 0 ? (double)a / ((double)proposals * chains) : NAN;
+    }
+}
 }  // namespace
 
 void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
@@ -287,47 +369,28 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
                  int64_t burn_in, int64_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate,
                  double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st) {
     const bool keys_path = N <= 64;
-    const int n_terms = (int)term_weight.size();
     const int rungs = (int)betas.size();
     const int64_t warps = ceil_div(chains, 32 / rungs), blocks = ceil_div(warps, WARPS);
     const size_t smem = sizeof(uint32_t) * (size_t)N * WARPS;
-    std::vector<float> w32(term_weight.begin(), term_weight.end());
-    std::vector<float> inc_w(inc.term.size());
-    for (size_t q = 0; q < inc.term.size(); ++q) inc_w[q] = inc.term[q] >= 0 ? (float)term_weight[inc.term[q]] : 0.f;
 
-    DevBuf<int32_t> rp, ot, ti;
-    DevBuf<float> ww, tw;
+    DeviceModel model(N, order, term_idx, term_weight, inc, betas, st);
     DevBuf<double> wstats;
     DevBuf<unsigned long long> keys, swaps;
-    rp.alloc(inc.row_ptr.size()); ot.alloc(inc.others.size()); ww.alloc(inc_w.size());
-    ti.alloc(std::max<size_t>(term_idx.size(), 1)); tw.alloc(std::max<size_t>(w32.size(), 1));
     wstats.alloc(warps * 6);
     if (rungs > 1) swaps.alloc(warps * (rungs - 1));
     if (keys_path) keys.alloc(n_samples);
-    GML_CUDA(cudaMemcpyAsync(rp.p, inc.row_ptr.data(), sizeof(int32_t) * inc.row_ptr.size(), cudaMemcpyHostToDevice, st));
-    GML_CUDA(cudaMemcpyAsync(ot.p, inc.others.data(), sizeof(int32_t) * inc.others.size(), cudaMemcpyHostToDevice, st));
-    GML_CUDA(cudaMemcpyAsync(ww.p, inc_w.data(), sizeof(float) * inc_w.size(), cudaMemcpyHostToDevice, st));
-    if (n_terms) {
-        GML_CUDA(cudaMemcpyAsync(ti.p, term_idx.data(), sizeof(int32_t) * term_idx.size(), cudaMemcpyHostToDevice, st));
-        GML_CUDA(cudaMemcpyAsync(tw.p, w32.data(), sizeof(float) * n_terms, cudaMemcpyHostToDevice, st));
-    }
     auto kernel = keys_path ? ladder_kernel<true>(rungs) : ladder_kernel<false>(rungs);
     GML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
-    McmcParams p{};
-    p.N = N; p.order = order; p.width = inc.width; p.n_terms = n_terms;
-    p.row_ptr = rp.p; p.others = ot.p; p.weight = ww.p; p.term_idx = ti.p; p.term_w = tw.p;
+    McmcParams& p = model.p;
     p.chains = chains; p.n = n_samples; p.burn_in = burn_in; p.thin = thin;
     p.records = ceil_div(n_samples, chains); p.full_records = n_samples / chains;
     p.seed = seed; p.keys = keys.p; p.warp_stats = wstats.p; p.swap_acc = swaps.p;
-    for (int k = 0; k < rungs; ++k) p.beta[k] = betas[k];
     const int64_t h = p.full_records / 2;
     p.inv_h = 1.0 / (double)h;
     p.inv_h1 = 1.0 / (double)(h - 1);
     const int64_t sweeps = burn_in + p.records * thin;
     std::vector<double> hs(warps * 6);
-    std::vector<unsigned long long> accepted(rungs > 1 ? warps * (rungs - 1) : 0);
-    auto with_parity = [](int64_t x, int par) { return par ? (x + 1) / 2 : x / 2; };   // sw in [1, x] with sw = par (mod 2)
     int64_t rows = 0;
     bool fits = true;
     for (int rep = 0; rep < replicates; ++rep) {
@@ -362,22 +425,71 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
                 rh[1] = split_rhat(acc[3], acc[4], acc[5], 2.0 * chains, (double)h);
             }
         }
-        if (out_swap_rate && rungs > 1) {                    // accepted / proposed swaps after burn_in, per pair
-            GML_CUDA(cudaMemcpyAsync(accepted.data(), swaps.p, sizeof(unsigned long long) * accepted.size(), cudaMemcpyDeviceToHost,
-                                     st));
-            GML_CUDA(cudaStreamSynchronize(st));
-            for (int k = 0; k + 1 < rungs; ++k) {
-                unsigned long long a = 0;
-                for (int64_t w = 0; w < warps; ++w) a += accepted[w * (rungs - 1) + k];
-                // the sweeps sw in (burn_in, sweeps] with sw = k (mod 2) propose pair k in every ladder
-                const int64_t proposals = with_parity(sweeps, k % 2) - with_parity(burn_in, k % 2);
-                out_swap_rate[(size_t)rep * (rungs - 1) + k] = proposals > 0 ? (double)a / ((double)proposals * chains) : NAN;
-            }
-        }
+        if (out_swap_rate && rungs > 1)
+            swap_rates(swaps.p, warps, rungs, chains, burn_in, sweeps, out_swap_rate + (size_t)rep * (rungs - 1), st);
     }
     GML_CUDA(cudaStreamSynchronize(st));
     GML_REQUIRE(!d_counts || fits, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(rows) +
                                    " rows of the replicates (out_K holds their sizes)");
+}
+
+void log_partition_tempering(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                             const Incidence& inc, const std::vector<double>& betas, int64_t chains, int64_t burn_in,
+                             int64_t sweeps, uint64_t seed, double* out_log_z, double* out_stderr, double* out_log_ratio,
+                             double* out_swap_rate, cudaStream_t st) {
+    const int rungs = (int)betas.size(), pairs = rungs - 1;
+    const int64_t warps = ceil_div(chains, 32 / rungs), blocks = ceil_div(warps, WARPS);
+    const size_t smem = sizeof(uint32_t) * (size_t)N * WARPS;
+
+    DeviceModel model(N, order, term_idx, term_weight, inc, betas, st);
+    DevBuf<double> wstats, bridge;
+    DevBuf<unsigned long long> swaps;
+    wstats.alloc(warps * 6);
+    swaps.alloc(warps * pairs);
+    bridge.alloc(chains * pairs * 2);
+    auto kernel = bridge_kernel(rungs);
+    GML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+
+    McmcParams& p = model.p;                          // no draws: every sweep after burn_in feeds the bridge sums
+    p.chains = chains; p.chain0 = 0; p.n = 0; p.burn_in = burn_in; p.thin = 1; p.records = sweeps; p.full_records = 0;
+    p.seed = seed; p.warp_stats = wstats.p; p.swap_acc = swaps.p; p.bridge = bridge.p;
+    kernel<<<(unsigned)blocks, WARPS * 32, smem, st>>>(p);
+    GML_LAUNCHED();
+    std::vector<double> ab(chains * pairs * 2);
+    GML_CUDA(cudaMemcpyAsync(ab.data(), bridge.p, sizeof(double) * ab.size(), cudaMemcpyDeviceToHost, st));
+    GML_CUDA(cudaStreamSynchronize(st));
+    if (out_swap_rate) swap_rates(swaps.p, warps, rungs, chains, burn_in, burn_in + sweeps, out_swap_rate, st);
+
+    // Over the L ladders, in ladder order: mean_k = logsumexp_c v_{c,k} - log L for v = a, b; log Z_k - log Z_{k+1} =
+    // mean_a - mean_b.  Delta method: u_{c,k} = e^{a_{c,k} - mean_a} - e^{b_{c,k} - mean_b}, stderr = std_c(u) / sqrt(L).
+    const double L = (double)chains, log_L = std::log(L);
+    std::vector<double> mean(pairs * 2), u_total(chains, 0.0), u(chains);
+    auto at = [&](int64_t c, int k, int ab_) { return ab[(c * pairs + k) * 2 + ab_]; };
+    auto stderr_of = [&](const std::vector<double>& x) {
+        double m = 0, q = 0;
+        for (double v : x) m += v;
+        m /= L;
+        for (double v : x) q += (v - m) * (v - m);
+        return std::sqrt(q / (L - 1.0) / L);
+    };
+    double log_z = N * std::log(2.0);
+    for (int k = 0; k < pairs; ++k) {
+        for (int h = 0; h < 2; ++h) {
+            double mx = -INFINITY, sum = 0;
+            for (int64_t c = 0; c < chains; ++c) mx = std::max(mx, at(c, k, h));
+            for (int64_t c = 0; c < chains; ++c) sum += std::exp(at(c, k, h) - mx);
+            mean[k * 2 + h] = mx + std::log(sum) - log_L;
+        }
+        for (int64_t c = 0; c < chains; ++c) {
+            u[c] = std::exp(at(c, k, 0) - mean[k * 2]) - std::exp(at(c, k, 1) - mean[k * 2 + 1]);
+            u_total[c] += u[c];
+        }
+        const double ratio = mean[k * 2] - mean[k * 2 + 1];
+        log_z += ratio;
+        if (out_log_ratio) { out_log_ratio[k * 2] = ratio; out_log_ratio[k * 2 + 1] = stderr_of(u); }
+    }
+    *out_log_z = log_z;
+    if (out_stderr) *out_stderr = stderr_of(u_total);
 }
 
 }  // namespace gml

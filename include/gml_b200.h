@@ -306,6 +306,37 @@ int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, i
                                      double* out_swap_rate /* nullable [replicates][n_rungs - 1] */, double* d_counts,
                                      int8_t* d_spins, int64_t ld, void* stream);
 
+/* Partition function by replica exchange: *out_log_z = log Z, Z = sum_s exp(sum_t w_t prod s), for the models of
+ * gml_b200_sample_tempering_device (N <= 4096, order <= 8) by bridge sampling between the adjacent rungs of ladders
+ * betas[0] = 1 > betas[1] > ... > betas[R-1] = 0; log Z(0) = N log 2 ties the chain of ratios to a known value.
+ *   - Each of `chains` ladders runs the replica-exchange kernel of gml_b200_sample_tempering_device (the same RNG streams
+ *     and swaps, no draws) for burn_in + sweeps sweeps.  On each of the last `sweeps` sweeps, before the swap, pair k
+ *     (dbeta_k = beta_k - beta_{k+1}) adds the fp64 energies E_{k+1} of rung k+1 and E_k of rung k to
+ *     a_{c,k} = log mean exp(+dbeta_k E_{k+1} / 2) and b_{c,k} = log mean exp(-dbeta_k E_k / 2) (running log-sum-exps).
+ *     Over the L ladders a_k = logsumexp_c a_{c,k} - log L, b_k likewise, and the geometric bridge (Meng & Wong 1996) gives
+ *     log Z_k - log Z_{k+1} = a_k - b_k and log Z = N log 2 + sum_k (a_k - b_k).
+ *   - *out_stderr (nullable): the delta-method standard error over the independent ladders, std_c(sum_k u_{c,k}) / sqrt(L)
+ *     with ddof = 1, u_{c,k} = exp(a_{c,k} - a_k) - exp(b_{c,k} - b_k).  out_log_ratio (nullable) [n_rungs-1][2]: per pair
+ *     the estimate a_k - b_k and its standard error (the same formula without the sum over k); the estimates sum to
+ *     log Z - N log 2.  out_swap_rate (nullable) [n_rungs-1]: the swap rates as gml_b200_sample_tempering_device.  The
+ *     reduction runs in ladder order: the result depends only on (terms, betas, chains, burn_in, sweeps, seed).
+ *   - n_rungs = 0 with betas = NULL selects GML_B200_LOG_Z_DEFAULT_RUNGS rungs evenly spaced, beta_k = 1 - k/31.
+ *     chains = 0 picks 2^17 / R ladders (4096 for 32 rungs).  Cost ~ chains * R * (burn_in + sweeps) site updates.
+ *   - Accuracy: the estimate is of the model with fp32-rounded weights, the model the chains sample; |log Z(w) -
+ *     log Z(fl32(w))| <= sum_t |w_t - fl32(w_t)|.  Each bridge is accurate while dbeta_k * (spread of E at rungs k, k+1)
+ *     stays of order 1; a ladder too coarse for the model shows as small swap rates and large per-pair standard errors,
+ *     and nothing is clamped.  At most 32 rungs.
+ *   - GML_B200_EINVAL: everything gml_b200_sample_tempering_device refuses that applies here (N, order, terms, weights,
+ *     the ladder), betas[n_rungs-1] != 0, chains < 0, chains == 1 (no standard error), burn_in < 0, sweeps < 1,
+ *     out_log_z == NULL, or (burn_in + sweeps) * N >= 2^62 site steps. */
+#define GML_B200_LOG_Z_DEFAULT_RUNGS 32
+int gml_b200_log_partition_tempering(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                     const double* term_weight, int32_t n_rungs, const double* betas /* [n_rungs] */,
+                                     int64_t chains, int32_t burn_in, int64_t sweeps, uint64_t seed, double* out_log_z,
+                                     double* out_stderr /* nullable */,
+                                     double* out_log_ratio /* nullable [n_rungs-1][2]: estimate, stderr */,
+                                     double* out_swap_rate /* nullable [n_rungs-1] */, void* stream);
+
 /* ---- sample-sharded mode (SURVEY 8e): histogram rows split over ranks, every rank solves all nodes; per pass
  * the int64 gradient sums and fp64 objective sums are combined with NCCL all-reduces on the solve stream.
  *   rank 0: gml_b200_comm_unique_id(id) -> broadcast the 128 bytes with any transport -> every rank:
