@@ -17,6 +17,7 @@ EXACT_MAX_N = 40   # GML_B200_EXACT_MAX_N
 MCMC_MAX_N = 4096  # GML_B200_MCMC_MAX_N
 TEMPERING_DEFAULT_RUNGS = 16  # GML_B200_TEMPERING_DEFAULT_RUNGS
 LOG_Z_DEFAULT_RUNGS = 32  # GML_B200_LOG_Z_DEFAULT_RUNGS
+KEYS_PAIRWISE = -1  # GML_B200_KEYS_PAIRWISE
 SOLVER_AUTO, SOLVER_NEWTON, SOLVER_FISTA_CC, SOLVER_FISTA_TC = 0, 1, 2, 3
 
 # every symbol include/gml_b200.h declares
@@ -31,6 +32,7 @@ EXPORTS = (
     "gml_b200_symmetrize_device",
     "gml_b200_sample_gibbs_device", "gml_b200_sample_gibbs_terms_device", "gml_b200_sample_exact_device",
     "gml_b200_sample_mcmc_device", "gml_b200_sample_tempering_device", "gml_b200_log_partition_tempering",
+    "gml_b200_moments_mcmc", "gml_b200_moments_exact", "gml_b200_moments_histogram",
     "gml_b200_build_histogram_device",
     "gml_b200_comm_unique_id", "gml_b200_comm_init", "gml_b200_comm_globalize_histogram", "gml_b200_comm_attach",
 )
@@ -129,6 +131,10 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
                                                      vp, vp, vp, c.c_int64, vp]
     lib.gml_b200_log_partition_tempering.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, vp,
                                                      c.c_int64, c.c_int32, c.c_int64, c.c_uint64, vp, vp, vp, vp, vp]
+    lib.gml_b200_moments_mcmc.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, vp, c.c_int64, c.c_int64,
+                                          c.c_int32, c.c_int32, c.c_uint64, c.c_int32, c.c_int32, vp, vp, vp, vp, vp, vp]
+    lib.gml_b200_moments_exact.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, c.c_int32, vp, vp, vp]
+    lib.gml_b200_moments_histogram.argtypes = [vp, c.c_int32, c.c_int32, vp, vp]
     lib.gml_b200_build_histogram_device.argtypes = [c.c_int32, vp, c.c_int64, c.c_int32, c.c_int64, vp, c.c_int64, vp,
                                                     c.POINTER(c.c_int64), vp]
     lib.gml_b200_comm_unique_id.argtypes = [vp]

@@ -576,6 +576,129 @@ def log_partition(gm: FactorGraph, sampler: Optional[GMLSampler] = None, sweeps:
     return log_z.value, stderr.value, info
 
 
+def _key_arrays(keys, N: int):
+    """A list of 1-based keys (tuples of 1..8 distinct spin labels in [1, N]) as the C ABI's key list: (key_order, key_idx
+    int32 [n_keys x key_order] 0-based, -1 padded, the keys as tuples)."""
+    keys = [tuple(int(i) for i in k) for k in keys]
+    if not keys:
+        raise ValueError("moments need at least one key")
+    for k in keys:
+        if not 1 <= len(k) <= 8 or len(set(k)) != len(k) or min(k) < 1 or max(k) > N:
+            raise ValueError(f"a key is a tuple of 1..8 distinct 1-based spin labels in [1, {N}], got {k}")
+    order = max(len(k) for k in keys)
+    idx = -np.ones((len(keys), order), dtype=np.int32)
+    for t, k in enumerate(keys):
+        idx[t, :len(k)] = np.asarray(k) - 1
+    return order, idx, keys
+
+
+def _keys_call(keys, N: int):
+    """((key_order, n_keys, key_idx pointer), key tuples or None, output shape, the key_idx array the pointer refers to)
+    of the C moments entries; keys is a key list or "pairwise" (the N x N output)."""
+    if isinstance(keys, str):
+        if keys != "pairwise":
+            raise ValueError(f'keys must be a list of tuples or "pairwise", got {keys!r}')
+        return (0, _lib.KEYS_PAIRWISE, None), None, (N, N), None
+    order, idx, tuples = _key_arrays(keys, N)
+    return (order, len(tuples), _ptr(idx)), tuples, (len(tuples),), idx
+
+
+def _moments_result(values, tuples, N: int):
+    """An N x N array (pairwise) as it is, or a FactorGraph over the key tuples"""
+    if tuples is None:
+        return values
+    return FactorGraph(max(len(k) for k in tuples), N, "spin", dict(zip(tuples, values.tolist())))
+
+
+def moments(gm: FactorGraph, sampler: Optional[GMLSampler] = None, number_sample: Optional[int] = None, keys=None):
+    """(mean, stderr): the model's moments <prod_{i in t} s_i> of keys t, the derivatives d log Z / d w_t.
+
+    - keys: None = gm's own keys in gm's order; a list of 1-based tuples (1..8 distinct spins each); both return two
+      FactorGraphs over those keys.  "pairwise" returns two N x N arrays laid out like learn()'s matrix: <s_i> on the
+      diagonal, <s_i s_j> off it.
+    - None or B200Exact: enumeration (N <= 40, gml_b200_moments_exact), exact in fp64, stderr all zeros; number_sample must
+      be None.  Cost ~2^N * (n_terms + n_keys): pairwise has N(N+1)/2 keys, ~5e11 operations at N = 30, ~9e14 at N = 40.
+    - B200Gibbs / B200Tempering (N <= 4096, gml_b200_moments_mcmc) need number_sample: the mean is over exactly the draws
+      that sample(gm, number_sample, 1, sampler) returns with the same sampler fields, bit for bit, without writing them;
+      stderr comes from G = min(32, warps) groups of chains (NaN with fewer than 2).  Sets last_rhat (and last_swap_rate)
+      as sample does.  The chains sample fp32-rounded weights: the moments of gm differ by at most e^{2 delta} - 1, delta =
+      sum_t |w_t - fl32(w_t)|."""
+    sampler = B200Exact() if sampler is None else sampler
+    if isinstance(sampler, Gibbs):
+        raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact(), "
+                                  "B200Gibbs() or B200Tempering()")
+    if not isinstance(sampler, (B200Exact, B200Gibbs, B200Tempering)):
+        raise TypeError("sampler must be a GMLSampler")
+    mcmc = not isinstance(sampler, B200Exact)
+    name = type(sampler).__name__
+    if gm.alphabet != "spin":
+        raise ValueError(f"moments are only supported for the spin alphabet, not {gm.alphabet!r}")
+    N = int(gm.varible_count)
+    cap = _lib.MCMC_MAX_N if mcmc else _lib.EXACT_MAX_N
+    if not 1 <= N <= cap:
+        raise ValueError(f"moments with {name} support 1 <= N <= {cap} spins, got {N}")
+    if mcmc and number_sample is None:
+        raise ValueError(f"{name} needs number_sample")
+    if not mcmc and number_sample is not None:
+        raise ValueError("B200Exact moments are exact: number_sample must be None")
+    if mcmc and (int(number_sample) < 1 or sampler.chains < 0 or sampler.burn_in < 0 or sampler.thin < 1):
+        raise ValueError(f"{name} needs number_sample >= 1, chains >= 0, burn_in >= 0 and thin >= 1")
+    betas = _ladder(sampler) if isinstance(sampler, B200Tempering) else None
+    key_args, tuples, shape, _keep = _keys_call(list(gm.terms) if keys is None else keys, N)
+    order, idx, wts = _term_arrays(gm)
+    lib = _lib.load()
+    seed = int(sampler.seed) & (2 ** 64 - 1)
+    mean, err = np.zeros(shape), np.zeros(shape)
+    model = (int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts))
+    if not mcmc:
+        _lib.check(lib.gml_b200_moments_exact(*model, *key_args, _ptr(mean), None))
+    else:
+        sampler.last_rhat = []
+        rhat = np.zeros(2)
+        if betas is None:
+            ladder, swap = (1, None), None
+        else:
+            ladder = (len(betas), _ptr(betas) if len(betas) else None)
+            swap = np.zeros((1, (len(betas) or _lib.TEMPERING_DEFAULT_RUNGS) - 1))
+            sampler.last_swap_rate = []
+        _lib.check(lib.gml_b200_moments_mcmc(*model, *ladder, int(number_sample), int(sampler.chains), int(sampler.burn_in),
+                                             int(sampler.thin), seed, *key_args, _ptr(mean), _ptr(err), _ptr(rhat),
+                                             None if swap is None else _ptr(swap), None))
+        sampler.last_rhat = [tuple(rhat.tolist())]
+        if swap is not None:
+            sampler.last_swap_rate = swap.tolist()
+    return _moments_result(mean, tuples, N), _moments_result(err, tuples, N)
+
+
+def empirical_moments(samples, keys="pairwise", device: int = 0):
+    """The data's moments sum_k c_k prod_{i in t} s_ki / M of a histogram (any `samples` learn() takes), on the device.
+    keys: "pairwise" (an N x N array laid out like learn()'s matrix: <s_i> on the diagonal, <s_i s_j> off it; the
+    tensor-core gradient pass at x = 0) or a list of 1-based tuples (a FactorGraph over them; raw counts summed in fp64, so
+    integer counts give exactly the MCMC moments of the same draws).  Session.moments does the same for a resident
+    histogram."""
+    counts, spins = pack_histogram(samples)
+    _keys_call(keys, spins.shape[0])                      # refuse bad keys before a device is needed
+    return Session(device).upload(counts, spins).moments(keys)
+
+
+def log_likelihood(gm: FactorGraph, samples, sampler: Optional[GMLSampler] = None, sweeps: int = 1000):
+    """(value, stderr): the mean log-likelihood of the rows of `samples` under gm, sum_t w_t <prod_{i in t} s_i>_data -
+    log Z.  The data term uses gm's fp64 weights and empirical_moments over gm's keys; log Z and the stderr come from
+    log_partition(gm, sampler, sweeps) with its samplers and defaults (None = B200Tempering(); B200Exact for N <= 40)."""
+    if not gm.terms:
+        raise ValueError("log_likelihood needs a model with at least one term")
+    counts, spins = pack_histogram(samples)
+    if spins.shape[0] != int(gm.varible_count):
+        raise ValueError(f"samples have {spins.shape[0]} spins, the model {gm.varible_count}")
+    keys = list(gm.terms)
+    _keys_call(keys, spins.shape[0])
+    log_z, err = log_partition(gm, sampler, sweeps)
+    device = 0 if sampler is None else int(sampler.device)
+    data = Session(device).upload(counts, spins).moments(keys)
+    energy = float(sum(w * m for w, m in zip(gm.terms.values(), data.terms.values())))
+    return energy - log_z, err
+
+
 class Session:
     """Handle API (include/gml_b200.h): keeps the histogram resident in HBM across calls."""
 
@@ -613,6 +736,14 @@ class Session:
     @property
     def num_samples(self) -> float:
         return float(self._lib.gml_b200_num_samples(self._h))
+
+    def moments(self, keys="pairwise"):
+        """The resident histogram's moments, as empirical_moments: an N x N array for "pairwise", else a FactorGraph over
+        the 1-based key tuples."""
+        key_args, tuples, shape, _keep = _keys_call(keys, self.N)
+        mean = np.zeros(shape)
+        _lib.check(self._lib.gml_b200_moments_histogram(self._h, *key_args, _ptr(mean)))
+        return _moments_result(mean, tuples, self.N)
 
     def _lam(self, formulation, lam: Optional[float]) -> float:
         """lam, by default the reference's lambda (:157) of the resident histogram"""

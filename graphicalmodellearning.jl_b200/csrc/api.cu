@@ -284,6 +284,64 @@ std::vector<double> tempering_ladder(int32_t n_rungs, const double* betas, std::
     return ladder;
 }
 
+// the sampling default of the replica-exchange entry points: geometric from 1 to 0.1
+std::vector<double> default_tempering_ladder() {
+    std::vector<double> ladder;
+    constexpr int R = GML_B200_TEMPERING_DEFAULT_RUNGS;
+    for (int k = 0; k < R; ++k) ladder.push_back(std::pow(0.1, (double)k / (R - 1)));
+    return ladder;
+}
+
+// The keys of a moments entry point: n_keys = GML_B200_KEYS_PAIRWISE with key_idx = NULL (the N x N output), or n_keys >= 1
+// rows of key_order <= 8 entries, each row 1..8 distinct 0-based spins in [0, N) padded with -1.
+MomentKeys moment_keys(int32_t N, int32_t key_order, int32_t n_keys, const int32_t* key_idx) {
+    MomentKeys k;
+    if (n_keys == GML_B200_KEYS_PAIRWISE) {
+        GML_REQUIRE(key_idx == nullptr, "GML_B200_KEYS_PAIRWISE goes with key_idx = NULL");
+        k.pairwise = true;
+        return k;
+    }
+    GML_REQUIRE(n_keys >= 1 && key_idx && key_order >= 1 && key_order <= 8,
+                "keys need n_keys >= 1 (or GML_B200_KEYS_PAIRWISE), key_idx and 1 <= key_order <= 8");
+    k.order = key_order; k.n_keys = n_keys;
+    k.idx.assign(key_idx, key_idx + (size_t)n_keys * key_order);
+    for (int t = 0; t < n_keys; ++t) {
+        const int32_t* key = k.idx.data() + (size_t)t * key_order;
+        int q = 0;
+        for (int m = 0; m < key_order; ++m) {
+            if (key[m] == -1) continue;
+            GML_REQUIRE(key[m] >= 0 && key[m] < N, "a key refers to a spin outside [0, N)");
+            for (int m2 = 0; m2 < m; ++m2) GML_REQUIRE(key[m2] != key[m], "a key repeats a spin");
+            ++q;
+        }
+        GML_REQUIRE(q >= 1, "a key has no spin");
+    }
+    return k;
+}
+
+// The term list of the exact entry points as spin masks, checked (N <= GML_B200_EXACT_MAX_N)
+void exact_model(int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx, const double* term_weight,
+                 std::vector<uint64_t>& masks, std::vector<double>& weights) {
+    GML_REQUIRE(N >= 1 && N <= GML_B200_EXACT_MAX_N, "exact sampler needs 1 <= N <= " + std::to_string(GML_B200_EXACT_MAX_N));
+    GML_REQUIRE(order >= 1 && order <= GML_B200_EXACT_MAX_N && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)),
+                "bad sampler argument");
+    masks.assign(n_terms, 0);
+    weights.assign(term_weight, term_weight + n_terms);
+    double abs_sum = 0.0;
+    for (int t = 0; t < n_terms; ++t) {
+        for (int m = 0; m < order; ++m) {
+            const int i = term_idx[(size_t)t * order + m];
+            if (i == -1) continue;
+            GML_REQUIRE(i >= 0 && i < N, "sampler term refers to a spin outside [0, N)");
+            GML_REQUIRE(!((masks[t] >> i) & 1ull), "sampler term repeats a spin");
+            masks[t] |= 1ull << i;
+        }
+        GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
+        abs_sum += std::fabs(weights[t]);
+    }
+    GML_REQUIRE(std::isfinite(abs_sum), "sum of |term weights| is not finite");
+}
+
 // The MCMC entry points (betas = {1}: gml_b200_sample_mcmc_device; R > 1 rungs: gml_b200_sample_tempering_device, whose
 // ladder the caller has checked): argument checks, then the sampler into the caller's buffers.
 void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx, const double* term_weight,
@@ -1239,26 +1297,12 @@ int gml_b200_sample_exact_device(int32_t device, int32_t N, int32_t order, int32
                                  int64_t* out_K, double* out_log_z, double* d_counts, int8_t* d_spins, int64_t ld,
                                  void* stream) {
     return guarded([&] {
-        GML_REQUIRE(N >= 1 && N <= GML_B200_EXACT_MAX_N, "exact sampler needs 1 <= N <= " + std::to_string(GML_B200_EXACT_MAX_N));
-        GML_REQUIRE(order >= 1 && order <= GML_B200_EXACT_MAX_N && n_terms >= 0 && (n_terms == 0 || (term_idx && term_weight)) && out_K,
-                    "bad sampler argument");
+        std::vector<uint64_t> masks;
+        std::vector<double> weights;
+        exact_model(N, order, n_terms, term_idx, term_weight, masks, weights);
+        GML_REQUIRE(out_K, "bad sampler argument");
         GML_REQUIRE(n_samples >= 1 && replicates >= 1 && n_samples <= (INT64_C(1) << 62) / replicates, "bad sampler sizes");
         GML_REQUIRE(!d_counts || (d_spins && ld >= 1), "d_counts needs d_spins and ld >= 1");
-        std::vector<uint64_t> masks(n_terms, 0);
-        std::vector<double> weights(term_weight, term_weight + n_terms);
-        double abs_sum = 0.0;
-        for (int t = 0; t < n_terms; ++t) {
-            for (int m = 0; m < order; ++m) {
-                const int i = term_idx[(size_t)t * order + m];
-                if (i == -1) continue;
-                GML_REQUIRE(i >= 0 && i < N, "sampler term refers to a spin outside [0, N)");
-                GML_REQUIRE(!((masks[t] >> i) & 1ull), "sampler term repeats a spin");
-                masks[t] |= 1ull << i;
-            }
-            GML_REQUIRE(std::isfinite(weights[t]), "sampler term weight is not finite");
-            abs_sum += std::fabs(weights[t]);
-        }
-        GML_REQUIRE(std::isfinite(abs_sum), "sum of |term weights| is not finite");
         GML_CUDA(cudaSetDevice(device));
         cudaStream_t st = (cudaStream_t)stream;
         double log_z = 0.0;
@@ -1285,10 +1329,7 @@ int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, i
                                      int64_t* out_K, double* out_rhat, double* out_swap_rate, double* d_counts, int8_t* d_spins,
                                      int64_t ld, void* stream) {
     return guarded([&] {
-        std::vector<double> fallback;               // the default ladder: geometric from 1 to 0.1
-        constexpr int R = GML_B200_TEMPERING_DEFAULT_RUNGS;
-        for (int k = 0; k < R; ++k) fallback.push_back(std::pow(0.1, (double)k / (R - 1)));
-        const std::vector<double> ladder = tempering_ladder(n_rungs, betas, fallback);
+        const std::vector<double> ladder = tempering_ladder(n_rungs, betas, default_tempering_ladder());
         run_mcmc(device, N, order, n_terms, term_idx, term_weight, ladder, n_samples, replicates, chains, burn_in, thin, seed,
                  out_K, out_rhat, out_swap_rate, d_counts, d_spins, ld, stream);
     });
@@ -1313,6 +1354,87 @@ int gml_b200_log_partition_tempering(int32_t device, int32_t N, int32_t order, i
         GML_CUDA(cudaSetDevice(device));
         log_partition_tempering(N, order, m.idx, m.weights, m.inc, ladder, chains, burn_in, sweeps, seed, out_log_z, out_stderr,
                                 out_log_ratio, out_swap_rate, (cudaStream_t)stream);
+    });
+}
+
+int gml_b200_moments_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                          const double* term_weight, int32_t n_rungs, const double* betas, int64_t n_samples, int64_t chains,
+                          int32_t burn_in, int32_t thin, uint64_t seed, int32_t key_order, int32_t n_keys, const int32_t* key_idx,
+                          double* out_mean, double* out_stderr, double* out_rhat, double* out_swap_rate, void* stream) {
+    return guarded([&] {
+        std::vector<double> ladder{1.0};            // n_rungs = 1, betas = NULL: single-site Gibbs
+        if (!(n_rungs == 1 && betas == nullptr)) ladder = tempering_ladder(n_rungs, betas, default_tempering_ladder());
+        const McmcModel m = mcmc_model(N, order, n_terms, term_idx, term_weight);
+        const MomentKeys keys = moment_keys(N, key_order, n_keys, key_idx);
+        GML_REQUIRE(out_mean, "null out_mean");
+        GML_REQUIRE(n_samples >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1, "bad sampler sizes");
+        const int rungs = (int)ladder.size();
+        if (chains == 0) chains = mcmc_auto_chains(n_samples, rungs);
+        GML_REQUIRE(((double)burn_in + (double)thin * (double)ceil_div(n_samples, chains)) * N < 0x1.0p62, "too many sweeps");
+        GML_CUDA(cudaSetDevice(device));
+        moments_mcmc(N, order, m.idx, m.weights, m.inc, ladder, n_samples, chains, burn_in, thin, seed, keys, out_mean, out_stderr,
+                     out_rhat, out_swap_rate, (cudaStream_t)stream);
+    });
+}
+
+int gml_b200_moments_exact(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                           const double* term_weight, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean,
+                           void* stream) {
+    return guarded([&] {
+        std::vector<uint64_t> masks;
+        std::vector<double> weights;
+        exact_model(N, order, n_terms, term_idx, term_weight, masks, weights);
+        const MomentKeys keys = moment_keys(N, key_order, n_keys, key_idx);
+        GML_REQUIRE(out_mean, "null out_mean");
+        std::vector<uint64_t> key_masks;
+        if (keys.pairwise) {                         // the upper triangle, row by row
+            for (int i = 0; i < N; ++i)
+                for (int j = i; j < N; ++j) key_masks.push_back((1ull << i) | (1ull << j));
+        } else {
+            for (int t = 0; t < keys.n_keys; ++t) {
+                uint64_t mk = 0;
+                for (int q = 0; q < keys.order; ++q)
+                    if (keys.idx[(size_t)t * keys.order + q] >= 0) mk |= 1ull << keys.idx[(size_t)t * keys.order + q];
+                key_masks.push_back(mk);
+            }
+        }
+        GML_CUDA(cudaSetDevice(device));
+        std::vector<double> mean(key_masks.size());
+        moments_exact(N, masks, weights, key_masks, mean.data(), (cudaStream_t)stream);
+        if (!keys.pairwise) { std::copy(mean.begin(), mean.end(), out_mean); return; }
+        size_t t = 0;
+        for (int i = 0; i < N; ++i)
+            for (int j = i; j < N; ++j, ++t) out_mean[(size_t)i * N + j] = out_mean[(size_t)j * N + i] = mean[t];
+    });
+}
+
+int gml_b200_moments_histogram(gml_b200_handle* h, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean) {
+    return guarded([&] {
+        GML_REQUIRE(h && out_mean, "null argument");
+        GML_REQUIRE(h->has_hist, "no histogram resident: call gml_b200_upload_histogram first");
+        GML_REQUIRE(h->hist.M_local == 0.0, "moments of a sample-sharded histogram are not supported");
+        const MomentKeys keys = moment_keys(h->hist.N, key_order, n_keys, key_idx);
+        g_launches = 0;
+        GML_CUDA(cudaSetDevice(h->device));
+        cudaStream_t st = h->own_stream;
+        if (!keys.pairwise) { moments_histogram_keys(h->hist, keys, out_mean, st); return; }
+        // the tensor-core gradient pass at x = 0: row u is -[C_u | m_u]; the diagonal takes m, then 0.5 (C + C')
+        const int N = h->hist.N;
+        gml_b200_opts o; fill_opts(o, nullptr);
+        o.solver = GML_B200_SOLVER_FISTA_TC;
+        NodeProblem p;
+        const std::unique_ptr<EvalBackend> be = eval_backend(h, GML_B200_RISE, o, p, st);
+        DevBuf<double> x, f, g, rows;
+        const size_t nx = (size_t)N * p.Fp;
+        x.alloc(nx); f.alloc(N); g.alloc(nx); rows.alloc((size_t)N * N);
+        GML_CUDA(cudaMemsetAsync(x.p, 0, sizeof(double) * nx, st));
+        be->eval(x.p, true, f.p, g.p, st);
+        pairwise_rows_kernel<<<N, 128, 0, st>>>(g.p, N, p.Fp, 0, rows.p);
+        GML_LAUNCHED();
+        launch_symmetrize(rows.p, N, st);
+        GML_CUDA(cudaMemcpyAsync(out_mean, rows.p, sizeof(double) * N * N, cudaMemcpyDeviceToHost, st));
+        GML_CUDA(cudaStreamSynchronize(st));
+        for (size_t e = 0; e < (size_t)N * N; ++e) out_mean[e] = -out_mean[e];
     });
 }
 

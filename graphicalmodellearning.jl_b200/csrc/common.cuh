@@ -89,6 +89,7 @@ struct Histogram {
     double K_total = 0.0;    // histogram rows over all ranks (= K unless sample-sharded)
     double wmax = 0.0;       // max_k c_k / M
     DevBuf<int8_t> base;
+    DevBuf<double> counts;   // [K] c_k as uploaded (the data moments sum them exactly)
     DevBuf<double> w64;      // [Kp] c_k / M
     DevBuf<float> w32;       // [Kp]
     int32_t mb_order = 0, mb_F = 0, mb_Fp = 0;
@@ -266,10 +267,33 @@ void log_partition_tempering(int N, int order, const std::vector<int32_t>& term_
                              int64_t sweeps, uint64_t seed, double* out_log_z, double* out_stderr, double* out_log_ratio,
                              double* out_swap_rate, cudaStream_t st);
 
+// --- moments.cu : moments <prod_{i in t} s_i> of keys t.  pairwise: all <s_i> (diagonal) and <s_i s_j> as an N x N
+// row-major matrix; otherwise n_keys keys of `order` 0-based spins, -1 padded ([n_keys x order]).
+struct MomentKeys {
+    bool pairwise = false;
+    int order = 0, n_keys = 0;
+    std::vector<int32_t> idx;
+};
+int64_t moment_outputs(const MomentKeys& keys, int N);
+// mean and stderr (nullable) of the keys over the draws of a record buffer of mcmc_kernel's RECORD mode
+void reduce_records(const uint32_t* rec, int N, int64_t records, int64_t warps, const MomentKeys& keys, double* out_mean,
+                    double* out_stderr, cudaStream_t st);
+// key-list moments of a resident histogram: sum_k c_k prod s / M
+void moments_histogram_keys(const Histogram& hist, const MomentKeys& keys, double* out_mean, cudaStream_t st);
+// The moments over exactly the n_samples draws that sample_mcmc(..., replicates = 1, ...) returns with the same arguments,
+// with their standard errors over G = min(32, warps) groups of warps, out_rhat [2] and out_swap_rate [R-1] as sample_mcmc.
+void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                  const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int64_t chains, int64_t burn_in,
+                  int64_t thin, uint64_t seed, const MomentKeys& keys, double* out_mean, double* out_stderr, double* out_rhat,
+                  double* out_swap_rate, cudaStream_t st);
+
 // --- exact_sampler.cu : iid draws from the exact distribution by enumeration (term t = spins of masks[t]); fills
 // out_K[replicates] and, when d_counts is set, the histograms at consecutive rows; returns log Z.  N <= GML_B200_EXACT_MAX_N.
 double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights, int64_t n_samples,
                     int replicates, uint64_t seed, int64_t* out_K, double* d_counts, int8_t* d_spins, int64_t ld,
                     cudaStream_t st);
+// exact moments of the keys (masks over spins 0..N-1; out_mean[keys]) by enumeration, N <= GML_B200_EXACT_MAX_N
+void moments_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights,
+                   const std::vector<uint64_t>& key_masks, double* out_mean, cudaStream_t st);
 
 }  // namespace gml

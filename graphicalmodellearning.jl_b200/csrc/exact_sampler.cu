@@ -11,6 +11,11 @@
 // Every reduction and scan has a fixed shape that depends on N only, so the output depends on (model, n, replicates,
 // seed) and not on the grid, the block scheduling or the device.  Cost: ~2^N * n_terms sign+add in fp64 for pass 1 (the
 // resolve pass only recomputes blocks that received draws); memory: 40 bytes per block plus 10 bytes per draw.
+// Moments (moments(gm) with B200Exact): pass 1 for the global max, then every configuration block recomputes its
+// energies, keeps p_c = exp(E_c - max) in shared memory, and thread t of the CTA adds sum_c p_c (-1)^popc(key & ~c) over
+// the block, in index order, to its CTA's partial for the keys t, t + 256, ...; the grid is fixed by N (CTA b takes blocks
+// b, b + grid, ...) and the partials are summed in CTA order, so the result depends only on (model, keys).  Cost: ~2^N *
+// (n_terms + n_keys) sign+add in fp64.
 #include <cmath>
 #include <cstring>
 
@@ -299,39 +304,123 @@ __global__ void __launch_bounds__(THREADS) exact_emit_kernel(int N, const ull* _
     }
 }
 
+// partial[blockIdx.x][k] += sum over the configurations of the CTA's blocks of p_c (-1)^popc(key_k & ~c); the last key
+// (mask 0) is the normaliser sum_c p_c.  key = the order key of the global max energy (max_kernel).
+template <class MaskT>
+__global__ void __launch_bounds__(THREADS) exact_moments_kernel(int N, int64_t nb, int n_terms, const uint64_t* __restrict__ hi,
+                                                                const double* __restrict__ w, const uint32_t* __restrict__ par,
+                                                                const ull* __restrict__ key, int n_keys,
+                                                                const uint64_t* __restrict__ key_masks, double* __restrict__ partial) {
+    __shared__ MaskT s_hi[TERM_CHUNK];
+    __shared__ double s_w[TERM_CHUNK];
+    __shared__ uint32_t s_par[TERM_CHUNK];
+    __shared__ double p[BLOCK_CFG];
+    const double gmax = from_order_key(*key);
+    for (int64_t b = blockIdx.x; b < nb; b += gridDim.x) {
+        const uint64_t cfg0 = ((uint64_t)b << BLOCK_BITS) + (uint64_t)PER_THREAD * threadIdx.x;
+        double e[PER_THREAD];
+        thread_energies<MaskT>(cfg0, n_terms, hi, w, par, s_hi, s_w, s_par, e);
+        mask_padding(cfg0, N, e);
+#pragma unroll
+        for (int k = 0; k < PER_THREAD; ++k) p[PER_THREAD * threadIdx.x + k] = exp(e[k] - gmax);
+        __syncthreads();
+        for (int k = threadIdx.x; k < n_keys; k += THREADS) {
+            const uint64_t m = key_masks[k];
+            const uint32_t lo = (uint32_t)(m & (BLOCK_CFG - 1));
+            const uint32_t par_hi = (uint32_t)__popcll((m >> BLOCK_BITS) & ~(uint64_t)b) & 1u;
+            double acc = 0.0;
+            for (uint32_t c = 0; c < BLOCK_CFG; ++c) {
+                const double v = p[c];
+                acc += ((__popc(lo & ~c) ^ par_hi) & 1u) ? -v : v;
+            }
+            partial[(int64_t)blockIdx.x * n_keys + k] += acc;
+        }
+        __syncthreads();
+    }
+}
+
+// mean[k] = sum over CTAs of partial[.][k] / the same sum for the normaliser (key n_keys - 1), in CTA order
+__global__ void exact_moments_finalize_kernel(const double* __restrict__ partial, int grid, int n_keys, double* __restrict__ mean) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_keys - 1) return;
+    double s = 0.0, z = 0.0;
+    for (int c = 0; c < grid; ++c) { s += partial[(int64_t)c * n_keys + k]; z += partial[(int64_t)c * n_keys + n_keys - 1]; }
+    mean[k] = s / z;
+}
+
+// the term arrays of the enumeration kernels: high mask bits, low-bit sign patterns and weights on the device
+struct ExactTerms {
+    DevBuf<uint64_t> hi;
+    DevBuf<uint32_t> par;
+    DevBuf<double> w;
+    ExactTerms(const std::vector<uint64_t>& masks, const std::vector<double>& weights, cudaStream_t st) {
+        const int n_terms = (int)masks.size();
+        std::vector<uint64_t> h_hi(std::max(n_terms, 1), 0);
+        std::vector<uint32_t> h_par(std::max(n_terms, 1), 0);
+        for (int t = 0; t < n_terms; ++t) {
+            h_hi[t] = masks[t] & ~0xFull;
+            for (int k = 0; k < PER_THREAD; ++k) h_par[t] |= (uint32_t)(__builtin_popcountll(masks[t] & 0xFull & ~(uint64_t)k) & 1) << k;
+        }
+        hi.alloc(h_hi.size()); par.alloc(h_par.size()); w.alloc(std::max(n_terms, 1));
+        GML_CUDA(cudaMemcpyAsync(hi.p, h_hi.data(), sizeof(uint64_t) * h_hi.size(), cudaMemcpyHostToDevice, st));
+        GML_CUDA(cudaMemcpyAsync(par.p, h_par.data(), sizeof(uint32_t) * h_par.size(), cudaMemcpyHostToDevice, st));
+        if (n_terms) GML_CUDA(cudaMemcpyAsync(w.p, weights.data(), sizeof(double) * n_terms, cudaMemcpyHostToDevice, st));
+        GML_CUDA(cudaStreamSynchronize(st));        // the host arrays go out of scope
+    }
+};
+
+// pass 1 (block max and sum) and the global max into *key
+void partition_pass(int N, int n_terms, const ExactTerms& t, int64_t nb, double* bmax, double* bsum, ull* key, cudaStream_t st) {
+    if (N <= 32) exact_partition_kernel<uint32_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, t.hi.p, t.w.p, t.par.p, bmax, bsum);
+    else exact_partition_kernel<uint64_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, t.hi.p, t.w.p, t.par.p, bmax, bsum);
+    GML_LAUNCHED();
+    GML_CUDA(cudaMemsetAsync(key, 0, sizeof(ull), st));
+    max_kernel<<<(unsigned)std::min<int64_t>(ceil_div(nb, THREADS), 1024), THREADS, 0, st>>>(bmax, nb, key);
+    GML_LAUNCHED();
+}
+
 }  // namespace
+
+void moments_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights,
+                   const std::vector<uint64_t>& key_masks, double* out_mean, cudaStream_t st) {
+    const int n_terms = (int)masks.size(), n_keys = (int)key_masks.size() + 1;
+    const int64_t nb = N > BLOCK_BITS ? (int64_t)1 << (N - BLOCK_BITS) : 1;
+    const int grid = (int)std::min<int64_t>(nb, 148 * 4);
+    ExactTerms terms(masks, weights, st);
+    std::vector<uint64_t> km(key_masks);
+    km.push_back(0);                                  // the normaliser
+    DevBuf<double> bmax, bsum, partial, mean;
+    DevBuf<ull> key;
+    DevBuf<uint64_t> d_km;
+    bmax.alloc(nb); bsum.alloc(nb); key.alloc(1); d_km.alloc(km.size());
+    partial.alloc((size_t)grid * n_keys); mean.alloc(n_keys);
+    GML_CUDA(cudaMemcpyAsync(d_km.p, km.data(), sizeof(uint64_t) * km.size(), cudaMemcpyHostToDevice, st));
+    GML_CUDA(cudaMemsetAsync(partial.p, 0, sizeof(double) * grid * n_keys, st));
+    partition_pass(N, n_terms, terms, nb, bmax.p, bsum.p, key.p, st);
+    if (N <= 32) exact_moments_kernel<uint32_t><<<grid, THREADS, 0, st>>>(N, nb, n_terms, terms.hi.p, terms.w.p, terms.par.p, key.p, n_keys, d_km.p, partial.p);
+    else exact_moments_kernel<uint64_t><<<grid, THREADS, 0, st>>>(N, nb, n_terms, terms.hi.p, terms.w.p, terms.par.p, key.p, n_keys, d_km.p, partial.p);
+    GML_LAUNCHED();
+    exact_moments_finalize_kernel<<<(unsigned)ceil_div(n_keys, 256), 256, 0, st>>>(partial.p, grid, n_keys, mean.p);
+    GML_LAUNCHED();
+    GML_CUDA(cudaMemcpyAsync(out_mean, mean.p, sizeof(double) * (n_keys - 1), cudaMemcpyDeviceToHost, st));
+    GML_CUDA(cudaStreamSynchronize(st));
+}
 
 double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights, int64_t n_samples,
                     int replicates, uint64_t seed, int64_t* out_K, double* d_counts, int8_t* d_spins, int64_t ld,
                     cudaStream_t st) {
     const int n_terms = (int)masks.size();
     const int64_t nb = N > BLOCK_BITS ? (int64_t)1 << (N - BLOCK_BITS) : 1;
-    std::vector<uint64_t> hi(std::max(n_terms, 1), 0);
-    std::vector<uint32_t> par(std::max(n_terms, 1), 0);
-    for (int t = 0; t < n_terms; ++t) {
-        hi[t] = masks[t] & ~0xFull;
-        for (int k = 0; k < PER_THREAD; ++k) par[t] |= (uint32_t)(__builtin_popcountll(masks[t] & 0xFull & ~(uint64_t)k) & 1) << k;
-    }
-    DevBuf<uint64_t> d_hi;
-    DevBuf<uint32_t> d_par;
-    DevBuf<double> d_w, bmax, cdf, dscan, resid;
+    ExactTerms terms(masks, weights, st);
+    DevBuf<double> bmax, cdf, dscan, resid;
     DevBuf<ull> key, cnt, cur, nz, uscan;
     DevBuf<uint16_t> cfg;
-    d_hi.alloc(hi.size()); d_par.alloc(par.size()); d_w.alloc(std::max(n_terms, 1));
     bmax.alloc(nb); cdf.alloc(nb); key.alloc(1); cnt.alloc(nb); cur.alloc(nb); nz.alloc(nb);
     dscan.alloc(scan_scratch<double>(nb)); uscan.alloc(scan_scratch<ull>(nb));
     resid.alloc(n_samples); cfg.alloc(n_samples);
-    GML_CUDA(cudaMemcpyAsync(d_hi.p, hi.data(), sizeof(uint64_t) * hi.size(), cudaMemcpyHostToDevice, st));
-    GML_CUDA(cudaMemcpyAsync(d_par.p, par.data(), sizeof(uint32_t) * par.size(), cudaMemcpyHostToDevice, st));
-    if (n_terms) GML_CUDA(cudaMemcpyAsync(d_w.p, weights.data(), sizeof(double) * n_terms, cudaMemcpyHostToDevice, st));
 
     // 1-2: block partition sums, global max, block CDF
-    if (N <= 32) exact_partition_kernel<uint32_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, d_hi.p, d_w.p, d_par.p, bmax.p, cdf.p);
-    else exact_partition_kernel<uint64_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, d_hi.p, d_w.p, d_par.p, bmax.p, cdf.p);
-    GML_LAUNCHED();
-    GML_CUDA(cudaMemsetAsync(key.p, 0, sizeof(ull), st));
-    max_kernel<<<(unsigned)std::min<int64_t>(ceil_div(nb, THREADS), 1024), THREADS, 0, st>>>(bmax.p, nb, key.p);
-    GML_LAUNCHED();
+    partition_pass(N, n_terms, terms, nb, bmax.p, cdf.p, key.p, st);
     rescale_kernel<<<(unsigned)ceil_div(nb, THREADS), THREADS, 0, st>>>(bmax.p, cdf.p, nb, key.p);
     GML_LAUNCHED();
     scan_inclusive(cdf.p, nb, dscan.p, st);
@@ -356,8 +445,8 @@ double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector
         scan_inclusive(cur.p, nb, uscan.p, st);
         scatter_draws_kernel<<<draw_grid, THREADS, 0, st>>>(cdf.p, nb, seed, d0, n_samples, cur.p, resid.p);
         GML_LAUNCHED();
-        if (N <= 32) exact_resolve_kernel<uint32_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, d_hi.p, d_w.p, d_par.p, cnt.p, cur.p, resid.p, cfg.p, nz.p);
-        else exact_resolve_kernel<uint64_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, d_hi.p, d_w.p, d_par.p, cnt.p, cur.p, resid.p, cfg.p, nz.p);
+        if (N <= 32) exact_resolve_kernel<uint32_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, terms.hi.p, terms.w.p, terms.par.p, cnt.p, cur.p, resid.p, cfg.p, nz.p);
+        else exact_resolve_kernel<uint64_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, terms.hi.p, terms.w.p, terms.par.p, cnt.p, cur.p, resid.p, cfg.p, nz.p);
         GML_LAUNCHED();
         scan_inclusive(nz.p, nb, uscan.p, st);
         ull K = 0;

@@ -28,6 +28,9 @@
 //     beta_{k+1}) to two running log-sum-exps (running maximum, so nothing overflows) and finally writes their log-means:
 //     the two halves of the geometric bridge log Z_k - log Z_{k+1} = log E_{k+1}[e^x] - log E_k[e^y] (Meng & Wong 1996).
 //     The RNG streams and the swap decisions are those of the sampler.
+//   - Moments (RECORD, moments(gm, sampler)): after every recording sweep each warp copies its N state words and a 32-bit
+//     mask of the lanes whose record is a draw (live && d < n && rung == 0) to column r * warps + warp of a spin-major
+//     record buffer [(N+1) x records * warps] (row N = the masks); nothing else is written.  moments.cu reduces it.
 #include <cmath>
 #include <type_traits>
 
@@ -80,6 +83,8 @@ struct McmcParams {
     unsigned long long* swap_acc;   // R > 1: [warps x (R-1)] swaps of pair (k, k+1) accepted after burn_in
     double beta[TEMPERING_MAX_RUNGS];  // R > 1: inverse temperature of each rung, beta[0] = 1
     double* bridge;            // BRIDGE: [chains x (R-1) x 2] per ladder and pair k the log-means of e^x and e^y
+    uint32_t* record;          // RECORD: [(N+1) x ld_rec] state words and draw masks, column r * rec_warps + warp
+    int64_t rec_warps, ld_rec; // RECORD: warps of the grid, records * rec_warps
 };
 
 // parity (1 = odd) of the down spins of lane `lane` among the members m of a list (entries < 0 are padding)
@@ -137,8 +142,9 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // R = 1: multi-sample Gibbs, one chain per lane.  R > 1: one ladder of R rungs per R consecutive lanes (see the top);
-// BRIDGE adds the sums of the log Z estimator (a separate instantiation: the sampler's registers stay as they are).
-template <bool KEYS, int R, bool BRIDGE = false>
+// BRIDGE adds the sums of the log Z estimator, RECORD the record buffer of the moments (separate instantiations: the
+// sampler's registers stay as they are).
+template <bool KEYS, int R, bool BRIDGE = false, bool RECORD = false>
 __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
     using Energy = typename std::conditional<R == 1, float, double>::type;
     constexpr int LADDERS = 32 / R;                           // ladders (chains) per warp
@@ -203,6 +209,13 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
                 if (KEYS) cfg |= (unsigned long long)bit << i;
                 else if (out && p.spins) p.spins[(int64_t)i * p.ld + d] = bit ? 1 : -1;
             }
+        }
+        if (RECORD && rec) {
+            const uint32_t draws = __ballot_sync(FULL, out);
+            uint32_t* dst = p.record + r * p.rec_warps + warp + lane * p.ld_rec;
+#pragma unroll 1
+            for (int i = lane; i < N; i += 32, dst += 32 * p.ld_rec) *dst = s[i];
+            if (lane == 0) p.record[N * p.ld_rec + r * p.rec_warps + warp] = draws;
         }
         double energy_now = 0;                                // R > 1: the energy of every lane, for the swap test
         if constexpr (R > 1) energy_now = term_energy<double>(s, p, p.n_terms, lane);
@@ -319,6 +332,17 @@ void (*bridge_kernel(int rungs))(McmcParams) {
     }
 }
 
+void (*record_kernel(int rungs))(McmcParams) {
+    switch (rungs) {
+        case 1: return mcmc_kernel<false, 1, false, true>;
+        case 2: return mcmc_kernel<false, 2, false, true>;
+        case 4: return mcmc_kernel<false, 4, false, true>;
+        case 8: return mcmc_kernel<false, 8, false, true>;
+        case 16: return mcmc_kernel<false, 16, false, true>;
+        default: return mcmc_kernel<false, 32, false, true>;
+    }
+}
+
 // A model on the device for mcmc_kernel: the incidence lists and the term list with weights rounded once to fp32, and the
 // parameters that describe the model and the ladder.  The caller fills in the run.
 struct DeviceModel {
@@ -346,6 +370,20 @@ struct DeviceModel {
         for (size_t k = 0; k < betas.size(); ++k) p.beta[k] = betas[k];
     }
 };
+
+// split-R-hat (energy, magnetisation) into rh[2] from the per-warp sums of warp_stats over half-chains of h records
+void rhat_of(const double* warp_stats, int64_t warps, int64_t chains, int64_t h, double* rh, cudaStream_t st) {
+    rh[0] = rh[1] = NAN;
+    if (h < 2) return;
+    std::vector<double> hs(warps * 6);
+    GML_CUDA(cudaMemcpyAsync(hs.data(), warp_stats, sizeof(double) * hs.size(), cudaMemcpyDeviceToHost, st));
+    GML_CUDA(cudaStreamSynchronize(st));
+    double acc[6] = {0, 0, 0, 0, 0, 0};
+    for (int64_t w = 0; w < warps; ++w)
+        for (int k = 0; k < 6; ++k) acc[k] += hs[w * 6 + k];
+    rh[0] = split_rhat(acc[0], acc[1], acc[2], 2.0 * chains, (double)h);
+    rh[1] = split_rhat(acc[3], acc[4], acc[5], 2.0 * chains, (double)h);
+}
 
 // per adjacent pair, accepted / proposed swaps after burn_in from the per-warp counts of swap_acc
 void swap_rates(const unsigned long long* swap_acc, int64_t warps, int rungs, int64_t chains, int64_t burn_in, int64_t sweeps,
@@ -390,7 +428,6 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
     p.inv_h = 1.0 / (double)h;
     p.inv_h1 = 1.0 / (double)(h - 1);
     const int64_t sweeps = burn_in + p.records * thin;
-    std::vector<double> hs(warps * 6);
     int64_t rows = 0;
     bool fits = true;
     for (int rep = 0; rep < replicates; ++rep) {
@@ -412,25 +449,46 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
         out_K[rep] = K;
         fits = fits && rows + K <= ld;
         rows += K;
-        if (out_rhat) {
-            double* rh = out_rhat + 2 * rep;
-            rh[0] = rh[1] = NAN;
-            if (h >= 2) {
-                GML_CUDA(cudaMemcpyAsync(hs.data(), wstats.p, sizeof(double) * hs.size(), cudaMemcpyDeviceToHost, st));
-                GML_CUDA(cudaStreamSynchronize(st));
-                double acc[6] = {0, 0, 0, 0, 0, 0};
-                for (int64_t w = 0; w < warps; ++w)
-                    for (int k = 0; k < 6; ++k) acc[k] += hs[w * 6 + k];
-                rh[0] = split_rhat(acc[0], acc[1], acc[2], 2.0 * chains, (double)h);
-                rh[1] = split_rhat(acc[3], acc[4], acc[5], 2.0 * chains, (double)h);
-            }
-        }
+        if (out_rhat) rhat_of(wstats.p, warps, chains, h, out_rhat + 2 * rep, st);
         if (out_swap_rate && rungs > 1)
             swap_rates(swaps.p, warps, rungs, chains, burn_in, sweeps, out_swap_rate + (size_t)rep * (rungs - 1), st);
     }
     GML_CUDA(cudaStreamSynchronize(st));
     GML_REQUIRE(!d_counts || fits, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(rows) +
                                    " rows of the replicates (out_K holds their sizes)");
+}
+
+void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                  const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int64_t chains, int64_t burn_in,
+                  int64_t thin, uint64_t seed, const MomentKeys& keys, double* out_mean, double* out_stderr, double* out_rhat,
+                  double* out_swap_rate, cudaStream_t st) {
+    const int rungs = (int)betas.size();
+    const int64_t warps = ceil_div(chains, 32 / rungs), blocks = ceil_div(warps, WARPS);
+    const size_t smem = sizeof(uint32_t) * (size_t)N * WARPS;
+
+    DeviceModel model(N, order, term_idx, term_weight, inc, betas, st);
+    DevBuf<double> wstats;
+    DevBuf<unsigned long long> swaps;
+    DevBuf<uint32_t> record;
+    McmcParams& p = model.p;
+    p.chains = chains; p.chain0 = 0; p.n = n_samples; p.burn_in = burn_in; p.thin = thin;
+    p.records = ceil_div(n_samples, chains); p.full_records = n_samples / chains;
+    const int64_t h = p.full_records / 2;
+    p.inv_h = 1.0 / (double)h;
+    p.inv_h1 = 1.0 / (double)(h - 1);
+    p.rec_warps = warps; p.ld_rec = p.records * warps;
+    wstats.alloc(warps * 6);
+    if (rungs > 1) swaps.alloc(warps * (rungs - 1));
+    record.alloc((size_t)(N + 1) * p.ld_rec);
+    p.seed = seed; p.warp_stats = wstats.p; p.swap_acc = swaps.p; p.record = record.p;
+    auto kernel = record_kernel(rungs);
+    GML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<(unsigned)blocks, WARPS * 32, smem, st>>>(p);
+    GML_LAUNCHED();
+    if (out_rhat) rhat_of(wstats.p, warps, chains, h, out_rhat, st);
+    if (out_swap_rate && rungs > 1)
+        swap_rates(swaps.p, warps, rungs, chains, burn_in, burn_in + p.records * thin, out_swap_rate, st);
+    reduce_records(record.p, N, p.records, warps, keys, out_mean, out_stderr, st);
 }
 
 void log_partition_tempering(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,

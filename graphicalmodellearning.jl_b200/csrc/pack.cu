@@ -151,6 +151,7 @@ void hist_from_device(Histogram& h, const double* d_counts, const int8_t* d_spin
     h.Kp = round_up(K, KPAD);
     h.Fb = (int32_t)round_up(N + 1, FPAD);
     h.base.alloc((size_t)h.Fb * h.Kp);
+    h.counts.alloc(K);
     h.w64.alloc(h.Kp);
     h.w32.alloc(h.Kp);
     h.mb_order = 0; h.P_of = nullptr; h.Qb_of = nullptr;
@@ -164,6 +165,7 @@ void hist_from_device(Histogram& h, const double* d_counts, const int8_t* d_spin
     dim3 grid((unsigned)ceil_div(h.Kp, 16 * 256), h.Fb);
     pack_spins_kernel<<<grid, 256, 0, st>>>(d_spins, ld, K, h.Kp, N, h.Fb, h.base.p, flags.p);
     GML_LAUNCHED();
+    GML_CUDA(cudaMemcpyAsync(h.counts.p, d_counts, sizeof(double) * K, cudaMemcpyDeviceToDevice, st));
     const int nb = (int)std::min<int64_t>(ceil_div(K, 256), 148 * 8);
     count_stats_kernel<<<nb, 256, 0, st>>>(d_counts, K, scal.p, scal.p + 1, flags.p);
     GML_LAUNCHED();

@@ -337,6 +337,41 @@ int gml_b200_log_partition_tempering(int32_t device, int32_t N, int32_t order, i
                                      double* out_log_ratio /* nullable [n_rungs-1][2]: estimate, stderr */,
                                      double* out_swap_rate /* nullable [n_rungs-1] */, void* stream);
 
+/* ---- moments <prod_{i in t} s_i> of keys t: the model's (MCMC or exact) and the data's (resident histogram) --------
+ * Keys: n_keys >= 1 rows of key_idx [n_keys x key_order], key_order <= 8, each row 1..8 distinct 0-based spins in
+ * [0, N) padded with -1 (the layout of term_idx); out_mean [n_keys].  n_keys = GML_B200_KEYS_PAIRWISE with key_idx =
+ * NULL selects all <s_i> and <s_i s_j>: out_mean [N x N] row-major, <s_i> on the diagonal, symmetric.
+ *
+ * gml_b200_moments_mcmc: the mean of prod_{i in t} s_i over exactly the n_samples draws that
+ * gml_b200_sample_mcmc_device (n_rungs = 1, betas = NULL) or gml_b200_sample_tempering_device (otherwise, the same
+ * ladder rules) with replicates = 1 and the same sizes and seed returns: the same chains, RNG streams, records and swaps.
+ *   - The kernel copies each warp's N state words and a mask of the lanes whose record is a draw to a record buffer of
+ *     records * warps * (N + 1) * 4 bytes, one bit per spin and chain record (R bits per draw with R rungs), and
+ *     integer popcount reductions sum it: the sums are exact, so the mean is the draws' mean bit for bit.
+ *   - out_stderr (nullable): the warps are split into G = min(32, warps) contiguous groups of whole warps with sums S_g
+ *     over n_g draws; stderr = sqrt(G/(G-1) sum_g (S_g - mean n_g)^2) / sum n_g, NaN when G < 2.
+ *   - out_rhat (nullable) [2] and out_swap_rate (nullable) [n_rungs-1]: as the sampler reports them.
+ *   - Pairwise cost: an XNOR-popcount bit-GEMM of N^2/2 * records * warps 32-bit popcounts and G * N^2 * 8 bytes of sums.
+ *   - The chains sample fp32-rounded weights: |<f>(w) - <f>(fl32(w))| <= e^{2 delta} - 1, delta = sum_t |w_t - fl32(w_t)|.
+ *   - GML_B200_EINVAL: what the sampler entry points refuse, bad keys, n_samples < 1, out_mean == NULL.
+ * gml_b200_moments_exact: sum_c e^{E_c} prod s / Z by enumeration for the models of gml_b200_sample_exact_device
+ *   (N <= 40), in fp64; the result depends only on (terms, keys).  Cost ~2^N * (n_terms + n_keys) sign+add: pairwise
+ *   has N(N+1)/2 keys, ~5e11 operations at N = 30 and ~9e14 at N = 40.
+ * gml_b200_moments_histogram: sum_k c_k prod s_k / M over the resident histogram.  Key lists sum the raw counts in fp64
+ *   (exact for integer counts below 2^53 in total, so equal to the MCMC mean of the same draws bit for bit); pairwise is the
+ *   tensor-core gradient pass at x = 0 (the mean-field warm start's), symmetrised as 0.5 (C + C').  Not for a
+ *   sample-sharded histogram. */
+#define GML_B200_KEYS_PAIRWISE (-1)
+int gml_b200_moments_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                          const double* term_weight, int32_t n_rungs, const double* betas /* [n_rungs] */, int64_t n_samples,
+                          int64_t chains, int32_t burn_in, int32_t thin, uint64_t seed, int32_t key_order, int32_t n_keys,
+                          const int32_t* key_idx, double* out_mean, double* out_stderr /* nullable */,
+                          double* out_rhat /* nullable [2] */, double* out_swap_rate /* nullable [n_rungs-1] */, void* stream);
+int gml_b200_moments_exact(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                           const double* term_weight, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean,
+                           void* stream);
+int gml_b200_moments_histogram(gml_b200_handle* h, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean);
+
 /* ---- sample-sharded mode (SURVEY 8e): histogram rows split over ranks, every rank solves all nodes; per pass
  * the int64 gradient sums and fp64 objective sums are combined with NCCL all-reduces on the solve stream.
  *   rank 0: gml_b200_comm_unique_id(id) -> broadcast the 128 bytes with any transport -> every rank:
