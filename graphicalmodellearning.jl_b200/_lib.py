@@ -18,6 +18,8 @@ MCMC_MAX_N = 4096  # GML_B200_MCMC_MAX_N
 TEMPERING_DEFAULT_RUNGS = 16  # GML_B200_TEMPERING_DEFAULT_RUNGS
 LOG_Z_DEFAULT_RUNGS = 32  # GML_B200_LOG_Z_DEFAULT_RUNGS
 KEYS_PAIRWISE = -1  # GML_B200_KEYS_PAIRWISE
+FIT_STEP_SIZE = 0.1  # default eta_0 of fit_likelihood with B200Gibbs
+FIT_STEP_S0 = 100.0  # eta_s = eta_0 (1 + s / FIT_STEP_S0)^-0.6 (FIT_STEP_S0 in csrc/common.cuh)
 SOLVER_AUTO, SOLVER_NEWTON, SOLVER_FISTA_CC, SOLVER_FISTA_TC = 0, 1, 2, 3
 
 # every symbol include/gml_b200.h declares
@@ -33,6 +35,7 @@ EXPORTS = (
     "gml_b200_sample_gibbs_device", "gml_b200_sample_gibbs_terms_device", "gml_b200_sample_exact_device",
     "gml_b200_sample_mcmc_device", "gml_b200_sample_tempering_device", "gml_b200_log_partition_tempering",
     "gml_b200_moments_mcmc", "gml_b200_moments_exact", "gml_b200_moments_histogram",
+    "gml_b200_fit_likelihood_mcmc", "gml_b200_fit_likelihood_exact",
     "gml_b200_build_histogram_device",
     "gml_b200_comm_unique_id", "gml_b200_comm_init", "gml_b200_comm_globalize_histogram", "gml_b200_comm_attach",
 )
@@ -135,6 +138,10 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
                                           c.c_int32, c.c_int32, c.c_uint64, c.c_int32, c.c_int32, vp, vp, vp, vp, vp, vp]
     lib.gml_b200_moments_exact.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, c.c_int32, vp, vp, vp]
     lib.gml_b200_moments_histogram.argtypes = [vp, c.c_int32, c.c_int32, vp, vp]
+    lib.gml_b200_fit_likelihood_mcmc.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, vp, c.c_double, c.c_int64,
+                                                 c.c_int32, c.c_int32, c.c_int64, c.c_double, c.c_uint64, vp, vp, vp, vp]
+    lib.gml_b200_fit_likelihood_exact.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, vp, c.c_double, c.c_double,
+                                                  c.c_int32, vp, vp, vp, vp]
     lib.gml_b200_build_histogram_device.argtypes = [c.c_int32, vp, c.c_int64, c.c_int32, c.c_int64, vp, c.c_int64, vp,
                                                     c.POINTER(c.c_int64), vp]
     lib.gml_b200_comm_unique_id.argtypes = [vp]

@@ -699,6 +699,99 @@ def log_likelihood(gm: FactorGraph, samples, sampler: Optional[GMLSampler] = Non
     return energy - log_z, err
 
 
+def fit_likelihood(gm: FactorGraph, samples, sampler: Optional[GMLSampler] = None, regularizer: float = 0.0,
+                   steps: int = 2000, step_size: Optional[float] = None, tol: float = 1e-10, max_iter: int = 100000,
+                   return_info: bool = False):
+    """Maximum-likelihood refit of gm's weights on gm's own terms: a FactorGraph with gm's keys in gm's order whose weights
+    maximise  l(w) = sum_t w_t m^_t - log Z(w) - lambda sum_{|t| >= 2} |w_t|,  starting from gm's weights.  m^_t are the
+    data moments of `samples` (any input learn() takes) over gm's keys (terms of at most 8 spins), lambda =
+    regularizer_lambda(regularizer, N, M) (fields are not penalised; the default 0 refits on the given support).  Keys
+    whose weight in gm is 0 are fitted too.  At the maximum the model's moments equal m^ on every unpenalised term, which
+    removes the shrinkage of an L1-penalised RISE / RPLE fit: select the support with learn(), refit it here.
+
+    - None or B200Exact: FISTA with backtracking on the exact objective (gml_b200_fit_likelihood_exact, N <= 40; each
+      iteration enumerates 2^N configurations once or twice, so it is practical to about N = 28).  Stops when the max-norm
+      of the prox-gradient mapping is <= tol; GMLB200Error (code ENOTCONV) after max_iter iterations.
+    - B200Gibbs: stochastic maximum likelihood with persistent chains (gml_b200_fit_likelihood_mcmc, N <= 4096).  The
+      sampler's seed, device, chains (0 = 2^17), burn_in and thin (sweeps per step) describe the chains.  `steps`
+      preconditioned proximal steps of size step_size (1 + s / 100)^-0.6 (None = the library default, 0.1) run on the
+      device; the result is the mean of the weights over the second half of the steps.  The chains sample fl32(w).
+    - B200Tempering is refused: persistent replica-exchange ladders are not built.
+    - return_info adds a dict: lambda and data_moments (m^ in gm's key order); for B200Gibbs also model_moments (the
+      chains' mean moments over the averaged steps), trace (max_t |m^_t - m_t| of every step) and step_sizes; for
+      B200Exact the objective l at the result and the iterations run."""
+    sampler = B200Exact() if sampler is None else sampler
+    if isinstance(sampler, Gibbs):
+        raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact() or "
+                                  "B200Gibbs()")
+    if isinstance(sampler, B200Tempering):
+        raise ValueError("fit_likelihood does not take B200Tempering: persistent replica-exchange ladders are not built; "
+                         "pass B200Gibbs() or B200Exact()")
+    if not isinstance(sampler, (B200Exact, B200Gibbs)):
+        raise TypeError("sampler must be B200Exact or B200Gibbs")
+    mcmc = isinstance(sampler, B200Gibbs)
+    name = type(sampler).__name__
+    if gm.alphabet != "spin":
+        raise ValueError(f"fit_likelihood is only supported for the spin alphabet, not {gm.alphabet!r}")
+    if not gm.terms:
+        raise ValueError("fit_likelihood needs a model with at least one term")
+    N = int(gm.varible_count)
+    cap = _lib.MCMC_MAX_N if mcmc else _lib.EXACT_MAX_N
+    if not 1 <= N <= cap:
+        raise ValueError(f"fit_likelihood with {name} supports 1 <= N <= {cap} spins, got {N}")
+    counts, spins = pack_histogram(samples)
+    if spins.shape[0] != N:
+        raise ValueError(f"samples have {spins.shape[0]} spins, the model {N}")
+    M = float(counts.sum())
+    if not (math.isfinite(M) and M > 0 and (counts >= 0).all()):
+        raise ValueError("sample counts must be non-negative with a positive finite total")
+    regularizer = float(regularizer)
+    if not (math.isfinite(regularizer) and regularizer >= 0):
+        raise ValueError("regularizer must be finite and >= 0")
+    lam = regularizer_lambda(regularizer, N, M)
+    steps, max_iter = int(steps), int(max_iter)
+    eta0 = _lib.FIT_STEP_SIZE if step_size is None else float(step_size)
+    if mcmc:
+        if steps < 1 or not (math.isfinite(eta0) and eta0 >= 0):
+            raise ValueError("B200Gibbs fits need steps >= 1 and a finite step_size >= 0")
+        if sampler.chains < 0 or sampler.chains > 2 ** 31 or sampler.burn_in < 0 or sampler.thin < 1:
+            raise ValueError("B200Gibbs needs 0 <= chains <= 2^31, burn_in >= 0 and thin >= 1")
+        if sampler.burn_in >= 2 ** 31 or sampler.thin >= 2 ** 31 or (sampler.burn_in + steps * sampler.thin) * N >= 2 ** 62:
+            raise ValueError("too many sweeps")
+    elif not (math.isfinite(float(tol)) and tol > 0 and 1 <= max_iter < 2 ** 31):
+        raise ValueError("B200Exact fits need a finite tol > 0 and 1 <= max_iter < 2^31")
+    keys = list(gm.terms)
+    _keys_call(keys, N)
+    order, idx, wts = _term_arrays(gm)
+    data = np.array(list(Session(int(sampler.device)).upload(counts, spins).moments(keys).terms.values()), dtype=np.float64)
+    sizes = np.array([len(k) for k in keys])
+    if not (np.isfinite(data).all() and (np.abs(data) <= 1).all()):
+        raise ValueError("the data moments are not in [-1, 1]")
+    unbounded = (np.abs(data) == 1) & ~((sizes >= 2) & (lam > 0))
+    if unbounded.any():
+        k = keys[int(np.argmax(unbounded))]
+        raise ValueError(f"the data moment of {k} is +-1 and lambda does not bound its weight: the likelihood has no "
+                         "finite maximum")
+    lib = _lib.load()
+    out = np.zeros(len(keys))
+    model = (int(sampler.device), N, order, len(keys), _ptr(idx), _ptr(wts), _ptr(data), lam)
+    info = {"lambda": lam, "data_moments": data.tolist()}
+    if mcmc:
+        mm, trace = np.zeros(len(keys)), np.zeros(steps)
+        _lib.check(lib.gml_b200_fit_likelihood_mcmc(*model, int(sampler.chains), int(sampler.burn_in), int(sampler.thin), steps,
+                                                    eta0, int(sampler.seed) & (2 ** 64 - 1), _ptr(out), _ptr(mm), _ptr(trace),
+                                                    None))
+        info.update(model_moments=mm.tolist(), trace=trace.tolist(),
+                    step_sizes=[eta0 * (1.0 + s / _lib.FIT_STEP_S0) ** -0.6 for s in range(steps)])
+    else:
+        obj, iters = ctypes.c_double(0.0), ctypes.c_int32(0)
+        _lib.check(lib.gml_b200_fit_likelihood_exact(*model, float(tol), max_iter, _ptr(out), ctypes.byref(obj),
+                                                     ctypes.byref(iters), None))
+        info.update(objective=obj.value, iterations=iters.value)
+    fg = FactorGraph(gm.order, N, "spin", dict(zip(keys, out.tolist())))
+    return (fg, info) if return_info else fg
+
+
 class Session:
     """Handle API (include/gml_b200.h): keeps the histogram resident in HBM across calls."""
 

@@ -371,6 +371,25 @@ void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const i
     });
 }
 
+// The fit targets of a fit_likelihood entry point, checked: per term whether lambda |w_t| applies (terms of >= 2 spins).
+// Every data moment lies in [-1, 1]; |m^_t| = 1 leaves l(w) without a finite maximum unless lambda bounds the term.
+std::vector<uint8_t> fit_targets(int32_t order, int32_t n_terms, const int32_t* term_idx, const double* data_mean,
+                                 double lambda, const double* out_weight) {
+    GML_REQUIRE(n_terms >= 1 && data_mean && out_weight, "fit_likelihood needs n_terms >= 1, data_mean and out_weight");
+    GML_REQUIRE(std::isfinite(lambda) && lambda >= 0.0, "lambda must be finite and >= 0");
+    std::vector<uint8_t> pen(n_terms);
+    for (int t = 0; t < n_terms; ++t) {
+        int q = 0;
+        for (int k = 0; k < order; ++k) q += term_idx[(size_t)t * order + k] >= 0;
+        pen[t] = q >= 2;
+        const double m = data_mean[t];
+        GML_REQUIRE(std::isfinite(m) && std::fabs(m) <= 1.0, "a data moment is outside [-1, 1] or not finite");
+        GML_REQUIRE(std::fabs(m) < 1.0 || (pen[t] && lambda > 0.0),
+                    "a data moment of +-1 on a term lambda does not bound: the likelihood has no finite maximum");
+    }
+    return pen;
+}
+
 void throw_if_unconverged(int n_unconverged) {
     if (n_unconverged == 0) return;
     set_error("solver did not reach tol within max_iter for " + std::to_string(n_unconverged) + " node(s)");
@@ -1405,6 +1424,45 @@ int gml_b200_moments_exact(int32_t device, int32_t N, int32_t order, int32_t n_t
         size_t t = 0;
         for (int i = 0; i < N; ++i)
             for (int j = i; j < N; ++j, ++t) out_mean[(size_t)i * N + j] = out_mean[(size_t)j * N + i] = mean[t];
+    });
+}
+
+int gml_b200_fit_likelihood_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                 const double* init_weight, const double* data_mean, double lambda, int64_t chains, int32_t burn_in,
+                                 int32_t thin, int64_t steps, double step_size, uint64_t seed, double* out_weight,
+                                 double* out_model_moments, double* out_trace, void* stream) {
+    return guarded([&] {
+        const McmcModel m = mcmc_model(N, order, n_terms, term_idx, init_weight);
+        const std::vector<uint8_t> pen = fit_targets(order, n_terms, term_idx, data_mean, lambda, out_weight);
+        GML_REQUIRE(chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1 && steps >= 1, "bad sampler sizes");
+        GML_REQUIRE(std::isfinite(step_size) && step_size >= 0.0, "step_size must be finite and >= 0");
+        GML_REQUIRE(((double)burn_in + (double)steps * (double)thin) * N < 0x1.0p62, "too many sweeps");
+        if (chains == 0) chains = MCMC_AUTO_CHAINS;
+        GML_CUDA(cudaSetDevice(device));
+        fit_likelihood_mcmc(N, order, m.idx, m.weights, m.inc, std::vector<double>(data_mean, data_mean + n_terms), pen, lambda,
+                            chains, burn_in, thin, steps, step_size, seed, out_weight, out_model_moments, out_trace,
+                            (cudaStream_t)stream);
+    });
+}
+
+int gml_b200_fit_likelihood_exact(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                  const double* init_weight, const double* data_mean, double lambda, double tol, int32_t max_iter,
+                                  double* out_weight, double* out_objective, int32_t* out_iterations, void* stream) {
+    return guarded([&] {
+        std::vector<uint64_t> masks;
+        std::vector<double> weights;
+        exact_model(N, order, n_terms, term_idx, init_weight, masks, weights);
+        const std::vector<uint8_t> pen = fit_targets(order, n_terms, term_idx, data_mean, lambda, out_weight);
+        GML_REQUIRE(std::isfinite(tol) && tol > 0.0 && max_iter >= 1, "tol must be finite and > 0, max_iter >= 1");
+        GML_CUDA(cudaSetDevice(device));
+        int iterations = 0;
+        const bool ok = fit_likelihood_exact(N, masks, weights, std::vector<double>(data_mean, data_mean + n_terms), pen, lambda,
+                                             tol, max_iter, out_weight, out_objective, &iterations, (cudaStream_t)stream);
+        if (out_iterations) *out_iterations = iterations;
+        if (!ok) {
+            set_error("fit_likelihood: the prox-gradient mapping did not reach tol within max_iter iterations");
+            throw CudaError{GML_B200_ENOTCONV};
+        }
     });
 }
 

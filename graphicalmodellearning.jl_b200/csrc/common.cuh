@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdio>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -267,6 +268,24 @@ void log_partition_tempering(int N, int order, const std::vector<int32_t>& term_
                              int64_t sweeps, uint64_t seed, double* out_log_z, double* out_stderr, double* out_log_ratio,
                              double* out_swap_rate, cudaStream_t st);
 
+// Persistent Gibbs chains (PERSIST instantiation of mcmc_kernel, fit_likelihood): `chains` chains of the model with
+// fp32 weights in the device buffers term_w [n_terms] and weight [incidence entries], which a caller may rewrite between
+// launches.  run(sweep0, k) advances every chain by sweeps sweep0 + 1 .. sweep0 + k of one long run (sweep0 = 0: from the
+// random start of sweep 0) and leaves the final state in `record`, a record buffer [(N+1) x warps] of one record (the
+// layout reduce_records reads, the live lanes as draws); it is also the state the next launch resumes from.
+struct PersistentChains {
+    struct Impl;
+    std::unique_ptr<Impl> impl;
+    int64_t warps = 0;
+    const uint32_t* record = nullptr;
+    float* term_w = nullptr;
+    float* weight = nullptr;
+    PersistentChains(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
+                     const Incidence& inc, int64_t chains, uint64_t seed, cudaStream_t st);
+    ~PersistentChains();
+    void run(int64_t sweep0, int64_t sweeps, cudaStream_t st);
+};
+
 // --- moments.cu : moments <prod_{i in t} s_i> of keys t.  pairwise: all <s_i> (diagonal) and <s_i s_j> as an N x N
 // row-major matrix; otherwise n_keys keys of `order` 0-based spins, -1 padded ([n_keys x order]).
 struct MomentKeys {
@@ -278,6 +297,11 @@ int64_t moment_outputs(const MomentKeys& keys, int N);
 // mean and stderr (nullable) of the keys over the draws of a record buffer of mcmc_kernel's RECORD mode
 void reduce_records(const uint32_t* rec, int N, int64_t records, int64_t warps, const MomentKeys& keys, double* out_mean,
                     double* out_stderr, cudaStream_t st);
+// the integer sums behind reduce_records' key-list means, left on the device: n_g [G] draws and S [G x n_keys] key sums
+// of the G = record_groups(warps) groups of warps (d_key_idx [n_keys x order] on the device)
+int record_groups(int64_t warps);
+void record_key_sums(const uint32_t* rec, int N, int64_t records, int64_t warps, int order, int n_keys, const int32_t* d_key_idx,
+                     long long* d_n_g, long long* d_S, cudaStream_t st);
 // key-list moments of a resident histogram: sum_k c_k prod s / M
 void moments_histogram_keys(const Histogram& hist, const MomentKeys& keys, double* out_mean, cudaStream_t st);
 // The moments over exactly the n_samples draws that sample_mcmc(..., replicates = 1, ...) returns with the same arguments,
@@ -287,13 +311,30 @@ void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const 
                   int64_t thin, uint64_t seed, const MomentKeys& keys, double* out_mean, double* out_stderr, double* out_rhat,
                   double* out_swap_rate, cudaStream_t st);
 
+// --- likelihood.cu : maximum-likelihood refit of the weights of a term list from data moments data_mean (fit_likelihood).
+// penalised[t] = 1 marks the terms of >= 2 spins, which carry lambda |w_t|.
+constexpr double FISHER_FLOOR = 1e-2;    // floor of the diagonal preconditioner 1 - m^_t^2 of the MCMC steps
+constexpr double FIT_STEP_S0 = 100.0;    // eta_s = eta_0 (1 + s / FIT_STEP_S0)^-0.6
+double fit_step_size(double eta0, int64_t s);
+// persistent-chain stochastic maximum likelihood; out_weight [n_terms] = the Polyak-Ruppert mean over steps >= steps / 2,
+// out_model_moments (nullable) [n_terms] = the chains' mean moments over the same steps, out_trace (nullable) [steps]
+void fit_likelihood_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& init_weight,
+                         const Incidence& inc, const std::vector<double>& data_mean, const std::vector<uint8_t>& penalised,
+                         double lambda, int64_t chains, int64_t burn_in, int64_t thin, int64_t steps, double eta0, uint64_t seed,
+                         double* out_weight, double* out_model_moments, double* out_trace, cudaStream_t st);
+// FISTA on the exact objective (term t = spins of masks[t]); false when the prox-gradient mapping did not reach tol
+bool fit_likelihood_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& init_weight,
+                          const std::vector<double>& data_mean, const std::vector<uint8_t>& penalised, double lambda, double tol,
+                          int max_iter, double* out_weight, double* out_objective, int* out_iterations, cudaStream_t st);
+
 // --- exact_sampler.cu : iid draws from the exact distribution by enumeration (term t = spins of masks[t]); fills
 // out_K[replicates] and, when d_counts is set, the histograms at consecutive rows; returns log Z.  N <= GML_B200_EXACT_MAX_N.
 double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights, int64_t n_samples,
                     int replicates, uint64_t seed, int64_t* out_K, double* d_counts, int8_t* d_spins, int64_t ld,
                     cudaStream_t st);
-// exact moments of the keys (masks over spins 0..N-1; out_mean[keys]) by enumeration, N <= GML_B200_EXACT_MAX_N
+// exact moments of the keys (masks over spins 0..N-1; out_mean[keys]) by enumeration, N <= GML_B200_EXACT_MAX_N, and
+// (nullable out_log_z) log Z from the same pass
 void moments_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights,
-                   const std::vector<uint64_t>& key_masks, double* out_mean, cudaStream_t st);
+                   const std::vector<uint64_t>& key_masks, double* out_mean, cudaStream_t st, double* out_log_z = nullptr);
 
 }  // namespace gml

@@ -15,7 +15,7 @@
 // energies, keeps p_c = exp(E_c - max) in shared memory, and thread t of the CTA adds sum_c p_c (-1)^popc(key & ~c) over
 // the block, in index order, to its CTA's partial for the keys t, t + 256, ...; the grid is fixed by N (CTA b takes blocks
 // b, b + grid, ...) and the partials are summed in CTA order, so the result depends only on (model, keys).  Cost: ~2^N *
-// (n_terms + n_keys) sign+add in fp64.
+// (n_terms + n_keys) sign+add in fp64.  log Z = global max + log(normaliser) comes with the same pass.
 #include <cmath>
 #include <cstring>
 
@@ -339,13 +339,14 @@ __global__ void __launch_bounds__(THREADS) exact_moments_kernel(int N, int64_t n
     }
 }
 
-// mean[k] = sum over CTAs of partial[.][k] / the same sum for the normaliser (key n_keys - 1), in CTA order
+// mean[k] = sum over CTAs of partial[.][k] / the same sum z for the normaliser (key n_keys - 1), in CTA order; mean[n_keys - 1]
+// = z
 __global__ void exact_moments_finalize_kernel(const double* __restrict__ partial, int grid, int n_keys, double* __restrict__ mean) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n_keys - 1) return;
+    if (k >= n_keys) return;
     double s = 0.0, z = 0.0;
     for (int c = 0; c < grid; ++c) { s += partial[(int64_t)c * n_keys + k]; z += partial[(int64_t)c * n_keys + n_keys - 1]; }
-    mean[k] = s / z;
+    mean[k] = k == n_keys - 1 ? z : s / z;
 }
 
 // the term arrays of the enumeration kernels: high mask bits, low-bit sign patterns and weights on the device
@@ -369,6 +370,13 @@ struct ExactTerms {
     }
 };
 
+double host_from_order_key(ull k) {
+    const uint64_t b = (k >> 63) ? (k & ~(1ull << 63)) : ~k;
+    double x;
+    std::memcpy(&x, &b, sizeof(double));
+    return x;
+}
+
 // pass 1 (block max and sum) and the global max into *key
 void partition_pass(int N, int n_terms, const ExactTerms& t, int64_t nb, double* bmax, double* bsum, ull* key, cudaStream_t st) {
     if (N <= 32) exact_partition_kernel<uint32_t><<<(unsigned)nb, THREADS, 0, st>>>(N, n_terms, t.hi.p, t.w.p, t.par.p, bmax, bsum);
@@ -382,7 +390,7 @@ void partition_pass(int N, int n_terms, const ExactTerms& t, int64_t nb, double*
 }  // namespace
 
 void moments_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights,
-                   const std::vector<uint64_t>& key_masks, double* out_mean, cudaStream_t st) {
+                   const std::vector<uint64_t>& key_masks, double* out_mean, cudaStream_t st, double* out_log_z) {
     const int n_terms = (int)masks.size(), n_keys = (int)key_masks.size() + 1;
     const int64_t nb = N > BLOCK_BITS ? (int64_t)1 << (N - BLOCK_BITS) : 1;
     const int grid = (int)std::min<int64_t>(nb, 148 * 4);
@@ -403,7 +411,14 @@ void moments_exact(int N, const std::vector<uint64_t>& masks, const std::vector<
     exact_moments_finalize_kernel<<<(unsigned)ceil_div(n_keys, 256), 256, 0, st>>>(partial.p, grid, n_keys, mean.p);
     GML_LAUNCHED();
     GML_CUDA(cudaMemcpyAsync(out_mean, mean.p, sizeof(double) * (n_keys - 1), cudaMemcpyDeviceToHost, st));
+    double z = 0.0;
+    ull hkey = 0;
+    if (out_log_z) {
+        GML_CUDA(cudaMemcpyAsync(&z, mean.p + n_keys - 1, sizeof(double), cudaMemcpyDeviceToHost, st));
+        GML_CUDA(cudaMemcpyAsync(&hkey, key.p, sizeof(ull), cudaMemcpyDeviceToHost, st));
+    }
     GML_CUDA(cudaStreamSynchronize(st));
+    if (out_log_z) *out_log_z = host_from_order_key(hkey) + std::log(z);
 }
 
 double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector<double>& weights, int64_t n_samples,
@@ -429,7 +444,7 @@ double sample_exact(int N, const std::vector<uint64_t>& masks, const std::vector
     GML_CUDA(cudaMemcpyAsync(&total, cdf.p + nb - 1, sizeof(double), cudaMemcpyDeviceToHost, st));
     GML_CUDA(cudaMemcpyAsync(&hkey, key.p, sizeof(ull), cudaMemcpyDeviceToHost, st));
     GML_CUDA(cudaStreamSynchronize(st));
-    { const uint64_t b = (hkey >> 63) ? (hkey & ~(1ull << 63)) : ~hkey; std::memcpy(&gmax, &b, sizeof(double)); }
+    gmax = host_from_order_key(hkey);
     const double log_z = gmax + std::log(total);
 
     // 3-4 per replicate: draws [r*n, (r+1)*n) of the stream

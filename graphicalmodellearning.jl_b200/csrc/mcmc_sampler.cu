@@ -31,6 +31,11 @@
 //   - Moments (RECORD, moments(gm, sampler)): after every recording sweep each warp copies its N state words and a 32-bit
 //     mask of the lanes whose record is a draw (live && d < n && rung == 0) to column r * warps + warp of a spin-major
 //     record buffer [(N+1) x records * warps] (row N = the masks); nothing else is written.  moments.cu reduces it.
+//   - Persistent chains (PERSIST, R = 1, fit_likelihood(gm, samples, B200Gibbs())): a launch runs sweeps sweep0 + 1 ..
+//     sweep0 + thin of the chains of one long run, so the site counters sweep * N + site continue across launches while
+//     the caller rewrites the weights between them.  The state lives in a record buffer [(N+1) x warps]: a launch with
+//     sweep0 > 0 loads its warp's column, and every launch stores its final state words and the mask of its live lanes
+//     there (one record per launch, column = warp).  No draws, energies or R-hat sums.
 #include <cmath>
 #include <type_traits>
 
@@ -85,6 +90,7 @@ struct McmcParams {
     double* bridge;            // BRIDGE: [chains x (R-1) x 2] per ladder and pair k the log-means of e^x and e^y
     uint32_t* record;          // RECORD: [(N+1) x ld_rec] state words and draw masks, column r * rec_warps + warp
     int64_t rec_warps, ld_rec; // RECORD: warps of the grid, records * rec_warps
+    int64_t sweep0;            // PERSIST: the sweeps of this launch are sweep0 + 1 .. sweep0 + thin
 };
 
 // parity (1 = odd) of the down spins of lane `lane` among the members m of a list (entries < 0 are padding)
@@ -142,9 +148,9 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // R = 1: multi-sample Gibbs, one chain per lane.  R > 1: one ladder of R rungs per R consecutive lanes (see the top);
-// BRIDGE adds the sums of the log Z estimator, RECORD the record buffer of the moments (separate instantiations: the
-// sampler's registers stay as they are).
-template <bool KEYS, int R, bool BRIDGE = false, bool RECORD = false>
+// BRIDGE adds the sums of the log Z estimator, RECORD the record buffer of the moments, PERSIST (R = 1) the persistent
+// chains of fit_likelihood (separate instantiations: the sampler's registers stay as they are).
+template <bool KEYS, int R, bool BRIDGE = false, bool RECORD = false, bool PERSIST = false>
 __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
     using Energy = typename std::conditional<R == 1, float, double>::type;
     constexpr int LADDERS = 32 / R;                           // ladders (chains) per warp
@@ -170,9 +176,15 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
         beta = (float)p.beta[slot];
     }
 
-    for (int i = 0; i < N; ++i) {                             // random start (sweep 0)
-        const uint32_t w = __ballot_sync(FULL, rand32(key, (uint64_t)i) >> 31);
-        if (lane == 0) s[i] = w;
+    if (PERSIST && p.sweep0 > 0) {                            // resume from the state the previous launch stored
+        const uint32_t* src = p.record + warp;
+#pragma unroll 1
+        for (int i = lane; i < N; i += 32) s[i] = src[(int64_t)i * p.ld_rec];
+    } else {
+        for (int i = 0; i < N; ++i) {                         // random start (sweep 0)
+            const uint32_t w = __ballot_sync(FULL, rand32(key, (uint64_t)i) >> 31);
+            if (lane == 0) s[i] = w;
+        }
     }
     __syncwarp();
 
@@ -180,10 +192,10 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
     double es0 = 0, eq0 = 0, es1 = 0, eq1 = 0, ms0 = 0, mq0 = 0, ms1 = 0, mq1 = 0;
     Energy e_first = 0;                                       // the statistics of the chain's first record
     int m_first = 0;
-    const int64_t sweeps = p.burn_in + p.records * p.thin;
+    const int64_t sweeps = PERSIST ? p.sweep0 + p.thin : p.burn_in + p.records * p.thin;
     int64_t next_rec = p.burn_in + p.thin, r = -1;           // the sweep that ends with the next record, its index
-    for (int64_t sw = 1; sw <= sweeps; ++sw) {
-        const bool rec = sw == next_rec;                      // warp-uniform
+    for (int64_t sw = PERSIST ? p.sweep0 + 1 : 1; sw <= sweeps; ++sw) {
+        const bool rec = !PERSIST && sw == next_rec;          // warp-uniform
         if (rec) { ++r; next_rec += p.thin; }
         const int64_t d = r * p.chains + c;
         const bool out = rec && live && d < p.n && rung == 0;
@@ -264,6 +276,14 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
         }
     }
 
+    if constexpr (PERSIST) {                                  // the final state and the mask of the live lanes
+        const uint32_t live_mask = __ballot_sync(FULL, live);
+        uint32_t* dst = p.record + warp + lane * p.ld_rec;
+#pragma unroll 1
+        for (int i = lane; i < N; i += 32, dst += 32 * p.ld_rec) *dst = s[i];
+        if (lane == 0) p.record[N * p.ld_rec + warp] = live_mask;
+        return;
+    }
     if constexpr (R > 1) {                                    // per pair, the sum over the warp's ladders
 #pragma unroll
         for (int o = R; o < 32; o <<= 1) n_acc += __shfl_xor_sync(FULL, n_acc, o);
@@ -489,6 +509,38 @@ void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const 
     if (out_swap_rate && rungs > 1)
         swap_rates(swaps.p, warps, rungs, chains, burn_in, burn_in + p.records * thin, out_swap_rate, st);
     reduce_records(record.p, N, p.records, warps, keys, out_mean, out_stderr, st);
+}
+
+struct PersistentChains::Impl {
+    DeviceModel model;
+    DevBuf<uint32_t> record;
+    Impl(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight, const Incidence& inc,
+         cudaStream_t st)
+        : model(N, order, term_idx, term_weight, inc, {1.0}, st) {}
+};
+
+PersistentChains::PersistentChains(int N, int order, const std::vector<int32_t>& term_idx,
+                                   const std::vector<double>& term_weight, const Incidence& inc, int64_t chains, uint64_t seed,
+                                   cudaStream_t st)
+    : impl(new Impl(N, order, term_idx, term_weight, inc, st)), warps(ceil_div(chains, 32)) {
+    McmcParams& p = impl->model.p;
+    p.chains = chains; p.chain0 = 0; p.seed = seed; p.records = 1;
+    p.rec_warps = warps; p.ld_rec = warps;
+    impl->record.alloc((size_t)(N + 1) * warps);
+    p.record = impl->record.p;
+    record = impl->record.p; term_w = impl->model.tw.p; weight = impl->model.ww.p;
+    const size_t smem = sizeof(uint32_t) * (size_t)N * WARPS;
+    GML_CUDA(cudaFuncSetAttribute(mcmc_kernel<false, 1, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+}
+
+PersistentChains::~PersistentChains() = default;
+
+void PersistentChains::run(int64_t sweep0, int64_t sweeps, cudaStream_t st) {
+    McmcParams p = impl->model.p;
+    p.sweep0 = sweep0; p.thin = sweeps;
+    const size_t smem = sizeof(uint32_t) * (size_t)p.N * WARPS;
+    mcmc_kernel<false, 1, false, true, true><<<(unsigned)ceil_div(warps, WARPS), WARPS * 32, smem, st>>>(p);
+    GML_LAUNCHED();
 }
 
 void log_partition_tempering(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,

@@ -200,9 +200,21 @@ std::vector<int32_t> singletons(int N) {
 
 int64_t moment_outputs(const MomentKeys& keys, int N) { return keys.pairwise ? (int64_t)N * N : keys.n_keys; }
 
+int record_groups(int64_t warps) { return (int)std::min<int64_t>(MAX_GROUPS, warps); }
+
+void record_key_sums(const uint32_t* rec, int N, int64_t records, int64_t warps, int order, int n_keys, const int32_t* d_key_idx,
+                     long long* d_n_g, long long* d_S, cudaStream_t st) {
+    const int G = record_groups(warps);
+    const int64_t ld = records * warps;
+    group_draws_kernel<<<G, 32, 0, st>>>(rec, N, records, warps, ld, G, d_n_g);
+    GML_LAUNCHED();
+    key_sums_kernel<<<dim3((unsigned)ceil_div(n_keys, 4), G), 128, 0, st>>>(rec, N, records, warps, ld, G, order, n_keys, d_key_idx, d_S);
+    GML_LAUNCHED();
+}
+
 void reduce_records(const uint32_t* rec, int N, int64_t records, int64_t warps, const MomentKeys& keys, double* out_mean,
                     double* out_stderr, cudaStream_t st) {
-    const int G = (int)std::min<int64_t>(MAX_GROUPS, warps);
+    const int G = record_groups(warps);
     const int64_t ld = records * warps, n_out = moment_outputs(keys, N);
     const std::vector<int32_t> idx = keys.pairwise ? singletons(N) : keys.idx;
     const int order = keys.pairwise ? 1 : keys.order, n_keys = keys.pairwise ? N : keys.n_keys;
@@ -213,10 +225,7 @@ void reduce_records(const uint32_t* rec, int N, int64_t records, int64_t warps, 
     n_g.alloc(G); S.alloc((size_t)G * n_keys); d_idx.alloc(idx.size());
     mean.alloc(n_out); err.alloc(n_out);
     GML_CUDA(cudaMemcpyAsync(d_idx.p, idx.data(), sizeof(int32_t) * idx.size(), cudaMemcpyHostToDevice, st));
-    group_draws_kernel<<<G, 32, 0, st>>>(rec, N, records, warps, ld, G, n_g.p);
-    GML_LAUNCHED();
-    key_sums_kernel<<<dim3((unsigned)ceil_div(n_keys, 4), G), 128, 0, st>>>(rec, N, records, warps, ld, G, order, n_keys, d_idx.p, S.p);
-    GML_LAUNCHED();
+    record_key_sums(rec, N, records, warps, order, n_keys, d_idx.p, n_g.p, S.p, st);
     if (keys.pairwise) {
         A.alloc((size_t)G * N * N);
         const unsigned t = (unsigned)ceil_div(N, TILE);

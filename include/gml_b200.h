@@ -372,6 +372,44 @@ int gml_b200_moments_exact(int32_t device, int32_t N, int32_t order, int32_t n_t
                            void* stream);
 int gml_b200_moments_histogram(gml_b200_handle* h, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean);
 
+/* ---- maximum-likelihood refit of a model's weights on its own terms -----------------------------------------------
+ * Both entries maximise l(w) = sum_t w_t data_mean[t] - log Z(w) - lambda sum_{|t| >= 2} |w_t| over the weights of the
+ * n_terms terms of term_idx (the layout of gml_b200_sample_mcmc_device), starting at init_weight, and write the
+ * maximiser to out_weight [n_terms].  data_mean [n_terms] are the data moments <prod_{i in t} s_i> (for example from
+ * gml_b200_moments_histogram over the same keys).  Fields (terms of one spin) are not penalised.  At the maximum the
+ * model's moments equal data_mean on every unpenalised term.
+ *
+ * gml_b200_fit_likelihood_mcmc: stochastic maximum likelihood with persistent Gibbs chains, N <= 4096, order <= 8.
+ *   - `chains` chains (0 = 2^17) run burn_in sweeps at init_weight.  Then each of `steps` steps s advances them by `thin`
+ *     sweeps of one long run (the RNG streams of gml_b200_sample_mcmc_device with the same seed and chains), reduces their
+ *     final states to the model moments m_t over gm's terms, and updates every weight on the device:
+ *     w_t <- w_t + eta_s g_t / d_t, g_t = data_mean[t] - m_t, d_t = max(1 - data_mean[t]^2, 0.01), soft-thresholded by
+ *     eta_s lambda / d_t on terms of >= 2 spins, eta_s = step_size (1 + s / 100)^-0.6.  The chains sample fl32(w).
+ *   - out_weight is the mean of w over the steps s >= floor(steps / 2) (Polyak-Ruppert averaging).
+ *     out_model_moments (nullable) [n_terms] is the chains' mean moment over the draws of the same steps, sum S / sum n
+ *     of integer sums: with step_size = 0 it equals gml_b200_moments_mcmc with burn_in + floor(steps/2) * thin burn-in
+ *     sweeps, the same thin, chains and seed, and n_samples = (steps - floor(steps/2)) * chains, bit for bit.
+ *     out_trace (nullable) [steps] holds max_t |g_t| of every step.
+ *   - No host synchronisation between steps, and no atomics: the result depends only on the arguments.
+ * gml_b200_fit_likelihood_exact: FISTA with backtracking on -l with exact log Z and moments by enumeration (the models
+ *   of gml_b200_sample_exact_device, N <= 40; each iteration costs one or two passes of ~2^N * 2 n_terms sign+add).  It
+ *   stops when the max-norm of the prox-gradient mapping is <= tol; *out_objective (nullable) = l(out_weight),
+ *   *out_iterations (nullable) = the iterations run.  GML_B200_ENOTCONV (out_weight holds the last iterate) after max_iter.
+ *
+ * GML_B200_EINVAL: what gml_b200_moments_mcmc / gml_b200_moments_exact refuse for the model and sizes, n_terms < 1, a null
+ * data_mean or out_weight, a data_mean entry outside [-1, 1] or not finite, |data_mean[t]| = 1 on a term that lambda
+ * does not bound (a field, or lambda = 0: no finite maximum), lambda < 0 or not finite, steps < 1, step_size < 0 or not
+ * finite (step_size = 0 samples init_weight unchanged), (burn_in + steps * thin) * N >= 2^62, tol <= 0, max_iter < 1. */
+int gml_b200_fit_likelihood_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                 const double* init_weight, const double* data_mean, double lambda, int64_t chains, int32_t burn_in,
+                                 int32_t thin, int64_t steps, double step_size, uint64_t seed, double* out_weight,
+                                 double* out_model_moments /* nullable [n_terms] */, double* out_trace /* nullable [steps] */,
+                                 void* stream);
+int gml_b200_fit_likelihood_exact(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                  const double* init_weight, const double* data_mean, double lambda, double tol, int32_t max_iter,
+                                  double* out_weight, double* out_objective /* nullable */,
+                                  int32_t* out_iterations /* nullable */, void* stream);
+
 /* ---- sample-sharded mode (SURVEY 8e): histogram rows split over ranks, every rank solves all nodes; per pass
  * the int64 gradient sums and fp64 objective sums are combined with NCCL all-reduces on the solve stream.
  *   rank 0: gml_b200_comm_unique_id(id) -> broadcast the 128 bytes with any transport -> every rank:
