@@ -34,6 +34,7 @@ EXPORTS = (
     "gml_b200_symmetrize_device",
     "gml_b200_sample_gibbs_device", "gml_b200_sample_gibbs_terms_device", "gml_b200_sample_exact_device",
     "gml_b200_sample_mcmc_device", "gml_b200_sample_tempering_device", "gml_b200_log_partition_tempering",
+    "gml_b200_sample_cluster_device", "gml_b200_moments_cluster",
     "gml_b200_moments_mcmc", "gml_b200_moments_exact", "gml_b200_moments_histogram",
     "gml_b200_fit_likelihood_mcmc", "gml_b200_fit_likelihood_exact",
     "gml_b200_build_histogram_device",
@@ -129,6 +130,9 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
                                                  c.c_uint64, vp, vp, vp, vp, c.c_int64, vp]
     lib.gml_b200_sample_mcmc_device.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int64, c.c_int32,
                                                 c.c_int64, c.c_int32, c.c_int32, c.c_uint64, vp, vp, vp, vp, c.c_int64, vp]
+    lib.gml_b200_sample_cluster_device.argtypes = lib.gml_b200_sample_mcmc_device.argtypes
+    lib.gml_b200_moments_cluster.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int64, c.c_int64, c.c_int32,
+                                             c.c_int32, c.c_uint64, c.c_int32, c.c_int32, vp, vp, vp, vp, vp]
     lib.gml_b200_sample_tempering_device.argtypes = [c.c_int32, c.c_int32, c.c_int32, c.c_int32, vp, vp, c.c_int32, vp,
                                                      c.c_int64, c.c_int32, c.c_int64, c.c_int32, c.c_int32, c.c_uint64, vp, vp,
                                                      vp, vp, vp, c.c_int64, vp]

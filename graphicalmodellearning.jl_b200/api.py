@@ -401,6 +401,25 @@ class B200Tempering(GMLSampler):
     last_swap_rate: list = field(default_factory=list, repr=False, compare=False)
 
 
+@dataclass
+class B200SwendsenWang(GMLSampler):
+    """Swendsen-Wang cluster sampler on the device (csrc/mcmc_sampler.cu) for pairwise models (terms of one or two spins)
+    with N <= 4096, such as ferromagnets at or below the critical coupling, where B200Gibbs chains do not mix.  Each
+    update bonds the satisfied terms with probability 1 - e^{-2|w_t|} (fields bond to a ghost spin fixed at +1) and flips
+    every cluster without the ghost with probability 1/2; it is valid for any signs, but frustrated models gain nothing
+    over B200Gibbs.  Fields and schedule as B200Gibbs, one update per "sweep": `chains` chains (0 = min(round_up(
+    number_sample, 32), 2^17)) run `burn_in` updates from a random start, then record after every `thin`-th.  The draws
+    depend only on (model, number_sample, replicates, seed, chains, burn_in, thin).  The chains sample the fp64 weights to
+    within |dw_t| <= 2^-52 + 2^-64 e^{2|w_t|}.  last_rhat holds, per replicate of the last call, the split-R-hat (energy,
+    magnetisation) over the chains' halves."""
+    seed: int = 0
+    device: int = 0
+    chains: int = 0
+    burn_in: int = 200
+    thin: int = 10
+    last_rhat: list = field(default_factory=list, repr=False, compare=False)
+
+
 def _ladder(sampler: B200Tempering) -> np.ndarray:
     """The betas of a B200Tempering as float64 (empty: the library default); ValueError for a ladder the library refuses."""
     if sampler.betas is None:
@@ -427,6 +446,13 @@ def _term_arrays(gm: FactorGraph):
     return order, idx, wts
 
 
+def _pairwise_only(gm: FactorGraph) -> None:
+    """ValueError for a term of three or more spins, which B200SwendsenWang does not take"""
+    big = next((k for k in gm.terms if len(k) > 2), None)
+    if big is not None:
+        raise ValueError(f"B200SwendsenWang samples pairwise models only (terms of one or two spins), got the term {big}")
+
+
 def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, return_log_z: bool):
     """Validates the arguments of sample / sample_device and runs the sampler's C entry point into device buffers sized
     for the largest possible result (min(n, 2^N) rows per replicate).  Returns (counts, spins, K, log_z); log_z is None
@@ -436,9 +462,9 @@ def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, 
     if isinstance(sampler, Gibbs):
         raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact() "
                                   "(N <= 40) or B200Gibbs() (MCMC) as the sampler")
-    if not isinstance(sampler, (B200Exact, B200Gibbs, B200Tempering)):
+    if not isinstance(sampler, (B200Exact, B200Gibbs, B200Tempering, B200SwendsenWang)):
         raise TypeError("sampler must be a GMLSampler")
-    mcmc = isinstance(sampler, (B200Gibbs, B200Tempering))
+    mcmc = isinstance(sampler, (B200Gibbs, B200Tempering, B200SwendsenWang))
     tempering = isinstance(sampler, B200Tempering)
     name = type(sampler).__name__
     if mcmc:
@@ -462,6 +488,8 @@ def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, 
             raise ValueError(f"{name} builds the histogram of N <= 64 spins from fewer than 2^31 draws per replicate")
     betas = _ladder(sampler) if tempering else None
     order, idx, wts = _term_arrays(gm)
+    if isinstance(sampler, B200SwendsenWang):
+        _pairwise_only(gm)
     ld = reps * min(n, 1 << N)
     dev = f"cuda:{int(sampler.device)}"
     counts = torch.empty(ld, dtype=torch.float64, device=dev)
@@ -481,6 +509,8 @@ def _sample_call(gm: FactorGraph, number_sample: int, replicates: int, sampler, 
         _lib.check(lib.gml_b200_sample_tempering_device(*head[:6], len(betas), _ptr(betas) if len(betas) else None, *head[6:],
                                                         *run, _ptr(swap), *tail))
         sampler.last_swap_rate = swap.tolist()
+    elif isinstance(sampler, B200SwendsenWang):
+        _lib.check(lib.gml_b200_sample_cluster_device(*head, *run, *tail))
     else:
         _lib.check(lib.gml_b200_sample_mcmc_device(*head, *run, *tail))
     sampler.last_rhat = [tuple(r) for r in rhat.tolist()]
@@ -504,8 +534,8 @@ def sample(gm: FactorGraph, number_sample: int, replicates: int = 1, sampler: Op
            return_log_z: bool = False):
     """sample(gm, number_sample[, replicates[, sampler]]) -- src/sampling.jl:90-106.  Returns the reference's int64
     K x (N+1) matrix [count, s_1..s_N] (spin_i = 2*bit_i - 1), or a list of them when replicates > 1; learn() takes it as it
-    is.  Rows are in increasing configuration index, except for B200Gibbs and B200Tempering beyond 64 spins, whose rows
-    are the draws in order with count 1.  The default sampler is B200Exact(seed=0, device=0)."""
+    is.  Rows are in increasing configuration index, except for B200Gibbs, B200Tempering and B200SwendsenWang beyond 64
+    spins, whose rows are the draws in order with count 1.  The default sampler is B200Exact(seed=0, device=0)."""
     counts, spins, K, log_z = _sample_call(gm, number_sample, replicates, sampler, return_log_z)
     rows = int(K.sum())
     c = counts[:rows].cpu().numpy().astype(np.int64)
@@ -618,16 +648,16 @@ def moments(gm: FactorGraph, sampler: Optional[GMLSampler] = None, number_sample
       diagonal, <s_i s_j> off it.
     - None or B200Exact: enumeration (N <= 40, gml_b200_moments_exact), exact in fp64, stderr all zeros; number_sample must
       be None.  Cost ~2^N * (n_terms + n_keys): pairwise has N(N+1)/2 keys, ~5e11 operations at N = 30, ~9e14 at N = 40.
-    - B200Gibbs / B200Tempering (N <= 4096, gml_b200_moments_mcmc) need number_sample: the mean is over exactly the draws
-      that sample(gm, number_sample, 1, sampler) returns with the same sampler fields, bit for bit, without writing them;
-      stderr comes from G = min(32, warps) groups of chains (NaN with fewer than 2).  Sets last_rhat (and last_swap_rate)
-      as sample does.  The chains sample fp32-rounded weights: the moments of gm differ by at most e^{2 delta} - 1, delta =
-      sum_t |w_t - fl32(w_t)|."""
+    - B200Gibbs / B200Tempering (N <= 4096, gml_b200_moments_mcmc) and B200SwendsenWang (gml_b200_moments_cluster) need
+      number_sample: the mean is over exactly the draws that sample(gm, number_sample, 1, sampler) returns with the same
+      sampler fields, bit for bit, without writing them; stderr comes from G = min(32, warps) groups of chains (NaN with
+      fewer than 2).  Sets last_rhat (and last_swap_rate) as sample does.  The Gibbs chains sample fp32-rounded weights:
+      the moments of gm differ by at most e^{2 delta} - 1, delta = sum_t |w_t - fl32(w_t)|."""
     sampler = B200Exact() if sampler is None else sampler
     if isinstance(sampler, Gibbs):
         raise NotImplementedError("Gibbs is the reference's CPU sampler and is not available here; pass B200Exact(), "
                                   "B200Gibbs() or B200Tempering()")
-    if not isinstance(sampler, (B200Exact, B200Gibbs, B200Tempering)):
+    if not isinstance(sampler, (B200Exact, B200Gibbs, B200Tempering, B200SwendsenWang)):
         raise TypeError("sampler must be a GMLSampler")
     mcmc = not isinstance(sampler, B200Exact)
     name = type(sampler).__name__
@@ -644,6 +674,8 @@ def moments(gm: FactorGraph, sampler: Optional[GMLSampler] = None, number_sample
     if mcmc and (int(number_sample) < 1 or sampler.chains < 0 or sampler.burn_in < 0 or sampler.thin < 1):
         raise ValueError(f"{name} needs number_sample >= 1, chains >= 0, burn_in >= 0 and thin >= 1")
     betas = _ladder(sampler) if isinstance(sampler, B200Tempering) else None
+    if isinstance(sampler, B200SwendsenWang):
+        _pairwise_only(gm)
     key_args, tuples, shape, _keep = _keys_call(list(gm.terms) if keys is None else keys, N)
     order, idx, wts = _term_arrays(gm)
     lib = _lib.load()
@@ -652,6 +684,12 @@ def moments(gm: FactorGraph, sampler: Optional[GMLSampler] = None, number_sample
     model = (int(sampler.device), N, order, len(gm.terms), _ptr(idx), _ptr(wts))
     if not mcmc:
         _lib.check(lib.gml_b200_moments_exact(*model, *key_args, _ptr(mean), None))
+    elif isinstance(sampler, B200SwendsenWang):
+        sampler.last_rhat = []
+        rhat = np.zeros(2)
+        _lib.check(lib.gml_b200_moments_cluster(*model, int(number_sample), int(sampler.chains), int(sampler.burn_in),
+                                                int(sampler.thin), seed, *key_args, _ptr(mean), _ptr(err), _ptr(rhat), None))
+        sampler.last_rhat = [tuple(rhat.tolist())]
     else:
         sampler.last_rhat = []
         rhat = np.zeros(2)

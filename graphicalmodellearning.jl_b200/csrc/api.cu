@@ -342,12 +342,20 @@ void exact_model(int32_t N, int32_t order, int32_t n_terms, const int32_t* term_
     GML_REQUIRE(std::isfinite(abs_sum), "sum of |term weights| is not finite");
 }
 
-// The MCMC entry points (betas = {1}: gml_b200_sample_mcmc_device; R > 1 rungs: gml_b200_sample_tempering_device, whose
-// ladder the caller has checked): argument checks, then the sampler into the caller's buffers.
+// The bond list of the Swendsen-Wang entry points, refused before the device is touched when a term has three or more
+// spins or the counters sweep * (n_terms + N + 1) + ... of `sweeps` updates would reach 2^62
+ClusterBonds checked_bonds(const McmcModel& m, int32_t N, int32_t order, double sweeps) {
+    GML_REQUIRE(sweeps * ((double)m.weights.size() + N + 1) < 0x1.0p62, "too many sweeps");
+    return cluster_bonds(order, m.idx, m.weights);
+}
+
+// The MCMC entry points (betas = {1}: gml_b200_sample_mcmc_device, or gml_b200_sample_cluster_device with cluster; R > 1
+// rungs: gml_b200_sample_tempering_device, whose ladder the caller has checked): argument checks, then the sampler into the
+// caller's buffers.
 void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx, const double* term_weight,
               const std::vector<double>& betas, int64_t n_samples, int32_t replicates, int64_t chains, int32_t burn_in,
               int32_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate, double* d_counts,
-              int8_t* d_spins, int64_t ld, void* stream) {
+              int8_t* d_spins, int64_t ld, void* stream, bool cluster = false) {
     const McmcModel m = mcmc_model(N, order, n_terms, term_idx, term_weight);
     GML_REQUIRE(out_K, "bad sampler argument");
     GML_REQUIRE(n_samples >= 1 && replicates >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1,
@@ -358,6 +366,7 @@ void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const i
     if (chains == 0) chains = mcmc_auto_chains(n_samples, rungs);
     const double steps = ((double)burn_in + (double)thin * (double)ceil_div(n_samples, chains)) * N;
     GML_REQUIRE(steps * replicates < 0x1.0p62, "too many sweeps");
+    const ClusterBonds bonds = cluster ? checked_bonds(m, N, order, steps / N) : ClusterBonds{};
     if (N > 64 && d_counts && ld < n_samples * replicates) {
         for (int r = 0; r < replicates; ++r) out_K[r] = n_samples;
         GML_REQUIRE(false, "ld = " + std::to_string(ld) + " is smaller than the " + std::to_string(n_samples * replicates) +
@@ -367,7 +376,7 @@ void run_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_terms, const i
     cudaStream_t st = (cudaStream_t)stream;
     into_sample_buffers(d_counts, d_spins, ld, N, replicates, out_K, st, [&](double* c, int8_t* sp) {
         sample_mcmc(N, order, m.idx, m.weights, m.inc, betas, n_samples, replicates, chains, burn_in, thin, seed, out_K,
-                    out_rhat, out_swap_rate, c, sp, ld, st);
+                    out_rhat, out_swap_rate, c, sp, ld, st, cluster ? &bonds : nullptr);
     });
 }
 
@@ -1342,6 +1351,16 @@ int gml_b200_sample_mcmc_device(int32_t device, int32_t N, int32_t order, int32_
     });
 }
 
+int gml_b200_sample_cluster_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                   const double* term_weight, int64_t n_samples, int32_t replicates, int64_t chains,
+                                   int32_t burn_in, int32_t thin, uint64_t seed, int64_t* out_K, double* out_rhat,
+                                   double* d_counts, int8_t* d_spins, int64_t ld, void* stream) {
+    return guarded([&] {
+        run_mcmc(device, N, order, n_terms, term_idx, term_weight, {1.0}, n_samples, replicates, chains, burn_in, thin, seed,
+                 out_K, out_rhat, nullptr, d_counts, d_spins, ld, stream, true);
+    });
+}
+
 int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
                                      const double* term_weight, int32_t n_rungs, const double* betas, int64_t n_samples,
                                      int32_t replicates, int64_t chains, int32_t burn_in, int32_t thin, uint64_t seed,
@@ -1393,6 +1412,25 @@ int gml_b200_moments_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_te
         GML_CUDA(cudaSetDevice(device));
         moments_mcmc(N, order, m.idx, m.weights, m.inc, ladder, n_samples, chains, burn_in, thin, seed, keys, out_mean, out_stderr,
                      out_rhat, out_swap_rate, (cudaStream_t)stream);
+    });
+}
+
+int gml_b200_moments_cluster(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                             const double* term_weight, int64_t n_samples, int64_t chains, int32_t burn_in, int32_t thin,
+                             uint64_t seed, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean,
+                             double* out_stderr, double* out_rhat, void* stream) {
+    return guarded([&] {
+        const McmcModel m = mcmc_model(N, order, n_terms, term_idx, term_weight);
+        const MomentKeys keys = moment_keys(N, key_order, n_keys, key_idx);
+        GML_REQUIRE(out_mean, "null out_mean");
+        GML_REQUIRE(n_samples >= 1 && chains >= 0 && chains <= (INT64_C(1) << 31) && burn_in >= 0 && thin >= 1, "bad sampler sizes");
+        if (chains == 0) chains = mcmc_auto_chains(n_samples, 1);
+        const double sweeps = (double)burn_in + (double)thin * (double)ceil_div(n_samples, chains);
+        GML_REQUIRE(sweeps * N < 0x1.0p62, "too many sweeps");
+        const ClusterBonds bonds = checked_bonds(m, N, order, sweeps);
+        GML_CUDA(cudaSetDevice(device));
+        moments_mcmc(N, order, m.idx, m.weights, m.inc, {1.0}, n_samples, chains, burn_in, thin, seed, keys, out_mean, out_stderr,
+                     out_rhat, nullptr, (cudaStream_t)stream, &bonds);
     });
 }
 

@@ -256,10 +256,19 @@ Incidence build_incidence(int N, int order, int n_terms, const int32_t* term_idx
 constexpr int64_t MCMC_AUTO_CHAINS = 1 << 17;
 constexpr int TEMPERING_MAX_RUNGS = GML_B200_TEMPERING_MAX_RUNGS;
 int64_t mcmc_auto_chains(int64_t n_samples, int rungs);
+// The bond list of the Swendsen-Wang sampler (cluster_kernel): per term of one or two spins with a nonzero weight, its
+// nodes (node 0 = the ghost spin, node i + 1 = spin i) and sign, and q_t = e^{-2|w_t|} in units of 2^-64.  Refuses a term
+// of three or more spins.
+struct ClusterBonds {
+    std::vector<uint32_t> ends;
+    std::vector<unsigned long long> q;
+};
+ClusterBonds cluster_bonds(int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight);
+// bonds != nullptr (betas = {1}): Swendsen-Wang updates instead of Gibbs sweeps, with the same records and outputs
 void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
                  const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int replicates, int64_t chains,
                  int64_t burn_in, int64_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate,
-                 double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st);
+                 double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st, const ClusterBonds* bonds = nullptr);
 // log Z of the model by bridge sampling along a replica-exchange ladder betas[0] = 1 > ... > betas[R-1] = 0 (R > 1):
 // `chains` ladders, burn_in sweeps, then `sweeps` sweeps that feed the bridge sums; fills *out_log_z and the nullable
 // out_stderr, out_log_ratio [R-1][2] (estimate, stderr of log Z_k - log Z_{k+1}) and out_swap_rate [R-1].  chains >= 2.
@@ -309,7 +318,7 @@ void moments_histogram_keys(const Histogram& hist, const MomentKeys& keys, doubl
 void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
                   const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int64_t chains, int64_t burn_in,
                   int64_t thin, uint64_t seed, const MomentKeys& keys, double* out_mean, double* out_stderr, double* out_rhat,
-                  double* out_swap_rate, cudaStream_t st);
+                  double* out_swap_rate, cudaStream_t st, const ClusterBonds* bonds = nullptr);
 
 // --- likelihood.cu : maximum-likelihood refit of the weights of a term list from data moments data_mean (fit_likelihood).
 // penalised[t] = 1 marks the terms of >= 2 spins, which carry lambda |w_t|.

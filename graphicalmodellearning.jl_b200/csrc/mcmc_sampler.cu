@@ -312,6 +312,147 @@ __global__ void __launch_bounds__(WARPS * 32) mcmc_kernel(McmcParams p) {
     }
 }
 
+// --- Swendsen-Wang cluster sampler (B200SwendsenWang) for pairwise models, Edwards-Sokal form with a ghost spin -----
+// Node 0 is a ghost spin fixed at +1 and node i + 1 is spin i, so a field (i,) is a bond between i + 1 and the ghost.
+// One update (a "sweep" for burn_in and thin): term t = (a, b) with w_t s_a s_b > 0 bonds unless u_t < q_t =
+// e^{-2|w_t|} (u_t a 64-bit uniform, q_t = bond_q[t] / 2^64 from fp64 on the host); every cluster without the ghost
+// flips with probability 1/2.  The warp keeps mcmc_kernel's state words and updates its 32 chains one after another,
+// lanes striding over terms and sites: the union-find hooks the larger root under the smaller, so every root is the least
+// node of its cluster and the labels do not depend on the order of the hooks.  Counters per sweep: bond t at sw * S + t,
+// the flip of root r at sw * S + n_bonds + r, S = n_bonds + N + 1; sweep 0 is mcmc_kernel's random start.
+constexpr int CLUSTER_WARPS = 2;      // 24.6 KB of shared memory per warp at N = 4096: 4 blocks (8 warps) per SM
+
+struct ClusterParams {
+    McmcParams m;                      // the model's term list (energy pass), the run and the outputs, as for mcmc_kernel
+    int n_bonds;
+    const uint32_t* bond_ends;         // [n_bonds] node a | node b << 16 | (w_t < 0) << 31, a in [1, N], b in [0, N]
+    const unsigned long long* bond_q;  // [n_bonds] round(e^{-2|w_t|} 2^64)
+};
+
+// 64 random bits of step `ctr` of the chain with key `chain_key` (rand32 is their upper half)
+__device__ __forceinline__ uint64_t rand64(uint64_t chain_key, uint64_t ctr) {
+    return mix64(chain_key + (ctr + 1) * 0x9E3779B97F4A7C15ULL);
+}
+
+// the root of x; volatile: other lanes hook roots while this lane walks
+__device__ __forceinline__ int uf_find(const volatile uint16_t* par, int x) {
+    int p = par[x];
+    while (p != x) { x = p; p = par[x]; }
+    return x;
+}
+
+// joins the clusters of a and b: hooks the larger root under the smaller with a CAS, retrying when another lane moved it
+__device__ __forceinline__ void uf_union(uint16_t* par, int a, int b) {
+    while (true) {
+        a = uf_find(par, a);
+        b = uf_find(par, b);
+        if (a == b) return;
+        if (a < b) { const int t = a; a = b; b = t; }
+        if (atomicCAS(reinterpret_cast<unsigned short*>(par + a), (unsigned short)a, (unsigned short)b) == a) return;
+    }
+}
+
+template <bool KEYS, bool RECORD>
+__global__ void __launch_bounds__(CLUSTER_WARPS * 32, 1) cluster_kernel(ClusterParams cp) {
+    const McmcParams& p = cp.m;
+    extern __shared__ uint32_t smem[];
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int64_t warp = (int64_t)blockIdx.x * CLUSTER_WARPS + wib;
+    const int64_t c = warp * 32 + lane;
+    if (warp * 32 >= p.chains) return;
+    const bool live = c < p.chains;
+    const int N = p.N, n_bonds = cp.n_bonds;
+    uint32_t* s = smem + (size_t)wib * N;
+    uint16_t* par = reinterpret_cast<uint16_t*>(smem + (size_t)CLUSTER_WARPS * N) + (size_t)wib * (N + 1);
+    const int chains_here = p.chains - warp * 32 < 32 ? (int)(p.chains - warp * 32) : 32;   // live chains of the warp
+    const uint64_t key = mix64(p.seed * 0xD1B54A32D192ED03ULL + mix64((uint64_t)(p.chain0 + c) + 1));
+    for (int i = 0; i < N; ++i) {                             // random start (sweep 0), as mcmc_kernel's
+        const uint32_t w = __ballot_sync(FULL, rand32(key, (uint64_t)i) >> 31);
+        if (lane == 0) s[i] = w;
+    }
+    __syncwarp();
+
+    const int64_t h = p.full_records / 2;
+    double es0 = 0, eq0 = 0, es1 = 0, eq1 = 0, ms0 = 0, mq0 = 0, ms1 = 0, mq1 = 0;
+    float e_first = 0;
+    int m_first = 0;
+    const uint64_t stride = (uint64_t)n_bonds + N + 1;
+    const int64_t sweeps = p.burn_in + p.records * p.thin;
+    int64_t next_rec = p.burn_in + p.thin, r = -1;
+    for (int64_t sw = 1; sw <= sweeps; ++sw) {
+        const uint64_t ctr0 = (uint64_t)sw * stride;
+#pragma unroll 1
+        for (int cc = 0; cc < chains_here; ++cc) {
+            const uint64_t ck = __shfl_sync(FULL, (unsigned long long)key, cc);
+            for (int i = lane; i <= N; i += 32) par[i] = (uint16_t)i;
+            __syncwarp();
+            for (int t = lane; t < n_bonds; t += 32) {        // bonds of the satisfied terms
+                const uint32_t ends = __ldg(cp.bond_ends + t);
+                const int a = ends & 0xffff, b = (ends >> 16) & 0x7fff;
+                const uint32_t sa = (s[a - 1] >> cc) & 1u, sb = b ? (s[b - 1] >> cc) & 1u : 1u;
+                if ((sa ^ sb) != (ends >> 31)) continue;      // w_t s_a s_b < 0: never bonds
+                if (rand64(ck, ctr0 + t) < __ldg(cp.bond_q + t)) continue;   // u_t < q_t: no bond
+                uf_union(par, a, b);
+            }
+            __syncwarp();
+            for (int i = lane; i <= N; i += 32) par[i] = (uint16_t)uf_find(par, i);
+            __syncwarp();
+            for (int i = lane; i < N; i += 32) {              // flip the clusters whose root drew 1, never the ghost's
+                const int root = par[i + 1];
+                if (root != 0 && rand32(ck, ctr0 + n_bonds + root) >> 31) s[i] ^= 1u << cc;
+            }
+            __syncwarp();
+        }
+        if (sw != next_rec) continue;
+        ++r;
+        next_rec += p.thin;
+        const int64_t d = r * p.chains + c;
+        const bool out = live && d < p.n;
+        unsigned long long cfg = 0;
+        int ups = 0;
+        for (int i = 0; i < N; ++i) {
+            const uint32_t bit = (s[i] >> lane) & 1u;
+            ups += bit;
+            if (KEYS) cfg |= (unsigned long long)bit << i;
+            else if (out && p.spins) p.spins[(int64_t)i * p.ld + d] = bit ? 1 : -1;
+        }
+        if (RECORD) {
+            const uint32_t draws = __ballot_sync(FULL, out);
+            uint32_t* dst = p.record + r * p.rec_warps + warp + lane * p.ld_rec;
+#pragma unroll 1
+            for (int i = lane; i < N; i += 32, dst += 32 * p.ld_rec) *dst = s[i];
+            if (lane == 0) p.record[N * p.ld_rec + r * p.rec_warps + warp] = draws;
+        }
+        if (out) {
+            if (KEYS) p.keys[d] = cfg;
+            else if (p.counts) p.counts[d] = 1.0;
+        }
+        if (r < p.full_records && h >= 2) {
+            const float energy = term_energy<float>(s, p, p.n_terms, lane);
+            const int mag = 2 * ups - N;
+            if (r == 0) { e_first = energy; m_first = mag; }
+            add_half(r, h, p.full_records, (double)energy - (double)e_first, es0, eq0, es1, eq1);
+            add_half(r, h, p.full_records, (double)(mag - m_first), ms0, mq0, ms1, mq1);
+        }
+    }
+
+    if (h < 2) return;
+    double em = 0, em2 = 0, ev = 0, mm = 0, mm2 = 0, mv = 0;
+    if (live) {
+        double m0, v0, m1, v1;
+        half_moments(e_first, es0, eq0, p.inv_h, p.inv_h1, m0, v0); half_moments(e_first, es1, eq1, p.inv_h, p.inv_h1, m1, v1);
+        em = m0 + m1; em2 = m0 * m0 + m1 * m1; ev = v0 + v1;
+        half_moments(m_first, ms0, mq0, p.inv_h, p.inv_h1, m0, v0); half_moments(m_first, ms1, mq1, p.inv_h, p.inv_h1, m1, v1);
+        mm = m0 + m1; mm2 = m0 * m0 + m1 * m1; mv = v0 + v1;
+    }
+    em = warp_sum(em); em2 = warp_sum(em2); ev = warp_sum(ev);
+    mm = warp_sum(mm); mm2 = warp_sum(mm2); mv = warp_sum(mv);
+    if (lane == 0) {
+        double* o = p.warp_stats + warp * 6;
+        o[0] = em; o[1] = em2; o[2] = ev; o[3] = mm; o[4] = mm2; o[5] = mv;
+    }
+}
+
 // split-R-hat of one statistic from the sums over M half-chains of h records each (Gelman et al., BDA3 sec. 11.4).
 // W = 0 means every half-chain held one value throughout: R-hat is then 1 when all half-chains held the same value (a
 // constant statistic has nothing to diagnose; the 1e-12 relative slack only absorbs the rounding of the sums) and +inf
@@ -362,6 +503,30 @@ void (*record_kernel(int rungs))(McmcParams) {
         default: return mcmc_kernel<false, 32, false, true>;
     }
 }
+
+// The bond list of a cluster run on the device, and its launches
+struct ClusterRun {
+    DevBuf<uint32_t> ends;
+    DevBuf<unsigned long long> q;
+    int n_bonds;
+
+    ClusterRun(const ClusterBonds& b, cudaStream_t st) : n_bonds((int)b.ends.size()) {
+        ends.alloc(std::max<size_t>(b.ends.size(), 1)); q.alloc(std::max<size_t>(b.q.size(), 1));
+        if (n_bonds) {
+            GML_CUDA(cudaMemcpyAsync(ends.p, b.ends.data(), sizeof(uint32_t) * n_bonds, cudaMemcpyHostToDevice, st));
+            GML_CUDA(cudaMemcpyAsync(q.p, b.q.data(), sizeof(unsigned long long) * n_bonds, cudaMemcpyHostToDevice, st));
+        }
+    }
+
+    template <bool KEYS, bool RECORD> void launch(const McmcParams& p, int64_t warps, cudaStream_t st) const {
+        // per warp: N state words and N + 1 16-bit parents
+        const size_t smem = CLUSTER_WARPS * (sizeof(uint32_t) * (size_t)p.N + sizeof(uint16_t) * (size_t)(p.N + 1));
+        GML_CUDA(cudaFuncSetAttribute(cluster_kernel<KEYS, RECORD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        cluster_kernel<KEYS, RECORD><<<(unsigned)ceil_div(warps, CLUSTER_WARPS), CLUSTER_WARPS * 32, smem, st>>>(
+            ClusterParams{p, n_bonds, ends.p, q.p});
+        GML_LAUNCHED();
+    }
+};
 
 // A model on the device for mcmc_kernel: the incidence lists and the term list with weights rounded once to fp32, and the
 // parameters that describe the model and the ladder.  The caller fills in the run.
@@ -422,16 +587,36 @@ void swap_rates(const unsigned long long* swap_acc, int64_t warps, int rungs, in
 }
 }  // namespace
 
+ClusterBonds cluster_bonds(int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight) {
+    ClusterBonds b;
+    for (size_t t = 0; t < term_weight.size(); ++t) {
+        int node[2] = {0, 0}, k = 0;
+        for (int m = 0; m < order; ++m) {
+            const int i = term_idx[t * order + m];
+            if (i < 0) continue;
+            GML_REQUIRE(k < 2, "the Swendsen-Wang sampler takes terms of one or two spins only");
+            node[k++] = i + 1;
+        }
+        const double q = std::exp(-2.0 * std::fabs(term_weight[t]));
+        if (k == 0 || q == 1.0) continue;                      // a constant, or |w| < 2^-54: never bonds
+        const uint32_t a = std::max(node[0], node[1]), c = std::min(node[0], node[1]);   // c = 0: the ghost
+        b.ends.push_back(a | c << 16 | (term_weight[t] < 0.0 ? 1u << 31 : 0u));
+        b.q.push_back((unsigned long long)(q * 0x1p64));       // rounded down: exact for q >= 2^-11, within 2^-64 below
+    }
+    return b;
+}
+
 void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
                  const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int replicates, int64_t chains,
                  int64_t burn_in, int64_t thin, uint64_t seed, int64_t* out_K, double* out_rhat, double* out_swap_rate,
-                 double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st) {
+                 double* d_counts, int8_t* d_spins, int64_t ld, cudaStream_t st, const ClusterBonds* bonds) {
     const bool keys_path = N <= 64;
     const int rungs = (int)betas.size();
     const int64_t warps = ceil_div(chains, 32 / rungs), blocks = ceil_div(warps, WARPS);
     const size_t smem = sizeof(uint32_t) * (size_t)N * WARPS;
 
     DeviceModel model(N, order, term_idx, term_weight, inc, betas, st);
+    std::unique_ptr<ClusterRun> cluster(bonds ? new ClusterRun(*bonds, st) : nullptr);
     DevBuf<double> wstats;
     DevBuf<unsigned long long> keys, swaps;
     wstats.alloc(warps * 6);
@@ -456,8 +641,14 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
         p.spins = write ? d_spins + rows : nullptr;
         p.counts = write ? d_counts + rows : nullptr;
         p.ld = ld;
-        kernel<<<(unsigned)blocks, WARPS * 32, smem, st>>>(p);
-        GML_LAUNCHED();
+        if (!cluster) {
+            kernel<<<(unsigned)blocks, WARPS * 32, smem, st>>>(p);
+            GML_LAUNCHED();
+        } else if (keys_path) {
+            cluster->launch<true, false>(p, warps, st);
+        } else {
+            cluster->launch<false, false>(p, warps, st);
+        }
         int64_t K = n_samples;
         if (keys_path) {
             KeyRuns runs;
@@ -481,7 +672,7 @@ void sample_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const s
 void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const std::vector<double>& term_weight,
                   const Incidence& inc, const std::vector<double>& betas, int64_t n_samples, int64_t chains, int64_t burn_in,
                   int64_t thin, uint64_t seed, const MomentKeys& keys, double* out_mean, double* out_stderr, double* out_rhat,
-                  double* out_swap_rate, cudaStream_t st) {
+                  double* out_swap_rate, cudaStream_t st, const ClusterBonds* bonds) {
     const int rungs = (int)betas.size();
     const int64_t warps = ceil_div(chains, 32 / rungs), blocks = ceil_div(warps, WARPS);
     const size_t smem = sizeof(uint32_t) * (size_t)N * WARPS;
@@ -501,10 +692,15 @@ void moments_mcmc(int N, int order, const std::vector<int32_t>& term_idx, const 
     if (rungs > 1) swaps.alloc(warps * (rungs - 1));
     record.alloc((size_t)(N + 1) * p.ld_rec);
     p.seed = seed; p.warp_stats = wstats.p; p.swap_acc = swaps.p; p.record = record.p;
-    auto kernel = record_kernel(rungs);
-    GML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kernel<<<(unsigned)blocks, WARPS * 32, smem, st>>>(p);
-    GML_LAUNCHED();
+    std::unique_ptr<ClusterRun> cluster(bonds ? new ClusterRun(*bonds, st) : nullptr);
+    if (cluster) {
+        cluster->launch<false, true>(p, warps, st);
+    } else {
+        auto kernel = record_kernel(rungs);
+        GML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kernel<<<(unsigned)blocks, WARPS * 32, smem, st>>>(p);
+        GML_LAUNCHED();
+    }
     if (out_rhat) rhat_of(wstats.p, warps, chains, h, out_rhat, st);
     if (out_swap_rate && rungs > 1)
         swap_rates(swaps.p, warps, rungs, chains, burn_in, burn_in + p.records * thin, out_swap_rate, st);

@@ -263,6 +263,48 @@ end
 
 sample(gm::FactorGraph, number_sample::Integer, sampler::B200Gibbs) = sample(gm, number_sample, 1, sampler)[1]
 
+"""
+    B200SwendsenWang(; seed=0, device=0, chains=0, burn_in=200, thin=10)
+
+Swendsen-Wang cluster sampler on the GPU for pairwise models (terms of one or two spins) with N <= 4096, such as
+ferromagnets at or below the critical coupling, where B200Gibbs chains do not mix.  Each update bonds the satisfied terms
+with probability 1 - exp(-2|w_t|) (fields bond to a ghost spin fixed at +1) and flips every cluster without the ghost
+with probability 1/2; one update counts as one sweep for `burn_in` and `thin`.  Fields, chain counts, output layout and
+`rhat` as B200Gibbs; a term of three or more spins is refused.
+"""
+mutable struct B200SwendsenWang <: GMLSampler
+    seed::UInt64
+    device::Int
+    chains::Int
+    burn_in::Int
+    thin::Int
+    rhat::Vector{NTuple{2,Float64}}
+end
+B200SwendsenWang(; seed=0, device=0, chains=0, burn_in=200, thin=10) =
+    B200SwendsenWang(UInt64(seed), device, chains, burn_in, thin, NTuple{2,Float64}[])
+
+function sample(gm::FactorGraph{T}, number_sample::Integer, replicates::Integer, sampler::B200SwendsenWang) where T <: Real
+    num_spins = gm.varible_count
+    order, n_terms, term_idx, term_weight = _gml_b200_terms(gm)
+    rows = replicates * (num_spins <= 62 ? min(number_sample, 2^num_spins) : number_sample)
+    out_K = zeros(Int64, replicates)
+    rhat = zeros(Float64, 2, replicates)
+    counts = Array{Float64}(undef, rows)
+    spins = Array{Int8}(undef, rows, num_spins)
+    GC.@preserve term_idx term_weight out_K rhat counts spins begin
+        rc = ccall((:gml_b200_sample_cluster_device, _libgml_b200), Cint,
+                   (Int32, Int32, Int32, Int32, Ptr{Int32}, Ptr{Cdouble}, Int64, Int32, Int64, Int32, Int32, UInt64, Ptr{Int64},
+                    Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int8}, Int64, Ptr{Cvoid}),
+                   sampler.device, num_spins, order, n_terms, term_idx, term_weight, number_sample, replicates, sampler.chains,
+                   sampler.burn_in, sampler.thin, sampler.seed, out_K, rhat, counts, spins, rows, C_NULL)
+    end
+    _gml_b200_check(rc)
+    sampler.rhat = [(rhat[1, r], rhat[2, r]) for r in 1:replicates]
+    return _gml_b200_replicates(counts, spins, out_K)
+end
+
+sample(gm::FactorGraph, number_sample::Integer, sampler::B200SwendsenWang) = sample(gm, number_sample, 1, sampler)[1]
+
 const GML_B200_TEMPERING_DEFAULT_RUNGS = 16   # include/gml_b200.h
 
 """

@@ -306,6 +306,25 @@ int gml_b200_sample_tempering_device(int32_t device, int32_t N, int32_t order, i
                                      double* out_swap_rate /* nullable [replicates][n_rungs - 1] */, double* d_counts,
                                      int8_t* d_spins, int64_t ld, void* stream);
 
+/* Swendsen-Wang cluster sampler: gml_b200_sample_mcmc_device for pairwise models whose single-site Gibbs chains do not
+ * mix, such as ferromagnets at or below the critical coupling.  Edwards-Sokal form with a ghost spin fixed at +1 that
+ * carries the fields: each update bonds every term t = (i, j) or (i,) with w_t s_i s_j > 0 (s_ghost = +1) with probability
+ * 1 - e^{-2|w_t|} (unsatisfied terms never bond; bonds are per term, so repeated keys stay correct) and flips every
+ * cluster without the ghost with probability 1/2.  One update counts as one sweep for burn_in and thin.  Valid for any
+ * signs; on frustrated models it samples correctly without the speed-up.
+ *   - Arguments, output layout, out_K, out_rhat, the buffers and chains = 0 (min(round_up(n_samples, 32), 2^17)) as
+ *     gml_b200_sample_mcmc_device; the output depends only on (terms, n_samples, replicates, chains, burn_in, thin, seed).
+ *   - Accuracy: "no bond" is drawn when a 64-bit uniform lies below q_t = e^{-2|w_t|}, computed on the host in fp64
+ *     from the fp64 weights, so the chains sample the model with w'_t = -1/2 log q'_t, |w'_t - w_t| <= 2^-52 +
+ *     2^-64 e^{2|w_t|} (while that is <= 1/2).  Unlike the Gibbs samplers, no weight is rounded to fp32.
+ *   - GML_B200_EINVAL: everything gml_b200_sample_mcmc_device refuses, a term of three or more spins, or
+ *     (burn_in + ceil(n_samples / chains) * thin) * (n_terms + N + 1) >= 2^62 counters. */
+int gml_b200_sample_cluster_device(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                                   const double* term_weight, int64_t n_samples, int32_t replicates, int64_t chains,
+                                   int32_t burn_in, int32_t thin, uint64_t seed, int64_t* out_K /* [replicates] */,
+                                   double* out_rhat /* nullable, [replicates][2]: energy, magnetisation */,
+                                   double* d_counts, int8_t* d_spins, int64_t ld, void* stream);
+
 /* Partition function by replica exchange: *out_log_z = log Z, Z = sum_s exp(sum_t w_t prod s), for the models of
  * gml_b200_sample_tempering_device (N <= 4096, order <= 8) by bridge sampling between the adjacent rungs of ladders
  * betas[0] = 1 > betas[1] > ... > betas[R-1] = 0; log Z(0) = N log 2 ties the chain of ratios to a known value.
@@ -367,6 +386,14 @@ int gml_b200_moments_mcmc(int32_t device, int32_t N, int32_t order, int32_t n_te
                           int64_t chains, int32_t burn_in, int32_t thin, uint64_t seed, int32_t key_order, int32_t n_keys,
                           const int32_t* key_idx, double* out_mean, double* out_stderr /* nullable */,
                           double* out_rhat /* nullable [2] */, double* out_swap_rate /* nullable [n_rungs-1] */, void* stream);
+/* gml_b200_moments_cluster: gml_b200_moments_mcmc for gml_b200_sample_cluster_device, without a ladder: the mean over
+ * exactly the n_samples draws that gml_b200_sample_cluster_device with replicates = 1 and the same sizes and seed returns,
+ * with the same group standard errors and out_rhat.  GML_B200_EINVAL: what gml_b200_sample_cluster_device refuses, bad
+ * keys, n_samples < 1, out_mean == NULL. */
+int gml_b200_moments_cluster(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
+                             const double* term_weight, int64_t n_samples, int64_t chains, int32_t burn_in, int32_t thin,
+                             uint64_t seed, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean,
+                             double* out_stderr /* nullable */, double* out_rhat /* nullable [2] */, void* stream);
 int gml_b200_moments_exact(int32_t device, int32_t N, int32_t order, int32_t n_terms, const int32_t* term_idx,
                            const double* term_weight, int32_t key_order, int32_t n_keys, const int32_t* key_idx, double* out_mean,
                            void* stream);
